@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """bench.py — QPS of exact inner-product top-100 over a 21M x 1024 synthetic corpus on N B200s.
 
-Contract (see the task statement): `python bench.py --gpus N --steps K --warmup W` prints ONE JSON
-line on rank 0.  A "step" is one search of a batch of B queries against the whole corpus.
+`python bench.py --gpus N --steps K --warmup W` prints ONE JSON line on rank 0.  A "step" is one search
+of a batch of B queries against the whole corpus; the headline times K of them after W warm-up steps.
+`--dump-outputs DIR` writes what the last timed step returned (scores.npy float32, ids.npy float64).
 
   value   QPS with queries and results resident in HBM (kirag_index_search, device pointers)
   e2e     QPS through the reference-facing call with HOST buffers: pinned-host queries in,
@@ -51,7 +52,37 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the N=1 extras (other BASELINE configs, pooling, stress corpus, index I/O)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (scores, ids) as DIR/<name>.npy, "
+                         "so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+NPY_HEADER_BYTES = 4096  # upper bound of one .npy header (numpy writes 128 bytes for these shapes)
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each [n, ...] array as out_dir/<name>.npy: float32 stays float32, everything else becomes float64 (exact
+    for ids).  If the files would exceed DUMP_LIMIT_BYTES in all, headers included, the same fixed, seeded sample of
+    rows is taken from every array and its row numbers are written as rows.npy."""
+    import numpy as np
+
+    arrays = {name: np.asarray(a) for name, a in arrays.items()}
+    arrays = {name: a if a.dtype == np.float32 else a.astype(np.float64) for name, a in arrays.items()}
+    n = next(iter(arrays.values())).shape[0]
+    if sum(a.nbytes for a in arrays.values()) + NPY_HEADER_BYTES * len(arrays) > DUMP_LIMIT_BYTES:
+        row_bytes = sum(a.nbytes for a in arrays.values()) // n + 8  # + 8: the row number in rows.npy
+        keep = min(n, max(1, (DUMP_LIMIT_BYTES - NPY_HEADER_BYTES * (len(arrays) + 1)) // row_bytes))
+        rows = np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def load_peaks():
@@ -169,7 +200,7 @@ def cpu_baseline(batch: int, k: int, rows_total: int, sample_rows: int, steps: i
         times = []
         for _ in range(max(1, steps)):
             t0 = time.perf_counter()
-            ix.search(xq, k)
+            out = ix.search(xq, k)
             times.append(time.perf_counter() - t0)
         t = sorted(times)[len(times) // 2]
         qps = b / (t * (rows_total / sample_rows))
@@ -177,7 +208,7 @@ def cpu_baseline(batch: int, k: int, rows_total: int, sample_rows: int, steps: i
                 "sample": f"{b} queries x {sample_rows} rows x {D_MODEL} (of {batch} x {rows_total}), top-{k}, "
                           f"faiss {getattr(real_faiss, '__version__', '?')} IndexFlatIP.search, median of {len(times)} x "
                           f"{t:.3f}s, extrapolated linearly in rows"}
-        return qps, info, t
+        return qps, info, t, out
     # pick the faster host BLAS for the blocked sgemm (MKL through torch, OpenBLAS through numpy)
     best = None
     for use_torch in (True, False):
@@ -193,9 +224,9 @@ def cpu_baseline(batch: int, k: int, rows_total: int, sample_rows: int, steps: i
     for _ in range(max(1, steps)):
         t0 = time.perf_counter()
         if b < 20:
-            oracle.flat_ip_search(xb, xq, k)  # FAISS's n < 20 path: per-query scan, threads over queries
+            out = oracle.flat_ip_search(xb, xq, k)  # FAISS's n < 20 path: per-query scan, threads over queries
         else:
-            oracle.flat_ip_search_blas(xb, xq, k, use_torch=use_torch)
+            out = oracle.flat_ip_search_blas(xb, xq, k, use_torch=use_torch)
         times.append(time.perf_counter() - t0)
     t = sorted(times)[len(times) // 2]
     qps = b / (t * (rows_total / sample_rows))
@@ -204,15 +235,17 @@ def cpu_baseline(batch: int, k: int, rows_total: int, sample_rows: int, steps: i
                       f"{'MKL(torch.mm)' if use_torch else 'OpenBLAS(numpy)'} sgemm 4096x1024 tiles + heap, "
                       f"median of {len(times)} x {t:.3f}s, extrapolated linearly in rows",
             "note": "FAISS-equivalent CPU restatement; faiss-cpu is not installable in this image"}
-    return qps, info, t
+    return qps, info, t, out
 
 
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    qps, info, t = cpu_baseline(args.batch, args.k, args.rows, args.cpu_sample_rows or (1 << 20), steps=args.steps,
-                                warmup=min(args.warmup, 1))
+    qps, info, t, (D, I) = cpu_baseline(args.batch, args.k, args.rows, args.cpu_sample_rows or (1 << 20),
+                                        steps=args.steps, warmup=min(args.warmup, 1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"scores": D, "ids": I})
     line = {
         "impl": "reference", "metric": "QPS, exact IP top-%d over %dx%d" % (args.k, args.rows, D_MODEL),
         "value": qps, "unit": "queries/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -283,9 +316,11 @@ def measure_batch(sh, lib, q_all, batch, k, steps, warmup, device, dist_ok, peak
     def step():
         D, I = sh.search(q, k)
         stats_box["stats"] = dict(sh.index.last_stats)
+        stats_box["outputs"] = (D, I)
         return D, I
 
     ms = timed_steps(step, steps, warmup, device, dist_ok)
+    outputs = stats_box["outputs"]  # what the last timed step returned (the roofline pass below computes it again)
     # roofline pass: same steps again with per-launch CUDA events on the launching stream
     lib.kirag_profile_enable(1)
     for _ in range(steps):
@@ -330,7 +365,7 @@ def measure_batch(sh, lib, q_all, batch, k, steps, warmup, device, dist_ok, peak
                               "cuBLAS's sustained rate), see frac_of_burst_peak / frac_of_nominal",
                  "frac_of_nominal": (ach / 7700.0) if roof["bound"] == "hbm" else (ach / 2250.0)})
     return {"batch": batch, "ms_per_step": ms, "qps": batch / (ms * 1e-3), "roofline": roof,
-            "stats": stats_box.get("stats", {})}
+            "stats": stats_box.get("stats", {}), "outputs": outputs}
 
 
 def parity_check(sh, q_all, batch, k, device, dist_ok, n_sample):
@@ -647,6 +682,9 @@ def run_ours(args):
         sampler.start()
     head = measure_batch(sh, lib, q_all, B, k, args.steps, args.warmup, device, dist_ok, peaks, args.rows, world)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        D, I = head.pop("outputs")
+        dump_outputs(args.dump_outputs, {"scores": D.cpu().numpy(), "ids": I.cpu().numpy()})
 
     # where a multi-GPU step goes: every rank's LOCAL search time (no exchange) and the exchange alone.  The step
     # is paced by the slowest rank (GPUs of one box sit at different power-capped clocks), so max(local) + exchange

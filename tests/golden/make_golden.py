@@ -9,7 +9,8 @@ Runs in the BUILD container only (needs /root/reference).  Three fixtures:
                       end to end (last_hidden_state captured with a forward hook).
   aligner_golden.npz  inputs + outputs of the reference's aligner scoring expression
                       (knowledge_graph/models.py:1532-1538): torch.matmul + torch.topk on CPU.
-  search_golden.npz   seeded flat-IP search cases answered by the ORACLE (fp64 accumulate).  The
+  search_golden.npz, search_golden_1024.npz
+                      seeded flat-IP search cases answered by the ORACLE (fp64 accumulate).  The
                       reference's FAISS cannot run here, so this fixture pins the oracle against
                       regressions, not against FAISS ("parity unpinned", see oracle/flat_ip_oracle.c).
 
@@ -113,7 +114,10 @@ def make_search():
     xq = rng.integers(-2, 3, size=(4, 64)).astype(np.float32)
     D, I = oracle.flat_ip_search(xb, xq, 16, accum="f64")
     out["ties_xb"], out["ties_xq"], out["ties_D"], out["ties_I"], out["ties_k"] = xb, xq, D, I, np.int64(16)
+    # two files, each under 1 MB: the 256 x 1024 case on its own (tests/helpers.py:load_search_golden reads both)
+    big = {f: out.pop(f) for f in list(out) if f.startswith("unit_1024_")}
     np.savez_compressed(os.path.join(HERE, "search_golden.npz"), **out)
+    np.savez_compressed(os.path.join(HERE, "search_golden_1024.npz"), **big)
 
 
 if __name__ == "__main__":

@@ -1,5 +1,19 @@
 """Shared comparison logic for the parity tests."""
+import os
+
 import numpy as np
+
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+# the search fixture is stored in two files to keep each under 1 MB (the 256 x 1024 case alone fills most of one)
+SEARCH_GOLDEN_FILES = ("search_golden.npz", "search_golden_1024.npz")
+
+
+def load_search_golden():
+    """Every array of the search fixture, by name, from all its files."""
+    z = {}
+    for f in SEARCH_GOLDEN_FILES:
+        z.update(np.load(os.path.join(GOLD, f)))
+    return z
 
 
 def exact_topk_f64(xb, xq, k):

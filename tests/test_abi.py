@@ -36,7 +36,7 @@ def test_library_loads_and_exports_every_declared_symbol():
 
 
 def test_built_for_sm100a_with_tcgen05_and_tma():
-    cuobjdump = "/usr/local/cuda/bin/cuobjdump"
+    cuobjdump = os.path.join(os.path.dirname(_build.find_nvcc()), "cuobjdump")  # the toolkit that built the library
     if not os.path.exists(cuobjdump):
         pytest.skip("cuobjdump not available")
     elf = subprocess.run([cuobjdump, "-lelf", _build.LIB_PATH], capture_output=True, text=True).stdout

@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle
-from tests.helpers import assert_topk_parity, exact_topk_f64, int_corpus
+from tests.helpers import assert_topk_parity, exact_topk_f64, int_corpus, load_search_golden
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 LOWEST = np.float32(-3.4028234663852886e38)
@@ -84,7 +84,7 @@ def test_merge_matches_unsharded():
 
 
 def test_search_golden_fixture():
-    z = np.load(os.path.join(GOLD, "search_golden.npz"))
+    z = load_search_golden()
     for name in ("unit_64", "unit_1024", "kgtn", "ties"):
         xb, xq, k = z[f"{name}_xb"], z[f"{name}_xq"], int(z[f"{name}_k"])
         D, I = oracle.flat_ip_search(xb, xq, k, accum="f64")

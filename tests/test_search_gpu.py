@@ -6,7 +6,7 @@ import pytest
 
 from oracle import oracle
 from tests.conftest import unit_rows
-from tests.helpers import assert_topk_parity, exact_topk_f64, int_corpus
+from tests.helpers import assert_topk_parity, exact_topk_f64, int_corpus, load_search_golden
 
 pytestmark = pytest.mark.gpu
 
@@ -342,7 +342,7 @@ def test_save_load_roundtrip_and_container_is_ixfi(fa, tmp_path):
 
 
 def test_search_golden_fixture(fa):
-    z = np.load(os.path.join(GOLD, "search_golden.npz"))
+    z = load_search_golden()
     for name in ("unit_64", "unit_1024", "kgtn", "ties"):
         xb, xq, k = z[f"{name}_xb"], z[f"{name}_xq"], int(z[f"{name}_k"])
         ix = build(fa, xb)
