@@ -643,10 +643,8 @@ static int fast_search(kirag_index* h, const float* qd, int64_t nq, int k, float
     if (h->flags.ensure((size_t)nq * 4)) return 1;
     if (h->rescored.ensure((size_t)nq * fp.kprime * 4)) return 1;
     if (h->tauk.ensure((size_t)nq * 4)) return 1;
-    // rescoring skips candidates more than 2 eps below the k-th best approximate score (KIRAG_RESCORE_ALL=1: all k')
-    const bool skip_far = env_int("KIRAG_RESCORE_ALL", 0) == 0;
     // small batches (wide candidate buffer): last compaction + rescoring + final sort are ONE cluster kernel
-    const bool fuse_tail = cap == kWideCap && fp.kprime <= 2048 && env_int("KIRAG_FUSED_TAIL", 1) != 0;
+    const bool fuse_tail = cap == kWideCap && fp.kprime <= 2048;
     if ((nq % plan.bq) != 0)  // only the pad rows of the last query tile need zeroing
         KIRAG_CUDA_OK(cudaMemsetAsync(h->qshadow.p, 0, qs_bytes, st));
     KIRAG_CUDA_OK(launch_chained(init_search_state_kernel, dim3((unsigned)((nq_pad + 255) / 256)), dim3(256), 0, st,
@@ -654,7 +652,7 @@ static int fast_search(kirag_index* h, const float* qd, int64_t nq, int k, float
     KIRAG_LAUNCH_OK("init_search_state_kernel");
     prof_mark(0, st);
     float* const qcdot = h->qnorm.as<float>() + 2 * nq;
-    if (launch_convert_rows(qd, nq, d, 0, h->qshadow.p, plan.q_tile_rows, nullptr, h->qnorm.as<float>(),
+    if (launch_convert_rows(qd, nq, d, 0, h->qshadow.p, plan.bq / 2, nullptr, h->qnorm.as<float>(),
                             h->qnorm.as<float>() + nq, h->center, qcdot, st)) return 1;
     prof_mark(1, st);
 
@@ -687,7 +685,7 @@ static int fast_search(kirag_index* h, const float* qd, int64_t nq, int k, float
         const bool last = (hi == bounds.back());
         if (last && fuse_tail) break;  // the fused tail kernel below does this level's compaction itself
         if (launch_compact_topm(h->cand.as<Cand>(), cap, h->cnt.as<int>(), cap, (int)nq, fp.kprime,
-                                h->tau.as<float>(), h->overflow.as<int>(), (last && skip_far) ? h->tauk.as<float>() : nullptr,
+                                h->tau.as<float>(), h->overflow.as<int>(), last ? h->tauk.as<float>() : nullptr,
                                 k, st)) return 1;
         prof_mark(30 + levels, st);
         ++levels;
@@ -704,8 +702,9 @@ static int fast_search(kirag_index* h, const float* qd, int64_t nq, int k, float
         if (levels_out) *levels_out = levels;
         return 0;
     }
+    // rescoring skips candidates more than 2 eps below the k-th best approximate score
     if (launch_rescore(h->master, d, qd, h->cand.as<Cand>(), h->cnt.as<int>(), cap, fp.kprime,
-                       h->rescored.as<float>(), nq, skip_far ? h->tauk.as<float>() : nullptr, h->qnorm.as<float>(),
+                       h->rescored.as<float>(), nq, h->tauk.as<float>(), h->qnorm.as<float>(),
                        h->qnorm.as<float>() + nq, ce.a, ce.b, st)) return 1;
     prof_mark(50, st);
     if (launch_final(h->cand.as<Cand>(), cap, h->rescored.as<float>(), h->cnt.as<int>(), 0, fp.kprime,
@@ -763,7 +762,7 @@ static int rescan_search(kirag_index* h, const float* qsel, const float* qnorm_a
         h->overflow.as<int>());
     KIRAG_LAUNCH_OK("rescan_threshold_kernel");
     if ((nb % plan.bq) != 0) KIRAG_CUDA_OK(cudaMemsetAsync(h->qshadow.p, 0, qs_bytes, st));
-    if (launch_convert_rows(qsel, nb, d, 0, h->qshadow.p, plan.q_tile_rows, nullptr, nullptr, nullptr, nullptr, nullptr,
+    if (launch_convert_rows(qsel, nb, d, 0, h->qshadow.p, plan.bq / 2, nullptr, nullptr, nullptr, nullptr, nullptr,
                             st)) return 1;
     const int64_t n_tiles = (n + kTileRows - 1) / kTileRows;
     if (launch_scan_tc(h->shadow, n, d, h->qshadow.p, nb, plan, 0, n_tiles, n_tiles, 1, h->tau.as<float>(),
@@ -856,7 +855,7 @@ static int resolve_chunk(kirag_index* h, const float* qd, int64_t cq, int k, flo
     std::vector<int> exact;
     const bool no_rescan = env_int("KIRAG_NO_RESCAN", 0) != 0;
     const bool gentle_already = fp.growth_override > 0 && fp.growth_override <= 4 && fp.first_growth_override > 0;
-    if (!ovf.empty() && !gentle_already && !env_int("KIRAG_NO_RETRY", 0)) {
+    if (!ovf.empty() && !gentle_already) {
         const int64_t nb = (int64_t)ovf.size();
         if (h->qmap.ensure((size_t)nb * 4) || h->qsel.ensure((size_t)nb * d * 4)) return 1;
         if (h->D_tmp.ensure((size_t)nb * k * 4) || h->I_tmp.ensure((size_t)nb * k * 8)) return 1;
@@ -1325,20 +1324,13 @@ int kirag_index_debug_scores(kirag_index_t* h, const float* q_host, int64_t nq, 
     if (scan_tc_pick(nq, d, &plan)) return 1;
     const char* force = getenv("KIRAG_DEBUG_BQ");
     if (force && *force) {
-        // 32 / 64 / 128 / 256: single-CTA kernels (32 resident, the others streamed); 512: the 2-CTA kernel
-        // with 256-query tiles (2512 / 4512: two / four pairs per cluster with multicast query blocks); 1128: the
-        // 2-CTA kernel with a resident 128-query tile; 1064: resident 64 (single CTA); 2064: resident 64 (2-CTA)
-        plan.bq = atoi(force);
-        plan.pair = 0;
-        plan.multi = 1;
-        plan.resident = (plan.bq == 32) ? 1 : 0;
-        if (plan.bq == 512) { plan.bq = 256; plan.pair = 1; }
-        if (plan.bq == 2512) { plan.bq = 256; plan.pair = 1; plan.multi = 2; }  // two pairs per cluster, multicast queries
-        if (plan.bq == 4512) { plan.bq = 256; plan.pair = 1; plan.multi = 4; }
-        if (plan.bq == 1128) { plan.bq = 128; plan.pair = 1; plan.resident = 1; }
-        if (plan.bq == 1064) { plan.bq = 64; plan.resident = 1; }
-        if (plan.bq == 2064) { plan.bq = 64; plan.pair = 1; plan.resident = 1; }  // 2-CTA kernel, resident 64-query tile
-        plan.q_tile_rows = plan.pair ? plan.bq / 2 : plan.bq;
+        // query-tile width + r(esident) / s(treamed): one of the five scan kernels
+        static const struct { const char* name; int bq, resident; } kVariants[] = {
+            {"64r", 64, 1}, {"64s", 64, 0}, {"128r", 128, 1}, {"128s", 128, 0}, {"256s", 256, 0}};
+        bool found = false;
+        for (const auto& v : kVariants)
+            if (strcmp(force, v.name) == 0) { plan.bq = v.bq; plan.resident = v.resident; found = true; }
+        KIRAG_CHECK(found, "debug_scores: KIRAG_DEBUG_BQ=%s is not one of 64r, 64s, 128r, 128s, 256s", force);
     }
     const size_t qs_bytes = scan_tc_qshadow_bytes(nq, d, plan);
     const int64_t nq_pad = round_up(nq, 256);
@@ -1354,7 +1346,7 @@ int kirag_index_debug_scores(kirag_index_t* h, const float* q_host, int64_t nq, 
         if (cudaMemsetAsync(cnt.p, 0, (size_t)nq_pad * 4, st) != cudaSuccess) break;
         if (cudaMemsetAsync(dump.p, 0, (size_t)h->ntotal * nq * 4, st) != cudaSuccess) break;
         if (fill_f32(tau.as<float>(), INFINITY, nq_pad, st)) break;
-        if (launch_convert_rows(qd.as<float>(), nq, d, 0, qs.p, plan.q_tile_rows, nullptr, nullptr, nullptr, h->center,
+        if (launch_convert_rows(qd.as<float>(), nq, d, 0, qs.p, plan.bq / 2, nullptr, nullptr, nullptr, h->center,
                                 h->center ? cdot.as<float>() : nullptr, st)) break;
         if (launch_scan_tc_dump(h->shadow, h->ntotal, d, qs.p, nq, plan, tau.as<float>(), cnt.as<int>(),
                                 dump.as<float>(), nq, h->num_sms, st)) break;

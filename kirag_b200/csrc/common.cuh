@@ -234,12 +234,11 @@ int launch_merge(const float* D_all, const int64_t* I_all, int G, int64_t nq, in
                  int64_t* I_out, cudaStream_t st);
 int launch_fill_pad(float* D, int64_t* I, int64_t n, cudaStream_t st);
 // scan_tc.cu
+// The scan runs on CTA pairs (cta_group::2, M = 256 corpus rows per MMA); each CTA stages half of a query tile,
+// so the query shadow is laid out in half tiles of bq / 2 rows.
 struct ScanTcPlan {
-    int bq;           // query-tile width (UMMA N)
-    int resident;     // 1: query tile stays in shared memory for the whole launch
-    int pair;         // 1: 2-CTA (cta_group::2) kernel, M = 256 corpus rows per MMA
-    int multi;        // CTA pairs per cluster sharing multicast query blocks (streamed 2-CTA kernel only; 1, 2 or 4)
-    int q_tile_rows;  // rows per tile of the query shadow layout (bq, or bq/2 for the pair kernel)
+    int bq;        // query-tile width (UMMA N): 64, 128 or 256
+    int resident;  // 1: query tile stays in shared memory for the whole launch (64 and 128 only)
 };
 int scan_tc_supported(int d);
 int scan_tc_pick(int64_t nq, int d, ScanTcPlan* plan);

@@ -7,16 +7,20 @@
 // "does this score enter the running top-k'" test is fused into the
 // accumulator read-out, so the score matrix never exists in memory.
 //
-// Data flow per CTA of the single-CTA kernel (persistent, one CTA per SM):
+// One kernel (scan_tc_pair_kernel): two CTAs on the two SMs of a TPC form a cluster and issue
+// one tcgen05.mma.cta_group::2 of M=256 corpus rows (one 128-row tile per CTA) x N=PQ queries x
+// K=16 per K-step.  Each CTA stages its own corpus tile and HALF of the query operand (PQ/2 rows).
+// Data flow per CTA (persistent, one cluster per SM pair):
 //   warp 0   producer : cp.async.bulk (TMA engine, SASS UBLKCP) of 16 KB shadow
 //                       blocks [128 corpus rows x 64 k] into an N-stage ring;
 //                       blocks are stored in HBM as the exact SWIZZLE_128B
 //                       K-major shared-memory image, so each copy is one
-//                       contiguous 16 KB read
-//   warp 1   MMA      : tcgen05.mma.cta_group::1.kind::f16, M=128 (corpus rows)
-//                       x N=BQ (queries) x K=16, bf16 in, fp32 accumulate in
-//                       TMEM; two accumulator stages so the read-out of tile t
-//                       overlaps the MMAs of tile t+1
+//                       contiguous 16 KB read.  Streamed variant: the stage also
+//                       holds this CTA's half of the query block
+//   warp 1   leader   : MMA issuer, bf16 in, fp32 accumulate in TMEM; two
+//                       accumulator stages so the read-out of tile t overlaps
+//                       the MMAs of tile t+1
+//            peer     : forwarder (tells the leader that the peer's stage is full)
 //   warps 2+  filter  : tcgen05.ld 32x32b -> thread = one corpus row, registers
 //                       = scores against 32 queries; compare with tau[q] (held in
 //                       registers, fetched one work item ahead); survivors are
@@ -24,27 +28,24 @@
 // Warps 0 and 1 run their loops with all 32 lanes on warp-uniform values and predicate
 // only the issuing instructions on elect.sync (see elect_one); one lane polls the mbarriers.
 //
-// The kernels the plan actually picks (scan_tc_pick) are the 2-CTA ones further down
-// (scan_tc_pair_kernel, cta_group::2: one M=256 MMA per K-step for an SM pair, each CTA
-// stages its own corpus tile and half of the query operand):
-//   <= 64 queries   resident 64-query tile (32 queries = 64 KB per CTA, 10-stage ring)   HBM-bound
-//   <= 128 queries  resident 128-query tile (64 queries = 128 KB per CTA, 6-stage ring)  HBM-bound
-//   larger          streamed 256-query tiles (16 KB corpus + 16 KB query half per stage)  tensor-bound
-// The single-CTA kernel remains for KIRAG_SCAN_PAIR=0 / KIRAG_PAIR64=0 and the forced-variant tests.
+// Instantiations (scan_tc_pick):
+//   <= 64 queries   64-query tile, resident (32 queries = 64 KB per CTA at d = 1024, 10-stage ring)  HBM-bound
+//   <= 128 queries  128-query tile, resident (64 queries = 128 KB per CTA at d = 1024, 6-stage ring) HBM-bound
+//   larger          streamed 256-query tiles (16 KB corpus + 16 KB query half per stage)             tensor-bound
+// The 64- and 128-query tiles are streamed instead (query half-block in every stage) when the resident
+// query half leaves too short a ring: d > 2048 at <= 64 queries, d > 1280 at <= 128 queries.
 //
 // Roofline: HBM for small query batches (algorithmic bytes = rows * d * 2 per
 // launch, streamed exactly once), tensor pipe for large ones (2 * rows * nq * d
 // flops per launch).
 #include "common.cuh"
 #include <cstdio>
-#include <cstdlib>
 
 namespace kirag {
 
 constexpr int kMaxStages = 12;
 constexpr int kBlockBytes = kTileRows * 128;  // one [128 x 64] bf16 block = 16 KB
 constexpr int kSmemLimit = 227 * 1024;
-constexpr int kDefaultMulti = 1;  // pairs per cluster of the streamed 2-CTA kernel (KIRAG_SCAN_MULTI overrides)
 
 // ------------------------------------------------------------------ PTX ----
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -56,9 +57,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
                  : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
     uint32_t ok;
@@ -84,8 +82,8 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, int ta
     }
 }
 // Wait of a whole (converged) warp on one barrier: ONE lane polls, the others park at the warp barrier.  All 32 lanes
-// polling costs 32 shared-memory barrier reads per try_wait; in the HBM-bound single-CTA kernel that traffic sits next
-// to the filter warps' accumulator read-out (same-box A/B, profiles/r02_ab/r3f_ab.log: 6.1 -> 6.5 ms at 8 queries).
+// polling costs 32 shared-memory barrier reads per try_wait; in an HBM-bound scan that traffic sits next to the
+// filter warps' accumulator read-out (same-box A/B, profiles/r02_ab/r3f_ab.log: 6.1 -> 6.5 ms at 8 queries).
 __device__ __forceinline__ void mbar_wait_warp(uint64_t* bar, uint32_t parity, int tag, int lane) {
     if (lane == 0) mbar_wait(bar, parity, tag);
     __syncwarp();
@@ -117,11 +115,6 @@ __device__ __forceinline__ uint64_t policy_evict_last() {
     asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
     return p;
 }
-__device__ __forceinline__ uint64_t policy_evict_normal() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
 __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar,
                                          uint64_t policy) {
     asm volatile(
@@ -129,38 +122,8 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
         ::"r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
         : "memory");
 }
-// Pull a block into L2 ahead of the shared-memory ring (KIRAG_PF_TILES > 0).  Hypothesis tested in round 2: at the
-// ridge (B ~ 256) the ring (7 x 16 KB of corpus per SM) bounds the HBM bytes in flight (ncu r2a: DRAM 52 %, tensor
-// 57 %), and a prefetch needs no shared-memory slot.  Measured at 21M rows (profiles/r02_ab/r2c_knobs.log): SLOWER at every
-// batch size (B=256 14.6-14.9 vs 12.2-13.4 ms; the extra bulk requests load the same TMA / L2 path), so it is off.
-__device__ __forceinline__ void bulk_prefetch_l2(const void* src_gmem, uint32_t bytes) {
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src_gmem), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void tmem_alloc(uint32_t* holder_smem, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(holder_smem)),
-                 "r"(ncols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                          uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-                 : "memory");
-}
-// ---- 2-CTA (cta_group::2) variants -------------------------------------------------
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -201,21 +164,10 @@ __device__ __forceinline__ void umma_bf16_2cta(uint32_t tmem_d, uint64_t desc_a,
         : "memory");
 }
 // arrives on the barrier at this shared-memory offset in every CTA of the cluster whose rank bit is set in `mask`
-// (both CTAs of the pair; for the multi-pair kernel also the CTAs of the other pairs)
 __device__ __forceinline__ void umma_commit_2cta(uint64_t* bar, uint16_t mask) {
     asm volatile(
         "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
         ::"r"(smem_u32(bar)), "h"(mask)
-        : "memory");
-}
-// one bulk copy delivered to the same shared-memory offset of every CTA in `mask`; each destination's mbarrier at
-// the offset of `bar` receives the complete_tx of its copy
-__device__ __forceinline__ void bulk_g2s_multicast(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar,
-                                                   uint16_t mask, uint64_t policy) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster.L2::cache_hint "
-        "[%0], [%1], %2, [%3], %4, %5;"
-        ::"r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)), "h"(mask), "l"(policy)
         : "memory");
 }
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
@@ -256,7 +208,7 @@ __host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N) {
 
 struct ScanArgs {
     const uint8_t* shadow;   // corpus bf16 blocks
-    const uint8_t* qshadow;  // query bf16 blocks, tiles of BQ rows
+    const uint8_t* qshadow;  // query bf16 blocks, half tiles of PQ/2 rows
     int64_t n_rows;
     int d;
     int64_t nq;
@@ -266,12 +218,9 @@ struct ScanArgs {
     int* cnt;          // [nq]
     int cap;
     int n_stages;
-    int x_policy;      // L2 policy of corpus blocks that are re-read per query tile: 1 normal, 2 evict_last,
-                       // 3 evict_last + evict_first on the last read
     int q_dep;         // 1: the query shadow is written by the kernel right before this one in the chain
                        // (level 0): the producer must pdl_wait() too; 0: only the filter warps wait
-    int pf_tiles;      // L2 prefetch distance of the corpus stream, in corpus tiles of this CTA (0: off)
-    float* dump;       // optional [n_rows, dump_ld] dense approx scores (debug / tests)
+    float* dump;      // optional [n_rows, dump_ld] dense approx scores (debug / tests)
     int64_t dump_ld;
 };
 
@@ -480,222 +429,44 @@ template <int BQ> struct EpiCfg {
     static constexpr int kGroups = BQ / 32 / (kWarps / 4);  // 32-column groups per warp
 };
 
-template <int BQ, bool RESIDENT>
-__global__ void __launch_bounds__(EpiCfg<BQ>::kThreads, 1) scan_tc_kernel(const ScanArgs a) {
-    extern __shared__ uint8_t smem_raw[];
-    // 1024-byte alignment for the 128B swizzle atoms
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    const int KC = a.d >> 6;                           // 64-wide k-blocks per row
-    constexpr int kQBlockBytes = BQ * 128;             // one [BQ x 64] bf16 block
-    const int NS = a.n_stages;
-    const int stage_bytes = kBlockBytes + (RESIDENT ? 0 : kQBlockBytes);
-    uint8_t* stage_base = smem;
-    uint8_t* q_res = smem + (size_t)NS * stage_bytes;  // resident query tile (RESIDENT only)
-    uint8_t* tail = q_res + (RESIDENT ? (size_t)KC * kQBlockBytes : 0);
-    uint64_t* full_bar = reinterpret_cast<uint64_t*>(tail);
-    uint64_t* empty_bar = full_bar + kMaxStages;
-    uint64_t* tmem_full = empty_bar + kMaxStages;
-    uint64_t* tmem_empty = tmem_full + 2;
-    uint64_t* q_bar = tmem_empty + 2;
-    uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(q_bar + 1);
-
-    // HBM-bound variant (idle issue slots): release the dependents at once; the next kernel (compaction)
-    // waits for this whole grid anyway
-    pdl_launch_dependents();
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-    constexpr uint32_t kTmemCols = (2 * BQ <= 32) ? 32 : (2 * BQ <= 64) ? 64 : (2 * BQ <= 128) ? 128 : (2 * BQ <= 256) ? 256 : 512;
-    const int n_qt = (int)((a.nq + BQ - 1) / BQ);
-    // work item w = (walk position, query tile), query tile fastest so that a CTA re-reads its corpus
-    // tile from L2; every CTA takes one contiguous, equally sized range of w
-    const int64_t W = (a.tile_hi - a.tile_lo) * n_qt;
-    const int64_t w_lo = W * blockIdx.x / gridDim.x;
-    const int64_t w_hi = W * (blockIdx.x + 1) / gridDim.x;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < NS; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-        for (int s = 0; s < 2; ++s) { mbar_init(&tmem_full[s], 1); mbar_init(&tmem_empty[s], EpiCfg<BQ>::kWarps); }
-        mbar_init(q_bar, 1);
-        fence_barrier_init();
-    }
-    if (warp == 1) tmem_alloc(tmem_holder, kTmemCols);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_holder;
-
-    if (warp == 0) {
-        // =============================== producer ===============================
-        {
-            const uint64_t pol_x = (n_qt == 1) ? policy_evict_first() : (a.x_policy >= 2 ? policy_evict_last() : policy_evict_normal());
-            const uint64_t pol_q = policy_evict_last();
-            if (a.q_dep) pdl_wait();  // level 0: the query shadow is being written by the previous kernel
-            if (RESIDENT && elect_one()) {
-                mbar_expect_tx(q_bar, (uint32_t)(KC * kQBlockBytes));
-                bulk_g2s(q_res, a.qshadow, (uint32_t)(KC * kQBlockBytes), q_bar, pol_q);
-            }
-            __syncwarp();
-            int s = 0;
-            uint32_t ph = 0;
-            for (int64_t w = w_lo; w < w_hi; ++w) {
-                const int64_t tp = w / n_qt;
-                const int qt = (int)(w - tp * n_qt);
-                const int64_t tile = ((a.tile_lo + tp) * a.tile_mult) % a.n_tiles;
-                const uint8_t* xsrc = a.shadow + (size_t)tile * ((size_t)a.d * kTileRows * 2);
-                const uint8_t* qsrc = a.qshadow + (size_t)qt * ((size_t)a.d * BQ * 2);
-                const uint8_t* pfsrc = nullptr;  // the tile this CTA streams pf_tiles tiles from now
-                if (a.pf_tiles > 0 && qt == 0 && (tp + a.pf_tiles) * n_qt < w_hi) {
-                    const int64_t ptile = ((a.tile_lo + tp + a.pf_tiles) * a.tile_mult) % a.n_tiles;
-                    pfsrc = a.shadow + (size_t)ptile * ((size_t)a.d * kTileRows * 2);
-                }
-                for (int kc = 0; kc < KC; ++kc) {
-                    mbar_wait_warp(&empty_bar[s], ph ^ 1u, 100 + s, lane);
-                    uint8_t* dst = stage_base + (size_t)s * stage_bytes;
-                    if (elect_one()) {
-                        if (pfsrc) bulk_prefetch_l2(pfsrc + (size_t)kc * kBlockBytes, kBlockBytes);
-                        mbar_expect_tx(&full_bar[s], (uint32_t)stage_bytes);
-                        bulk_g2s(dst, xsrc + (size_t)kc * kBlockBytes, kBlockBytes, &full_bar[s], pol_x);
-                        if (!RESIDENT)
-                            bulk_g2s(dst + kBlockBytes, qsrc + (size_t)kc * kQBlockBytes, kQBlockBytes, &full_bar[s], pol_q);
-                    }
-                    __syncwarp();
-                    if (++s == NS) { s = 0; ph ^= 1u; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ================================= MMA ==================================
-        {
-            constexpr uint32_t idesc = make_idesc_bf16(kTileRows, BQ);
-            if (RESIDENT) mbar_wait_warp(q_bar, 0, 200, lane);
-            int s = 0;
-            uint32_t ph = 0;
-            uint32_t it = 0;
-            for (int64_t w = w_lo; w < w_hi; ++w, ++it) {
-                const uint32_t as = it & 1u;
-                const uint32_t aph = (it >> 1) & 1u;
-                mbar_wait_warp(&tmem_empty[as], aph ^ 1u, 300 + as, lane);
-                tc_fence_after();
-                const uint32_t d_tmem = tmem_base + as * BQ;
-                for (int kc = 0; kc < KC; ++kc) {
-                    mbar_wait_warp(&full_bar[s], ph, 400 + s, lane);
-                    tc_fence_after();
-                    const uint32_t xa = smem_u32(stage_base + (size_t)s * stage_bytes);
-                    const uint32_t qa = RESIDENT ? smem_u32(q_res + (size_t)kc * kQBlockBytes) : xa + kBlockBytes;
-                    const uint64_t da = make_sw128_desc(xa);
-                    const uint64_t db = make_sw128_desc(qa);
-                    if (elect_one()) {
-#pragma unroll
-                        for (int k4 = 0; k4 < 4; ++k4) {
-                            // +32 bytes (two 16-byte units) per K=16 step inside the 128-byte swizzle row
-                            umma_bf16(d_tmem, da + (uint64_t)(k4 * 2), db + (uint64_t)(k4 * 2), idesc,
-                                      (kc | k4) ? 1u : 0u);
-                        }
-                        umma_commit(&empty_bar[s]);  // frees the stage once these MMAs have read it
-                        if (kc == KC - 1) umma_commit(&tmem_full[as]);  // accumulator complete
-                    }
-                    __syncwarp();
-                    if (++s == NS) { s = 0; ph ^= 1u; }
-                }
-            }
-        }
-    } else {
-        // ================================ filter ================================
-        const int quad = warp & 3;  // TMEM lane quadrant this warp may read
-        const uint32_t lane_base = (uint32_t)(quad * 32) << 16;
-        constexpr int NG = EpiCfg<BQ>::kGroups;
-        const int col0 = ((warp - 2) >> 2) * (NG * 32);  // this warp's first column inside the query tile
-        uint32_t it = 0;
-        Stash pend, cur;
-        stash_clear(pend);
-        pdl_wait();  // tau / cand / cnt come from the previous compaction; the corpus stream did not have to wait
-        float mytau[NG];
-        int tau_qt = -1;
-        for (int64_t w = w_lo; w < w_hi; ++w, ++it) {
-            const int64_t tp = w / n_qt;
-            const int qt = (int)(w - tp * n_qt);
-            const int64_t tile = ((a.tile_lo + tp) * a.tile_mult) % a.n_tiles;
-            const int64_t row = tile * kTileRows + quad * 32 + lane;
-            const bool row_ok = row < a.n_rows;
-            const uint32_t as = it & 1u;
-            const uint32_t aph = (it >> 1) & 1u;
-            if (qt != tau_qt) {  // once per launch when the batch is a single query tile; in flight during the wait below
-#pragma unroll
-                for (int g = 0; g < NG; ++g) mytau[g] = __ldcg(a.tau + (int64_t)qt * BQ + col0 + g * 32 + lane);
-                tau_qt = qt;
-            }
-            mbar_wait(&tmem_full[as], aph, 500 + as);
-            tc_fence_after();
-            uint64_t* const ebar = &tmem_empty[as];
-            filter_item<NG>(a, tmem_base + lane_base + as * BQ + col0, (int64_t)qt * BQ + col0, row, row_ok, lane,
-                            cur, mytau, [=]() {
-                                // all of this warp's reads of the accumulator are done
-                                tc_fence_before();
-                                __syncwarp();
-                                if (lane == 0) mbar_arrive(ebar);
-                            });
-            stash_store(a, pend);    // slots reserved one item ago
-            stash_reserve(a, cur);   // atomics in flight until the next item has been read
-            pend = cur;
-        }
-        stash_store(a, pend);
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, kTmemCols);
-    }
-}
-
-// ------------------------------------------------------- 2-CTA pair kernel ----
-// Large query batches are tensor-bound, and with one CTA per tile the query operand makes
-// the L2 -> shared-memory traffic the limiter (48 KB per 128x256x64 MMA block).  Here two
-// CTAs on the two SMs of a TPC form a cluster and issue ONE tcgen05.mma.cta_group::2 of
-// M=256 (2 corpus tiles) x N=256 (queries) x K=16: each CTA stages only its own 16 KB corpus
-// block and HALF of the query block (16 KB), i.e. 32 KB per CTA for the same flops.
+// ------------------------------------------------------------- pair kernel ----
+// With one CTA per corpus tile the query operand made the L2 -> shared-memory traffic the limiter of
+// large batches (48 KB per 128x256x64 MMA block); the pair stages 16 KB of corpus and 16 KB of queries
+// per CTA for the same flops.
 //   rank 0 (leader): producer, MMA issuer, filter warps
 //   rank 1 (peer)  : producer, forwarder (tells the leader that the peer's stage is full),
 //                    filter warps
 // Barriers: full[s] lives in each CTA (leader: own expect_tx + the peer's forwarded arrive);
 // empty[s] and tmem_full[a] are signalled in both CTAs by a multicast tcgen05.commit;
-// tmem_empty[a] of the LEADER collects the 8 filter warps of both CTAs.
-// Three instantiations:
+// tmem_empty[a] of the LEADER collects the filter warps of both CTAs.
+// Instantiations:
 //   PQ = 256, streamed  : large batches (tensor-bound); corpus block + half query block per stage
-//   PQ = 128, RES       : 64 < batch <= 128 (HBM-bound); each CTA keeps ITS half of the single query
+//   PQ = 128, resident  : 64 < batch <= 128 (HBM-bound); each CTA keeps ITS half of the single query
 //                         tile (64 queries x d, 128 KB at d = 1024) resident in shared memory, so
 //                         only corpus blocks are streamed: L2 -> SM traffic equals the HBM traffic
-//   PQ = 64, RES        : batch <= 64 (HBM-bound, the default for KiRAG's 1-2 queries per retrieval):
-//                         32 queries = 64 KB resident per CTA, 10-stage ring, four filter warps
+//   PQ = 64, resident   : batch <= 64 (HBM-bound, the default for KiRAG's 1-2 queries per retrieval):
+//                         32 queries = 64 KB resident per CTA at d = 1024, 10-stage ring, four filter warps
+//   PQ = 128 / 64, streamed : the same batches at a d where the resident half leaves too short a ring
 template <int PQ, bool RES> struct PairCfg {
     static constexpr int kHalfQ = PQ / 2;                      // query rows staged per CTA
     static constexpr int kQHalfBytes = kHalfQ * 128;           // one [half x 64] bf16 block
     static constexpr int kStageBytes = kBlockBytes + (RES ? 0 : kQHalfBytes);
 };
 
-// NP = CTA pairs per cluster.  NP = 1 is the kernel described above.  NP > 1 (streamed variant only): the NP pairs
-// of a cluster work on different corpus tiles but on the SAME query tile and k-block at the same time, and the
-// 16 KB query half-block that the "same half" CTAs of all pairs need is fetched from L2 ONCE and multicast to them
-// (cp.async.bulk ... .multicast::cluster).  The streamed kernel is bound by the L2 -> SM fill path (32 KB per CTA
-// per 512 tensor cycles: the pipe was 84-85 % active with operands that all hit L2, ncu r01b / r2a — before the
-// warp-uniform issue loops, which turned out to be the actual cause; measured again after them: still slower), and half of
-// that traffic is the query operand; with NP pairs sharing it the fill drops to 16 + 16/NP KB per CTA and k-block.
-//   pair j's CTAs issue the query blocks of the k-blocks kc with kc % NP == j, for every pair;
-//   a stage may be refilled only when EVERY pair has consumed it: empty[s] collects one tcgen05.commit per pair
-//   (each commit is multicast to all 2 NP CTAs), so the pairs advance through the ring in lock-step.
-template <int PQ, bool RES, int NP>
-__device__ __forceinline__ void scan_pair_body(const ScanArgs& a) {
-    static_assert(NP == 1 || !RES, "query multicast is for the streamed variant");
-    constexpr int kPairQ = PQ;
-    constexpr int kPairHalfQ = PairCfg<PQ, RES>::kHalfQ;
+template <int PQ, bool RES>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(EpiCfg<PQ>::kThreads, 1)
+scan_tc_pair_kernel(const ScanArgs a) {
+    constexpr int kHalfQ = PairCfg<PQ, RES>::kHalfQ;
     constexpr int kQHalfBytes = PairCfg<PQ, RES>::kQHalfBytes;
-    constexpr int kPairStageBytes = PairCfg<PQ, RES>::kStageBytes;
+    constexpr int kStageBytes = PairCfg<PQ, RES>::kStageBytes;
+    constexpr uint16_t kPairMask = 0x3;  // both CTAs of the cluster
     extern __shared__ uint8_t smem_raw[];
+    // 1024-byte alignment for the 128B swizzle atoms
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    const int KC = a.d >> 6;
+    const int KC = a.d >> 6;  // 64-wide k-blocks per row
     const int NS = a.n_stages;
     uint8_t* stage_base = smem;
-    uint8_t* q_res = smem + (size_t)NS * kPairStageBytes;  // resident half query tile (RES only)
+    uint8_t* q_res = smem + (size_t)NS * kStageBytes;  // resident half query tile (RES only)
     uint8_t* tail = q_res + (RES ? (size_t)KC * kQHalfBytes : 0);
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(tail);
     uint64_t* empty_bar = full_bar + kMaxStages;
@@ -706,33 +477,21 @@ __device__ __forceinline__ void scan_pair_body(const ScanArgs& a) {
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();   // 0 .. 2 NP - 1
-    const uint32_t half = rank & 1u;            // 0: leader of its pair (issues the MMAs), 1: peer
-    const uint32_t pairc = rank >> 1;           // pair inside the cluster
-    const uint32_t leader = rank & ~1u;
-    constexpr int kCl = 2 * NP;                 // CTAs per cluster
-    constexpr uint16_t kMaskAll = (uint16_t)((1u << kCl) - 1u);
-    const uint16_t mask_pair = (uint16_t)(3u << leader);
-    uint16_t mask_half = 0;                     // the CTAs of every pair that stage the same query half as this one
-#pragma unroll
-    for (int j = 0; j < NP; ++j) mask_half |= (uint16_t)(1u << (2 * j + half));
-    const int64_t pair = blockIdx.x / kCl;       // work unit: the cluster
-    const int64_t n_pairs = gridDim.x / kCl;
+    const uint32_t rank = cluster_ctarank();  // 0: leader (issues the MMAs), 1: peer
+    const int64_t pair = blockIdx.x / 2;
+    const int64_t n_pairs = gridDim.x / 2;
     constexpr uint32_t kTmemCols = 2 * PQ;  // two accumulator stages of PQ columns
-    const int n_qt = (int)((a.nq + kPairQ - 1) / kPairQ);
-    // work item w = (pair of walk positions, 256-query tile), query tile fastest; every cluster takes
-    // one contiguous, equally sized range of w, so small levels still occupy all SM pairs
-    const int64_t W = ((a.tile_hi - a.tile_lo + kCl - 1) / kCl) * n_qt;
+    const int n_qt = (int)((a.nq + PQ - 1) / PQ);
+    // work item w = (pair of walk positions, query tile), query tile fastest so that a CTA re-reads its corpus tile
+    // from L2; every pair takes one contiguous, equally sized range of w, so small levels still occupy all SM pairs
+    const int64_t W = ((a.tile_hi - a.tile_lo + 1) / 2) * n_qt;
     const int64_t w_lo = W * pair / n_pairs;
     const int64_t w_hi = W * (pair + 1) / n_pairs;
 
     if (threadIdx.x == 0) {
-        for (int s = 0; s < NS; ++s) {
-            mbar_init(&full_bar[s], half == 0 ? 2 : 1);
-            mbar_init(&empty_bar[s], NP);  // one tcgen05.commit per pair of the cluster
-        }
-        for (int s = 0; s < 2; ++s) { mbar_init(&tmem_full[s], 1); mbar_init(&tmem_empty[s], 2 * EpiCfg<kPairQ>::kWarps); }
-        mbar_init(q_bar, half == 0 ? 2 : 1);
+        for (int s = 0; s < NS; ++s) { mbar_init(&full_bar[s], rank == 0 ? 2 : 1); mbar_init(&empty_bar[s], 1); }
+        for (int s = 0; s < 2; ++s) { mbar_init(&tmem_full[s], 1); mbar_init(&tmem_empty[s], 2 * EpiCfg<PQ>::kWarps); }
+        mbar_init(q_bar, rank == 0 ? 2 : 1);
         fence_barrier_init();
     }
     if (warp == 1) tmem_alloc2(tmem_holder, kTmemCols);
@@ -741,18 +500,22 @@ __device__ __forceinline__ void scan_pair_body(const ScanArgs& a) {
     tc_fence_after();
     const uint32_t tmem_base = *tmem_holder;
 
-    // tiles of this level are taken 2 NP at a time: walk position 2*NP*p + rank
+    // tiles of this level are taken two at a time: walk position 2 p + rank
     if (warp == 0) {
         // =============================== producer ===============================
         // (all lanes run the warp-uniform loop, one elected lane issues: see elect_one)
         {
-            const uint64_t pol_x = (n_qt == 1) ? policy_evict_first() : (a.x_policy >= 2 ? policy_evict_last() : policy_evict_normal());
+            // corpus blocks that are re-read once per query tile: evict_last, and evict_first on their LAST read (last
+            // query tile) so that dead tiles, not live ones, make room for the next tiles.  DRAM reads of a 21M-row step
+            // at batch 4096 (43.0 GB algorithmic; single-pass ncu, profiles/r02_ab/r2w, r2x): evict_normal 78.6 GB,
+            // evict_last 61.8 GB, with the demotion 54.3 GB; time unchanged (DRAM is at 6 %).
+            const uint64_t pol_x = (n_qt == 1) ? policy_evict_first() : policy_evict_last();
             const uint64_t pol_x_last = policy_evict_first();
             const uint64_t pol_q = policy_evict_last();
-            if (a.q_dep) pdl_wait();
+            if (a.q_dep) pdl_wait();  // level 0: the query shadow is being written by the previous kernel
             if (RES && elect_one()) {  // the batch is one query tile: this CTA's half stays in shared memory for the whole launch
                 mbar_expect_tx(q_bar, (uint32_t)(KC * kQHalfBytes));
-                bulk_g2s(q_res, a.qshadow + (size_t)half * ((size_t)a.d * kPairHalfQ * 2), (uint32_t)(KC * kQHalfBytes),
+                bulk_g2s(q_res, a.qshadow + (size_t)rank * ((size_t)a.d * kHalfQ * 2), (uint32_t)(KC * kQHalfBytes),
                          q_bar, pol_q);
             }
             __syncwarp();
@@ -761,34 +524,21 @@ __device__ __forceinline__ void scan_pair_body(const ScanArgs& a) {
             for (int64_t w = w_lo; w < w_hi; ++w) {
                 const int64_t p = w / n_qt;
                 const int qt = (int)(w - p * n_qt);
-                int64_t ti = a.tile_lo + kCl * p + rank;
+                int64_t ti = a.tile_lo + 2 * p + rank;
                 if (ti >= a.tile_hi) ti = a.tile_hi - 1;  // ragged tail: stage a valid tile, rows are masked later
                 const int64_t tile = (ti * a.tile_mult) % a.n_tiles;
                 const uint8_t* xsrc = a.shadow + (size_t)tile * ((size_t)a.d * kTileRows * 2);
-                // query shadow is stored in 128-row tiles: this CTA stages tile 2*qt + half
-                const uint8_t* qsrc = a.qshadow + (size_t)(2 * qt + half) * ((size_t)a.d * kPairHalfQ * 2);
-                const uint8_t* pfsrc = nullptr;  // the tile this CTA streams pf_tiles work items from now
-                if (a.pf_tiles > 0 && qt == 0 && (p + a.pf_tiles) * n_qt < w_hi) {
-                    int64_t pti = a.tile_lo + kCl * (p + a.pf_tiles) + rank;
-                    if (pti < a.tile_hi) pfsrc = a.shadow + (size_t)((pti * a.tile_mult) % a.n_tiles) * ((size_t)a.d * kTileRows * 2);
-                }
-                // x_policy 3: the LAST read of a corpus block (last query tile) demotes it to evict_first, so that dead
-                // tiles, not live ones, make room for the next tiles
-                const uint64_t pol_xw = (a.x_policy == 3 && n_qt > 1 && qt == n_qt - 1) ? pol_x_last : pol_x;
+                // query shadow is stored in half tiles of PQ/2 rows: this CTA stages half tile 2*qt + rank
+                const uint8_t* qsrc = a.qshadow + (size_t)(2 * qt + rank) * ((size_t)a.d * kHalfQ * 2);
+                const uint64_t pol_xw = (n_qt > 1 && qt == n_qt - 1) ? pol_x_last : pol_x;
                 for (int kc = 0; kc < KC; ++kc) {
                     mbar_wait_warp(&empty_bar[s], ph ^ 1u, 100 + s, lane);
-                    uint8_t* dst = stage_base + (size_t)s * kPairStageBytes;
+                    uint8_t* dst = stage_base + (size_t)s * kStageBytes;
                     if (elect_one()) {
-                        if (pfsrc) bulk_prefetch_l2(pfsrc + (size_t)kc * kBlockBytes, kBlockBytes);
-                        mbar_expect_tx(&full_bar[s], (uint32_t)kPairStageBytes);
+                        mbar_expect_tx(&full_bar[s], (uint32_t)kStageBytes);
                         bulk_g2s(dst, xsrc + (size_t)kc * kBlockBytes, kBlockBytes, &full_bar[s], pol_xw);
-                        if (!RES) {
-                            if (NP == 1)
-                                bulk_g2s(dst + kBlockBytes, qsrc + (size_t)kc * kQHalfBytes, kQHalfBytes, &full_bar[s], pol_q);
-                            else if ((uint32_t)(kc % NP) == pairc)  // this pair's turn: one L2 read for all NP pairs
-                                bulk_g2s_multicast(dst + kBlockBytes, qsrc + (size_t)kc * kQHalfBytes, kQHalfBytes, &full_bar[s],
-                                                   mask_half, pol_q);
-                        }
+                        if (!RES)
+                            bulk_g2s(dst + kBlockBytes, qsrc + (size_t)kc * kQHalfBytes, kQHalfBytes, &full_bar[s], pol_q);
                     }
                     __syncwarp();
                     if (++s == NS) { s = 0; ph ^= 1u; }
@@ -799,24 +549,24 @@ __device__ __forceinline__ void scan_pair_body(const ScanArgs& a) {
         {
             int s = 0;
             uint32_t ph = 0;
-            if (half == 1) {
+            if (rank == 1) {
                 // ============================= forwarder =============================
                 if (RES) {
                     mbar_wait_warp(q_bar, 0, 650, lane);                          // this CTA's half of the query tile has landed
-                    if (elect_one()) mbar_arrive_cluster(map_to_rank(q_bar, leader));   // tell the leader
+                    if (elect_one()) mbar_arrive_cluster(map_to_rank(q_bar, 0));  // tell the leader
                     __syncwarp();
                 }
                 for (int64_t w = w_lo; w < w_hi; ++w) {
                     for (int kc = 0; kc < KC; ++kc) {
-                        mbar_wait_warp(&full_bar[s], ph, 600 + s, lane);               // this CTA's stage has landed
-                        if (elect_one()) mbar_arrive_cluster(map_to_rank(&full_bar[s], leader));  // tell the leader
+                        mbar_wait_warp(&full_bar[s], ph, 600 + s, lane);                    // this CTA's stage has landed
+                        if (elect_one()) mbar_arrive_cluster(map_to_rank(&full_bar[s], 0));  // tell the leader
                         __syncwarp();
                         if (++s == NS) { s = 0; ph ^= 1u; }
                     }
                 }
             } else {
                 // ================================ MMA ================================
-                constexpr uint32_t idesc = make_idesc_bf16(2 * kTileRows, kPairQ);
+                constexpr uint32_t idesc = make_idesc_bf16(2 * kTileRows, PQ);
                 if (RES) mbar_wait_warp(q_bar, 0, 200, lane);  // both halves of the query tile are resident
                 uint32_t it = 0;
                 for (int64_t w = w_lo; w < w_hi; ++w, ++it) {
@@ -824,20 +574,21 @@ __device__ __forceinline__ void scan_pair_body(const ScanArgs& a) {
                     const uint32_t aph = (it >> 1) & 1u;
                     mbar_wait_warp(&tmem_empty[as], aph ^ 1u, 300 + as, lane);
                     tc_fence_after();
-                    const uint32_t d_tmem = tmem_base + as * kPairQ;
+                    const uint32_t d_tmem = tmem_base + as * PQ;
                     for (int kc = 0; kc < KC; ++kc) {
                         mbar_wait_warp(&full_bar[s], ph, 400 + s, lane);  // own bytes + the peer's forward
                         tc_fence_after();
-                        const uint32_t xa = smem_u32(stage_base + (size_t)s * kPairStageBytes);
+                        const uint32_t xa = smem_u32(stage_base + (size_t)s * kStageBytes);
                         const uint64_t da = make_sw128_desc(xa);
                         const uint64_t db = make_sw128_desc(RES ? smem_u32(q_res + (size_t)kc * kQHalfBytes) : xa + kBlockBytes);
                         if (elect_one()) {
 #pragma unroll
                             for (int k4 = 0; k4 < 4; ++k4)
+                                // +32 bytes (two 16-byte units) per K=16 step inside the 128-byte swizzle row
                                 umma_bf16_2cta(d_tmem, da + (uint64_t)(k4 * 2), db + (uint64_t)(k4 * 2), idesc,
                                                (kc | k4) ? 1u : 0u);
-                            umma_commit_2cta(&empty_bar[s], kMaskAll);  // every CTA of the cluster: the stage is free for this pair
-                            if (kc == KC - 1) umma_commit_2cta(&tmem_full[as], mask_pair);
+                            umma_commit_2cta(&empty_bar[s], kPairMask);  // frees the stage in both CTAs once read
+                            if (kc == KC - 1) umma_commit_2cta(&tmem_full[as], kPairMask);  // accumulator complete
                         }
                         __syncwarp();
                         if (++s == NS) { s = 0; ph ^= 1u; }
@@ -847,17 +598,17 @@ __device__ __forceinline__ void scan_pair_body(const ScanArgs& a) {
         }
     } else {
         // ================================ filter ================================
-        const int quad = warp & 3;
+        const int quad = warp & 3;  // TMEM lane quadrant this warp may read
         const uint32_t lane_base = (uint32_t)(quad * 32) << 16;
         uint32_t leader_empty[2];
-        leader_empty[0] = map_to_rank(&tmem_empty[0], leader);
-        leader_empty[1] = map_to_rank(&tmem_empty[1], leader);
-        constexpr int NG = EpiCfg<kPairQ>::kGroups;
-        const int col0 = ((warp - 2) >> 2) * (NG * 32);
+        leader_empty[0] = map_to_rank(&tmem_empty[0], 0);
+        leader_empty[1] = map_to_rank(&tmem_empty[1], 0);
+        constexpr int NG = EpiCfg<PQ>::kGroups;
+        const int col0 = ((warp - 2) >> 2) * (NG * 32);  // this warp's first column inside the query tile
         uint32_t it = 0;
         Stash pend, cur;
         stash_clear(pend);
-        pdl_wait();
+        pdl_wait();  // tau / cand / cnt come from the previous compaction; the corpus stream did not have to wait
         // Thresholds of this warp's columns: lane l holds tau of column g*32 + l.  They are fetched through L2 one
         // work item AHEAD (the streamed variant changes query tile with every item): ncu r2a at B = 256 had the
         // filter warps spend 52 % of their time on the in-loop tau loads — with the memory system saturated by the
@@ -868,12 +619,12 @@ __device__ __forceinline__ void scan_pair_body(const ScanArgs& a) {
             const int qt0 = RES ? 0 : (int)(w_lo % n_qt);
 #pragma unroll
             for (int g = 0; g < NG; ++g)
-                mytau[g] = (w_lo < w_hi) ? __ldcg(a.tau + (int64_t)qt0 * kPairQ + col0 + g * 32 + lane) : 0.f;
+                mytau[g] = (w_lo < w_hi) ? __ldcg(a.tau + (int64_t)qt0 * PQ + col0 + g * 32 + lane) : 0.f;
         }
         for (int64_t w = w_lo; w < w_hi; ++w, ++it) {
             const int64_t p = w / n_qt;
             const int qt = (int)(w - p * n_qt);
-            const int64_t ti = a.tile_lo + kCl * p + rank;
+            const int64_t ti = a.tile_lo + 2 * p + rank;
             const bool tile_ok = ti < a.tile_hi;
             const int64_t tile = ((tile_ok ? ti : a.tile_hi - 1) * a.tile_mult) % a.n_tiles;
             const int64_t row = tile * kTileRows + quad * 32 + lane;
@@ -884,20 +635,21 @@ __device__ __forceinline__ void scan_pair_body(const ScanArgs& a) {
             const bool fetch = !RES && n_qt > 1 && w + 1 < w_hi;
 #pragma unroll
             for (int g = 0; g < NG; ++g)
-                nxtau[g] = fetch ? __ldcg(a.tau + (int64_t)qt_next * kPairQ + col0 + g * 32 + lane) : mytau[g];
+                nxtau[g] = fetch ? __ldcg(a.tau + (int64_t)qt_next * PQ + col0 + g * 32 + lane) : mytau[g];
             mbar_wait(&tmem_full[as], aph, 500 + as);
             tc_fence_after();
             const uint32_t ebar = leader_empty[as];
-            filter_item<NG>(a, tmem_base + lane_base + as * kPairQ + col0, (int64_t)qt * kPairQ + col0, row, row_ok,
+            filter_item<NG>(a, tmem_base + lane_base + as * PQ + col0, (int64_t)qt * PQ + col0, row, row_ok,
                             lane, cur, mytau, [=]() {
+                                // all of this warp's reads of the accumulator are done
                                 tc_fence_before();
                                 __syncwarp();
                                 if (lane == 0) mbar_arrive_cluster(ebar);
                             });
 #pragma unroll
             for (int g = 0; g < NG; ++g) mytau[g] = nxtau[g];
-            stash_store(a, pend);
-            stash_reserve(a, cur);
+            stash_store(a, pend);    // slots reserved one item ago
+            stash_reserve(a, cur);   // atomics in flight until the next item has been read
             pend = cur;
         }
         stash_store(a, pend);
@@ -914,58 +666,8 @@ __device__ __forceinline__ void scan_pair_body(const ScanArgs& a) {
     }
 }
 
-template <int PQ, bool RES>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(EpiCfg<PQ>::kThreads, 1)
-scan_tc_pair_kernel(const ScanArgs a) {
-    scan_pair_body<PQ, RES, 1>(a);
-}
-
-// NP pairs per cluster (cluster size 2 NP, given at launch): the streamed 256-query kernel with multicast query blocks
-template <int NP>
-__global__ void __launch_bounds__(EpiCfg<256>::kThreads, 1)
-scan_tc_multi_kernel(const ScanArgs a) {
-    scan_pair_body<256, false, NP>(a);
-}
-
 // ------------------------------------------------------------------ host ----
 int scan_tc_supported(int d) { return (d % 64 == 0 && d >= 64 && d <= 4096) ? 1 : 0; }
-
-static size_t scan_smem_bytes(int bq, bool resident, int d, int n_stages) {
-    const size_t stage = kBlockBytes + (resident ? 0 : (size_t)bq * 128);
-    size_t total = 1024 /* alignment slack */ + (size_t)n_stages * stage;
-    if (resident) total += (size_t)(d / 64) * bq * 128;
-    total += (2 * kMaxStages + 5) * 8 + 16;
-    return total;
-}
-
-static int pick_stages(int bq, bool resident, int d) {
-    int ns = kMaxStages;
-    while (ns > 0 && scan_smem_bytes(bq, resident, d, ns) > (size_t)kSmemLimit) --ns;
-    return ns;
-}
-
-static int env_flag(const char* name, int dflt) {
-    const char* v = getenv(name);
-    return (v && *v) ? atoi(v) : dflt;
-}
-
-// Grid of a scan launch: one CTA (pair) per SM (pair) with equal contiguous work ranges.  ncu (r2a, B = 256)
-// shows sm__cycles_active between 0.99M and 1.43M of 1.44M elapsed cycles, which suggested cutting long levels
-// into more CTAs than SMs so that the hardware block scheduler balances them (KIRAG_SCAN_WAVES > 1: up to that
-// many ranges per SM, none shorter than `min_items` work items).  Measured at 21M rows (profiles/r02_ab/r2c_knobs.log):
-// no gain at any batch size (B=256 13.3 vs 13.4 ms, B=512 20.5 vs 19.2 ms), so the default stays 1.
-constexpr int64_t kWaveItems = 48;  // corpus tiles (or tile pairs) per range, times the number of query tiles
-static int64_t scan_grid_limit(int64_t work_items, int64_t slots, int64_t min_items) {
-    int waves = env_flag("KIRAG_SCAN_WAVES", 1);
-    if (waves < 1) waves = 1;
-    int64_t limit = slots;
-    if (waves > 1 && min_items > 0) {
-        int64_t ranges = work_items / min_items;  // ranges of at least min_items items
-        if (ranges > slots * waves) ranges = slots * waves;
-        if (ranges > limit) limit = ranges / slots * slots;  // whole waves only
-    }
-    return limit;
-}
 
 template <int PQ, bool RES>
 static size_t pair_fixed_bytes(int d) {
@@ -980,25 +682,12 @@ static int pair_stages(int d) {
 
 int scan_tc_pick(int64_t nq, int d, ScanTcPlan* plan) {
     KIRAG_CHECK(scan_tc_supported(d), "scan_tc: dimension %d is not supported (need a multiple of 64, <= 4096)", d);
-    const int pair_ok = env_flag("KIRAG_SCAN_PAIR", 1) ? 1 : 0;
-    plan->pair = 0;
-    plan->multi = 1;
-    // up to 64 queries: the 2-CTA kernel with a resident 64-query tile (32 queries = 64 KB per CTA, 10 stages).  Same-box
-    // A/B against the single-CTA resident kernels at 21M rows (profiles/r02_ab/r3j_ab.log, r3k_ab.log): 5.85 vs 6.2 ms at
-    // 1-32 queries (7.3 TB/s whole-step), 6.1 vs 6.4 ms at 48, 6.2-6.6 vs 6.6-6.7 ms at 64.  KIRAG_PAIR64=0: single CTA.
-    if (nq <= 64 && pair_ok && env_flag("KIRAG_PAIR64", 1) && pair_stages<64, true>(d) >= 6) { plan->bq = 64; plan->resident = 1; plan->pair = 1; }
-    else if (nq <= 32 && pick_stages(32, true, d) >= 4) { plan->bq = 32; plan->resident = 1; }
-    else if (nq <= 64 && pick_stages(64, true, d) >= 4) { plan->bq = 64; plan->resident = 1; }  // 128 KB of queries + >= 4 stages
-    else if (nq <= 64) { plan->bq = 64; plan->resident = 0; }
-    else if (nq <= 128 && pair_ok && pair_stages<128, true>(d) >= 4) { plan->bq = 128; plan->resident = 1; plan->pair = 1; }
-    else if (nq <= 128) { plan->bq = 128; plan->resident = 0; }
-    else {
-        plan->bq = 256; plan->resident = 0; plan->pair = pair_ok;
-        // pairs per cluster sharing one multicast copy of every query block (1: no sharing)
-        const int multi = env_flag("KIRAG_SCAN_MULTI", kDefaultMulti);
-        plan->multi = (pair_ok && (multi == 2 || multi == 4)) ? multi : 1;
-    }
-    plan->q_tile_rows = plan->pair ? plan->bq / 2 : plan->bq;
+    // up to 64 queries: a resident 64-query tile (32 queries = 64 KB per CTA at d = 1024, 10 stages).  Same-box A/B
+    // against the single-CTA resident kernels it replaced, 21M rows (profiles/r02_ab/r3j_ab.log, r3k_ab.log): 5.85 vs
+    // 6.2 ms at 1-32 queries (7.3 TB/s whole-step), 6.1 vs 6.4 ms at 48, 6.2-6.6 vs 6.6-6.7 ms at 64.
+    if (nq <= 64) { plan->bq = 64; plan->resident = pair_stages<64, true>(d) >= 6; }
+    else if (nq <= 128) { plan->bq = 128; plan->resident = pair_stages<128, true>(d) >= 4; }
+    else { plan->bq = 256; plan->resident = 0; }
     return 0;
 }
 
@@ -1007,6 +696,9 @@ size_t scan_tc_qshadow_bytes(int64_t nq, int d, const ScanTcPlan& plan) {
     return (size_t)tiles * plan.bq * d * 2;
 }
 
+// one pair per SM pair with equal contiguous work ranges.  More, shorter ranges for the hardware block scheduler to
+// balance (ncu r2a, B = 256: sm__cycles_active 0.99M-1.43M of 1.44M elapsed) gained nothing at 21M rows
+// (profiles/r02_ab/r2c_knobs.log: B=256 13.3 vs 13.4 ms, B=512 20.5 vs 19.2 ms).
 template <int PQ, bool RES>
 static int launch_scan_pair(const ScanArgs& args_in, int num_sms, cudaStream_t st) {
     ScanArgs args = args_in;
@@ -1017,87 +709,19 @@ static int launch_scan_pair(const ScanArgs& args_in, int num_sms, cudaStream_t s
     const size_t smem = pair_fixed_bytes<PQ, RES>(args.d) + (size_t)ns * PairCfg<PQ, RES>::kStageBytes;
     if (ensure_dynamic_smem(scan_tc_pair_kernel<PQ, RES>, kSmemLimit)) return 1;
     int64_t pairs = ((args.tile_hi - args.tile_lo + 1) / 2) * ((args.nq + PQ - 1) / PQ);  // work items
-    const int64_t max_pairs = scan_grid_limit(pairs, num_sms / 2, ((args.nq + PQ - 1) / PQ) * kWaveItems);
-    if (pairs > max_pairs) pairs = max_pairs;
+    if (pairs > num_sms / 2) pairs = num_sms / 2;
     if (pairs <= 0) return 0;
     KIRAG_CUDA_OK(launch_chained(scan_tc_pair_kernel<PQ, RES>, dim3((unsigned)(2 * pairs)), dim3(EpiCfg<PQ>::kThreads), smem, st, args));
     KIRAG_LAUNCH_OK("scan_tc_pair_kernel");
     return 0;
 }
 
-// cluster kernel with NP pairs per cluster: as many clusters as the GPU can hold at once (GPCs whose TPC count is not a
-// multiple of NP leave a TPC unused), each taking an equal contiguous range of (tile group, query tile) work items
-template <int NP>
-static int launch_scan_multi(const ScanArgs& args_in, int num_sms, cudaStream_t st) {
-    ScanArgs args = args_in;
-    const int ns = pair_stages<256, false>(args.d);
-    KIRAG_CHECK(ns >= 2, "scan_tc multi: no room for a shared-memory pipeline");
-    args.n_stages = ns;
-    const size_t smem = pair_fixed_bytes<256, false>(args.d) + (size_t)ns * PairCfg<256, false>::kStageBytes;
-    if (ensure_dynamic_smem(scan_tc_multi_kernel<NP>, kSmemLimit)) return 1;
-    constexpr int kCl = 2 * NP;
-    cudaLaunchConfig_t cfg = {};
-    cfg.blockDim = dim3(EpiCfg<256>::kThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = kCl;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    static int max_clusters[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // per NP, queried once (one GPU model per process)
-    if (max_clusters[NP] == 0) {
-        cfg.gridDim = dim3((unsigned)(kCl * (num_sms / kCl)));
-        cfg.numAttrs = 1;
-        int n = 0;
-        if (cudaOccupancyMaxActiveClusters(&n, scan_tc_multi_kernel<NP>, &cfg) != cudaSuccess || n <= 0) {
-            cudaGetLastError();
-            n = num_sms / kCl / 2;  // conservative: co-residency of the whole grid is not required for correctness
-            if (n < 1) n = 1;
-        }
-        max_clusters[NP] = n;
-    }
-    int64_t clusters = ((args.tile_hi - args.tile_lo + kCl - 1) / kCl) * ((args.nq + 255) / 256);  // work items
-    if (clusters > max_clusters[NP]) clusters = max_clusters[NP];
-    if (clusters <= 0) return 0;
-    cfg.gridDim = dim3((unsigned)(kCl * clusters));
-    cfg.numAttrs = pdl_enabled() ? 2 : 1;
-    KIRAG_CUDA_OK(cudaLaunchKernelEx(&cfg, scan_tc_multi_kernel<NP>, args));
-    KIRAG_LAUNCH_OK("scan_tc_multi_kernel");
-    return 0;
-}
-
-template <int BQ, bool RESIDENT>
-static int launch_scan_t(const ScanArgs& args_in, int num_sms, cudaStream_t st) {
-    ScanArgs args = args_in;
-    args.n_stages = pick_stages(BQ, RESIDENT, args.d);
-    KIRAG_CHECK(args.n_stages >= 2, "scan_tc: d=%d leaves no room for a shared-memory pipeline", args.d);
-    const size_t smem = scan_smem_bytes(BQ, RESIDENT, args.d, args.n_stages);
-    if (ensure_dynamic_smem(scan_tc_kernel<BQ, RESIDENT>, kSmemLimit)) return 1;
-    const int64_t n_qt = (args.nq + BQ - 1) / BQ;
-    int64_t grid = (args.tile_hi - args.tile_lo) * n_qt;  // work items
-    const int64_t max_grid = scan_grid_limit(grid, num_sms, n_qt * kWaveItems);
-    if (grid > max_grid) grid = max_grid;
-    if (grid <= 0) return 0;
-    KIRAG_CUDA_OK(launch_chained(scan_tc_kernel<BQ, RESIDENT>, dim3((unsigned)grid), dim3(EpiCfg<BQ>::kThreads), smem, st, args));
-    KIRAG_LAUNCH_OK("scan_tc_kernel");
-    return 0;
-}
-
 static int launch_scan_args(const ScanArgs& args, const ScanTcPlan& plan, int num_sms, cudaStream_t st) {
-    if (plan.pair && plan.bq == 256 && !plan.resident && plan.multi == 2) return launch_scan_multi<2>(args, num_sms, st);
-    if (plan.pair && plan.bq == 256 && !plan.resident && plan.multi == 4) return launch_scan_multi<4>(args, num_sms, st);
-    if (plan.pair && plan.bq == 256 && !plan.resident) return launch_scan_pair<256, false>(args, num_sms, st);
-    if (plan.pair && plan.bq == 128 && plan.resident) return launch_scan_pair<128, true>(args, num_sms, st);
-    if (plan.pair && plan.bq == 64 && plan.resident) return launch_scan_pair<64, true>(args, num_sms, st);
-    if (plan.bq == 32 && plan.resident) return launch_scan_t<32, true>(args, num_sms, st);
-    if (plan.bq == 64 && plan.resident) return launch_scan_t<64, true>(args, num_sms, st);
-    if (plan.bq == 64 && !plan.resident) return launch_scan_t<64, false>(args, num_sms, st);
-    if (plan.bq == 128 && !plan.resident) return launch_scan_t<128, false>(args, num_sms, st);
-    if (plan.bq == 256 && !plan.resident) return launch_scan_t<256, false>(args, num_sms, st);
+    if (plan.bq == 64 && plan.resident) return launch_scan_pair<64, true>(args, num_sms, st);
+    if (plan.bq == 64 && !plan.resident) return launch_scan_pair<64, false>(args, num_sms, st);
+    if (plan.bq == 128 && plan.resident) return launch_scan_pair<128, true>(args, num_sms, st);
+    if (plan.bq == 128 && !plan.resident) return launch_scan_pair<128, false>(args, num_sms, st);
+    if (plan.bq == 256 && !plan.resident) return launch_scan_pair<256, false>(args, num_sms, st);
     set_error("scan_tc: no kernel for plan (bq=%d resident=%d)", plan.bq, plan.resident);
     return 1;
 }
@@ -1123,12 +747,6 @@ int launch_scan_tc(const void* shadow, int64_t n_rows, int d, const void* qshado
     args.cap = cap;
     args.dump = nullptr;
     args.dump_ld = 0;
-    // corpus blocks that are re-read once per query tile: evict_last, and evict_first on their LAST read so that dead
-    // tiles make room instead of live ones.  DRAM reads of a 21M-row step at batch 4096 (43.0 GB algorithmic; single-pass
-    // ncu, profiles/r02_ab/r2w, r2x): evict_normal 78.6 GB, evict_last 61.8 GB, with the demotion 54.3 GB; time unchanged
-    // (DRAM is at 6 %).
-    args.x_policy = env_flag("KIRAG_X_POLICY", 3);
-    args.pf_tiles = env_flag("KIRAG_PF_TILES", 0);
     return launch_scan_args(args, plan, num_sms, st);
 }
 

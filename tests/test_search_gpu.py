@@ -77,7 +77,9 @@ def test_argument_errors(fa):
 
 # ------------------------------------------------------ tensor-core scores ---
 @pytest.mark.parametrize("n,d,nq", [(300, 64, 5), (1000, 128, 32), (777, 1024, 3), (4096, 1024, 40), (513, 256, 100),
-                                    (300, 192, 200)])
+                                    (300, 192, 200),
+                                    # large d, where the plan streams the 64- / 128-query tiles
+                                    (1000, 2560, 5), (1000, 2560, 40), (600, 1536, 100), (300, 4096, 1), (300, 4096, 128)])
 def test_tcgen05_scores_match_bf16_reference(fa, n, d, nq):
     """The MMA itself (descriptors, swizzled layout, TMEM read-out): dense approximate scores equal the
     fp32-accumulated product of the bf16-rounded operands."""
@@ -92,14 +94,17 @@ def test_tcgen05_scores_match_bf16_reference(fa, n, d, nq):
     assert np.max(np.abs(got - ref) / scale) < 2e-6  # fp32 accumulation of exact bf16 products
 
 
-@pytest.mark.parametrize("code,nq", [("32", 5), ("64", 40), ("1064", 40), ("2064", 40), ("2064", 1), ("128", 100),
-                                     ("1128", 100), ("256", 200), ("512", 300)])
-def test_every_scan_kernel_variant_scores_match_bf16_reference(fa, monkeypatch, code, nq):
+@pytest.mark.parametrize("code,n,d,nq", [("64r", 1300, 256, 1), ("64r", 1300, 256, 40), ("64s", 1300, 256, 5),
+                                         ("64s", 1300, 256, 40), ("128r", 1300, 256, 100), ("128s", 1300, 256, 65),
+                                         ("128s", 1300, 256, 100), ("256s", 1300, 256, 200), ("256s", 1300, 256, 300),
+                                         # ragged tile groups at three d
+                                         ("256s", 3000, 128, 260), ("256s", 1100, 1024, 600), ("256s", 129, 64, 257)])
+def test_every_scan_kernel_variant_scores_match_bf16_reference(fa, monkeypatch, code, n, d, nq):
     """Every instantiation of the scan kernel, forced through KIRAG_DEBUG_BQ (the default plan only exercises the ones
-    it picks): single-CTA 32 / 64 resident and 64 / 128 / 256 streamed, 2-CTA resident 64 / 128 and streamed 256."""
+    it picks at the dimension of the index): 64 / 128-query tiles resident (r) and streamed (s), 256-query tiles
+    streamed."""
     monkeypatch.setenv("KIRAG_DEBUG_BQ", code)
-    rng = np.random.default_rng(int(code) + nq)
-    n, d = 1300, 256
+    rng = np.random.default_rng(n + d + nq + len(code))
     xb = rng.standard_normal((n, d)).astype(np.float32)
     xq = rng.standard_normal((nq, d)).astype(np.float32)
     got = build(fa, xb).debug_scores(xq)
@@ -111,11 +116,16 @@ def test_every_scan_kernel_variant_scores_match_bf16_reference(fa, monkeypatch, 
     assert np.array_equal(goti, (xi.astype(np.float64) @ qi.astype(np.float64).T).astype(np.float32))
 
 
-@pytest.mark.parametrize("pair64", ["0", "1"])
-def test_small_batches_on_both_resident_kernels(fa, monkeypatch, pair64):
-    """Batches of up to 64 queries through the 2-CTA resident-64 kernel (default) and through the single-CTA resident
-    kernels (KIRAG_PAIR64=0): same exact answer."""
-    monkeypatch.setenv("KIRAG_PAIR64", pair64)
+def test_unknown_scan_kernel_variant_is_an_error(fa, monkeypatch):
+    monkeypatch.setenv("KIRAG_DEBUG_BQ", "512")
+    rng = np.random.default_rng(3)
+    ix = build(fa, rng.standard_normal((300, 64)).astype(np.float32))
+    with pytest.raises(RuntimeError):
+        ix.debug_scores(rng.standard_normal((4, 64)).astype(np.float32))
+
+
+def test_small_batches_on_the_resident_64_kernel(fa):
+    """Batches of up to 64 queries (the resident 64-query tile) and just above: exact answers."""
     rng = np.random.default_rng(77)
     xb = unit_rows(rng, 60000, 128)
     ix = build(fa, xb)
@@ -123,7 +133,32 @@ def test_small_batches_on_both_resident_kernels(fa, monkeypatch, pair64):
         xq = unit_rows(rng, nq, 128)
         D, I, st = ix.search_ex(xq, 10, path=AUTO)
         assert st["n_fast"] == nq, st
-        assert_topk_parity(D, I, xb, xq, 10, what=f"pair64={pair64} nq={nq} {st}")
+        assert_topk_parity(D, I, xb, xq, 10, what=f"nq={nq} {st}")
+
+
+@pytest.mark.parametrize("d", [2560, 4096])
+def test_large_d_batches_on_the_streamed_small_tiles(fa, d):
+    """At d = 2560 / 4096 the default plan streams the 64- and 128-query tiles (the resident query half would leave
+    too short a ring).  Each query has k planted neighbours far above the rest, so every first pass certifies and
+    the streamed kernels answer every query."""
+    rng = np.random.default_rng(d)
+    n, k, batches = 40000, 10, (1, 40, 100)
+    xb = unit_rows(rng, n, d)
+    xq_all = unit_rows(rng, sum(batches), d)
+    tgt = rng.choice(n, (len(xq_all), k), replace=False)
+    for i in range(len(xq_all)):
+        near = xq_all[i][None, :] + 0.3 * unit_rows(rng, k, d)
+        xb[tgt[i]] = near / np.linalg.norm(near, axis=1, keepdims=True)
+    ix = build(fa, xb)
+    q0 = 0
+    for nq in batches:
+        xq = xq_all[q0:q0 + nq]
+        D, I, st = ix.search_ex(xq, k, path=AUTO)
+        assert st["n_fast"] == nq, (nq, st)
+        assert all(set(I[r]) == set(tgt[q0 + r]) for r in range(nq)), nq
+        De, Ie, _ = ix.search_ex(xq, k, path=EXACT)
+        assert np.array_equal(I, Ie) and np.array_equal(D, De), (nq, st)
+        q0 += nq
 
 
 def test_tcgen05_scores_exact_on_integers(fa):
@@ -655,26 +690,9 @@ def test_growth_without_virtual_memory_api_still_works(fa, monkeypatch):
         assert np.array_equal(np.load(out), I0)
 
 
-# ----------------------------------------- multi-pair cluster kernel (multicast query blocks) ---
-@pytest.mark.parametrize("code", ["512", "2512", "4512"])
-@pytest.mark.parametrize("n,d,nq", [(3000, 128, 260), (1100, 1024, 600), (129, 64, 257)])
-def test_multi_pair_cluster_kernel_scores_match_bf16_reference(fa, monkeypatch, code, n, d, nq):
-    """The streamed 2-CTA kernel with 1 / 2 / 4 CTA pairs per cluster (query blocks multicast to the pairs): dense
-    approximate scores equal the fp32-accumulated product of the bf16-rounded operands, ragged tile groups included."""
-    monkeypatch.setenv("KIRAG_DEBUG_BQ", code)
-    rng = np.random.default_rng(n + d + nq)
-    xb = rng.standard_normal((n, d)).astype(np.float32)
-    xq = rng.standard_normal((nq, d)).astype(np.float32)
-    got = build(fa, xb).debug_scores(xq)
-    ref = bf16_round(xb).astype(np.float64) @ bf16_round(xq).astype(np.float64).T
-    scale = np.linalg.norm(xb, axis=1)[:, None] * np.linalg.norm(xq, axis=1)[None, :]
-    assert np.max(np.abs(got - ref) / scale) < 2e-6
-
-
-@pytest.mark.parametrize("multi", ["2", "4"])
-def test_multi_pair_cluster_kernel_full_search(fa, monkeypatch, multi):
-    monkeypatch.setenv("KIRAG_SCAN_MULTI", multi)
-    rng = np.random.default_rng(50 + int(multi))
+# ------------------------------------------------------------ streamed 256-query tiles ---
+def test_streamed_pair_kernel_full_search(fa):
+    rng = np.random.default_rng(52)
     xb, xq = unit_rows(rng, 90000, 256), unit_rows(rng, 700, 256)
     ix = build(fa, xb)
     D, I, st = ix.search_ex(xq, 20, path=AUTO)

@@ -45,7 +45,7 @@ for (n,d,nq) in ((300,64,40),(1000,128,100),(2000,1024,200),(1000,256,600)):
 """,
     "tc_scores_pair": """
 import os, numpy as np
-os.environ['KIRAG_DEBUG_BQ']='512'
+os.environ['KIRAG_DEBUG_BQ']='256s'
 from kirag_b200 import faiss_api
 rng=np.random.default_rng(0)
 for (n,d,nq) in ((256,64,256),(300,64,40),(1000,128,300),(2100,1024,520),(128,64,256),(129,256,1)):

@@ -68,8 +68,7 @@ static void case_scan() {
     kirag_index_t* h = nullptr;
     CK(kirag_index_create(d, KIRAG_METRIC_INNER_PRODUCT, 0, &h));
     CK(kirag_index_add(h, xb.data(), n, 0, nullptr));
-    const struct { const char* bq; int nq; } variants[] = {{"32", 5},   {"64", 40},   {"1064", 40}, {"2064", 40}, {"128", 100},
-                                                           {"1128", 100}, {"256", 200}, {"512", 300}, {"2512", 300}};
+    const struct { const char* bq; int nq; } variants[] = {{"64r", 40}, {"64s", 40}, {"128r", 100}, {"128s", 100}, {"256s", 300}};
     for (const auto& v : variants) {
         setenv("KIRAG_DEBUG_BQ", v.bq, 1);
         auto xq = unit_rows(rng, v.nq, d);
