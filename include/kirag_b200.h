@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define KIRAG_ABI_VERSION 6
+#define KIRAG_ABI_VERSION 7
 
 /* metric ids; only inner product is implemented, as only inner product is
  * ever constructed by the reference (retrieve.py:112, faiss_index_corpus.py:29) */
@@ -147,6 +147,28 @@ int kirag_index_search(kirag_index_t* h, const float* q, int64_t nq, int k,
 int kirag_index_search_ex(kirag_index_t* h, const float* q, int64_t nq, int k,
                           float* D, int64_t* I, int ptrs_are_device, int64_t id_offset,
                           int path, kirag_search_stats_t* stats, void* stream);
+
+/* index.range_search(x, radius)             (faiss IndexFlatIP::range_search; no reference call site)
+ * Every row j with canonical fp32 score s_qj > radius (strict, FAISS's rule for inner product).  NaN scores are never
+ * returned; a NaN or +inf radius gives empty lists, -inf every row whose score is a number above -inf.  Scores are
+ * bit-identical to what kirag_index_search returns for the same (query, row); each query's list is ordered by
+ * (score descending, id ascending) (FAISS leaves the order unspecified); `id_offset` is added to every id.
+ * Layout is FAISS's: query i owns entries [lims[i], lims[i+1]) of D (float32) / I (int64), lims[nq] in all.
+ * q: float32 [nq, d], host or device (q_is_device).  lims_out: HOST int64 [nq + 1].  Synchronous.
+ * path: KIRAG_PATH_AUTO / KIRAG_PATH_FAST one bf16 filter pass with the threshold radius - eps(q) (complete by
+ *       construction) + fp32 rescoring, a second pass for queries with more survivors than the candidate buffer
+ *       holds (stats: n_fast / n_overflow, levels 1 or 2); the exact fp32 scan for shapes the filter cannot take
+ *       (d % 64 != 0, more than 0x7fffff00 rows); KIRAG_PATH_EXACT the fp32 scan.  AUTO and EXACT agree bit for bit.
+ * The D/I entries stay in the handle (grow-only workspaces, no allocation once warm) until kirag_index_range_fetch;
+ * the next search, add or range search on the handle drops them.  A call that fails (e.g. a result that does not fit
+ * in device memory) holds nothing. */
+int kirag_index_range_search(kirag_index_t* h, const float* q, int64_t nq, float radius, int q_is_device,
+                             int64_t id_offset, int path, int64_t* lims_out, kirag_search_stats_t* stats,
+                             void* stream);
+/* Copies the lims_out[nq] entries of the last range search into D (float32) / I (int64), host or device
+ * (ptrs_are_device), and releases the held result (a second fetch is an error).  Synchronous.  An error if nothing is
+ * held. */
+int kirag_index_range_fetch(kirag_index_t* h, float* D, int64_t* I, int ptrs_are_device, void* stream);
 
 /* Stream-ordered half of a device-pointer search (KIRAG_PATH_AUTO, nq <= 16384): enqueues every kernel of the
  * first attempt (filter levels, fp32 rescoring, final sort, certificate) and the copy of the certificate flags to

@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("KIRAG_B200_LIB") or os.path.join(HERE, "libkirag_b200.so")
 
 # constants mirrored from the header
-ABI_VERSION = 6
+ABI_VERSION = 7
 METRIC_INNER_PRODUCT = 0
 METRIC_L2 = 1
 PATH_AUTO, PATH_EXACT, PATH_FAST = 0, 1, 2
@@ -66,6 +66,9 @@ SIGNATURES = {
     "kirag_index_search": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_int, c_int64, c_void_p]),
     "kirag_index_search_ex": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_int, c_int64, c_int,
                                       POINTER(SearchStats), c_void_p]),
+    "kirag_index_range_search": (c_int, [c_void_p, c_void_p, c_int64, c_float, c_int, c_int64, c_int, c_void_p,
+                                         POINTER(SearchStats), c_void_p]),
+    "kirag_index_range_fetch": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "kirag_index_search_async": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_int64, c_void_p]),
     "kirag_index_search_finish": (c_int, [c_void_p, POINTER(SearchStats), POINTER(c_int64)]),
     "kirag_index_search_flags": (c_int, [c_void_p, POINTER(c_void_p)]),

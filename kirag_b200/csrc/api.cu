@@ -23,6 +23,7 @@
 
 #include <cuda.h>  // driver-API TYPES only: the entry points are fetched with cudaGetDriverEntryPoint (no -lcuda)
 
+#include <algorithm>
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
@@ -332,6 +333,12 @@ struct kirag_index {
     PendingSearch captured;  // the asynchronous search most recently captured into a CUDA graph (kirag_index_search_rearm)
     bool has_captured = false;
     cudaEvent_t pending_ev = nullptr;
+    // range search: item arrays (+ the second buffer of the run merges), per-query counts / cursors / offsets, the
+    // long-segment table, and the result held for kirag_index_range_fetch (range_n entries of rD / rI, the chunks
+    // back to back).  Grow-only like every workspace: a call allocates only when it needs more than any call before.
+    DevBuf ritems, ritems2, rcount, rcursor, roff, rtab, rD, rI;
+    int64_t range_n = 0;
+    bool range_valid = false;
 };
 
 static int64_t round_up(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
@@ -931,8 +938,16 @@ static void fill_stats(kirag_search_stats_t* stats, int64_t nq, const SearchCoun
     stats->kernel_launches = g_launches.load() - launches0;
 }
 
+static void drop_range_result(kirag_index* h) {
+    h->range_n = 0;
+    h->range_valid = false;
+}
+
 // Completes an asynchronous search whose certificate has not been looked at yet (kirag_index_search_async).
+// Every call that uses the search workspaces or changes the rows comes through here: a held range-search
+// result is dropped as well.
 static int finish_pending(kirag_index* h, kirag_search_stats_t* stats, int64_t* n_changed) {
+    drop_range_result(h);
     if (n_changed) *n_changed = 0;
     PendingSearch& p = h->pending;
     if (!p.active) {
@@ -1004,6 +1019,321 @@ static int search_impl(kirag_index* h, const float* q, int64_t nq, int k, float*
         }
     }
     fill_stats(stats, nq, c, fast_ok, path, launches0);
+    return 0;
+}
+
+// ------------------------------------------------------------ range search ----
+// index.range_search(x, radius): every row with canonical score > radius (DESIGN.md §3, "Range search").
+//   filter path  one bf16 pass over the whole shadow with tau_q = radius - eps(q) - <q, c> collects a superset of the
+//                answer (|approx - canonical| <= eps(q)); fp32 rescoring keeps the exact answer.  The scan counts
+//                survivors past the buffer, so a query whose buffer overflowed knows its exact survivor count: it is
+//                scanned once more (pass 2) in a group whose buffer holds that many.
+//   exact path   the fp32 scan, kExactNQ queries at a time, dense scores filtered by the same test.
+// Both append each query's hits to an item array (one segment per query) and share the sort / write (range.cu).
+constexpr size_t kRangeGroupBytes = (size_t)1 << 30;  // pass-2 candidate buffers (Cand + rescored score, 12 B an entry)
+
+struct RangeChunk {
+    std::vector<int64_t> src_off, count;  // per chunk query: its segment in ritems
+    int64_t used = 0;                     // items appended so far
+};
+
+// Grows a device buffer to `need` bytes keeping its first `used` bytes.
+static int grow_keep(DevBuf& b, size_t used, size_t need, cudaStream_t st) {
+    if (need <= b.bytes) return 0;
+    size_t want = b.bytes + b.bytes / 2;
+    if (want < need) want = need;
+    want = (want + ((size_t)1 << 20) - 1) & ~(((size_t)1 << 20) - 1);
+    void* p = nullptr;
+    cudaError_t e = cudaMalloc(&p, want);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        set_error("range_search: cudaMalloc(%zu) for the collected entries failed: %s", want, cudaGetErrorString(e));
+        return 1;
+    }
+    if (used) KIRAG_CUDA_OK(cudaMemcpyAsync(p, b.p, used, cudaMemcpyDeviceToDevice, st));
+    KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    b.release();
+    b.p = p;
+    b.bytes = want;
+    return 0;
+}
+
+// Reserves segments for the source rows i with chunk_q[i] >= 0 (counts[i] entries each) and uploads the per-row
+// cursors for the collect kernel.  Synchronises the stream (the cursor vector is pageable).
+static int range_reserve(kirag_index* h, RangeChunk& rc, const std::vector<int>& counts, const std::vector<int>& chunk_q,
+                         cudaStream_t st) {
+    const size_t nsrc = counts.size();
+    std::vector<int64_t> cursor(nsrc, 0);
+    int64_t add = 0;
+    for (size_t i = 0; i < nsrc; ++i) {
+        if (chunk_q[i] < 0) continue;
+        cursor[i] = rc.used + add;
+        rc.src_off[(size_t)chunk_q[i]] = cursor[i];
+        rc.count[(size_t)chunk_q[i]] = counts[i];
+        add += counts[i];
+    }
+    if (grow_keep(h->ritems, (size_t)rc.used * 8, (size_t)(rc.used + add) * 8, st)) return 1;
+    rc.used += add;
+    if (h->rcursor.ensure(nsrc * 8)) return 1;
+    KIRAG_CUDA_OK(cudaMemcpyAsync(h->rcursor.p, cursor.data(), nsrc * 8, cudaMemcpyHostToDevice, st));
+    KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+static int range_scan(kirag_index* h, const ScanTcPlan& plan, int64_t nq, int cap, cudaStream_t st) {
+    const int64_t n = h->ntotal;
+    const int64_t n_tiles = (n + kTileRows - 1) / kTileRows;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    if (g_prof.on) {
+        KIRAG_CUDA_OK(cudaEventCreate(&e0));
+        KIRAG_CUDA_OK(cudaEventCreate(&e1));
+        KIRAG_CUDA_OK(cudaEventRecord(e0, st));
+    }
+    if (launch_scan_tc(h->shadow, n, h->d, h->qshadow.p, nq, plan, 0, n_tiles, n_tiles, 1, h->tau.as<float>(),
+                       h->cand.as<Cand>(), h->cnt.as<int>(), cap, h->num_sms, 1, st)) return 1;
+    if (g_prof.on) {
+        KIRAG_CUDA_OK(cudaEventRecord(e1, st));
+        g_prof.ev.emplace_back(e0, e1);
+        g_prof.rows += (double)n;
+        g_prof.launch_rows.push_back((double)n);
+        g_prof.queries = (double)nq;
+    }
+    return 0;
+}
+
+// One filter pass for nb queries qs (device [nb, d]) into the candidate workspace with buffer `cap`, rescored, and
+// counted; then the queries whose buffer held every survivor are collected.  qmap (device, may be null = identity)
+// maps a row of qs to its chunk query for the norms of the first conversion (h->qnorm).  Returns, per row, the
+// survivor count in *cnt_out; rows with cnt_out[i] > cap are left to the caller.
+static int range_filter_pass(kirag_index* h, const float* qs, int64_t nb, const int* qmap_dev,
+                             const std::vector<int>& chunk_q_of_row, int64_t cq, float radius, int cap, bool first,
+                             RangeChunk& rc, std::vector<int>* cnt_out, cudaStream_t st) {
+    const int d = h->d;
+    ScanTcPlan plan;
+    if (scan_tc_pick(nb, d, &plan)) return 1;
+    const size_t qs_bytes = scan_tc_qshadow_bytes(nb, d, plan);
+    const int64_t nb_pad = round_up(nb, 256);
+    if (h->qshadow.ensure(qs_bytes)) return 1;
+    if (h->cand.ensure((size_t)nb * cap * sizeof(Cand))) return 1;
+    if (h->cnt.ensure((size_t)nb_pad * 4) || h->tau.ensure((size_t)nb_pad * 4) || h->rcount.ensure((size_t)nb * 4)) return 1;
+    if ((nb % plan.bq) != 0) KIRAG_CUDA_OK(cudaMemsetAsync(h->qshadow.p, 0, qs_bytes, st));
+    float* const qn = h->qnorm.as<float>();
+    // the first pass measures the norms (+ rounding-error norms, + <q, c>) of the chunk; a second pass reuses them
+    if (launch_convert_rows(qs, nb, d, 0, h->qshadow.p, plan.bq / 2, nullptr, first ? qn : nullptr,
+                            first ? qn + cq : nullptr, first ? h->center : nullptr, first ? qn + 2 * cq : nullptr,
+                            st)) return 1;
+    const CertEps ce = cert_eps(h);
+    if (launch_range_threshold(qmap_dev, qn, qn + cq, qn + 2 * cq, radius, ce.a, ce.b, nb, nb_pad, h->tau.as<float>(),
+                               h->cnt.as<int>(), st)) return 1;
+    if (range_scan(h, plan, nb, cap, st)) return 1;
+    // the survivor counts size the rescoring: m = the largest complete buffer of the batch, not cap (~100-200 rows
+    // per query against 8192-32768 slots when the radius selects ~100 rows)
+    cnt_out->assign((size_t)nb, 0);
+    KIRAG_CUDA_OK(cudaMemcpyAsync(cnt_out->data(), h->cnt.p, (size_t)nb * 4, cudaMemcpyDeviceToHost, st));
+    KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    int m = 1;
+    for (int64_t i = 0; i < nb; ++i)
+        if ((*cnt_out)[(size_t)i] <= cap) m = std::max(m, (*cnt_out)[(size_t)i]);
+    if (h->rescored.ensure((size_t)nb * m * 4)) return 1;
+    if (launch_rescore(h->master, d, qs, h->cand.as<Cand>(), h->cnt.as<int>(), cap, m, h->rescored.as<float>(), nb,
+                       nullptr, nullptr, nullptr, 0.f, 0.f, st)) return 1;
+    if (launch_range_count_cand(h->cand.as<Cand>(), cap, h->rescored.as<float>(), m, h->cnt.as<int>(), nb, radius,
+                                h->rcount.as<int>(), st)) return 1;
+    std::vector<int> counts((size_t)nb);
+    KIRAG_CUDA_OK(cudaMemcpyAsync(counts.data(), h->rcount.p, (size_t)nb * 4, cudaMemcpyDeviceToHost, st));
+    KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    std::vector<int> keep(chunk_q_of_row);
+    for (int64_t i = 0; i < nb; ++i)
+        if ((*cnt_out)[(size_t)i] > cap) keep[(size_t)i] = -1;
+    if (range_reserve(h, rc, counts, keep, st)) return 1;
+    return launch_range_collect_cand(h->cand.as<Cand>(), cap, h->rescored.as<float>(), m, h->cnt.as<int>(), nb, radius,
+                                     h->rcursor.as<unsigned long long>(), h->ritems.as<uint64_t>(), st);
+}
+
+static int range_filter_chunk(kirag_index* h, const float* qd, int64_t cq, float radius, int cap, RangeChunk& rc,
+                              SearchCounters* c, cudaStream_t st) {
+    const int d = h->d;
+    if (h->qnorm.ensure((size_t)cq * 12)) return 1;
+    std::vector<int> rows((size_t)cq), cnt;
+    for (int64_t i = 0; i < cq; ++i) rows[(size_t)i] = (int)i;
+    if (range_filter_pass(h, qd, cq, nullptr, rows, cq, radius, cap, true, rc, &cnt, st)) return 1;
+    // pass 2: (survivor count, chunk query) of every query whose buffer overflowed
+    std::vector<std::pair<int, int>> pend;
+    for (int64_t i = 0; i < cq; ++i)
+        if (cnt[(size_t)i] > cap) pend.emplace_back(cnt[(size_t)i], (int)i);
+    c->n_overflow += (int64_t)pend.size();
+    c->n_fast += cq - (int64_t)pend.size();
+    c->levels = std::max(c->levels, pend.empty() ? 1 : 2);  // 2 if any chunk needed a second pass
+    // the scan of a group reproduces the first pass's survivors (same shadow, same threshold); the loop only guards
+    // against a count that differs between query-tile widths
+    for (int round = 0; !pend.empty(); ++round) {
+        KIRAG_CHECK(round < 4, "range_search: survivor counts did not settle between bf16 passes");
+        std::sort(pend.begin(), pend.end(), [](const std::pair<int, int>& a, const std::pair<int, int>& b) {
+            return a.first != b.first ? a.first > b.first : a.second < b.second;
+        });
+        std::vector<std::pair<int, int>> next;
+        for (size_t i0 = 0; i0 < pend.size();) {
+            const int cap2 = pend[i0].first;  // the largest count of the group (the list is sorted)
+            int64_t g = (int64_t)(kRangeGroupBytes / ((size_t)cap2 * 12));
+            if (g < 1) g = 1;
+            if (g > (int64_t)(pend.size() - i0)) g = (int64_t)(pend.size() - i0);
+            if (g > kQChunk) g = kQChunk;
+            std::vector<int> qmap((size_t)g);
+            for (int64_t j = 0; j < g; ++j) qmap[(size_t)j] = pend[i0 + (size_t)j].second;
+            if (h->qmap.ensure((size_t)g * 4) || h->qsel.ensure((size_t)g * d * 4)) return 1;
+            KIRAG_CUDA_OK(cudaMemcpyAsync(h->qmap.p, qmap.data(), (size_t)g * 4, cudaMemcpyHostToDevice, st));
+            gather_rows_kernel<<<(unsigned)g, 256, 0, st>>>(qd, h->qmap.as<int>(), d, h->qsel.as<float>());
+            KIRAG_LAUNCH_OK("gather_rows_kernel");
+            std::vector<int> cnt2;
+            if (range_filter_pass(h, h->qsel.as<float>(), g, h->qmap.as<int>(), qmap, cq, radius, cap2, false, rc, &cnt2,
+                                  st)) return 1;
+            for (int64_t j = 0; j < g; ++j)
+                if (cnt2[(size_t)j] > cap2) next.emplace_back(cnt2[(size_t)j], qmap[(size_t)j]);
+            i0 += (size_t)g;
+        }
+        pend.swap(next);
+    }
+    return 0;
+}
+
+static int range_exact_chunk(kirag_index* h, const float* qd, int64_t cq, float radius, RangeChunk& rc,
+                             SearchCounters* c, cudaStream_t st) {
+    const int64_t n = h->ntotal;
+    const int d = h->d;
+    const int64_t ld = round_up(n, 32);
+    if (h->dense.ensure((size_t)kExactNQ * ld * sizeof(float)) || h->rcount.ensure((size_t)kExactNQ * 4)) return 1;
+    for (int64_t g0 = 0; g0 < cq; g0 += kExactNQ) {
+        const int gq = (int)((cq - g0 < kExactNQ) ? (cq - g0) : kExactNQ);
+        if (launch_scan_exact(h->master, n, d, qd + g0 * d, gq, h->dense.as<float>(), ld, h->num_sms, st)) return 1;
+        if (launch_range_count_dense(h->dense.as<float>(), ld, n, gq, radius, h->rcount.as<int>(), st)) return 1;
+        std::vector<int> counts((size_t)gq), rows((size_t)gq);
+        KIRAG_CUDA_OK(cudaMemcpyAsync(counts.data(), h->rcount.p, (size_t)gq * 4, cudaMemcpyDeviceToHost, st));
+        KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+        for (int i = 0; i < gq; ++i) rows[(size_t)i] = (int)(g0 + i);
+        if (range_reserve(h, rc, counts, rows, st)) return 1;
+        if (launch_range_collect_dense(h->dense.as<float>(), ld, n, gq, radius, h->rcursor.as<unsigned long long>(),
+                                       h->ritems.as<uint64_t>(), st)) return 1;
+    }
+    c->n_exact += cq;
+    c->levels = 0;
+    return 0;
+}
+
+// Sorts the chunk's segments into the held result after its first `base` entries; lims_out[0..cq) receive base + the
+// chunk's offsets, *chunk_total its entry count.
+static int range_emit_chunk(kirag_index* h, RangeChunk& rc, int64_t cq, int64_t id_offset, int64_t base,
+                            int64_t* lims_out, int64_t* chunk_total, cudaStream_t st) {
+    std::vector<int64_t> lims((size_t)cq + 1);
+    lims[0] = 0;
+    for (int64_t i = 0; i < cq; ++i) lims[(size_t)i + 1] = lims[(size_t)i] + rc.count[(size_t)i];
+    for (int64_t i = 0; i < cq; ++i) lims_out[i] = base + lims[(size_t)i];
+    const int64_t total = lims[(size_t)cq];
+    *chunk_total = total;
+    if (total == 0) return 0;
+    if (grow_keep(h->rD, (size_t)base * 4, (size_t)(base + total) * 4, st) ||
+        grow_keep(h->rI, (size_t)base * 8, (size_t)(base + total) * 8, st)) {
+        set_error("range_search: the result of %lld entries (%lld MiB) does not fit in device memory",
+                  (long long)(base + total), (long long)(((base + total) * 12) >> 20));
+        return 1;
+    }
+    // segments longer than one sort run: table seg_src [n], seg_dst [n], seg_len [n], seg_e0 [n + 1] (flat offsets)
+    std::vector<int64_t> seg;
+    int64_t longest = 0, total_long = 0;
+    for (int64_t i = 0; i < cq; ++i)
+        if (rc.count[(size_t)i] > kRangeRun) seg.push_back(i);
+    const int n_seg = (int)seg.size();
+    std::vector<int64_t> tab(n_seg ? (size_t)4 * n_seg + 1 : 0);
+    for (int s = 0; s < n_seg; ++s) {
+        const size_t i = (size_t)seg[(size_t)s];
+        tab[(size_t)s] = rc.src_off[i];
+        tab[(size_t)n_seg + s] = lims[i];
+        tab[(size_t)2 * n_seg + s] = rc.count[i];
+        tab[(size_t)3 * n_seg + s] = total_long;
+        total_long += rc.count[i];
+        longest = std::max(longest, rc.count[i]);
+    }
+    if (n_seg) {
+        tab[(size_t)4 * n_seg] = total_long;
+        if (h->ritems2.ensure((size_t)rc.used * 8) || h->rtab.ensure(tab.size() * 8)) return 1;
+        KIRAG_CUDA_OK(cudaMemcpyAsync(h->rtab.p, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice, st));
+    }
+    // [cq] segment offsets, then [cq + 1] result offsets
+    if (h->roff.ensure(((size_t)cq * 2 + 1) * 8)) return 1;
+    KIRAG_CUDA_OK(cudaMemcpyAsync(h->roff.p, rc.src_off.data(), (size_t)cq * 8, cudaMemcpyHostToDevice, st));
+    KIRAG_CUDA_OK(cudaMemcpyAsync(h->roff.as<int64_t>() + cq, lims.data(), ((size_t)cq + 1) * 8, cudaMemcpyHostToDevice, st));
+    if (launch_range_emit(h->ritems.as<uint64_t>(), h->ritems2.as<uint64_t>(), cq, h->roff.as<int64_t>(),
+                          h->roff.as<int64_t>() + cq, n_seg, longest, total_long, h->rtab.as<int64_t>(), id_offset,
+                          h->rD.as<float>() + base, h->rI.as<int64_t>() + base, st)) return 1;
+    KIRAG_CUDA_OK(cudaStreamSynchronize(st));  // the host vectors above are read by the copies
+    return 0;
+}
+
+static int range_search_impl(kirag_index* h, const float* q, int64_t nq, float radius, int q_is_device,
+                             int64_t id_offset, int path, int64_t* lims_out, kirag_search_stats_t* stats,
+                             cudaStream_t st) {
+    KIRAG_CHECK(nq >= 0, "range_search: negative nq");
+    KIRAG_CHECK(h != nullptr, "range_search: null index");
+    KIRAG_CHECK(lims_out != nullptr, "range_search: null lims");
+    KIRAG_CHECK(path >= 0 && path <= 2, "range_search: unknown path %d", path);
+    if (finish_pending(h, nullptr, nullptr)) return 1;  // also drops the previous range result
+    if (stats) memset(stats, 0, sizeof(*stats));
+    for (int64_t i = 0; i <= nq; ++i) lims_out[i] = 0;
+    const bool fast_ok = path != KIRAG_PATH_EXACT && h->shadow && scan_tc_supported(h->d) && h->ntotal <= 0x7fffff00LL;
+    // NaN or +inf: nothing is strictly above it
+    if (nq == 0 || h->ntotal == 0 || !(radius < INFINITY)) {
+        h->range_valid = true;
+        if (stats) { stats->nq = nq; stats->path = fast_ok ? path : KIRAG_PATH_EXACT; }
+        return 0;
+    }
+    KIRAG_CHECK(q != nullptr, "range_search: null queries");
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return 1;
+    const long long launches0 = g_launches.load();
+    const int d = h->d;
+    FastParams fp{};
+    fp.cap_override = env_int("KIRAG_CAND_CAP", 0);
+    SearchCounters c;
+    int64_t base = 0;
+    for (int64_t q0 = 0; q0 < nq; q0 += kQChunk) {
+        const int64_t cq = (nq - q0 < kQChunk) ? (nq - q0) : kQChunk;
+        const float* qd = q + q0 * d;
+        if (!q_is_device) {
+            if (h->q_dev.ensure((size_t)cq * d * 4)) return 1;
+            KIRAG_CUDA_OK(cudaMemcpyAsync(h->q_dev.p, qd, (size_t)cq * d * 4, cudaMemcpyHostToDevice, st));
+            qd = h->q_dev.as<float>();
+        }
+        RangeChunk rc;
+        rc.src_off.assign((size_t)cq, 0);
+        rc.count.assign((size_t)cq, 0);
+        if (fast_ok ? range_filter_chunk(h, qd, cq, radius, pick_cap(fp, cq), rc, &c, st)
+                    : range_exact_chunk(h, qd, cq, radius, rc, &c, st)) return 1;
+        int64_t chunk_total = 0;
+        if (range_emit_chunk(h, rc, cq, id_offset, base, lims_out + q0, &chunk_total, st)) return 1;
+        base += chunk_total;
+    }
+    lims_out[nq] = base;
+    h->range_n = base;
+    h->range_valid = true;
+    fill_stats(stats, nq, c, fast_ok, path, launches0);
+    return 0;
+}
+
+static int range_fetch_impl(kirag_index* h, float* D, int64_t* I, int ptrs_are_device, cudaStream_t st) {
+    KIRAG_CHECK(h != nullptr, "range_fetch: null index");
+    KIRAG_CHECK(h->range_valid, "range_fetch: no range-search result is held (the last call on this index was not "
+                                "kirag_index_range_search, or its result was fetched already)");
+    const int64_t total = h->range_n;
+    if (total > 0) {
+        KIRAG_CHECK(D && I, "range_fetch: null buffer");
+        DeviceGuard guard(h->device);
+        if (!guard.ok) return 1;
+        const cudaMemcpyKind kind = ptrs_are_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+        KIRAG_CUDA_OK(cudaMemcpyAsync(D, h->rD.p, (size_t)total * 4, kind, st));
+        KIRAG_CUDA_OK(cudaMemcpyAsync(I, h->rI.p, (size_t)total * 8, kind, st));
+        // the held buffers are workspaces of the handle: the next call on any stream may overwrite them
+        KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    }
+    drop_range_result(h);
     return 0;
 }
 
@@ -1168,7 +1498,8 @@ int kirag_index_destroy(kirag_index_t* h) {
     if (h->center) cudaFree(h->center);
     DevBuf* bufs[] = {&h->q_dev, &h->D_dev, &h->I_dev, &h->qshadow, &h->qnorm, &h->cand, &h->cnt, &h->tau, &h->tauk,
                       &h->overflow, &h->flags, &h->rescored, &h->dense, &h->stage_a, &h->stage_b, &h->qmap, &h->qsel, &h->qnorm2, &h->t_dev, &h->center_sums,
-                      &h->D_tmp, &h->I_tmp};
+                      &h->D_tmp, &h->I_tmp, &h->ritems, &h->ritems2, &h->rcount, &h->rcursor, &h->roff, &h->rtab,
+                      &h->rD, &h->rI};
     for (DevBuf* b : bufs) b->release();
     if (h->host_flags) cudaFreeHost(h->host_flags);
     if (h->pending_ev) cudaEventDestroy(h->pending_ev);
@@ -1214,6 +1545,19 @@ int kirag_index_search_ex(kirag_index_t* h, const float* q, int64_t nq, int k, f
                           int ptrs_are_device, int64_t id_offset, int path, kirag_search_stats_t* stats,
                           void* stream) {
     return search_impl(h, q, nq, k, D, I, ptrs_are_device, id_offset, path, stats, (cudaStream_t)stream);
+}
+
+int kirag_index_range_search(kirag_index_t* h, const float* q, int64_t nq, float radius, int q_is_device,
+                             int64_t id_offset, int path, int64_t* lims_out, kirag_search_stats_t* stats,
+                             void* stream) {
+    const int rc = range_search_impl(h, q, nq, radius, q_is_device, id_offset, path, lims_out, stats,
+                                     (cudaStream_t)stream);
+    if (rc && h) drop_range_result(h);  // no partial result
+    return rc;
+}
+
+int kirag_index_range_fetch(kirag_index_t* h, float* D, int64_t* I, int ptrs_are_device, void* stream) {
+    return range_fetch_impl(h, D, I, ptrs_are_device, (cudaStream_t)stream);
 }
 
 int kirag_index_search_async(kirag_index_t* h, const float* q, int64_t nq, int k, float* D, int64_t* I,

@@ -189,6 +189,22 @@ __device__ __forceinline__ float warp_butterfly_sum(float v) {
     v = __fadd_rn(v, __shfl_xor_sync(0xffffffffu, v, 1));
     return v;
 }
+
+// In-place descending bitonic sort of P (a power of two) 64-bit items in shared memory by the whole CTA.
+__device__ __forceinline__ void bitonic_sort_desc(uint64_t* s, int P) {
+    for (int size = 2; size <= P; size <<= 1) {
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            for (int t = threadIdx.x; t < (P >> 1); t += blockDim.x) {
+                const int pos = 2 * t - (t & (stride - 1));
+                const int par = pos + stride;
+                const bool desc = ((pos & size) == 0);
+                const uint64_t a = s[pos], b = s[par];
+                if ((a < b) == desc) { s[pos] = b; s[par] = a; }
+            }
+            __syncthreads();
+        }
+    }
+}
 #endif
 
 // ------------------------------------------------------ kernel launchers ---
@@ -250,6 +266,30 @@ int launch_scan_tc(const void* shadow, int64_t n_rows, int d, const void* qshado
 int launch_scan_tc_dump(const void* shadow, int64_t n_rows, int d, const void* qshadow, int64_t nq,
                         const ScanTcPlan& plan, const float* tau_inf, int* cnt_scratch, float* dump,
                         int64_t dump_ld, int num_sms, cudaStream_t st);
+// range.cu — range search: collect every entry with score > radius, then sort each query's segment
+constexpr int kRangeRun = 8192;  // segments up to this length are sorted by one CTA; longer ones in runs of it + merges
+// tau[i] = radius - eps(q) - <q, c> with q = qmap[i] (qmap == nullptr: q = i); +inf on the pad up to nb_pad; cnt zeroed
+int launch_range_threshold(const int* qmap, const float* qnorm, const float* qerr, const float* qcdot, float radius,
+                           float eps_a, float eps_b, int64_t nb, int64_t nb_pad, float* tau, int* cnt, cudaStream_t st);
+// candidate buffer [nq, cap] of a filter scan, rescored [nq, m] its canonical scores (m >= every count <= cap; a query
+// with cnt > cap overflowed and counts as empty): counts[q] = entries with score > radius; collect appends them at
+// cursor[q] (advanced)
+int launch_range_count_cand(const Cand* cand, int cap, const float* rescored, int m, const int* cnt, int64_t nq,
+                            float radius, int* counts, cudaStream_t st);
+int launch_range_collect_cand(const Cand* cand, int cap, const float* rescored, int m, const int* cnt, int64_t nq,
+                              float radius, unsigned long long* cursor, uint64_t* items, cudaStream_t st);
+// dense exact scores scores[q * ld + row], rows [0, n)
+int launch_range_count_dense(const float* scores, int64_t ld, int64_t n, int nq, float radius, int* counts,
+                             cudaStream_t st);
+int launch_range_collect_dense(const float* scores, int64_t ld, int64_t n, int nq, float radius,
+                               unsigned long long* cursor, uint64_t* items, cudaStream_t st);
+// Query q's items[src_off[q] .. + lims[q+1] - lims[q]) -> D / I [lims[q], lims[q+1]) by (score desc, id asc), ids +
+// id_offset.  Segments of at most kRangeRun items: one CTA each.  The n_seg longer ones are listed in the device table
+// tab = seg_src [n_seg] (item offset), seg_dst [n_seg] (result offset), seg_len [n_seg], seg_e0 [n_seg + 1] (prefix of
+// the lengths, total_long in all); they are sorted in items / items2 (same offsets).  Stream-ordered.
+int launch_range_emit(uint64_t* items, uint64_t* items2, int64_t nq, const int64_t* src_off, const int64_t* lims,
+                      int n_seg, int64_t longest, int64_t total_long, const int64_t* tab, int64_t id_offset, float* D,
+                      int64_t* I, cudaStream_t st);
 // pool.cu
 int launch_pool_normalize(const void* hidden, const void* mask, float* out, void* out_lp, float* pooled_norm,
                           int64_t B, int64_t S, int64_t H, int64_t sb, int64_t ss, int64_t mb,

@@ -13,21 +13,6 @@
 
 namespace kirag {
 
-__device__ __forceinline__ void bitonic_sort_desc(uint64_t* s, int P) {
-    for (int size = 2; size <= P; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            for (int t = threadIdx.x; t < (P >> 1); t += blockDim.x) {
-                const int pos = 2 * t - (t & (stride - 1));
-                const int par = pos + stride;
-                const bool desc = ((pos & size) == 0);
-                const uint64_t a = s[pos], b = s[par];
-                if ((a < b) == desc) { s[pos] = b; s[par] = a; }
-            }
-            __syncthreads();
-        }
-    }
-}
-
 __device__ __forceinline__ int next_pow2(int v) {
     int p = 32;
     while (p < v) p <<= 1;

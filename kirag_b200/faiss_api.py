@@ -7,6 +7,7 @@ Reference call sites (all in /root/reference/retriever/index.py):
     index.is_trained / index.train  :30-31        -> True / no-op
     index.add(x)                    :32           -> kirag_index_add
     index.search(x, k)              :47           -> kirag_index_search
+    index.range_search(x, radius)   (no call site) -> kirag_index_range_search + kirag_index_range_fetch
     faiss.write_index(index, path)  :62           -> kirag_index_save   ("IxFI" container)
     faiss.read_index(path, flags)   :73           -> kirag_index_load
     index.ntotal                    :74, :79      -> kirag_index_ntotal
@@ -120,6 +121,25 @@ class IndexFlatIP:
         self.last_stats = stats.as_dict()
         return D, I, self.last_stats
 
+    def range_search(self, x, radius: float) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """faiss IndexFlatIP.range_search: every row with score > radius.  Returns (lims int64 [n+1], D float32,
+        I int64); query i owns D/I[lims[i]:lims[i+1]], ordered by (score desc, id asc).  Honours KIRAG_PATH."""
+        x = np.ascontiguousarray(x, dtype=np.float32)
+        assert x.ndim == 2, "range_search expects a 2-D array"
+        n, d = x.shape
+        assert d == self.d, f"range_search: queries have dimension {d}, index has {self.d}"
+        path = int(os.environ.get("KIRAG_PATH", _lib.PATH_AUTO))
+        lims = np.zeros(n + 1, dtype=np.int64)
+        stats = _lib.SearchStats()
+        _lib.check(self._lib.kirag_index_range_search(self._h, _ptr(x), n, float(radius), 0, 0, path, _ptr(lims),
+                                                      ctypes.byref(stats), None), "range_search")
+        total = int(lims[n])
+        D = np.empty(total, dtype=np.float32)
+        I = np.empty(total, dtype=np.int64)
+        _lib.check(self._lib.kirag_index_range_fetch(self._h, _ptr(D), _ptr(I), 0, None), "range_search")
+        self.last_stats = stats.as_dict()
+        return lims, D, I
+
     def reconstruct_n(self, i0: int = 0, n: int = -1) -> np.ndarray:
         if n < 0:
             n = self.ntotal - i0
@@ -186,6 +206,27 @@ class IndexFlatIP:
             )
         self.last_stats = stats.as_dict()
         return D, I
+
+    def range_search_device(self, q, radius: float, id_offset: int = 0, path: int = _lib.PATH_AUTO):
+        """range_search on a float32 CUDA tensor [n, d]; returns CUDA tensors (lims int64 [n+1], D f32, I i64).  The
+        call is synchronous: the result size is only known once the survivors have been counted."""
+        import torch
+
+        q = self._own_tensor(q, "range_search_device")
+        n = q.shape[0]
+        lims = np.zeros(n + 1, dtype=np.int64)
+        stats = _lib.SearchStats()
+        st = ctypes.c_void_p(torch.cuda.current_stream(q.device).cuda_stream)
+        _lib.check(self._lib.kirag_index_range_search(self._h, ctypes.c_void_p(q.data_ptr()), n, float(radius), 1,
+                                                      int(id_offset), int(path), _ptr(lims), ctypes.byref(stats), st),
+                   "range_search_device")
+        total = int(lims[n])
+        D = torch.empty(total, dtype=torch.float32, device=q.device)
+        I = torch.empty(total, dtype=torch.int64, device=q.device)
+        _lib.check(self._lib.kirag_index_range_fetch(self._h, ctypes.c_void_p(D.data_ptr()),
+                                                     ctypes.c_void_p(I.data_ptr()), 1, st), "range_search_device")
+        self.last_stats = stats.as_dict()
+        return torch.from_numpy(lims).to(q.device), D, I
 
     def search_device_async(self, q, k: int, id_offset: int = 0):
         """Stream-ordered first half of search_device (kirag_index_search_async): no host synchronisation, CUDA-graph

@@ -322,6 +322,40 @@ class ShardedFlatIP:
         D_loc, I_loc = self.search_local(q, k, path=path)
         return self.exchange_merge(D_loc, I_loc)
 
+    def range_search(self, q: torch.Tensor, radius: float) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """q [nq, d] replicated on every rank -> (lims [nq+1], D, I) over the whole corpus, identical on every rank:
+        every global row with score > radius, per query ordered by (score desc, id asc).  Each rank answers its shard
+        (global ids), the per-query counts and the padded D/I arrays are all-gathered, and the lists are assembled
+        here: shard ranges are contiguous and ascending in rank order, so a stable sort by score over the rank-ordered
+        concatenation keeps equal scores in ascending id order."""
+        lims_l, D_l, I_l = self.index.range_search_device(q, radius, id_offset=self.lo)
+        if self.world_size == 1:
+            return lims_l, D_l, I_l
+        nq = q.shape[0]
+        counts = (lims_l[1:] - lims_l[:-1]).contiguous()
+        all_counts = [torch.empty_like(counts) for _ in range(self.world_size)]
+        dist.all_gather(all_counts, counts, group=self.group)
+        totals = [int(c.sum()) for c in all_counts]
+        width = max(max(totals), 1)
+        D_pad = torch.zeros(width, dtype=D_l.dtype, device=D_l.device)
+        I_pad = torch.zeros(width, dtype=I_l.dtype, device=I_l.device)
+        D_pad[:D_l.numel()] = D_l
+        I_pad[:I_l.numel()] = I_l
+        all_D = [torch.empty_like(D_pad) for _ in range(self.world_size)]
+        all_I = [torch.empty_like(I_pad) for _ in range(self.world_size)]
+        dist.all_gather(all_D, D_pad, group=self.group)
+        dist.all_gather(all_I, I_pad, group=self.group)
+        qids = torch.arange(nq, device=counts.device)
+        D = torch.cat([d[:t] for d, t in zip(all_D, totals)])
+        I = torch.cat([i[:t] for i, t in zip(all_I, totals)])
+        owner = torch.cat([torch.repeat_interleave(qids, c) for c in all_counts])
+        order = torch.sort(D, descending=True, stable=True).indices
+        order = order[torch.sort(owner[order], stable=True).indices]
+        per_query = torch.stack(all_counts).sum(dim=0)
+        lims = torch.zeros(nq + 1, dtype=torch.int64, device=counts.device)
+        lims[1:] = torch.cumsum(per_query, dim=0)
+        return lims, D[order], I[order]
+
     def search_graph(self, q: torch.Tensor, k: int) -> Tuple[torch.Tensor, torch.Tensor]:
         """search() for small query batches with the whole chain — local search, exchange+merge kernel, flag
         read-back — replayed from ONE CUDA graph per (nq, k): a graph launch and a stream synchronisation are all the
