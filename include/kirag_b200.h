@@ -34,12 +34,19 @@
 extern "C" {
 #endif
 
-#define KIRAG_ABI_VERSION 7
+#define KIRAG_ABI_VERSION 8
 
 /* metric ids; only inner product is implemented, as only inner product is
  * ever constructed by the reference (retrieve.py:112, faiss_index_corpus.py:29) */
 #define KIRAG_METRIC_INNER_PRODUCT 0
 #define KIRAG_METRIC_L2 1
+
+/* index flags for kirag_index_create_ex() / kirag_index_load_ex() */
+#define KIRAG_INDEX_HOST_MASTER 1 /* fp32 master in pinned host memory mapped into the device's address space (same
+                                   * address on both sides); the bf16 shadow, the workspaces and every scan stay in
+                                   * HBM.  Needs the bf16 shadow (d % 64 == 0).  Rescoring reads only the rows that can
+                                   * still reach the top-k over PCIe; the exact fp32 scan stages the master through HBM
+                                   * in chunks.  Results are bit-identical to an index with a device master. */
 
 /* search path selectors for kirag_index_search_ex() */
 #define KIRAG_PATH_AUTO 0   /* tcgen05 bf16 filter scan + fp32 rescoring, certified; exact fp32 scan for uncertified queries */
@@ -104,8 +111,13 @@ int kirag_profile_read_timeline(int* tags_out, double* ms_since_first, int64_t m
 
 /* ---- flat inner-product index  (replaces faiss.IndexFlatIP) ------------ */
 
-/* faiss.IndexFlatIP(d)                      retriever/index.py:13,23 */
+/* faiss.IndexFlatIP(d)                      retriever/index.py:13,23
+ * Same as kirag_index_create_ex(d, metric, device, 0, out). */
 int kirag_index_create(int d, int metric, int device, kirag_index_t** out);
+
+/* flags: 0 or KIRAG_INDEX_HOST_MASTER.  Unknown flag bits and KIRAG_INDEX_HOST_MASTER with d % 64 != 0 are rejected
+ * before any device is looked at. */
+int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_t** out);
 
 /* destructor of the faiss index object */
 int kirag_index_destroy(kirag_index_t* h);
@@ -204,7 +216,8 @@ int kirag_index_search_rearm(kirag_index_t* h, void* stream);
  * replay a graph only while the token equals the one read right after the capture. */
 int kirag_index_state_token(const kirag_index_t* h, uint64_t* token);
 
-/* index.reconstruct_n(i0, n): copy rows [i0, i0+n) of the fp32 master out. */
+/* index.reconstruct_n(i0, n): copy rows [i0, i0+n) of the fp32 master out (from host memory with
+ * KIRAG_INDEX_HOST_MASTER). */
 int kirag_index_reconstruct(const kirag_index_t* h, int64_t i0, int64_t n, float* out,
                             int out_is_device, void* stream);
 
@@ -212,12 +225,22 @@ int kirag_index_reconstruct(const kirag_index_t* h, int64_t i0, int64_t n, float
  * Writes the FAISS "IxFI" flat-index container (see DESIGN.md). */
 int kirag_index_save(const kirag_index_t* h, const char* path);
 
-/* faiss.read_index(path, flags)             retriever/index.py:73 */
+/* faiss.read_index(path, flags)             retriever/index.py:73
+ * Same as kirag_index_load_ex(path, device, 0, out). */
 int kirag_index_load(const char* path, int device, kirag_index_t** out);
+
+/* flags as for kirag_index_create_ex (these are index flags, not FAISS IO flags).  The file format does not depend on
+ * where the master lives: a file written by either kind of index loads into either kind. */
+int kirag_index_load_ex(const char* path, int device, int flags, kirag_index_t** out);
+
+/* Bytes of corpus storage currently mapped (device) or pinned (host): fp32 master plus bf16 shadow, workspaces not
+ * counted.  Either output may be NULL. */
+int kirag_index_storage_bytes(const kirag_index_t* h, int64_t* device_bytes, int64_t* host_bytes);
 
 /* Raw device pointers of the index storage (for zero-copy integration and
  * for the benchmark's synthetic-corpus generator).  fp32 master is row-major
- * [ntotal, d]. */
+ * [ntotal, d].  With KIRAG_INDEX_HOST_MASTER, master_f32 is a pinned HOST address that the device can dereference
+ * (the same address on both sides). */
 int kirag_index_device_ptrs(const kirag_index_t* h, const float** master_f32, const void** shadow_bf16);
 
 /* Test hook (host only, no device needed): the level schedule of the filter path for a search of nq queries

@@ -16,7 +16,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("KIRAG_B200_LIB") or os.path.join(HERE, "libkirag_b200.so")
 
 # constants mirrored from the header
-ABI_VERSION = 7
+ABI_VERSION = 8
+INDEX_HOST_MASTER = 1
 METRIC_INNER_PRODUCT = 0
 METRIC_L2 = 1
 PATH_AUTO, PATH_EXACT, PATH_FAST = 0, 1, 2
@@ -58,6 +59,7 @@ SIGNATURES = {
     "kirag_profile_read_launches": (c_int, [POINTER(ctypes.c_double), POINTER(ctypes.c_double), c_int64]),
     "kirag_profile_read_timeline": (c_int, [POINTER(c_int), POINTER(ctypes.c_double), c_int64]),
     "kirag_index_create": (c_int, [c_int, c_int, c_int, POINTER(c_void_p)]),
+    "kirag_index_create_ex": (c_int, [c_int, c_int, c_int, c_int, POINTER(c_void_p)]),
     "kirag_index_destroy": (c_int, [c_void_p]),
     "kirag_index_reserve": (c_int, [c_void_p, c_int64]),
     "kirag_index_add": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p]),
@@ -77,6 +79,8 @@ SIGNATURES = {
     "kirag_index_reconstruct": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int, c_void_p]),
     "kirag_index_save": (c_int, [c_void_p, c_char_p]),
     "kirag_index_load": (c_int, [c_char_p, c_int, POINTER(c_void_p)]),
+    "kirag_index_load_ex": (c_int, [c_char_p, c_int, c_int, POINTER(c_void_p)]),
+    "kirag_index_storage_bytes": (c_int, [c_void_p, POINTER(c_int64), POINTER(c_int64)]),
     "kirag_index_device_ptrs": (c_int, [c_void_p, POINTER(c_void_p), POINTER(c_void_p)]),
     "kirag_debug_level_schedule": (c_int, [c_int64, c_int64, c_int, c_int, POINTER(c_int64), c_int, POINTER(c_int),
                                            POINTER(c_int)]),

@@ -34,6 +34,9 @@
 #include <new>
 #include <vector>
 
+#include <sys/mman.h>
+#include <unistd.h>
+
 namespace kirag {
 
 static thread_local char g_err[768] = "";
@@ -277,6 +280,97 @@ struct VmBuffer {
     }
 };
 
+// ------------------------------------------------------------- pinned host storage ---
+// The fp32 master of a KIRAG_INDEX_HOST_MASTER index: ONE range of host address space, reserved once (PROT_NONE,
+// MAP_NORESERVE: no memory behind it) for as many bytes as the machine has RAM, and made usable chunk by chunk as the
+// index grows — mprotect read/write, then page-locked and mapped into the device's address space with
+// cudaHostRegister.  Like VmBuffer, growing never copies and the base never moves, and the device address of every
+// byte equals its host address, so kernels index `master + row * d` exactly as for a device master and fread /
+// fwrite / memcpy work on the same pointer.
+struct HostBuffer {
+    uint8_t* base = nullptr;
+    size_t reserved = 0, mapped = 0;
+    static constexpr size_t kGran = (size_t)2 << 20;
+    std::vector<std::pair<size_t, size_t>> chunks;  // (offset, bytes) of every registered chunk
+
+    int reserve() {
+        const long pages = sysconf(_SC_PHYS_PAGES), page = sysconf(_SC_PAGE_SIZE);
+        if (pages <= 0 || page <= 0) { set_error("host master: cannot read the size of physical memory"); return 1; }
+        reserved = ((size_t)pages * (size_t)page + kGran - 1) / kGran * kGran;
+        void* p = mmap(nullptr, reserved, PROT_NONE, MAP_PRIVATE | MAP_ANONYMOUS | MAP_NORESERVE, -1, 0);
+        if (p == MAP_FAILED) {
+            set_error("host master: reserving %zu MiB of address space failed", reserved >> 20);
+            reserved = 0;
+            return 1;
+        }
+        base = static_cast<uint8_t*>(p);
+        return 0;
+    }
+    // make [0, bytes) usable; 0 ok, 1 failed (error set) — nothing is changed then
+    int ensure(size_t bytes) {
+        if (bytes <= mapped) return 0;
+        const size_t want = (bytes + kGran - 1) / kGran * kGran;
+        if (want > reserved) {
+            set_error("%zu MiB exceed the %zu MiB of physical memory", want >> 20, reserved >> 20);
+            return 1;
+        }
+        uint8_t* p = base + mapped;
+        const size_t sz = want - mapped;
+        if (mprotect(p, sz, PROT_READ | PROT_WRITE) != 0) {
+            set_error("mprotect of %zu MiB failed", sz >> 20);
+            return 1;
+        }
+        cudaError_t e = cudaHostRegister(p, sz, cudaHostRegisterMapped | cudaHostRegisterPortable);
+        if (e == cudaSuccess) {
+            void* dp = nullptr;
+            e = cudaHostGetDevicePointer(&dp, p, 0);
+            if (e == cudaSuccess && dp != (void*)p) {
+                cudaHostUnregister(p);
+                set_error("the device maps pinned host memory at another address than the host "
+                          "(cudaDevAttrCanUseHostPointerForRegisteredMem is 0): a host master needs both to agree");
+                madvise(p, sz, MADV_DONTNEED);
+                mprotect(p, sz, PROT_NONE);
+                return 1;
+            }
+        }
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            set_error("pinning %zu MiB (cudaHostRegister) failed: %s", sz >> 20, cudaGetErrorString(e));
+            madvise(p, sz, MADV_DONTNEED);
+            mprotect(p, sz, PROT_NONE);
+            return 1;
+        }
+        chunks.emplace_back(mapped, sz);
+        mapped = want;
+        return 0;
+    }
+    // cudaMemcpyAsync between the device and [host, host + bytes) of this range.  A copy must not cross from one
+    // registration into the next (the runtime rejects it), so it is split at chunk boundaries; kernels read across
+    // them through the mapping without restriction.
+    cudaError_t copy(void* dev, uint8_t* host, size_t bytes, bool to_device, cudaStream_t st) const {
+        size_t pos = (size_t)(host - base), done = 0;
+        for (const auto& c : chunks) {
+            if (done == bytes) break;
+            if (pos >= c.first + c.second) continue;
+            const size_t len = std::min(bytes - done, c.first + c.second - pos);
+            uint8_t* d = static_cast<uint8_t*>(dev) + done;
+            const cudaError_t e = to_device ? cudaMemcpyAsync(d, base + pos, len, cudaMemcpyHostToDevice, st)
+                                            : cudaMemcpyAsync(base + pos, d, len, cudaMemcpyDeviceToHost, st);
+            if (e != cudaSuccess) return e;
+            done += len;
+            pos += len;
+        }
+        return done == bytes ? cudaSuccess : cudaErrorInvalidValue;
+    }
+    void release() {
+        for (auto& c : chunks) cudaHostUnregister(base + c.first);
+        chunks.clear();
+        if (base) munmap(base, reserved);
+        base = nullptr;
+        reserved = mapped = 0;
+    }
+};
+
 struct FastParams {
     int kprime;
     int growth_override;  // KIRAG_LEVEL_GROWTH (0: automatic)
@@ -317,6 +411,11 @@ struct kirag_index {
     uint8_t* shadow = nullptr;  // bf16 tiles, capacity rounded up to 128 rows (null if d % 64)
     VmBuffer vm_master, vm_shadow;  // where master / shadow live when virtual-memory growth is available
     bool use_vmm = false;
+    bool host_master = false;   // KIRAG_INDEX_HOST_MASTER: master lives in hm (pinned host memory, same address)
+    HostBuffer hm;
+    DevBuf mstage[2];                 // host master: device staging of master pieces (convert, exact scan)
+    cudaStream_t copy_st = nullptr;   // host master: copies of the staged exact scan
+    cudaEvent_t stage_ev[5] = {};     // host master: [0,1] piece copied, [2,3] piece consumed, [4] scan entry
     unsigned* maxnorm2_bits = nullptr;  // device: [0] max ||y||^2, [1] max ||y - bf16(y)||^2, [2] max ||x||^2 (float bits)
     float maxnorm = 0.f;                // max_j ||y_j||, y = x - center (= x without a centre): what the shadow holds
     float maxerr = 0.f;                 // max_j ||y_j - bf16(y_j)||
@@ -402,16 +501,22 @@ static int decide_center(kirag_index* h, int64_t rows_available, cudaStream_t st
 static int index_grow(kirag_index* h, int64_t need_rows, cudaStream_t st) {
     if (need_rows <= h->capacity) return 0;
     const bool want_shadow = scan_tc_supported(h->d) != 0;
+    const bool host = h->host_master;  // master in pinned host memory (h->hm), only the shadow in HBM
     const size_t row_m = (size_t)h->d * sizeof(float), row_s = (size_t)h->d * 2;
-    if (h->capacity == 0 && !h->master && vmm_api().ok) {
-        // address space for the largest index this GPU could ever hold (the whole device memory as fp32 rows)
+    if (host && !h->master) {
+        if (h->hm.reserve()) return 1;
+        h->master = reinterpret_cast<float*>(h->hm.base);
+    }
+    if (h->capacity == 0 && (host ? !h->use_vmm : !h->master) && vmm_api().ok) {
+        // address space for the largest index this GPU could ever hold (the whole device memory as fp32 rows; as
+        // bf16 rows when only the shadow lives there)
         size_t free_b = 0, total_b = 0;
         if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && total_b > 0) {
-            const size_t max_rows = (size_t)round_up((int64_t)(total_b / row_m) + kTileRows, kTileRows);
-            if (h->vm_master.reserve(h->device, max_rows * row_m) == 0 &&
+            const size_t max_rows = (size_t)round_up((int64_t)(total_b / (host ? row_s : row_m)) + kTileRows, kTileRows);
+            if ((host || h->vm_master.reserve(h->device, max_rows * row_m) == 0) &&
                 (!want_shadow || h->vm_shadow.reserve(h->device, max_rows * row_s) == 0)) {
                 h->use_vmm = true;
-                h->master = static_cast<float*>(h->vm_master.ptr());
+                if (!host) h->master = static_cast<float*>(h->vm_master.ptr());
                 h->shadow = want_shadow ? static_cast<uint8_t*>(h->vm_shadow.ptr()) : nullptr;
             } else {
                 h->vm_master.release();
@@ -424,11 +529,24 @@ static int index_grow(kirag_index* h, int64_t need_rows, cudaStream_t st) {
     // not fit any more, by exactly what is needed
     int64_t cap = round_up(need_rows > h->capacity + h->capacity / 4 ? need_rows : h->capacity + h->capacity / 4, kTileRows);
     const int64_t exact = round_up(need_rows, kTileRows);
+    // host master: pinned chunk by chunk like the device buffers; a failure names the host side
+    auto host_fail = [&](int64_t rows) {
+        char why[512];
+        snprintf(why, sizeof(why), "%s", kirag_last_error());
+        set_error("index storage for %lld rows x %d does not fit: the fp32 master in pinned host memory (%zu MiB "
+                  "pinned now): %s", (long long)rows, h->d, h->hm.mapped >> 20, why);
+        return 1;
+    };
     if (h->use_vmm) {
         for (int attempt = 0; attempt < 2; ++attempt) {
             const int64_t c = attempt == 0 ? cap : exact;
             // nothing has to be undone on failure: a mapped-but-unused tail of the master is just capacity
-            if (h->vm_master.ensure((size_t)c * row_m) == 0 && (!want_shadow || h->vm_shadow.ensure((size_t)c * row_s) == 0)) {
+            if (host && h->hm.ensure((size_t)c * row_m)) {
+                if (c == exact) return host_fail(exact);
+                continue;
+            }
+            if ((host || h->vm_master.ensure((size_t)c * row_m) == 0) &&
+                (!want_shadow || h->vm_shadow.ensure((size_t)c * row_s) == 0)) {
                 h->capacity = c;
                 return 0;
             }
@@ -436,8 +554,9 @@ static int index_grow(kirag_index* h, int64_t need_rows, cudaStream_t st) {
         }
         size_t free_b = 0, total_b = 0;
         cudaMemGetInfo(&free_b, &total_b);
-        set_error("index storage for %lld rows x %d (fp32 master%s) does not fit: %zu MiB free of %zu MiB",
-                  (long long)exact, h->d, want_shadow ? " + bf16 shadow" : "", free_b >> 20, total_b >> 20);
+        set_error("index storage for %lld rows x %d (%s) does not fit: %zu MiB free of %zu MiB",
+                  (long long)exact, h->d, host ? "bf16 shadow" : want_shadow ? "fp32 master + bf16 shadow" : "fp32 master",
+                  free_b >> 20, total_b >> 20);
         cudaGetLastError();
         return 1;
     }
@@ -467,29 +586,27 @@ static int index_grow(kirag_index* h, int64_t need_rows, cudaStream_t st) {
         cap = c;  // the second buffer must not be larger than the first
         return 0;
     };
-    if (regrow((void**)&h->master, row_m, (size_t)h->ntotal, "fp32 master")) return 1;
+    if (host) {
+        if (h->hm.ensure((size_t)cap * row_m)) {
+            if (cap == exact || h->hm.ensure((size_t)exact * row_m)) return host_fail(exact);
+            cap = exact;
+        }
+    } else if (regrow((void**)&h->master, row_m, (size_t)h->ntotal, "fp32 master")) return 1;
     if (want_shadow && regrow((void**)&h->shadow, row_s, (size_t)round_up(h->ntotal, kTileRows), "bf16 shadow")) return 1;
     h->capacity = cap;
     return 0;
 }
 
 // ------------------------------------------------------------ exact path ----
-// Answers queries qsub[0..nsub) (device, contiguous [nsub, d]) with the exact
-// fp32 scan.  Output row of query i is out_row0 + i, or qmap_dev[i] if given.
-static int exact_search(kirag_index* h, const float* qsub, int64_t nsub, int k, float* D, int64_t* I,
-                        int64_t out_row0, const int* qmap_dev, int64_t id_offset, cudaStream_t st) {
-    const int64_t n = h->ntotal;
-    const int d = h->d;
+// Top-k of gq <= kExactNQ queries from their dense scores (rows [0, n) of dense, leading dimension ld) into D / I:
+// row g0 + i of the output block (out_row0 + g0 + i, or qmap_dev[g0 + i] if given).
+static int select_dense_topk(kirag_index* h, const float* dense, int64_t ld, int64_t n, int gq, int k, float* D,
+                             int64_t* I, int64_t out_row0, const int* qmap_dev, int64_t g0, int64_t id_offset,
+                             cudaStream_t st) {
     const int m = (int)((k < n) ? k : n);  // at most n real results
-    const int64_t ld = round_up(n, 32);
-    if (h->dense.ensure((size_t)kExactNQ * ld * sizeof(float))) return 1;
-    const int64_t n_seg = (n + kSelectSeg - 1) / kSelectSeg;
-    if (h->stage_a.ensure((size_t)kExactNQ * n_seg * m * sizeof(Cand))) return 1;
-    for (int64_t g0 = 0; g0 < nsub; g0 += kExactNQ) {
-        const int gq = (int)((nsub - g0 < kExactNQ) ? (nsub - g0) : kExactNQ);
-        if (launch_scan_exact(h->master, n, d, qsub + g0 * d, gq, h->dense.as<float>(), ld, h->num_sms, st)) return 1;
+    {
         int nseg_i = 0;
-        if (launch_select_dense(h->dense.as<float>(), ld, n, gq, m, h->stage_a.as<Cand>(), &nseg_i, st)) return 1;
+        if (launch_select_dense(dense, ld, n, gq, m, h->stage_a.as<Cand>(), &nseg_i, st)) return 1;
         Cand* cur = h->stage_a.as<Cand>();
         int64_t cur_stride = (int64_t)nseg_i * m;
         int cur_count = (int)cur_stride;
@@ -511,6 +628,100 @@ static int exact_search(kirag_index* h, const float* qsub, int64_t nsub, int k, 
                          qmap_dev ? D : D + (out_row0 + g0) * k, qmap_dev ? I : I + (out_row0 + g0) * k,
                          id_offset, nullptr, nullptr, nullptr, nullptr, 0.f, 0.f, 0, nullptr, nullptr,
                          qmap_dev ? qmap_dev + g0 : nullptr, st)) return 1;
+    }
+    return 0;
+}
+
+// Host master: the exact scan must not stream the master over PCIe once per kExactNQ queries.  Queries are taken in
+// groups of as many as kExactGroupBytes of dense scores hold (at most kExactGroupMax); for each group the master
+// crosses PCIe ONCE, in pieces of ~kStageBytes copied into one of two device staging buffers on h->copy_st while the
+// previous piece is being scanned.  Each piece is scanned by the same kernel for every kExactNQ-query subgroup, writing
+// the piece's columns of the group's dense rows; a score is one warp's canonical dot of one row, whichever launch
+// computes it, so the dense scores are bit-identical to the unstaged scan.
+constexpr size_t kStageBytes = (size_t)64 << 20;
+constexpr size_t kExactGroupBytes = (size_t)4 << 30;
+constexpr int64_t kExactGroupMax = 512;
+
+static int64_t stage_rows(const kirag_index* h) {
+    int64_t r = (int64_t)(kStageBytes / ((size_t)h->d * 4)) / 32 * 32;
+    return r < 32 ? 32 : r;
+}
+
+static int64_t exact_group_queries(int64_t ld) {
+    int64_t g = (int64_t)(kExactGroupBytes / ((size_t)ld * 4)) / kExactNQ * kExactNQ;
+    if (g < kExactNQ) g = kExactNQ;
+    return g < kExactGroupMax ? g : kExactGroupMax;
+}
+
+static int ensure_stage(kirag_index* h) {
+    const size_t bytes = (size_t)stage_rows(h) * h->d * 4;
+    if (h->mstage[0].ensure(bytes) || h->mstage[1].ensure(bytes)) return 1;
+    if (!h->copy_st) KIRAG_CUDA_OK(cudaStreamCreateWithFlags(&h->copy_st, cudaStreamNonBlocking));
+    for (auto& e : h->stage_ev)
+        if (!e) KIRAG_CUDA_OK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    return 0;
+}
+
+// dense[i * ld + r] = canonical score of query i (of q [nq, d], nq <= the group size) and row r, all rows
+static int scan_exact_staged(kirag_index* h, const float* q, int64_t nq, float* dense, int64_t ld, cudaStream_t st) {
+    const int64_t n = h->ntotal;
+    const int d = h->d;
+    if (ensure_stage(h)) return 1;
+    const int64_t piece = stage_rows(h);
+    cudaEvent_t* ev = h->stage_ev;
+    // the staging buffers may still be read by earlier work on st
+    KIRAG_CUDA_OK(cudaEventRecord(ev[4], st));
+    KIRAG_CUDA_OK(cudaStreamWaitEvent(h->copy_st, ev[4], 0));
+    int64_t i = 0;
+    for (int64_t r0 = 0; r0 < n; r0 += piece, ++i) {
+        const int b = (int)(i & 1);
+        const int64_t rows = (n - r0 < piece) ? (n - r0) : piece;
+        if (i >= 2) KIRAG_CUDA_OK(cudaStreamWaitEvent(h->copy_st, ev[2 + b], 0));  // piece i - 2 has been scanned
+        KIRAG_CUDA_OK(h->hm.copy(h->mstage[b].p, reinterpret_cast<uint8_t*>(h->master + r0 * d), (size_t)rows * d * 4, true,
+                                 h->copy_st));
+        KIRAG_CUDA_OK(cudaEventRecord(ev[b], h->copy_st));
+        KIRAG_CUDA_OK(cudaStreamWaitEvent(st, ev[b], 0));
+        for (int64_t s0 = 0; s0 < nq; s0 += kExactNQ) {
+            const int gq = (int)((nq - s0 < kExactNQ) ? (nq - s0) : kExactNQ);
+            if (launch_scan_exact(h->mstage[b].as<float>(), rows, d, q + s0 * d, gq, dense + s0 * ld + r0, ld, h->num_sms,
+                                  st)) return 1;
+        }
+        KIRAG_CUDA_OK(cudaEventRecord(ev[2 + b], st));
+    }
+    return 0;
+}
+
+// Answers queries qsub[0..nsub) (device, contiguous [nsub, d]) with the exact
+// fp32 scan.  Output row of query i is out_row0 + i, or qmap_dev[i] if given.
+static int exact_search(kirag_index* h, const float* qsub, int64_t nsub, int k, float* D, int64_t* I,
+                        int64_t out_row0, const int* qmap_dev, int64_t id_offset, cudaStream_t st) {
+    const int64_t n = h->ntotal;
+    const int d = h->d;
+    const int m = (int)((k < n) ? k : n);  // at most n real results
+    const int64_t ld = round_up(n, 32);
+    const int64_t n_seg = (n + kSelectSeg - 1) / kSelectSeg;
+    if (h->host_master) {
+        const int64_t G = exact_group_queries(ld);
+        const int64_t gmax = nsub < G ? round_up(nsub, kExactNQ) : G;
+        if (h->dense.ensure((size_t)gmax * ld * sizeof(float))) return 1;
+        if (h->stage_a.ensure((size_t)kExactNQ * n_seg * m * sizeof(Cand))) return 1;
+        for (int64_t g0 = 0; g0 < nsub; g0 += G) {
+            const int64_t gn = (nsub - g0 < G) ? (nsub - g0) : G;
+            if (scan_exact_staged(h, qsub + g0 * d, gn, h->dense.as<float>(), ld, st)) return 1;
+            for (int64_t s0 = 0; s0 < gn; s0 += kExactNQ) {
+                const int gq = (int)((gn - s0 < kExactNQ) ? (gn - s0) : kExactNQ);
+                if (select_dense_topk(h, h->dense.as<float>() + s0 * ld, ld, n, gq, k, D, I, out_row0, qmap_dev, g0 + s0,
+                                      id_offset, st)) return 1;
+            }
+        }
+        return 0;
+    }
+    if (h->dense.ensure((size_t)kExactNQ * ld * sizeof(float))) return 1;
+    if (h->stage_a.ensure((size_t)kExactNQ * n_seg * m * sizeof(Cand))) return 1;
+    for (int64_t g0 = 0; g0 < nsub; g0 += kExactNQ) {
+        const int gq = (int)((nsub - g0 < kExactNQ) ? (nsub - g0) : kExactNQ);
+        if (launch_scan_exact(h->master, n, d, qsub + g0 * d, gq, h->dense.as<float>(), ld, h->num_sms, st)) return 1;
+        if (select_dense_topk(h, h->dense.as<float>(), ld, n, gq, k, D, I, out_row0, qmap_dev, g0, id_offset, st)) return 1;
     }
     return 0;
 }
@@ -651,7 +862,9 @@ static int fast_search(kirag_index* h, const float* qd, int64_t nq, int k, float
     if (h->rescored.ensure((size_t)nq * fp.kprime * 4)) return 1;
     if (h->tauk.ensure((size_t)nq * 4)) return 1;
     // small batches (wide candidate buffer): last compaction + rescoring + final sort are ONE cluster kernel
-    const bool fuse_tail = cap == kWideCap && fp.kprime <= 2048;
+    // (not with a host master: the fused tail rescores all k' survivors, the three-launch tail only those that can still
+    // reach the top-k, and every row rescored crosses PCIe there)
+    const bool fuse_tail = cap == kWideCap && fp.kprime <= 2048 && !h->host_master;
     if ((nq % plan.bq) != 0)  // only the pad rows of the last query tile need zeroing
         KIRAG_CUDA_OK(cudaMemsetAsync(h->qshadow.p, 0, qs_bytes, st));
     KIRAG_CUDA_OK(launch_chained(init_search_state_kernel, dim3((unsigned)((nq_pad + 255) / 256)), dim3(256), 0, st,
@@ -710,9 +923,12 @@ static int fast_search(kirag_index* h, const float* qd, int64_t nq, int k, float
         return 0;
     }
     // rescoring skips candidates more than 2 eps below the k-th best approximate score
-    if (launch_rescore(h->master, d, qd, h->cand.as<Cand>(), h->cnt.as<int>(), cap, fp.kprime,
-                       h->rescored.as<float>(), nq, h->tauk.as<float>(), h->qnorm.as<float>(),
-                       h->qnorm.as<float>() + nq, ce.a, ce.b, st)) return 1;
+    if (h->host_master ? launch_rescore_host(h->master, d, qd, h->cand.as<Cand>(), h->cnt.as<int>(), cap, fp.kprime,
+                                             h->rescored.as<float>(), nq, h->tauk.as<float>(), nullptr,
+                                             h->qnorm.as<float>(), h->qnorm.as<float>() + nq, ce.a, ce.b, st)
+                       : launch_rescore(h->master, d, qd, h->cand.as<Cand>(), h->cnt.as<int>(), cap, fp.kprime,
+                                        h->rescored.as<float>(), nq, h->tauk.as<float>(), h->qnorm.as<float>(),
+                                        h->qnorm.as<float>() + nq, ce.a, ce.b, st)) return 1;
     prof_mark(50, st);
     if (launch_final(h->cand.as<Cand>(), cap, h->rescored.as<float>(), h->cnt.as<int>(), 0, fp.kprime,
                      (int)nq, k, D, I, id_offset, h->tau.as<float>(), h->qnorm.as<float>(), h->qnorm.as<float>() + nq,
@@ -774,11 +990,23 @@ static int rescan_search(kirag_index* h, const float* qsel, const float* qnorm_a
     const int64_t n_tiles = (n + kTileRows - 1) / kTileRows;
     if (launch_scan_tc(h->shadow, n, d, h->qshadow.p, nb, plan, 0, n_tiles, n_tiles, 1, h->tau.as<float>(),
                        h->cand.as<Cand>(), h->cnt.as<int>(), cap, h->num_sms, 1, st)) return 1;
-    if (launch_rescore(h->master, d, qsel, h->cand.as<Cand>(), h->cnt.as<int>(), cap, cap, h->rescored.as<float>(), nb,
-                       nullptr, nullptr, nullptr, 0.f, 0.f, st)) return 1;
     // overflow = appended count beyond the buffer
     std::vector<int> counts((size_t)nb);
-    KIRAG_CUDA_OK(cudaMemcpyAsync(counts.data(), h->cnt.p, (size_t)nb * 4, cudaMemcpyDeviceToHost, st));
+    if (h->host_master) {
+        // rows cross PCIe: rescore only the collected rows that can still reach the top-k, with the skip of the first
+        // attempt.  s~_k = the k-th best approximate score of the collected set (a compaction that keeps every entry;
+        // it rewrites cnt, so the survivor counts are read first).  Its qnorm / qerr are the chunk's, through qmap.
+        if (h->tauk.ensure((size_t)nb * 4)) return 1;
+        KIRAG_CUDA_OK(cudaMemcpyAsync(counts.data(), h->cnt.p, (size_t)nb * 4, cudaMemcpyDeviceToHost, st));
+        if (launch_compact_topm(h->cand.as<Cand>(), cap, h->cnt.as<int>(), cap, (int)nb, cap, h->tau.as<float>(),
+                                h->overflow.as<int>(), h->tauk.as<float>(), k, st)) return 1;
+        if (launch_rescore_host(h->master, d, qsel, h->cand.as<Cand>(), h->cnt.as<int>(), cap, cap, h->rescored.as<float>(),
+                                nb, h->tauk.as<float>(), qmap_dev, qnorm_all, qerr_all, ce.a, ce.b, st)) return 1;
+    } else {
+        if (launch_rescore(h->master, d, qsel, h->cand.as<Cand>(), h->cnt.as<int>(), cap, cap, h->rescored.as<float>(), nb,
+                           nullptr, nullptr, nullptr, 0.f, 0.f, st)) return 1;
+        KIRAG_CUDA_OK(cudaMemcpyAsync(counts.data(), h->cnt.p, (size_t)nb * 4, cudaMemcpyDeviceToHost, st));
+    }
     if (launch_final(h->cand.as<Cand>(), cap, h->rescored.as<float>(), h->cnt.as<int>(), 0, cap, (int)nb, k, D, I,
                      id_offset, nullptr, nullptr, nullptr, nullptr, 0.f, 0.f, 0, nullptr, nullptr, qmap_dev, st)) return 1;
     KIRAG_CUDA_OK(cudaStreamSynchronize(st));
@@ -1135,8 +1363,10 @@ static int range_filter_pass(kirag_index* h, const float* qs, int64_t nb, const 
     for (int64_t i = 0; i < nb; ++i)
         if ((*cnt_out)[(size_t)i] <= cap) m = std::max(m, (*cnt_out)[(size_t)i]);
     if (h->rescored.ensure((size_t)nb * m * 4)) return 1;
-    if (launch_rescore(h->master, d, qs, h->cand.as<Cand>(), h->cnt.as<int>(), cap, m, h->rescored.as<float>(), nb,
-                       nullptr, nullptr, nullptr, 0.f, 0.f, st)) return 1;
+    if (h->host_master ? launch_rescore_host(h->master, d, qs, h->cand.as<Cand>(), h->cnt.as<int>(), cap, m,
+                                             h->rescored.as<float>(), nb, nullptr, nullptr, nullptr, nullptr, 0.f, 0.f, st)
+                       : launch_rescore(h->master, d, qs, h->cand.as<Cand>(), h->cnt.as<int>(), cap, m,
+                                        h->rescored.as<float>(), nb, nullptr, nullptr, nullptr, 0.f, 0.f, st)) return 1;
     if (launch_range_count_cand(h->cand.as<Cand>(), cap, h->rescored.as<float>(), m, h->cnt.as<int>(), nb, radius,
                                 h->rcount.as<int>(), st)) return 1;
     std::vector<int> counts((size_t)nb);
@@ -1201,6 +1431,31 @@ static int range_exact_chunk(kirag_index* h, const float* qd, int64_t cq, float 
     const int64_t n = h->ntotal;
     const int d = h->d;
     const int64_t ld = round_up(n, 32);
+    if (h->host_master) {
+        // the staged scan of exact_search: the master crosses PCIe once per query group
+        const int64_t G = exact_group_queries(ld);
+        const int64_t gmax = cq < G ? round_up(cq, kExactNQ) : G;
+        if (h->dense.ensure((size_t)gmax * ld * sizeof(float)) || h->rcount.ensure((size_t)kExactNQ * 4)) return 1;
+        for (int64_t g0 = 0; g0 < cq; g0 += G) {
+            const int64_t gn = (cq - g0 < G) ? (cq - g0) : G;
+            if (scan_exact_staged(h, qd + g0 * d, gn, h->dense.as<float>(), ld, st)) return 1;
+            for (int64_t s0 = 0; s0 < gn; s0 += kExactNQ) {
+                const int gq = (int)((gn - s0 < kExactNQ) ? (gn - s0) : kExactNQ);
+                const float* dense = h->dense.as<float>() + s0 * ld;
+                if (launch_range_count_dense(dense, ld, n, gq, radius, h->rcount.as<int>(), st)) return 1;
+                std::vector<int> counts((size_t)gq), rows((size_t)gq);
+                KIRAG_CUDA_OK(cudaMemcpyAsync(counts.data(), h->rcount.p, (size_t)gq * 4, cudaMemcpyDeviceToHost, st));
+                KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+                for (int i = 0; i < gq; ++i) rows[(size_t)i] = (int)(g0 + s0 + i);
+                if (range_reserve(h, rc, counts, rows, st)) return 1;
+                if (launch_range_collect_dense(dense, ld, n, gq, radius, h->rcursor.as<unsigned long long>(),
+                                               h->ritems.as<uint64_t>(), st)) return 1;
+            }
+        }
+        c->n_exact += cq;
+        c->levels = 0;
+        return 0;
+    }
     if (h->dense.ensure((size_t)kExactNQ * ld * sizeof(float)) || h->rcount.ensure((size_t)kExactNQ * 4)) return 1;
     for (int64_t g0 = 0; g0 < cq; g0 += kExactNQ) {
         const int gq = (int)((cq - g0 < kExactNQ) ? (cq - g0) : kExactNQ);
@@ -1338,8 +1593,10 @@ static int range_fetch_impl(kirag_index* h, float* D, int64_t* I, int ptrs_are_d
 }
 
 // Rows [r0, r0 + n) of the master are in place: (re)decide the centre if it is time, convert them to the shadow
-// and refresh the norm maxima.  One pass, one synchronisation.
-static int finalize_rows(kirag_index* h, int64_t r0, int64_t n, cudaStream_t st) {
+// and refresh the norm maxima.  One pass, one synchronisation.  src: the same rows in device memory, or null for a
+// host master whose rows are then streamed through a device staging buffer (each crosses PCIe once; the centre
+// decision, <= kCenterSampleRows rows, and the re-conversion of < kCenterMinRows rows read the mapping directly).
+static int finalize_rows(kirag_index* h, int64_t r0, int64_t n, const float* src, cudaStream_t st) {
     if (h->shadow && !h->center_decided && r0 + n >= kCenterMinRows) {
         if (decide_center(h, r0 + n, st)) return 1;
         h->center_decided = true;
@@ -1349,8 +1606,20 @@ static int finalize_rows(kirag_index* h, int64_t r0, int64_t n, cudaStream_t st)
                                     nullptr, st)) return 1;
         }
     }
-    if (launch_convert_rows(h->master + r0 * (int64_t)h->d, n, h->d, r0, h->shadow, kTileRows, h->maxnorm2_bits, nullptr,
-                            nullptr, h->center, nullptr, st)) return 1;
+    if (src) {
+        if (launch_convert_rows(src, n, h->d, r0, h->shadow, kTileRows, h->maxnorm2_bits, nullptr, nullptr, h->center,
+                                nullptr, st)) return 1;
+    } else {
+        const int64_t piece = stage_rows(h);
+        if (h->mstage[0].ensure((size_t)piece * h->d * 4)) return 1;
+        for (int64_t i = 0; i < n; i += piece) {
+            const int64_t rows = (n - i < piece) ? (n - i) : piece;
+            KIRAG_CUDA_OK(h->hm.copy(h->mstage[0].p, reinterpret_cast<uint8_t*>(h->master + (r0 + i) * (int64_t)h->d),
+                                     (size_t)rows * h->d * 4, true, st));
+            if (launch_convert_rows(h->mstage[0].as<float>(), rows, h->d, r0 + i, h->shadow, kTileRows, h->maxnorm2_bits,
+                                    nullptr, nullptr, h->center, nullptr, st)) return 1;
+        }
+    }
     if (h->shadow && ((r0 + n) % kTileRows) != 0) {
         // rows of the last tile beyond ntotal: masked by the scan, but newly mapped memory is not zeroed — keep them
         // finite.  In the block layout rows rr..127 of a tile are the tail of each of its d/64 16-KB blocks.
@@ -1448,11 +1717,20 @@ int kirag_profile_read(double* scan_ms, int64_t* scan_launches, double* scan_row
 }
 
 int kirag_index_create(int d, int metric, int device, kirag_index_t** out) {
+    return kirag_index_create_ex(d, metric, device, 0, out);
+}
+
+int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_t** out) {
     KIRAG_CHECK(out != nullptr, "index_create: null out pointer");
     *out = nullptr;
     KIRAG_CHECK(d > 0 && d <= 16384, "index_create: unsupported dimension %d", d);
     KIRAG_CHECK(metric == KIRAG_METRIC_INNER_PRODUCT,
                 "index_create: only the inner-product metric is implemented (got %d)", metric);
+    KIRAG_CHECK((flags & ~KIRAG_INDEX_HOST_MASTER) == 0, "index_create: unknown flag bits 0x%x",
+                (unsigned)(flags & ~KIRAG_INDEX_HOST_MASTER));
+    // without a shadow every search would be an fp32 scan of the master over PCIe
+    KIRAG_CHECK(!(flags & KIRAG_INDEX_HOST_MASTER) || scan_tc_supported(d),
+                "index_create: host master needs the bf16 shadow (d %% 64 == 0, got d=%d)", d);
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev == 0) {
@@ -1474,6 +1752,7 @@ int kirag_index_create(int d, int metric, int device, kirag_index_t** out) {
     h->metric = metric;
     h->device = device;
     h->num_sms = prop.multiProcessorCount;
+    h->host_master = (flags & KIRAG_INDEX_HOST_MASTER) != 0;
     if (cudaMalloc((void**)&h->maxnorm2_bits, 12) != cudaSuccess || cudaMemset(h->maxnorm2_bits, 0, 12) != cudaSuccess) {
         set_error("index_create: cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
         delete h;
@@ -1487,13 +1766,22 @@ int kirag_index_destroy(kirag_index_t* h) {
     if (!h) return 0;
     DeviceGuard guard(h->device);
     cudaDeviceSynchronize();
-    if (h->use_vmm) {
+    if (h->host_master) {
+        h->hm.release();
+        if (h->use_vmm) h->vm_shadow.release();
+        else if (h->shadow) cudaFree(h->shadow);
+    } else if (h->use_vmm) {
         h->vm_master.release();
         h->vm_shadow.release();
     } else {
         if (h->master) cudaFree(h->master);
         if (h->shadow) cudaFree(h->shadow);
     }
+    h->mstage[0].release();
+    h->mstage[1].release();
+    if (h->copy_st) cudaStreamDestroy(h->copy_st);
+    for (auto e : h->stage_ev)
+        if (e) cudaEventDestroy(e);
     if (h->maxnorm2_bits) cudaFree(h->maxnorm2_bits);
     if (h->center) cudaFree(h->center);
     DevBuf* bufs[] = {&h->q_dev, &h->D_dev, &h->I_dev, &h->qshadow, &h->qnorm, &h->cand, &h->cnt, &h->tau, &h->tauk,
@@ -1527,9 +1815,19 @@ int kirag_index_add(kirag_index_t* h, const float* x, int64_t n, int x_is_device
     KIRAG_CHECK(h->ntotal + n <= 0x7fffff00LL, "index_add: more than 2^31 rows per device are not supported");
     if (index_grow(h, h->ntotal + n, st)) return 1;
     float* dst = h->master + h->ntotal * (int64_t)h->d;
-    KIRAG_CUDA_OK(cudaMemcpyAsync(dst, x, (size_t)n * h->d * sizeof(float),
-                                  x_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
-    return finalize_rows(h, h->ntotal, n, st);
+    const size_t bytes = (size_t)n * h->d * sizeof(float);
+    if (h->host_master) {
+        // device rows: the shadow is converted from x itself and x goes to the host once; host rows: a plain memcpy
+        // into the pinned master, from where finalize_rows streams them to the device for the convert pass
+        if (x_is_device) {
+            KIRAG_CUDA_OK(h->hm.copy(const_cast<float*>(x), reinterpret_cast<uint8_t*>(dst), bytes, false, st));
+            return finalize_rows(h, h->ntotal, n, x, st);
+        }
+        memcpy(dst, x, bytes);
+        return finalize_rows(h, h->ntotal, n, nullptr, st);
+    }
+    KIRAG_CUDA_OK(cudaMemcpyAsync(dst, x, bytes, x_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
+    return finalize_rows(h, h->ntotal, n, dst, st);
 }
 
 int64_t kirag_index_ntotal(const kirag_index_t* h) { return h ? h->ntotal : -1; }
@@ -1649,8 +1947,15 @@ int kirag_index_reconstruct(const kirag_index_t* h, int64_t i0, int64_t n, float
     DeviceGuard guard(h->device);
     if (!guard.ok) return 1;
     cudaStream_t st = (cudaStream_t)stream;
-    KIRAG_CUDA_OK(cudaMemcpyAsync(out, h->master + i0 * (int64_t)h->d, (size_t)n * h->d * 4,
-                                  out_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
+    if (h->host_master && !out_is_device) {
+        memcpy(out, h->master + i0 * (int64_t)h->d, (size_t)n * h->d * 4);
+        return 0;
+    }
+    if (h->host_master)
+        KIRAG_CUDA_OK(h->hm.copy(out, reinterpret_cast<uint8_t*>(h->master + i0 * (int64_t)h->d), (size_t)n * h->d * 4, true, st));
+    else
+        KIRAG_CUDA_OK(cudaMemcpyAsync(out, h->master + i0 * (int64_t)h->d, (size_t)n * h->d * 4,
+                                      out_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
     if (!out_is_device) KIRAG_CUDA_OK(cudaStreamSynchronize(st));
     return 0;
 }
@@ -1747,6 +2052,17 @@ int kirag_debug_level_schedule(int64_t n_rows, int64_t nq, int k, int d, int64_t
     return (int)b.size();
 }
 
+int kirag_index_storage_bytes(const kirag_index_t* h, int64_t* device_bytes, int64_t* host_bytes) {
+    KIRAG_CHECK(h != nullptr, "index_storage_bytes: null index");
+    const size_t row_m = (size_t)h->d * 4, row_s = (size_t)h->d * 2;
+    size_t dev = 0;
+    if (h->use_vmm) dev = (h->host_master ? 0 : h->vm_master.mapped) + h->vm_shadow.mapped;
+    else dev = (h->host_master || !h->master ? 0 : (size_t)h->capacity * row_m) + (h->shadow ? (size_t)h->capacity * row_s : 0);
+    if (device_bytes) *device_bytes = (int64_t)dev;
+    if (host_bytes) *host_bytes = (int64_t)h->hm.mapped;
+    return 0;
+}
+
 int kirag_index_device_ptrs(const kirag_index_t* h, const float** master_f32, const void** shadow_bf16) {
     KIRAG_CHECK(h != nullptr, "index_device_ptrs: null index");
     if (master_f32) *master_f32 = h->master;
@@ -1775,6 +2091,16 @@ int kirag_index_save(const kirag_index_t* h, const char* path) {
     ok = ok && fwrite(&fourcc, 4, 1, f) == 1 && fwrite(&d, 4, 1, f) == 1 && fwrite(&ntotal, 8, 1, f) == 1 &&
          fwrite(&dummy, 8, 1, f) == 1 && fwrite(&dummy, 8, 1, f) == 1 && fwrite(&trained, 1, 1, f) == 1 &&
          fwrite(&metric, 4, 1, f) == 1 && fwrite(&words, 8, 1, f) == 1;
+    if (h->host_master) {
+        // the master is host memory already: written as it is, the same bytes as a device-master index's file
+        for (int64_t r = 0; ok && r < ntotal; r += (int64_t)kIoChunkRows) {
+            const size_t n_el = (size_t)((ntotal - r < (int64_t)kIoChunkRows) ? (ntotal - r) : (int64_t)kIoChunkRows) * d;
+            ok = fwrite(h->master + r * d, 4, n_el, f) == n_el;
+        }
+        if (fclose(f) != 0) ok = false;
+        KIRAG_CHECK(ok, "index_save: write to %s failed", path);
+        return 0;
+    }
     // two pinned buffers: the device -> host copy of piece i+1 runs while piece i is being written
     float* stage[2] = {nullptr, nullptr};
     cudaEvent_t copied[2] = {nullptr, nullptr};
@@ -1825,8 +2151,13 @@ int kirag_index_save(const kirag_index_t* h, const char* path) {
 // pinned buffers and copied while the next piece is being read (no per-piece synchronisation: the host only waits
 // for the piece that used the same buffer two pieces ago), then ONE convert pass builds the bf16 shadow.  The
 // IO_FLAG_MMAP the reference passes asks FAISS not to read the file eagerly; it has no meaning for a device-resident
-// index and is accepted and ignored.
+// index and is accepted and ignored.  A host-master index (flags) reads the payload straight into its pinned master
+// and streams it to the device once for the convert pass.
 int kirag_index_load(const char* path, int device, kirag_index_t** out) {
+    return kirag_index_load_ex(path, device, 0, out);
+}
+
+int kirag_index_load_ex(const char* path, int device, int flags, kirag_index_t** out) {
     KIRAG_CHECK(path != nullptr && out != nullptr, "index_load: null argument");
     *out = nullptr;
     FILE* f = fopen(path, "rb");
@@ -1851,7 +2182,7 @@ int kirag_index_load(const char* path, int device, kirag_index_t** out) {
         return 1;
     }
     kirag_index_t* h = nullptr;
-    if (kirag_index_create(d, KIRAG_METRIC_INNER_PRODUCT, device, &h)) { fclose(f); return 1; }
+    if (kirag_index_create_ex(d, KIRAG_METRIC_INNER_PRODUCT, device, flags, &h)) { fclose(f); return 1; }
     if (ntotal == 0) { fclose(f); *out = h; return 0; }
     DeviceGuard guard(device);
     float* stage[2] = {nullptr, nullptr};
@@ -1862,6 +2193,21 @@ int kirag_index_load(const char* path, int device, kirag_index_t** out) {
         if (!guard.ok) break;
         if (kirag_index_reserve(h, ntotal)) break;
         const size_t row_bytes = (size_t)d * 4;
+        if (h->host_master) {
+            bool io_ok = true;
+            for (int64_t r = 0; r < ntotal && io_ok; r += (int64_t)kIoChunkRows) {
+                const size_t rows = (size_t)((ntotal - r < (int64_t)kIoChunkRows) ? (ntotal - r) : (int64_t)kIoChunkRows);
+                if (fread(h->master + r * d, row_bytes, rows, f) != rows) {
+                    set_error("index_load: %s is truncated", path);
+                    io_ok = false;
+                }
+            }
+            if (!io_ok) break;
+            if (cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) != cudaSuccess) { set_error("index_load: cudaStreamCreate failed"); break; }
+            if (finalize_rows(h, 0, ntotal, nullptr, st)) break;
+            rc = 0;
+            break;
+        }
         int64_t piece_rows = (int64_t)(((size_t)64 << 20) / row_bytes);
         if (piece_rows < 1) piece_rows = 1;
         if (piece_rows > ntotal) piece_rows = ntotal;
@@ -1889,7 +2235,7 @@ int kirag_index_load(const char* path, int device, kirag_index_t** out) {
             }
         }
         if (!io_ok) { cudaStreamSynchronize(st); break; }
-        if (finalize_rows(h, 0, ntotal, st)) break;
+        if (finalize_rows(h, 0, ntotal, h->master, st)) break;
         rc = 0;
     } while (0);
     for (int i = 0; i < 2; ++i) {
@@ -2010,7 +2356,7 @@ int kirag_topk_ip(const float* q, int64_t nq, const float* t, int64_t nt, int d,
         if (index_grow(h, nt, st)) return 1;
         float* const own_master = h->master;
         h->master = const_cast<float*>(t);
-        rc = finalize_rows(h, 0, nt, st);
+        rc = finalize_rows(h, 0, nt, t, st);
         if (!rc) rc = kirag_index_search(h, q, nq, k, D, I, ptrs_are_device, 0, stream);
         h->master = own_master;
         return rc;

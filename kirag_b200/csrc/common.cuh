@@ -226,6 +226,11 @@ int launch_scan_exact(const float* master, int64_t n, int d, const float* q, int
 int launch_rescore(const float* master, int d, const float* q, const Cand* cand, const int* cnt,
                    int cand_stride, int m, float* out_scores, int64_t nq, const float* tauk, const float* qnorm,
                    const float* qerr, float eps_a, float eps_b, cudaStream_t st);
+// Same scores from a host-resident master (pinned, mapped at the same address): a row's loads are all issued before
+// they are consumed.  The skip's qnorm / qerr are indexed by qmap[q] when qmap is given (else by q).
+int launch_rescore_host(const float* master, int d, const float* q, const Cand* cand, const int* cnt,
+                        int cand_stride, int m, float* out_scores, int64_t nq, const float* tauk, const int* qmap,
+                        const float* qnorm, const float* qerr, float eps_a, float eps_b, cudaStream_t st);
 // select.cu
 constexpr int kSelectSeg = 8192;
 constexpr int kWideCap = 32768;  // candidate buffer of small query batches (fewer, longer levels)

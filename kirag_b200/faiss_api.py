@@ -36,16 +36,28 @@ def _ptr(a: np.ndarray) -> ctypes.c_void_p:
     return ctypes.c_void_p(a.ctypes.data)
 
 
+def _master_flags(master: Optional[str]) -> int:
+    """Index flags for where the fp32 master lives: "device" (HBM, the default) or "host" (pinned host memory mapped
+    into the device; only the bf16 shadow takes HBM).  None reads KIRAG_MASTER, "device" when it is unset."""
+    if master is None:
+        master = os.environ.get("KIRAG_MASTER") or "device"
+    assert master in ("device", "host"), f"master must be 'device' or 'host', got {master!r}"
+    return _lib.INDEX_HOST_MASTER if master == "host" else 0
+
+
 class IndexFlatIP:
-    """Exact inner-product index; corpus lives in HBM (fp32 master + bf16 shadow)."""
+    """Exact inner-product index; corpus lives in HBM (fp32 master + bf16 shadow).  master="host" keeps the fp32 master
+    in pinned host memory instead (only the shadow in HBM), with bit-identical results."""
 
     metric_type = METRIC_INNER_PRODUCT
     is_trained = True
 
-    def __init__(self, d: int, device: Optional[int] = None, _handle: Optional[int] = None):
+    def __init__(self, d: int, device: Optional[int] = None, master: Optional[str] = None,
+                 _handle: Optional[int] = None):
         self._h = None
         self._pending = None
         self.last_stats: dict = {}
+        self._flags = _master_flags(master)
         self._lib = _lib.load()
         if _handle is not None:
             self._h = ctypes.c_void_p(_handle)
@@ -57,9 +69,21 @@ class IndexFlatIP:
         self.d = d
         self.device = _lib.default_device() if device is None else int(device)
         h = ctypes.c_void_p()
-        _lib.check(self._lib.kirag_index_create(d, METRIC_INNER_PRODUCT, self.device, ctypes.byref(h)),
+        _lib.check(self._lib.kirag_index_create_ex(d, METRIC_INNER_PRODUCT, self.device, self._flags, ctypes.byref(h)),
                    "IndexFlatIP")
         self._h = h
+
+    @property
+    def master(self) -> str:
+        """Where the fp32 master lives: "device" or "host"."""
+        return "host" if self._flags & _lib.INDEX_HOST_MASTER else "device"
+
+    def storage_bytes(self) -> dict:
+        """Corpus storage (fp32 master + bf16 shadow, no workspaces) now held: {"device": HBM bytes, "host": pinned
+        host bytes}."""
+        dev, host = ctypes.c_int64(0), ctypes.c_int64(0)
+        _lib.check(self._lib.kirag_index_storage_bytes(self._h, ctypes.byref(dev), ctypes.byref(host)), "storage_bytes")
+        return {"device": int(dev.value), "host": int(host.value)}
 
     # -- faiss surface -----------------------------------------------------
     @property
@@ -155,7 +179,8 @@ class IndexFlatIP:
     def reset(self) -> None:
         self._destroy()
         h = ctypes.c_void_p()
-        _lib.check(self._lib.kirag_index_create(self.d, METRIC_INNER_PRODUCT, self.device, ctypes.byref(h)), "reset")
+        _lib.check(self._lib.kirag_index_create_ex(self.d, METRIC_INNER_PRODUCT, self.device, self._flags,
+                                                   ctypes.byref(h)), "reset")
         self._h = h
 
     # -- device-resident entry points (additions, not part of faiss) --------
@@ -366,12 +391,14 @@ def write_index(index: IndexFlatIP, path) -> None:
     _lib.check(index._lib.kirag_index_save(index._h, os.fspath(path).encode()), "write_index")
 
 
-def read_index(path, flags: int = 0, device: Optional[int] = None) -> IndexFlatIP:
+def read_index(path, flags: int = 0, device: Optional[int] = None, master: Optional[str] = None) -> IndexFlatIP:
+    """`flags` are FAISS IO flags (IO_FLAG_MMAP is accepted and ignored); `master` as for IndexFlatIP."""
+    index_flags = _master_flags(master)
     lib = _lib.load()
     dev = _lib.default_device() if device is None else int(device)
     h = ctypes.c_void_p()
-    _lib.check(lib.kirag_index_load(os.fspath(path).encode(), dev, ctypes.byref(h)), "read_index")
-    return IndexFlatIP(0, device=dev, _handle=h.value)
+    _lib.check(lib.kirag_index_load_ex(os.fspath(path).encode(), dev, index_flags, ctypes.byref(h)), "read_index")
+    return IndexFlatIP(0, device=dev, master="host" if index_flags else "device", _handle=h.value)
 
 
 def omp_get_max_threads() -> int:

@@ -233,7 +233,7 @@ class ShardedFlatIP:
     def __init__(self, d: int, n_total: int, rank: Optional[int] = None, world_size: Optional[int] = None,
                  device: Optional[int] = None, group=None,
                  local_index=None, merge_fn: Optional[Callable] = None, exchange: Optional[str] = None,
-                 max_nq: int = 16384, max_k: int = 128, weights=None):
+                 max_nq: int = 16384, max_k: int = 128, weights=None, master: Optional[str] = None):
         self.d = d
         self.group = group
         self.rank = dist.get_rank(group) if rank is None else rank
@@ -244,7 +244,7 @@ class ShardedFlatIP:
         if local_index is None:
             from .faiss_api import IndexFlatIP
 
-            local_index = IndexFlatIP(d, device=device)
+            local_index = IndexFlatIP(d, device=device, master=master)
             local_index.reserve(max(self.hi - self.lo, 1))
         self.index = local_index
         self.merge_fn = merge_fn or merge_topk_device

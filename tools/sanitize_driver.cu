@@ -3,7 +3,7 @@
 // under the tool.  Built and run by tools/sanitize.sh on the GPU box; every case checks its result against a host
 // computation, so a "passed" under the sanitizer is also a correctness pass.
 //
-//   ./sanitize_driver [case]     case = scan | search | pool | exchange | topk | all (default)
+//   ./sanitize_driver [case]     case = scan | search | pool | exchange | topk | host_rescore | host_exact | all (default)
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -269,6 +269,77 @@ static void case_topk() {
     CK(kirag_topk_ip_release());
 }
 
+// host-resident master (KIRAG_INDEX_HOST_MASTER): 140k rows x 128, more than one 64-MB staging piece
+static kirag_index_t* host_master_index(const std::vector<float>& xb, int n, int d) {
+    kirag_index_t* h = nullptr;
+    CK(kirag_index_create_ex(d, KIRAG_METRIC_INNER_PRODUCT, 0, KIRAG_INDEX_HOST_MASTER, &h));
+    CK(kirag_index_add(h, xb.data(), n, 0, nullptr));
+    int64_t dev_b = 0, host_b = 0;
+    CK(kirag_index_storage_bytes(h, &dev_b, &host_b));
+    if (host_b < (int64_t)n * d * 4 || dev_b >= (int64_t)n * d * 4) {
+        printf("host master storage: device %lld B, host %lld B BAD\n", (long long)dev_b, (long long)host_b);
+        exit(3);
+    }
+    return h;
+}
+
+// the rescoring gather from pinned host rows: three-launch tail of the filter path, every batch size
+static void case_host_rescore() {
+    std::mt19937 rng(6);
+    const int n = 140000, d = 128, k = 10;
+    auto xb = unit_rows(rng, n, d);
+    kirag_index_t* h = host_master_index(xb, n, d);
+    for (int nq : {1, 40, 200}) {
+        auto xq = unit_rows(rng, nq, d);
+        std::vector<float> D((size_t)nq * k);
+        std::vector<int64_t> I((size_t)nq * k), Ih;
+        kirag_search_stats_t st;
+        CK(kirag_index_search_ex(h, xq.data(), nq, k, D.data(), I.data(), 0, 0, KIRAG_PATH_AUTO, &st, nullptr));
+        host_topk(xb, n, xq, nq, d, k, &Ih);
+        int diff = 0;
+        double worst = 0;
+        for (int q = 0; q < nq; ++q)
+            for (int j = 0; j < k; ++j) {
+                const size_t i = (size_t)q * k + j;
+                diff += I[i] != Ih[i];
+                double a = 0;
+                for (int c = 0; c < d; ++c) a += (double)xq[(size_t)q * d + c] * xb[(size_t)I[i] * d + c];
+                worst = std::max(worst, std::fabs(a - D[i]));
+            }
+        printf("host-master search nq=%d: fast=%lld, ids vs host fp64 %d, max |score - fp64| = %.2e %s\n", nq,
+               (long long)st.n_fast, diff, worst, diff <= 2 && worst < 1e-5 ? "ok" : "BAD");
+        if (diff > 2 || !(worst < 1e-5)) exit(3);
+    }
+    CK(kirag_index_destroy(h));
+}
+
+// the exact fp32 scan of a host master, staged through HBM in pieces (two pieces here)
+static void case_host_exact() {
+    std::mt19937 rng(7);
+    const int n = 140000, d = 128, k = 10, nq = 20;
+    auto xb = unit_rows(rng, n, d);
+    kirag_index_t* h = host_master_index(xb, n, d);
+    auto xq = unit_rows(rng, nq, d);
+    std::vector<float> D((size_t)nq * k);
+    std::vector<int64_t> I((size_t)nq * k), Ih;
+    CK(kirag_index_search_ex(h, xq.data(), nq, k, D.data(), I.data(), 0, 0, KIRAG_PATH_EXACT, nullptr, nullptr));
+    host_topk(xb, n, xq, nq, d, k, &Ih);
+    int diff = 0;
+    double worst = 0;
+    for (int q = 0; q < nq; ++q)
+        for (int j = 0; j < k; ++j) {
+            const size_t i = (size_t)q * k + j;
+            diff += I[i] != Ih[i];
+            double a = 0;
+            for (int c = 0; c < d; ++c) a += (double)xq[(size_t)q * d + c] * xb[(size_t)I[i] * d + c];
+            worst = std::max(worst, std::fabs(a - D[i]));
+        }
+    printf("host-master staged exact scan nq=%d: ids vs host fp64 %d, max |score - fp64| = %.2e %s\n", nq, diff, worst,
+           diff <= 1 && worst < 1e-5 ? "ok" : "BAD");
+    if (diff > 1 || !(worst < 1e-5)) exit(3);
+    CK(kirag_index_destroy(h));
+}
+
 int main(int argc, char** argv) {
     const std::string which = argc > 1 ? argv[1] : "all";
     if (which == "scan" || which == "all") case_scan();
@@ -276,6 +347,8 @@ int main(int argc, char** argv) {
     if (which == "pool" || which == "all") case_pool();
     if (which == "exchange" || which == "all") case_exchange();
     if (which == "topk" || which == "all") case_topk();
+    if (which == "host_rescore" || which == "all") case_host_rescore();
+    if (which == "host_exact" || which == "all") case_host_exact();
     CU(cudaDeviceSynchronize());
     printf("sanitize_driver %s: passed\n", which.c_str());
     return 0;
