@@ -21,7 +21,8 @@
  *     copies on add(), reference call site retriever/index.py:32).
  *   - threading: calls on DIFFERENT index handles may run concurrently from different host threads;
  *     calls on the SAME handle must be serialised by the caller (search workspaces belong to the
- *     handle).  KiRAG's callers are single-threaded Python (retriever/retrievers.py:250-275).
+ *     handle).  KiRAG's callers are single-threaded Python (retriever/retrievers.py:250-275).  A
+ *     multi-device index (kirag_index_create_multi) runs its shards from worker threads of its own.
  *   - there is NO CPU fallback.  If no CUDA device is usable every call fails
  *     with a non-zero status.
  */
@@ -34,7 +35,7 @@
 extern "C" {
 #endif
 
-#define KIRAG_ABI_VERSION 8
+#define KIRAG_ABI_VERSION 9
 
 /* metric ids; only inner product is implemented, as only inner product is
  * ever constructed by the reference (retrieve.py:112, faiss_index_corpus.py:29) */
@@ -69,7 +70,11 @@ extern "C" {
 
 typedef struct kirag_index kirag_index_t;
 
-/* per-call search statistics (all counts are queries unless noted) */
+/* per-call search statistics (all counts are queries unless noted).  For a multi-device index: nq is the number of
+ * queries; n_fast, n_exact, n_cert_fail, n_overflow, n_rescan and n_retry are summed over the shards (a query counts
+ * once per shard); levels is the maximum over the shards; path is the shards' path if they agree, else
+ * KIRAG_PATH_EXACT; kernel_launches counts the launches of the call's shard workers and of the calling thread (the
+ * merge), on every device; concurrent calls of other threads are not counted. */
 typedef struct kirag_search_stats {
     int64_t nq;              /* queries in the call */
     int64_t n_fast;          /* answered by the tcgen05 filter path with a passing certificate (first attempt) */
@@ -98,7 +103,8 @@ int kirag_device_count(void);
  * events recorded on the launching stream; used by bench.py for the roofline
  * line.  enable(1) clears and starts recording, read() returns the summed
  * duration (ms), the number of launches and the corpus rows they streamed,
- * then clears. */
+ * then clears.  The recorder is guarded by a mutex: the shards of a multi-device
+ * index record into it from their worker threads (their launches all land in it). */
 int kirag_profile_enable(int on);
 int kirag_profile_read(double* scan_ms, int64_t* scan_launches, double* scan_rows);
 /* Per-launch durations (ms) and corpus rows of the recorded scan launches, up to max_n entries;
@@ -118,6 +124,37 @@ int kirag_index_create(int d, int metric, int device, kirag_index_t** out);
 /* flags: 0 or KIRAG_INDEX_HOST_MASTER.  Unknown flag bits and KIRAG_INDEX_HOST_MASTER with d % 64 != 0 are rejected
  * before any device is looked at. */
 int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_t** out);
+
+/* Multi-device index: the rows are striped over n_devices shards (1 <= n_devices <= 16), 128 rows at a time: global
+ * row r lives in shard s = (r / 128) mod G at local row (r / (128 G)) * 128 + r mod 128.  devices[0] is the HOME device:
+ * device pointers given to the calls below are on it, and the shard results are merged there by kernels that read them
+ * through peer pointers.  Every distinct device must be peer-accessible from the home device (peer access is enabled
+ * here; a device without it is an error).  A device may be repeated: [0, 0, 0] is three shards on one GPU, which gives
+ * no speed-up but runs every part of the multi-device logic on a box with one GPU.
+ * flags as for kirag_index_create_ex; with KIRAG_INDEX_HOST_MASTER every shard has its own host master.  n_devices,
+ * unknown flag bits and the host flag with d % 64 != 0 are checked before any device is looked at.
+ * The handle owns one ordinary index per shard (the existing single-device code runs each of them unchanged) and one
+ * worker thread per shard, started here and joined by kirag_index_destroy: a call hands every shard its part, all
+ * shards run at once (each on its own stream), the calling thread waits for them and merges.  Results are bit-identical
+ * to a single-device index with the same rows.
+ * Accepted: add, ntotal, dim, reserve, search, search_ex, range_search, range_fetch, reconstruct, save, storage_bytes
+ * (summed over shards), destroy.  An error: search_async, search_finish, search_flags, search_rearm, state_token (no CUDA
+ * graph across devices), device_ptrs, debug_scores. */
+int kirag_index_create_multi(int d, int metric, const int* devices, int n_devices, int flags, kirag_index_t** out);
+
+/* faiss.read_index into a multi-device index: the file is streamed once and every piece split over the shards. */
+int kirag_index_load_multi(const char* path, const int* devices, int n_devices, int flags, kirag_index_t** out);
+
+/* Returns the number of shards G (1 for a single-device index, -1 with kirag_last_error() set on a null handle) and
+ * writes the device and the row count of the first min(G, max) shards (either output may be NULL). */
+int kirag_index_shards(const kirag_index_t* h, int* devices_out, int64_t* rows_out, int max);
+
+/* Test hooks (host only, no device needed): the stripe arithmetic of a multi-device index with G shards.  map: shard,
+ * local row and the global row computed back from them, for each of n global rows; rows: rows of each shard of an index
+ * of ntotal rows. */
+int kirag_debug_stripe_map(int G, const int64_t* global_ids, int64_t n, int* shard_out, int64_t* local_out,
+                           int64_t* global_out);
+int kirag_debug_stripe_rows(int64_t ntotal, int G, int64_t* rows_out);
 
 /* destructor of the faiss index object */
 int kirag_index_destroy(kirag_index_t* h);

@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("KIRAG_B200_LIB") or os.path.join(HERE, "libkirag_b200.so")
 
 # constants mirrored from the header
-ABI_VERSION = 8
+ABI_VERSION = 9
 INDEX_HOST_MASTER = 1
 METRIC_INNER_PRODUCT = 0
 METRIC_L2 = 1
@@ -60,6 +60,11 @@ SIGNATURES = {
     "kirag_profile_read_timeline": (c_int, [POINTER(c_int), POINTER(ctypes.c_double), c_int64]),
     "kirag_index_create": (c_int, [c_int, c_int, c_int, POINTER(c_void_p)]),
     "kirag_index_create_ex": (c_int, [c_int, c_int, c_int, c_int, POINTER(c_void_p)]),
+    "kirag_index_create_multi": (c_int, [c_int, c_int, POINTER(c_int), c_int, c_int, POINTER(c_void_p)]),
+    "kirag_index_load_multi": (c_int, [c_char_p, POINTER(c_int), c_int, c_int, POINTER(c_void_p)]),
+    "kirag_index_shards": (c_int, [c_void_p, POINTER(c_int), POINTER(c_int64), c_int]),
+    "kirag_debug_stripe_map": (c_int, [c_int, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
+    "kirag_debug_stripe_rows": (c_int, [c_int64, c_int, POINTER(c_int64)]),
     "kirag_index_destroy": (c_int, [c_void_p]),
     "kirag_index_reserve": (c_int, [c_void_p, c_int64]),
     "kirag_index_add": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p]),

@@ -30,8 +30,12 @@
 #include <cstdlib>
 #include <cstring>
 #include <cmath>
+#include <condition_variable>
+#include <type_traits>
+#include <memory>
 #include <mutex>
 #include <new>
+#include <thread>
 #include <vector>
 
 #include <sys/mman.h>
@@ -41,6 +45,9 @@ namespace kirag {
 
 static thread_local char g_err[768] = "";
 static std::atomic<long long> g_launches{0};
+// launches made by this thread: the statistics of a multi-device call add up its workers' and its own, which other
+// threads' concurrent calls on other handles do not disturb
+static thread_local long long g_thread_launches = 0;
 
 void set_error(const char* fmt, ...) {
     va_list ap;
@@ -48,7 +55,10 @@ void set_error(const char* fmt, ...) {
     vsnprintf(g_err, sizeof(g_err), fmt, ap);
     va_end(ap);
 }
-void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
+void count_launch(int n) {
+    g_launches.fetch_add(n, std::memory_order_relaxed);
+    g_thread_launches += n;
+}
 
 // Chained (programmatic dependent) launches pay off where the kernels of a search are short: measured
 // 12% at 430k rows, 4% at 2.6M rows x 32 queries, nothing at 1024 queries, and a slight LOSS at 4096
@@ -94,9 +104,10 @@ int ensure_dynamic_smem_impl(const void* kernel, size_t bytes) {
 
 // Optional per-kernel timing of the dominant kernel (the tcgen05 filter scan): CUDA events
 // recorded on the launching stream around every scan launch while enabled.  bench.py uses
-// it for the roofline line; it is off by default.
+// it for the roofline line; it is off by default.  The shards of a multi-device index search from one worker thread
+// each, so every access to the recorder holds g_prof_mu.
 struct ScanProfile {
-    bool on = false;
+    std::atomic<bool> on{false};
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev;
     std::vector<double> launch_rows;
     std::vector<std::pair<int, cudaEvent_t>> marks;  // (tag, event) timeline of the search phases
@@ -104,6 +115,7 @@ struct ScanProfile {
     double queries = 0.0;
 };
 static ScanProfile g_prof;
+static std::mutex g_prof_mu;
 
 // timeline tags: 0 start, 1 after convert/init, 10+l after scan of level l, 30+l after select of
 // level l, 50 after rescore, 51 after final, 52 after certificate readback
@@ -112,6 +124,7 @@ static void prof_mark(int tag, cudaStream_t st) {
     cudaEvent_t e = nullptr;
     if (cudaEventCreate(&e) != cudaSuccess) return;
     cudaEventRecord(e, st);
+    std::lock_guard<std::mutex> lock(g_prof_mu);
     g_prof.marks.emplace_back(tag, e);
 }
 
@@ -400,7 +413,10 @@ struct PendingSearch {
     FastParams fp{};
 };
 
+struct MultiIndex;
+
 struct kirag_index {
+    MultiIndex* multi = nullptr;  // a multi-device index (kirag_index_create_multi): the shards hold everything else
     int d = 0;
     int metric = 0;
     int device = 0;
@@ -441,6 +457,14 @@ struct kirag_index {
 };
 
 static int64_t round_up(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
+
+// multi-device index (defined with its orchestration below)
+static int multi_search(kirag_index* h, const float* q, int64_t nq, int k, float* D, int64_t* I, int ptrs_are_device,
+                        int64_t id_offset, int path, kirag_search_stats_t* stats, cudaStream_t st);
+static int multi_range_search(kirag_index* h, const float* q, int64_t nq, float radius, int q_is_device,
+                              int64_t id_offset, int path, int64_t* lims_out, kirag_search_stats_t* stats,
+                              cudaStream_t st);
+static int multi_range_fetch(kirag_index* h, float* D, int64_t* I, int ptrs_are_device, cudaStream_t st);
 
 static int env_int(const char* name, int dflt) {
     const char* v = getenv(name);
@@ -895,6 +919,7 @@ static int fast_search(kirag_index* h, const float* qd, int64_t nq, int k, float
                            levels == 0 ? 1 : 0, st)) return 1;
         if (g_prof.on) {
             KIRAG_CUDA_OK(cudaEventRecord(e1, st));
+            std::lock_guard<std::mutex> lock(g_prof_mu);
             g_prof.ev.emplace_back(e0, e1);
             int64_t r1 = hi * kTileRows; if (r1 > n) r1 = n;
             g_prof.rows += (double)(r1 - lo * kTileRows);
@@ -1202,6 +1227,7 @@ static int search_impl(kirag_index* h, const float* q, int64_t nq, int k, float*
     KIRAG_CHECK(k <= 2048, "search: k=%d exceeds the supported maximum of 2048", k);
     KIRAG_CHECK(nq >= 0, "search: negative nq");
     KIRAG_CHECK(path >= 0 && path <= 2, "search: unknown path %d", path);
+    if (h->multi) return multi_search(h, q, nq, k, D, I, ptrs_are_device, id_offset, path, stats, st);
     if (finish_pending(h, nullptr, nullptr)) return 1;  // an unfinished asynchronous search owns the workspaces
     if (stats) memset(stats, 0, sizeof(*stats));
     if (nq == 0) return 0;
@@ -1321,6 +1347,7 @@ static int range_scan(kirag_index* h, const ScanTcPlan& plan, int64_t nq, int ca
                        h->cand.as<Cand>(), h->cnt.as<int>(), cap, h->num_sms, 1, st)) return 1;
     if (g_prof.on) {
         KIRAG_CUDA_OK(cudaEventRecord(e1, st));
+        std::lock_guard<std::mutex> lock(g_prof_mu);
         g_prof.ev.emplace_back(e0, e1);
         g_prof.rows += (double)n;
         g_prof.launch_rows.push_back((double)n);
@@ -1530,6 +1557,7 @@ static int range_search_impl(kirag_index* h, const float* q, int64_t nq, float r
     KIRAG_CHECK(h != nullptr, "range_search: null index");
     KIRAG_CHECK(lims_out != nullptr, "range_search: null lims");
     KIRAG_CHECK(path >= 0 && path <= 2, "range_search: unknown path %d", path);
+    if (h->multi) return multi_range_search(h, q, nq, radius, q_is_device, id_offset, path, lims_out, stats, st);
     if (finish_pending(h, nullptr, nullptr)) return 1;  // also drops the previous range result
     if (stats) memset(stats, 0, sizeof(*stats));
     for (int64_t i = 0; i <= nq; ++i) lims_out[i] = 0;
@@ -1575,6 +1603,7 @@ static int range_search_impl(kirag_index* h, const float* q, int64_t nq, float r
 
 static int range_fetch_impl(kirag_index* h, float* D, int64_t* I, int ptrs_are_device, cudaStream_t st) {
     KIRAG_CHECK(h != nullptr, "range_fetch: null index");
+    if (h->multi) return multi_range_fetch(h, D, I, ptrs_are_device, st);
     KIRAG_CHECK(h->range_valid, "range_fetch: no range-search result is held (the last call on this index was not "
                                 "kirag_index_range_search, or its result was fetched already)");
     const int64_t total = h->range_n;
@@ -1642,6 +1671,376 @@ static int finalize_rows(kirag_index* h, int64_t r0, int64_t n, const float* src
     return 0;
 }
 
+// ------------------------------------------------------------ multi-device index ----
+// kirag_index_create_multi: G shard indexes, rows striped over them (common.cuh::stripe_*), one persistent worker
+// thread per shard.  A call hands one job to every worker; each makes the ordinary single-device call on its shard on
+// its own stream (search with its escalation ladder, range search with its read-backs, add, reserve, reconstruct), so
+// every phase runs on all devices at once.  The calling thread waits for all of them, then merges the shard results on
+// the home device (devices[0]) with one kernel that reads them in place through peer pointers (multi.cu).
+struct MultiShard {
+    int device = 0;
+    kirag_index_t* h = nullptr;
+    cudaStream_t st = nullptr;
+    std::thread th;
+    int rc = 0;
+    char err[768] = "";
+    DevBuf q, D, I, rD, rI, stage;  // on the shard's device, grow-only
+    std::vector<int64_t> lims;      // the last range search's lims
+    kirag_search_stats_t stats{};   // accumulated over the query chunks of a call
+    long long launches = 0;         // kernels the worker launched during the call
+};
+
+struct MultiIndex {
+    int G = 0;
+    std::vector<std::unique_ptr<MultiShard>> sh;
+    std::mutex mu;
+    std::condition_variable cv_job, cv_done;
+    int (*job_fn)(void*, MultiShard&, int) = nullptr;  // the job of the current call: job_fn(job_ctx, shard, s)
+    void* job_ctx = nullptr;
+    uint64_t gen = 0;
+    int pending = 0;
+    bool quit = false;
+    int64_t ntotal = 0;
+    DevBuf ws, D_out, I_out, lims_dev;  // on the home device: merge workspace, host-output staging, shard + global lims
+    bool range_valid = false;
+    int64_t range_n = 0, range_nq = 0, range_max = 0, range_id_offset = 0;
+};
+
+static void multi_worker(MultiIndex* m, int s) {
+    MultiShard& sh = *m->sh[(size_t)s];
+    cudaSetDevice(sh.device);
+    uint64_t seen = 0;
+    for (;;) {
+        {
+            std::unique_lock<std::mutex> lk(m->mu);
+            m->cv_job.wait(lk, [&] { return m->quit || m->gen != seen; });
+            if (m->quit) return;
+            seen = m->gen;
+        }
+        g_err[0] = '\0';
+        const long long launches0 = g_thread_launches;
+        int rc = 1;
+        try {
+            rc = m->job_fn(m->job_ctx, sh, s);  // the job only changes once every worker has reported
+        } catch (const std::exception& e) {
+            set_error("%s", e.what());
+        }
+        std::lock_guard<std::mutex> lk(m->mu);
+        sh.rc = rc;
+        sh.launches += g_thread_launches - launches0;
+        if (rc) snprintf(sh.err, sizeof(sh.err), "%s", g_err);  // g_err is per thread: carried to the caller
+        if (--m->pending == 0) m->cv_done.notify_all();
+    }
+}
+
+// Runs fn(shard, s) on every worker and waits for all of them; the first failure becomes the caller's error.
+template <typename F>
+static int multi_run(MultiIndex* m, F&& fn) {
+    {
+        std::lock_guard<std::mutex> lk(m->mu);
+        m->job_fn = [](void* ctx, MultiShard& sh, int s) -> int { return (*static_cast<std::remove_reference_t<F>*>(ctx))(sh, s); };
+        m->job_ctx = &fn;
+        m->pending = m->G;
+        ++m->gen;
+    }
+    m->cv_job.notify_all();
+    {
+        std::unique_lock<std::mutex> lk(m->mu);
+        m->cv_done.wait(lk, [&] { return m->pending == 0; });
+    }
+    for (int s = 0; s < m->G; ++s) {
+        const MultiShard& sh = *m->sh[(size_t)s];
+        KIRAG_CHECK(sh.rc == 0, "shard %d (device %d): %s", s, sh.device, sh.err);
+    }
+    return 0;
+}
+
+static void multi_destroy(MultiIndex* m) {
+    {
+        std::lock_guard<std::mutex> lk(m->mu);
+        m->quit = true;
+    }
+    m->cv_job.notify_all();
+    for (auto& sh : m->sh)
+        if (sh->th.joinable()) sh->th.join();
+    for (auto& sh : m->sh) {
+        DeviceGuard guard(sh->device);
+        if (sh->st) { cudaStreamSynchronize(sh->st); cudaStreamDestroy(sh->st); }
+        DevBuf* bufs[] = {&sh->q, &sh->D, &sh->I, &sh->rD, &sh->rI, &sh->stage};
+        for (DevBuf* b : bufs) b->release();
+        kirag_index_destroy(sh->h);
+    }
+    if (!m->sh.empty()) {
+        DeviceGuard guard(m->sh[0]->device);
+        DevBuf* bufs[] = {&m->ws, &m->D_out, &m->I_out, &m->lims_dev};
+        for (DevBuf* b : bufs) b->release();
+    }
+    delete m;
+}
+
+// Rows [a, b) of the striped sequence that belong to shard s, copied between `glob` (row a at glob, row-major [., d])
+// and `local` (contiguous, in order): the partial stripes at either end one copy each, the full stripes in between one
+// 2D copy with a source pitch of G stripes.  Any pair of host / device pointers (cudaMemcpyDefault).
+static int stripe_copy(float* glob, float* local, int64_t a, int64_t b, int s, int G, int d, bool to_local,
+                       cudaStream_t st) {
+    const size_t row = (size_t)d * 4;
+    const int64_t R = kStripeRows;
+    int64_t t = a / R;
+    t += ((s - t % G) % G + G) % G;  // first stripe of shard s at or after row a
+    int64_t out = 0;
+    auto copy = [&](int64_t lo, int64_t hi) -> cudaError_t {
+        float* g = glob + (lo - a) * d;
+        float* l = local + out * d;
+        out += hi - lo;
+        return cudaMemcpyAsync(to_local ? l : g, to_local ? g : l, (size_t)(hi - lo) * row, cudaMemcpyDefault, st);
+    };
+    if (t * R < a) {
+        KIRAG_CUDA_OK(copy(a, b < t * R + R ? b : t * R + R));
+        t += G;
+    }
+    const int64_t last_full = b / R - 1;
+    if (t * R < b && t <= last_full) {
+        const int64_t nfull = (last_full - t) / G + 1;
+        float* g = glob + (t * R - a) * d;
+        float* l = local + out * d;
+        const size_t gp = (size_t)G * R * row, lp = (size_t)R * row;
+        KIRAG_CUDA_OK(cudaMemcpy2DAsync(to_local ? l : g, to_local ? lp : gp, to_local ? g : l, to_local ? gp : lp,
+                                        (size_t)R * row, (size_t)nfull, cudaMemcpyDefault, st));
+        out += nfull * R;
+        t += nfull * G;
+    }
+    if (t * R < b) KIRAG_CUDA_OK(copy(t * R, b));
+    return 0;
+}
+
+// global rows per round of add / reconstruct: about kStageBytes per shard, whole stripes
+static int64_t multi_piece_rows(const MultiIndex* m, int d) {
+    int64_t per = (int64_t)(kStageBytes / ((size_t)d * 4)) / kStripeRows * kStripeRows;
+    if (per < kStripeRows) per = kStripeRows;
+    return per * m->G;
+}
+
+static void multi_drop_range(MultiIndex* m) {
+    m->range_valid = false;
+    m->range_n = 0;
+}
+
+static int multi_add(kirag_index* h, const float* x, int64_t n, int x_is_device, cudaStream_t st) {
+    MultiIndex* m = h->multi;
+    multi_drop_range(m);
+    const int d = h->d, G = m->G;
+    if (x_is_device) {  // x is written on the caller's stream; the workers read it on theirs
+        DeviceGuard guard(h->device);
+        if (!guard.ok) return 1;
+        KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    }
+    const int64_t piece = multi_piece_rows(m, d);
+    for (int64_t a = 0; a < n; a += piece) {
+        const int64_t len = (n - a < piece) ? (n - a) : piece;
+        const int64_t g0 = m->ntotal;
+        const float* src = x + a * d;
+        if (multi_run(m, [&](MultiShard& sh, int s) -> int {
+                const int64_t rows = stripe_rows(g0 + len, s, G) - stripe_rows(g0, s, G);
+                if (rows == 0) return 0;
+                if (sh.stage.ensure((size_t)rows * d * 4)) return 1;
+                if (stripe_copy(const_cast<float*>(src), sh.stage.as<float>(), g0, g0 + len, s, G, d, true, sh.st))
+                    return 1;
+                return kirag_index_add(sh.h, sh.stage.as<float>(), rows, 1, sh.st);
+            })) return 1;
+        m->ntotal = g0 + len;
+    }
+    return 0;
+}
+
+static int multi_reserve(kirag_index* h, int64_t n_total) {
+    MultiIndex* m = h->multi;
+    return multi_run(m, [&](MultiShard& sh, int s) { return kirag_index_reserve(sh.h, stripe_rows(n_total, s, m->G)); });
+}
+
+static int multi_reconstruct(const kirag_index* h, int64_t i0, int64_t n, float* out) {
+    MultiIndex* m = h->multi;
+    const int d = h->d, G = m->G;
+    const int64_t piece = multi_piece_rows(m, d);
+    for (int64_t a = i0; a < i0 + n; a += piece) {
+        const int64_t b = (i0 + n - a < piece) ? (i0 + n) : a + piece;
+        float* dst = out + (a - i0) * d;
+        if (multi_run(m, [&](MultiShard& sh, int s) -> int {
+                const int64_t l0 = stripe_rows(a, s, G), rows = stripe_rows(b, s, G) - l0;
+                if (rows == 0) return 0;
+                if (sh.stage.ensure((size_t)rows * d * 4)) return 1;
+                if (kirag_index_reconstruct(sh.h, l0, rows, sh.stage.as<float>(), 1, sh.st)) return 1;
+                if (stripe_copy(dst, sh.stage.as<float>(), a, b, s, G, d, false, sh.st)) return 1;
+                KIRAG_CUDA_OK(cudaStreamSynchronize(sh.st));
+                return 0;
+            })) return 1;
+    }
+    return 0;
+}
+
+static void add_stats(kirag_search_stats_t& acc, const kirag_search_stats_t& s) {
+    acc.n_fast += s.n_fast;
+    acc.n_exact += s.n_exact;
+    acc.n_cert_fail += s.n_cert_fail;
+    acc.n_overflow += s.n_overflow;
+    acc.n_rescan += s.n_rescan;
+    acc.n_retry += s.n_retry;
+    if (s.levels > acc.levels) acc.levels = s.levels;
+    acc.path = s.path;
+}
+
+// stats of a multi-device call: per-shard counts summed (a query counts once per shard), levels the maximum, the path
+// the shards' if they agree (else KIRAG_PATH_EXACT), kernel launches those of the workers and of the calling thread
+// (the merge) during the call.  launches0: the calling thread's count at the start of the call.
+static void multi_fill_stats(const MultiIndex* m, kirag_search_stats_t* stats, int64_t nq, long long launches0) {
+    if (!stats) return;
+    memset(stats, 0, sizeof(*stats));
+    stats->nq = nq;
+    for (int s = 0; s < m->G; ++s) {
+        const kirag_search_stats_t& ss = m->sh[(size_t)s]->stats;
+        const int path = stats->path;
+        add_stats(*stats, ss);
+        if (s > 0 && ss.path != path) stats->path = KIRAG_PATH_EXACT;
+    }
+    stats->kernel_launches = g_thread_launches - launches0;
+    for (const auto& sh : m->sh) stats->kernel_launches += sh->launches;
+}
+
+static int multi_search(kirag_index* h, const float* q, int64_t nq, int k, float* D, int64_t* I, int ptrs_are_device,
+                        int64_t id_offset, int path, kirag_search_stats_t* stats, cudaStream_t st) {
+    MultiIndex* m = h->multi;
+    multi_drop_range(m);
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (nq == 0) return 0;
+    KIRAG_CHECK(q && D && I, "search: null buffer");
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return 1;
+    const long long launches0 = g_thread_launches;
+    const int d = h->d, G = m->G;
+    if (ptrs_are_device) KIRAG_CUDA_OK(cudaStreamSynchronize(st));  // q is written on the caller's stream
+    for (auto& sh : m->sh) {
+        sh->stats = kirag_search_stats_t{};
+        sh->launches = 0;
+    }
+    const float* Dsh[kMaxShards];
+    const int64_t* Ish[kMaxShards];
+    for (int64_t q0 = 0; q0 < nq; q0 += kQChunk) {
+        const int64_t cq = (nq - q0 < kQChunk) ? (nq - q0) : kQChunk;
+        const float* qc = q + q0 * d;
+        if (multi_run(m, [&](MultiShard& sh, int) -> int {
+                if (sh.q.ensure((size_t)cq * d * 4) || sh.D.ensure((size_t)cq * k * 4) || sh.I.ensure((size_t)cq * k * 8))
+                    return 1;
+                KIRAG_CUDA_OK(cudaMemcpyAsync(sh.q.p, qc, (size_t)cq * d * 4, cudaMemcpyDefault, sh.st));
+                kirag_search_stats_t ss;
+                if (kirag_index_search_ex(sh.h, sh.q.as<float>(), cq, k, sh.D.as<float>(), sh.I.as<int64_t>(), 1, 0, path,
+                                          &ss, sh.st)) return 1;
+                KIRAG_CUDA_OK(cudaStreamSynchronize(sh.st));
+                add_stats(sh.stats, ss);
+                return 0;
+            })) return 1;
+        for (int s = 0; s < G; ++s) { Dsh[s] = m->sh[(size_t)s]->D.as<float>(); Ish[s] = m->sh[(size_t)s]->I.as<int64_t>(); }
+        float* Dd = D + q0 * k;
+        int64_t* Id = I + q0 * k;
+        if (!ptrs_are_device) {
+            if (m->D_out.ensure((size_t)cq * k * 4) || m->I_out.ensure((size_t)cq * k * 8)) return 1;
+            Dd = m->D_out.as<float>();
+            Id = m->I_out.as<int64_t>();
+        }
+        const size_t ws = multi_merge_ws_bytes(G, k, cq);
+        if (ws && m->ws.ensure(ws)) return 1;
+        if (launch_multi_merge(Dsh, Ish, G, cq, k, id_offset, Dd, Id, m->ws.p, st)) return 1;
+        if (!ptrs_are_device) {
+            KIRAG_CUDA_OK(cudaMemcpyAsync(D + q0 * k, Dd, (size_t)cq * k * 4, cudaMemcpyDeviceToHost, st));
+            KIRAG_CUDA_OK(cudaMemcpyAsync(I + q0 * k, Id, (size_t)cq * k * 8, cudaMemcpyDeviceToHost, st));
+        }
+        KIRAG_CUDA_OK(cudaStreamSynchronize(st));  // the next round's shard searches overwrite what the merge reads
+    }
+    multi_fill_stats(m, stats, nq, launches0);
+    return 0;
+}
+
+static int multi_range_search(kirag_index* h, const float* q, int64_t nq, float radius, int q_is_device,
+                              int64_t id_offset, int path, int64_t* lims_out, kirag_search_stats_t* stats,
+                              cudaStream_t st) {
+    MultiIndex* m = h->multi;
+    multi_drop_range(m);
+    if (stats) memset(stats, 0, sizeof(*stats));
+    for (int64_t i = 0; i <= nq; ++i) lims_out[i] = 0;
+    const int d = h->d, G = m->G;
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return 1;
+    const long long launches0 = g_thread_launches;
+    for (auto& sh : m->sh) sh->launches = 0;
+    if (nq > 0) {
+        KIRAG_CHECK(q != nullptr, "range_search: null queries");
+        if (q_is_device) KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    }
+    if (multi_run(m, [&](MultiShard& sh, int) -> int {
+            sh.stats = kirag_search_stats_t{};
+            sh.lims.assign((size_t)nq + 1, 0);
+            if (nq == 0) return 0;
+            if (sh.q.ensure((size_t)nq * d * 4)) return 1;
+            KIRAG_CUDA_OK(cudaMemcpyAsync(sh.q.p, q, (size_t)nq * d * 4, cudaMemcpyDefault, sh.st));
+            if (kirag_index_range_search(sh.h, sh.q.as<float>(), nq, radius, 1, 0, path, sh.lims.data(), &sh.stats,
+                                         sh.st)) return 1;
+            const int64_t total = sh.lims[(size_t)nq];
+            if (sh.rD.ensure((size_t)total * 4 + 4) || sh.rI.ensure((size_t)total * 8 + 8)) return 1;
+            return kirag_index_range_fetch(sh.h, sh.rD.as<float>(), sh.rI.as<int64_t>(), 1, sh.st);
+        })) return 1;
+    int64_t max_n = 0;
+    for (int64_t i = 0; i <= nq; ++i)
+        for (int s = 0; s < G; ++s) lims_out[i] += m->sh[(size_t)s]->lims[(size_t)i];
+    for (int s = 0; s < G; ++s) max_n = std::max(max_n, m->sh[(size_t)s]->lims[(size_t)nq]);
+    if (lims_out[nq] > 0) {
+        const size_t row = (size_t)(nq + 1) * 8;
+        if (m->lims_dev.ensure(row * (G + 1))) return 1;
+        for (int s = 0; s < G; ++s)
+            KIRAG_CUDA_OK(cudaMemcpyAsync(m->lims_dev.as<uint8_t>() + row * s, m->sh[(size_t)s]->lims.data(), row,
+                                          cudaMemcpyHostToDevice, st));
+        KIRAG_CUDA_OK(cudaMemcpyAsync(m->lims_dev.as<uint8_t>() + row * G, lims_out, row, cudaMemcpyHostToDevice, st));
+        KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    }
+    m->range_valid = true;
+    m->range_n = lims_out[nq];
+    m->range_nq = nq;
+    m->range_max = max_n;
+    m->range_id_offset = id_offset;
+    multi_fill_stats(m, stats, nq, launches0);
+    return 0;
+}
+
+static int multi_range_fetch(kirag_index* h, float* D, int64_t* I, int ptrs_are_device, cudaStream_t st) {
+    MultiIndex* m = h->multi;
+    KIRAG_CHECK(m->range_valid, "range_fetch: no range-search result is held (the last call on this index was not "
+                                "kirag_index_range_search, or its result was fetched already)");
+    const int64_t total = m->range_n, nq = m->range_nq;
+    const int G = m->G;
+    if (total > 0) {
+        KIRAG_CHECK(D && I, "range_fetch: null buffer");
+        DeviceGuard guard(h->device);
+        if (!guard.ok) return 1;
+        float* Dd = D;
+        int64_t* Id = I;
+        if (!ptrs_are_device) {
+            if (m->D_out.ensure((size_t)total * 4) || m->I_out.ensure((size_t)total * 8)) return 1;
+            Dd = m->D_out.as<float>();
+            Id = m->I_out.as<int64_t>();
+        }
+        const float* Dsh[kMaxShards];
+        const int64_t* Ish[kMaxShards];
+        for (int s = 0; s < G; ++s) { Dsh[s] = m->sh[(size_t)s]->rD.as<float>(); Ish[s] = m->sh[(size_t)s]->rI.as<int64_t>(); }
+        const int64_t* lims = m->lims_dev.as<int64_t>();
+        if (launch_multi_range_merge(Dsh, Ish, lims, lims + (size_t)G * (nq + 1), G, nq, m->range_max, m->range_id_offset,
+                                     Dd, Id, st)) return 1;
+        if (!ptrs_are_device) {
+            KIRAG_CUDA_OK(cudaMemcpyAsync(D, Dd, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
+            KIRAG_CUDA_OK(cudaMemcpyAsync(I, Id, (size_t)total * 8, cudaMemcpyDeviceToHost, st));
+        }
+        KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    }
+    multi_drop_range(m);
+    return 0;
+}
+
 // ================================================================= C ABI ====
 extern "C" {
 
@@ -1656,6 +2055,7 @@ int kirag_device_count(void) {
 }
 
 int kirag_profile_enable(int on) {
+    std::lock_guard<std::mutex> lock(g_prof_mu);
     for (auto& pr : g_prof.ev) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
     g_prof.ev.clear();
     g_prof.launch_rows.clear();
@@ -1668,6 +2068,7 @@ int kirag_profile_enable(int on) {
 
 int kirag_profile_read_timeline(int* tags_out, double* ms_since_first, int64_t max_n) {
     // timeline of the recorded search phases (does not clear); ms are relative to the first mark
+    std::lock_guard<std::mutex> lock(g_prof_mu);
     int64_t i = 0;
     for (auto& mk : g_prof.marks) {
         if (i >= max_n) break;
@@ -1683,6 +2084,7 @@ int kirag_profile_read_timeline(int* tags_out, double* ms_since_first, int64_t m
 
 int kirag_profile_read_launches(double* ms_out, double* rows_out, int64_t max_n) {
     // per-launch durations (does not clear; call before kirag_profile_read)
+    std::lock_guard<std::mutex> lock(g_prof_mu);
     int64_t i = 0;
     for (auto& pr : g_prof.ev) {
         if (i >= max_n) break;
@@ -1697,6 +2099,7 @@ int kirag_profile_read_launches(double* ms_out, double* rows_out, int64_t max_n)
 }
 
 int kirag_profile_read(double* scan_ms, int64_t* scan_launches, double* scan_rows) {
+    std::lock_guard<std::mutex> lock(g_prof_mu);
     double ms = 0.0;
     for (auto& pr : g_prof.ev) {
         KIRAG_CUDA_OK(cudaEventSynchronize(pr.second));
@@ -1720,30 +2123,44 @@ int kirag_index_create(int d, int metric, int device, kirag_index_t** out) {
     return kirag_index_create_ex(d, metric, device, 0, out);
 }
 
-int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_t** out) {
-    KIRAG_CHECK(out != nullptr, "index_create: null out pointer");
-    *out = nullptr;
-    KIRAG_CHECK(d > 0 && d <= 16384, "index_create: unsupported dimension %d", d);
-    KIRAG_CHECK(metric == KIRAG_METRIC_INNER_PRODUCT,
-                "index_create: only the inner-product metric is implemented (got %d)", metric);
-    KIRAG_CHECK((flags & ~KIRAG_INDEX_HOST_MASTER) == 0, "index_create: unknown flag bits 0x%x",
+// Checks of kirag_index_create_ex / _multi that need no device.
+static int check_index_args(const char* what, int d, int metric, int flags) {
+    KIRAG_CHECK(d > 0 && d <= 16384, "%s: unsupported dimension %d", what, d);
+    KIRAG_CHECK(metric == KIRAG_METRIC_INNER_PRODUCT, "%s: only the inner-product metric is implemented (got %d)", what,
+                metric);
+    KIRAG_CHECK((flags & ~KIRAG_INDEX_HOST_MASTER) == 0, "%s: unknown flag bits 0x%x", what,
                 (unsigned)(flags & ~KIRAG_INDEX_HOST_MASTER));
     // without a shadow every search would be an fp32 scan of the master over PCIe
     KIRAG_CHECK(!(flags & KIRAG_INDEX_HOST_MASTER) || scan_tc_supported(d),
-                "index_create: host master needs the bf16 shadow (d %% 64 == 0, got d=%d)", d);
+                "%s: host master needs the bf16 shadow (d %% 64 == 0, got d=%d)", what, d);
+    return 0;
+}
+
+// The device must exist and be an sm_100 part.
+static int check_device(const char* what, int device, int* num_sms) {
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev == 0) {
-        set_error("index_create: no CUDA device available (%s); this library has no CPU path",
+        set_error("%s: no CUDA device available (%s); this library has no CPU path", what,
                   e == cudaSuccess ? "device count is 0" : cudaGetErrorString(e));
         cudaGetLastError();
         return 1;
     }
-    KIRAG_CHECK(device >= 0 && device < ndev, "index_create: device %d out of range [0,%d)", device, ndev);
+    KIRAG_CHECK(device >= 0 && device < ndev, "%s: device %d out of range [0,%d)", what, device, ndev);
     cudaDeviceProp prop;
     KIRAG_CUDA_OK(cudaGetDeviceProperties(&prop, device));
-    KIRAG_CHECK(prop.major == 10, "index_create: device %d is sm_%d%d; this library is built for sm_100a only",
-                device, prop.major, prop.minor);
+    KIRAG_CHECK(prop.major == 10, "%s: device %d is sm_%d%d; this library is built for sm_100a only", what, device,
+                prop.major, prop.minor);
+    if (num_sms) *num_sms = prop.multiProcessorCount;
+    return 0;
+}
+
+int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_t** out) {
+    KIRAG_CHECK(out != nullptr, "index_create: null out pointer");
+    *out = nullptr;
+    if (check_index_args("index_create", d, metric, flags)) return 1;
+    int num_sms = 0;
+    if (check_device("index_create", device, &num_sms)) return 1;
     DeviceGuard guard(device);
     if (!guard.ok) return 1;
     kirag_index* h = new (std::nothrow) kirag_index();
@@ -1751,7 +2168,7 @@ int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_
     h->d = d;
     h->metric = metric;
     h->device = device;
-    h->num_sms = prop.multiProcessorCount;
+    h->num_sms = num_sms;
     h->host_master = (flags & KIRAG_INDEX_HOST_MASTER) != 0;
     if (cudaMalloc((void**)&h->maxnorm2_bits, 12) != cudaSuccess || cudaMemset(h->maxnorm2_bits, 0, 12) != cudaSuccess) {
         set_error("index_create: cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -1762,8 +2179,100 @@ int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_
     return 0;
 }
 
+int kirag_index_create_multi(int d, int metric, const int* devices, int n_devices, int flags, kirag_index_t** out) {
+    KIRAG_CHECK(out != nullptr, "index_create_multi: null out pointer");
+    *out = nullptr;
+    KIRAG_CHECK(devices != nullptr && n_devices >= 1, "index_create_multi: empty device list");
+    KIRAG_CHECK(n_devices <= kMaxShards, "index_create_multi: %d devices exceed the maximum of %d", n_devices, kMaxShards);
+    if (check_index_args("index_create_multi", d, metric, flags)) return 1;
+    for (int s = 0; s < n_devices; ++s)
+        if (check_device("index_create_multi", devices[s], nullptr)) return 1;
+    // the merges run on the home device and read every shard's results in place
+    const int home = devices[0];
+    for (int s = 1; s < n_devices; ++s) {
+        if (devices[s] == home) continue;
+        int can = 0;
+        KIRAG_CUDA_OK(cudaDeviceCanAccessPeer(&can, home, devices[s]));
+        KIRAG_CHECK(can, "index_create_multi: device %d cannot access device %d's memory (no peer access)", home,
+                    devices[s]);
+        DeviceGuard guard(home);
+        if (!guard.ok) return 1;
+        const cudaError_t e = cudaDeviceEnablePeerAccess(devices[s], 0);
+        if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) {
+            set_error("index_create_multi: cudaDeviceEnablePeerAccess(%d -> %d) failed: %s", home, devices[s],
+                      cudaGetErrorString(e));
+            cudaGetLastError();
+            return 1;
+        }
+        cudaGetLastError();
+    }
+    MultiIndex* m = new (std::nothrow) MultiIndex();
+    KIRAG_CHECK(m != nullptr, "index_create_multi: out of host memory");
+    m->G = n_devices;
+    for (int s = 0; s < n_devices; ++s) {
+        MultiShard* sh = new (std::nothrow) MultiShard();
+        if (sh) {
+            try {
+                m->sh.emplace_back(sh);
+            } catch (const std::exception&) {
+                delete sh;
+                sh = nullptr;
+            }
+        }
+        if (!sh) { multi_destroy(m); set_error("index_create_multi: out of host memory"); return 1; }
+        sh->device = devices[s];
+        if (kirag_index_create_ex(d, metric, devices[s], flags, &sh->h)) { multi_destroy(m); return 1; }
+        DeviceGuard guard(devices[s]);
+        if (!guard.ok || cudaStreamCreateWithFlags(&sh->st, cudaStreamNonBlocking) != cudaSuccess) {
+            set_error("index_create_multi: cudaStreamCreate on device %d failed: %s", devices[s],
+                      cudaGetErrorString(cudaGetLastError()));
+            sh->st = nullptr;
+            multi_destroy(m);
+            return 1;
+        }
+    }
+    for (int s = 0; s < n_devices; ++s) {
+        try {
+            m->sh[(size_t)s]->th = std::thread(multi_worker, m, s);
+        } catch (const std::exception& e) {
+            multi_destroy(m);  // joins the workers started so far
+            set_error("index_create_multi: starting the worker of shard %d failed: %s", s, e.what());
+            return 1;
+        }
+    }
+    kirag_index* h = new (std::nothrow) kirag_index();
+    if (!h) { multi_destroy(m); set_error("index_create_multi: out of host memory"); return 1; }
+    h->multi = m;
+    h->d = d;
+    h->metric = metric;
+    h->device = home;
+    h->host_master = (flags & KIRAG_INDEX_HOST_MASTER) != 0;
+    *out = h;
+    return 0;
+}
+
+int kirag_index_shards(const kirag_index_t* h, int* devices_out, int64_t* rows_out, int max) {
+    if (!h) { set_error("index_shards: null index"); return -1; }
+    if (!h->multi) {
+        if (max >= 1 && devices_out) devices_out[0] = h->device;
+        if (max >= 1 && rows_out) rows_out[0] = h->ntotal;
+        return 1;
+    }
+    const MultiIndex* m = h->multi;
+    for (int s = 0; s < m->G && s < max; ++s) {
+        if (devices_out) devices_out[s] = m->sh[(size_t)s]->device;
+        if (rows_out) rows_out[s] = kirag_index_ntotal(m->sh[(size_t)s]->h);
+    }
+    return m->G;
+}
+
 int kirag_index_destroy(kirag_index_t* h) {
     if (!h) return 0;
+    if (h->multi) {
+        multi_destroy(h->multi);
+        delete h;
+        return 0;
+    }
     DeviceGuard guard(h->device);
     cudaDeviceSynchronize();
     if (h->host_master) {
@@ -1798,6 +2307,7 @@ int kirag_index_destroy(kirag_index_t* h) {
 int kirag_index_reserve(kirag_index_t* h, int64_t n_total) {
     KIRAG_CHECK(h != nullptr, "index_reserve: null index");
     KIRAG_CHECK(n_total >= 0, "index_reserve: negative size");
+    if (h->multi) return multi_reserve(h, n_total);
     DeviceGuard guard(h->device);
     if (!guard.ok) return 1;
     return index_grow(h, n_total, 0);
@@ -1808,6 +2318,7 @@ int kirag_index_add(kirag_index_t* h, const float* x, int64_t n, int x_is_device
     KIRAG_CHECK(n >= 0, "index_add: negative n");
     if (n == 0) return 0;
     KIRAG_CHECK(x != nullptr, "index_add: null data");
+    if (h->multi) return multi_add(h, x, n, x_is_device, (cudaStream_t)stream);
     DeviceGuard guard(h->device);
     if (!guard.ok) return 1;
     cudaStream_t st = (cudaStream_t)stream;
@@ -1830,7 +2341,7 @@ int kirag_index_add(kirag_index_t* h, const float* x, int64_t n, int x_is_device
     return finalize_rows(h, h->ntotal, n, dst, st);
 }
 
-int64_t kirag_index_ntotal(const kirag_index_t* h) { return h ? h->ntotal : -1; }
+int64_t kirag_index_ntotal(const kirag_index_t* h) { return h ? (h->multi ? h->multi->ntotal : h->ntotal) : -1; }
 int kirag_index_dim(const kirag_index_t* h) { return h ? h->d : -1; }
 
 int kirag_index_search(kirag_index_t* h, const float* q, int64_t nq, int k, float* D, int64_t* I,
@@ -1850,7 +2361,10 @@ int kirag_index_range_search(kirag_index_t* h, const float* q, int64_t nq, float
                              void* stream) {
     const int rc = range_search_impl(h, q, nq, radius, q_is_device, id_offset, path, lims_out, stats,
                                      (cudaStream_t)stream);
-    if (rc && h) drop_range_result(h);  // no partial result
+    if (rc && h) {  // no partial result
+        drop_range_result(h);
+        if (h->multi) multi_drop_range(h->multi);
+    }
     return rc;
 }
 
@@ -1861,6 +2375,7 @@ int kirag_index_range_fetch(kirag_index_t* h, float* D, int64_t* I, int ptrs_are
 int kirag_index_search_async(kirag_index_t* h, const float* q, int64_t nq, int k, float* D, int64_t* I,
                              int64_t id_offset, void* stream) {
     KIRAG_CHECK(h != nullptr, "search_async: null index");
+    KIRAG_CHECK(!h->multi, "search_async: not supported on a multi-device index");
     KIRAG_CHECK(k > 0 && k <= 2048, "search_async: k=%d not in [1, 2048]", k);
     KIRAG_CHECK(nq >= 0 && nq <= kQChunk, "search_async: nq=%lld not in [0, %lld] (split larger batches)", (long long)nq,
                 (long long)kQChunk);
@@ -1895,6 +2410,7 @@ int kirag_index_search_async(kirag_index_t* h, const float* q, int64_t nq, int k
 
 int kirag_index_search_rearm(kirag_index_t* h, void* stream) {
     KIRAG_CHECK(h != nullptr, "search_rearm: null index");
+    KIRAG_CHECK(!h->multi, "search_rearm: not supported on a multi-device index");
     KIRAG_CHECK(h->has_captured, "search_rearm: no asynchronous search has been captured on this index");
     if (finish_pending(h, nullptr, nullptr)) return 1;
     h->pending = h->captured;
@@ -1908,6 +2424,7 @@ int kirag_index_search_rearm(kirag_index_t* h, void* stream) {
 // FNV-1a over everything a captured search has baked into its kernel arguments
 int kirag_index_state_token(const kirag_index_t* h, uint64_t* token) {
     KIRAG_CHECK(h != nullptr && token != nullptr, "state_token: null argument");
+    KIRAG_CHECK(!h->multi, "state_token: not supported on a multi-device index");
     uint64_t x = 1469598103934665603ULL;
     auto mix = [&x](uint64_t v) {
         for (int i = 0; i < 8; ++i) { x ^= (v >> (8 * i)) & 0xffu; x *= 1099511628211ULL; }
@@ -1929,11 +2446,13 @@ int kirag_index_state_token(const kirag_index_t* h, uint64_t* token) {
 
 int kirag_index_search_finish(kirag_index_t* h, kirag_search_stats_t* stats, int64_t* n_changed) {
     KIRAG_CHECK(h != nullptr, "search_finish: null index");
+    KIRAG_CHECK(!h->multi, "search_finish: not supported on a multi-device index");
     return finish_pending(h, stats, n_changed);
 }
 
 int kirag_index_search_flags(const kirag_index_t* h, const int** flags_dev) {
     KIRAG_CHECK(h != nullptr && flags_dev != nullptr, "search_flags: null argument");
+    KIRAG_CHECK(!h->multi, "search_flags: not supported on a multi-device index");
     *flags_dev = (h->pending.active && h->pending.mode == 1) ? h->flags.as<int>() : nullptr;
     return 0;
 }
@@ -1941,9 +2460,11 @@ int kirag_index_search_flags(const kirag_index_t* h, const int** flags_dev) {
 int kirag_index_reconstruct(const kirag_index_t* h, int64_t i0, int64_t n, float* out, int out_is_device,
                             void* stream) {
     KIRAG_CHECK(h != nullptr && out != nullptr, "index_reconstruct: null argument");
-    KIRAG_CHECK(i0 >= 0 && n >= 0 && i0 + n <= h->ntotal, "index_reconstruct: rows [%lld,%lld) out of range (ntotal=%lld)",
-                (long long)i0, (long long)(i0 + n), (long long)h->ntotal);
+    const int64_t ntotal = kirag_index_ntotal(h);
+    KIRAG_CHECK(i0 >= 0 && n >= 0 && i0 + n <= ntotal, "index_reconstruct: rows [%lld,%lld) out of range (ntotal=%lld)",
+                (long long)i0, (long long)(i0 + n), (long long)ntotal);
     if (n == 0) return 0;
+    if (h->multi) return multi_reconstruct(h, i0, n, out);
     DeviceGuard guard(h->device);
     if (!guard.ok) return 1;
     cudaStream_t st = (cudaStream_t)stream;
@@ -1963,6 +2484,7 @@ int kirag_index_reconstruct(const kirag_index_t* h, int64_t i0, int64_t n, float
 /* debug / test hook: dense approximate (bf16 tcgen05) scores, out is host [ntotal, nq] */
 int kirag_index_debug_scores(kirag_index_t* h, const float* q_host, int64_t nq, float* out_host) {
     KIRAG_CHECK(h && q_host && out_host, "debug_scores: null argument");
+    KIRAG_CHECK(!h->multi, "debug_scores: not supported on a multi-device index");
     KIRAG_CHECK(h->shadow && scan_tc_supported(h->d), "debug_scores: index has no bf16 shadow (d=%d)", h->d);
     KIRAG_CHECK(nq > 0 && h->ntotal > 0, "debug_scores: empty input");
     DeviceGuard guard(h->device);
@@ -2054,6 +2576,18 @@ int kirag_debug_level_schedule(int64_t n_rows, int64_t nq, int k, int d, int64_t
 
 int kirag_index_storage_bytes(const kirag_index_t* h, int64_t* device_bytes, int64_t* host_bytes) {
     KIRAG_CHECK(h != nullptr, "index_storage_bytes: null index");
+    if (h->multi) {  // summed over the shards
+        int64_t dev_sum = 0, host_sum = 0;
+        for (auto& sh : h->multi->sh) {
+            int64_t db = 0, hb = 0;
+            if (kirag_index_storage_bytes(sh->h, &db, &hb)) return 1;
+            dev_sum += db;
+            host_sum += hb;
+        }
+        if (device_bytes) *device_bytes = dev_sum;
+        if (host_bytes) *host_bytes = host_sum;
+        return 0;
+    }
     const size_t row_m = (size_t)h->d * 4, row_s = (size_t)h->d * 2;
     size_t dev = 0;
     if (h->use_vmm) dev = (h->host_master ? 0 : h->vm_master.mapped) + h->vm_shadow.mapped;
@@ -2065,6 +2599,7 @@ int kirag_index_storage_bytes(const kirag_index_t* h, int64_t* device_bytes, int
 
 int kirag_index_device_ptrs(const kirag_index_t* h, const float** master_f32, const void** shadow_bf16) {
     KIRAG_CHECK(h != nullptr, "index_device_ptrs: null index");
+    KIRAG_CHECK(!h->multi, "index_device_ptrs: not supported on a multi-device index (the rows are spread over shards)");
     if (master_f32) *master_f32 = h->master;
     if (shadow_bf16) *shadow_bf16 = h->shadow;
     return 0;
@@ -2073,6 +2608,35 @@ int kirag_index_device_ptrs(const kirag_index_t* h, const float** master_f32, co
 // ---- FAISS "IxFI" container (faiss 1.8.0 index_write.cpp: write_index_header
 //      + WRITEXBVECTOR(codes)); restated from the published format -------------
 static const size_t kIoChunkRows = 65536;
+static const uint32_t kIxFI = (uint32_t)'I' | ((uint32_t)'x' << 8) | ((uint32_t)'F' << 16) | ((uint32_t)'I' << 24);
+
+static bool write_ixfi_header(FILE* f, int32_t d, int64_t ntotal) {
+    const int64_t dummy = (int64_t)1 << 20;
+    const uint8_t trained = 1;
+    const int32_t metric = 0;  // METRIC_INNER_PRODUCT
+    const uint64_t words = (uint64_t)ntotal * (uint64_t)d;
+    return fwrite(&kIxFI, 4, 1, f) == 1 && fwrite(&d, 4, 1, f) == 1 && fwrite(&ntotal, 8, 1, f) == 1 &&
+           fwrite(&dummy, 8, 1, f) == 1 && fwrite(&dummy, 8, 1, f) == 1 && fwrite(&trained, 1, 1, f) == 1 &&
+           fwrite(&metric, 4, 1, f) == 1 && fwrite(&words, 8, 1, f) == 1;
+}
+
+// Reads the header up to the payload; 0 ok, 1 (error set) not an IxFI file or an inconsistent header.
+static int read_ixfi_header(FILE* f, const char* path, int32_t* d_out, int64_t* ntotal_out) {
+    uint32_t fourcc = 0; int32_t d = 0; int64_t ntotal = 0, dummy = 0; uint8_t trained = 0; int32_t metric = 0;
+    uint64_t words = 0;
+    bool ok = fread(&fourcc, 4, 1, f) == 1 && fread(&d, 4, 1, f) == 1 && fread(&ntotal, 8, 1, f) == 1 &&
+              fread(&dummy, 8, 1, f) == 1 && fread(&dummy, 8, 1, f) == 1 && fread(&trained, 1, 1, f) == 1 &&
+              fread(&metric, 4, 1, f) == 1;
+    KIRAG_CHECK(ok && fourcc == kIxFI, "index_load: %s is not an IxFI (IndexFlatIP) file (fourcc 0x%08x)", path, fourcc);
+    if (metric > 1) { float arg; ok = ok && fread(&arg, 4, 1, f) == 1; }
+    ok = ok && fread(&words, 8, 1, f) == 1;
+    KIRAG_CHECK(ok && metric == 0 && d > 0 && ntotal >= 0 && words == (uint64_t)ntotal * (uint64_t)d,
+                "index_load: %s has an inconsistent header (d=%d ntotal=%lld metric=%d words=%llu)", path, d,
+                (long long)ntotal, metric, (unsigned long long)words);
+    *d_out = d;
+    *ntotal_out = ntotal;
+    return 0;
+}
 
 int kirag_index_save(const kirag_index_t* h, const char* path) {
     KIRAG_CHECK(h != nullptr && path != nullptr, "index_save: null argument");
@@ -2080,17 +2644,35 @@ int kirag_index_save(const kirag_index_t* h, const char* path) {
     if (!guard.ok) return 1;
     FILE* f = fopen(path, "wb");
     KIRAG_CHECK(f != nullptr, "index_save: cannot open %s for writing", path);
-    bool ok = true;
-    const uint32_t fourcc = (uint32_t)'I' | ((uint32_t)'x' << 8) | ((uint32_t)'F' << 16) | ((uint32_t)'I' << 24);
+    if (h->multi) {
+        // the same bytes as a single-device index with the same rows: every shard reconstructs its part of a piece,
+        // the stripes are interleaved in a pinned host buffer, the piece is written
+        const int64_t ntotal = h->multi->ntotal, piece = multi_piece_rows(h->multi, h->d);
+        float* buf = nullptr;
+        bool ok = write_ixfi_header(f, h->d, ntotal);
+        if (ok && ntotal > 0 && cudaMallocHost((void**)&buf, (size_t)std::min(piece, ntotal) * h->d * 4) != cudaSuccess) {
+            set_error("index_save: pinned staging buffer: %s", cudaGetErrorString(cudaGetLastError()));
+            buf = nullptr;
+            ok = false;
+        }
+        for (int64_t r = 0; ok && r < ntotal; r += piece) {
+            const int64_t rows = (ntotal - r < piece) ? (ntotal - r) : piece;
+            if (multi_reconstruct(h, r, rows, buf)) { ok = false; break; }
+            ok = fwrite(buf, (size_t)h->d * 4, (size_t)rows, f) == (size_t)rows;
+        }
+        if (buf) cudaFreeHost(buf);
+        if (fclose(f) != 0) ok = false;
+        if (!ok) {
+            char why[512];
+            snprintf(why, sizeof(why), "%s", kirag_last_error());  // set_error writes the buffer kirag_last_error reads
+            set_error("index_save: write to %s failed: %s", path, why);
+            return 1;
+        }
+        return 0;
+    }
     const int32_t d = h->d;
     const int64_t ntotal = h->ntotal;
-    const int64_t dummy = (int64_t)1 << 20;
-    const uint8_t trained = 1;
-    const int32_t metric = 0;  // METRIC_INNER_PRODUCT
-    const uint64_t words = (uint64_t)ntotal * (uint64_t)d;
-    ok = ok && fwrite(&fourcc, 4, 1, f) == 1 && fwrite(&d, 4, 1, f) == 1 && fwrite(&ntotal, 8, 1, f) == 1 &&
-         fwrite(&dummy, 8, 1, f) == 1 && fwrite(&dummy, 8, 1, f) == 1 && fwrite(&trained, 1, 1, f) == 1 &&
-         fwrite(&metric, 4, 1, f) == 1 && fwrite(&words, 8, 1, f) == 1;
+    bool ok = write_ixfi_header(f, d, ntotal);
     if (h->host_master) {
         // the master is host memory already: written as it is, the same bytes as a device-master index's file
         for (int64_t r = 0; ok && r < ntotal; r += (int64_t)kIoChunkRows) {
@@ -2162,25 +2744,9 @@ int kirag_index_load_ex(const char* path, int device, int flags, kirag_index_t**
     *out = nullptr;
     FILE* f = fopen(path, "rb");
     KIRAG_CHECK(f != nullptr, "index_load: cannot open %s", path);
-    uint32_t fourcc = 0; int32_t d = 0; int64_t ntotal = 0, dummy = 0; uint8_t trained = 0; int32_t metric = 0;
-    uint64_t words = 0;
-    bool ok = fread(&fourcc, 4, 1, f) == 1 && fread(&d, 4, 1, f) == 1 && fread(&ntotal, 8, 1, f) == 1 &&
-              fread(&dummy, 8, 1, f) == 1 && fread(&dummy, 8, 1, f) == 1 && fread(&trained, 1, 1, f) == 1 &&
-              fread(&metric, 4, 1, f) == 1;
-    const uint32_t ixfi = (uint32_t)'I' | ((uint32_t)'x' << 8) | ((uint32_t)'F' << 16) | ((uint32_t)'I' << 24);
-    if (!ok || fourcc != ixfi) {
-        fclose(f);
-        set_error("index_load: %s is not an IxFI (IndexFlatIP) file (fourcc 0x%08x)", path, fourcc);
-        return 1;
-    }
-    if (metric > 1) { float arg; ok = ok && fread(&arg, 4, 1, f) == 1; }
-    ok = ok && fread(&words, 8, 1, f) == 1;
-    if (!ok || metric != 0 || d <= 0 || ntotal < 0 || words != (uint64_t)ntotal * (uint64_t)d) {
-        fclose(f);
-        set_error("index_load: %s has an inconsistent header (d=%d ntotal=%lld metric=%d words=%llu)", path, d,
-                  (long long)ntotal, metric, (unsigned long long)words);
-        return 1;
-    }
+    int32_t d = 0;
+    int64_t ntotal = 0;
+    if (read_ixfi_header(f, path, &d, &ntotal)) { fclose(f); return 1; }
     kirag_index_t* h = nullptr;
     if (kirag_index_create_ex(d, KIRAG_METRIC_INNER_PRODUCT, device, flags, &h)) { fclose(f); return 1; }
     if (ntotal == 0) { fclose(f); *out = h; return 0; }
@@ -2246,6 +2812,75 @@ int kirag_index_load_ex(const char* path, int device, int flags, kirag_index_t**
     fclose(f);
     if (rc) { kirag_index_destroy(h); return 1; }
     *out = h;
+    return 0;
+}
+
+// The file is streamed once, in 64 MB pieces read into one pinned buffer; every piece is split over the shards by the
+// stripe rule (one add per piece).
+int kirag_index_load_multi(const char* path, const int* devices, int n_devices, int flags, kirag_index_t** out) {
+    KIRAG_CHECK(path != nullptr && out != nullptr, "index_load: null argument");
+    *out = nullptr;
+    FILE* f = fopen(path, "rb");
+    KIRAG_CHECK(f != nullptr, "index_load: cannot open %s", path);
+    int32_t d = 0;
+    int64_t ntotal = 0;
+    kirag_index_t* h = nullptr;
+    if (read_ixfi_header(f, path, &d, &ntotal) ||
+        kirag_index_create_multi(d, KIRAG_METRIC_INNER_PRODUCT, devices, n_devices, flags, &h)) {
+        fclose(f);
+        return 1;
+    }
+    const size_t row_bytes = (size_t)d * 4;
+    int64_t piece = (int64_t)(((size_t)64 << 20) / row_bytes);
+    if (piece < 1) piece = 1;
+    if (piece > ntotal) piece = ntotal;
+    float* buf = nullptr;
+    int rc = 1;
+    do {
+        if (ntotal == 0) { rc = 0; break; }
+        if (kirag_index_reserve(h, ntotal)) break;
+        if (cudaMallocHost((void**)&buf, (size_t)piece * row_bytes) != cudaSuccess) {
+            set_error("index_load: pinned staging buffer: %s", cudaGetErrorString(cudaGetLastError()));
+            buf = nullptr;
+            break;
+        }
+        bool ok = true;
+        for (int64_t r = 0; ok && r < ntotal; r += piece) {
+            const int64_t rows = (ntotal - r < piece) ? (ntotal - r) : piece;
+            if (fread(buf, row_bytes, (size_t)rows, f) != (size_t)rows) {
+                set_error("index_load: %s is truncated", path);
+                ok = false;
+            } else if (kirag_index_add(h, buf, rows, 0, nullptr)) {
+                ok = false;
+            }
+        }
+        if (ok) rc = 0;
+    } while (0);
+    if (buf) cudaFreeHost(buf);
+    fclose(f);
+    if (rc) { kirag_index_destroy(h); return 1; }
+    *out = h;
+    return 0;
+}
+
+int kirag_debug_stripe_map(int G, const int64_t* global_ids, int64_t n, int* shard_out, int64_t* local_out,
+                           int64_t* global_out) {
+    KIRAG_CHECK(G >= 1 && n >= 0 && (n == 0 || global_ids), "debug_stripe_map: bad argument");
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t r = global_ids[i];
+        KIRAG_CHECK(r >= 0, "debug_stripe_map: negative row %lld", (long long)r);
+        const int s = stripe_shard(r, G);
+        const int64_t l = stripe_local(r, G);
+        if (shard_out) shard_out[i] = s;
+        if (local_out) local_out[i] = l;
+        if (global_out) global_out[i] = stripe_global(l, s, G);
+    }
+    return 0;
+}
+
+int kirag_debug_stripe_rows(int64_t ntotal, int G, int64_t* rows_out) {
+    KIRAG_CHECK(G >= 1 && ntotal >= 0 && rows_out, "debug_stripe_rows: bad argument");
+    for (int s = 0; s < G; ++s) rows_out[s] = stripe_rows(ntotal, s, G);
     return 0;
 }
 

@@ -205,7 +205,83 @@ __device__ __forceinline__ void bitonic_sort_desc(uint64_t* s, int P) {
         }
     }
 }
+
+// (key, id) total order of the result lists: larger key first, then lower id
+__device__ __forceinline__ bool item_before(uint32_t ka, int64_t ia, uint32_t kb, int64_t ib) {
+    return (ka > kb) || (ka == kb && ia < ib);
+}
+
+// number of items of the sorted list (keys[0..n), ids[0..n)) that come before (key, id)
+__device__ __forceinline__ int count_before(const uint32_t* keys, const int64_t* ids, int n, uint32_t key, int64_t id) {
+    int lo = 0, hi = n;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (item_before(keys[mid], ids[mid], key, id)) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+__device__ __forceinline__ void group_barrier(int id, int n_threads) {
+    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n_threads) : "memory");
+}
+
+// Pairwise merge tree of G lists sorted by (key desc, id asc), with distinct ids, run by one thread group (thread gt of
+// gthreads, named barrier bar_id).  Buffer b of keys_buf / ids_buf is [G*k] (list l at [l*k, l*k + nv[b][l])); the
+// lists start in buffer 0.  Two lists are merged by giving every element the rank "own position + number of elements
+// of the sibling list that precede it" (one binary search) and keeping ranks < k: the top-k of a union is in the union
+// of the top-k's, so truncating after every round is exact.  log2 G rounds, O(G k log k) steps, no sort.  Returns the
+// buffer that holds the merged list (nv[result][0] items).  The buffers may be shared or global memory.
+__device__ __forceinline__ int merge_tree(uint32_t* keys_buf, int64_t* ids_buf, int* const nv[2], int G, int k, int gt,
+                                          int gthreads, int bar_id) {
+    const size_t L = (size_t)G * k;
+    int cur = 0;
+    for (int n_lists = G; n_lists > 1; n_lists = (n_lists + 1) >> 1) {
+        const uint32_t* kin = keys_buf + (size_t)cur * L;
+        const int64_t* iin = ids_buf + (size_t)cur * L;
+        uint32_t* kout = keys_buf + (size_t)(cur ^ 1) * L;
+        int64_t* iout = ids_buf + (size_t)(cur ^ 1) * L;
+        const int* nin = nv[cur];
+        int* nout = nv[cur ^ 1];
+        for (int i = gt; i < n_lists * k; i += gthreads) {
+            const int l = i / k, j = i - l * k;
+            const int mate = l ^ 1;
+            const int n_own = nin[l];
+            const int n_mate = (mate < n_lists) ? nin[mate] : 0;
+            if (j == 0 && (l & 1) == 0) nout[l >> 1] = (n_own + n_mate < k) ? (n_own + n_mate) : k;
+            if (j >= n_own) continue;
+            const uint32_t key = kin[i];
+            const int64_t id = iin[i];
+            const int r = j + (n_mate ? count_before(kin + (size_t)mate * k, iin + (size_t)mate * k, n_mate, key, id) : 0);
+            if (r < k) {
+                kout[(size_t)(l >> 1) * k + r] = key;
+                iout[(size_t)(l >> 1) * k + r] = id;
+            }
+        }
+        group_barrier(bar_id, gthreads);
+        cur ^= 1;
+    }
+    return cur;
+}
 #endif
+
+// --------------------------------------------------- multi-device stripes ---
+// A multi-device index (kirag_index_create_multi) with G shards keeps global row r in shard (r / 128) mod G at local
+// row (r / (128 G)) * 128 + r mod 128.  Pure arithmetic: no id tables, shards within 128 rows of each other whatever
+// the add sizes, and local order within a shard is monotone in the global id.
+constexpr int kStripeRows = 128;
+__host__ __device__ __forceinline__ int stripe_shard(int64_t r, int G) { return (int)((r / kStripeRows) % G); }
+__host__ __device__ __forceinline__ int64_t stripe_local(int64_t r, int G) {
+    return r / ((int64_t)kStripeRows * G) * kStripeRows + r % kStripeRows;
+}
+__host__ __device__ __forceinline__ int64_t stripe_global(int64_t local, int s, int G) {
+    return (local / kStripeRows * G + s) * kStripeRows + local % kStripeRows;
+}
+// rows of shard s among the global rows [0, n)
+__host__ __device__ __forceinline__ int64_t stripe_rows(int64_t n, int s, int G) {
+    const int64_t span = (int64_t)kStripeRows * G;
+    const int64_t rem = n % span - (int64_t)s * kStripeRows;
+    return n / span * kStripeRows + (rem < 0 ? 0 : rem > kStripeRows ? kStripeRows : rem);
+}
 
 // ------------------------------------------------------ kernel launchers ---
 // convert.cu
@@ -295,6 +371,20 @@ int launch_range_collect_dense(const float* scores, int64_t ld, int64_t n, int n
 int launch_range_emit(uint64_t* items, uint64_t* items2, int64_t nq, const int64_t* src_off, const int64_t* lims,
                       int n_seg, int64_t longest, int64_t total_long, const int64_t* tab, int64_t id_offset, float* D,
                       int64_t* I, cudaStream_t st);
+// multi.cu — merges of a multi-device index's shard results on the home device (shard buffers read in place, through
+// peer pointers)
+constexpr int kMaxShards = 16;
+// D_sh[s] / I_sh[s]: shard s's top-k [nq, k] (local ids, padding id -1).  Out: the global top-k [nq, k] with global
+// ids + id_offset, padding (-FLT_MAX, -1).  ws: workspace of multi_merge_ws_bytes(G, k, nq) bytes (may be null if 0).
+size_t multi_merge_ws_bytes(int G, int k, int64_t nq);
+int launch_multi_merge(const float* const* D_sh, const int64_t* const* I_sh, int G, int64_t nq, int k, int64_t id_offset,
+                       float* D_out, int64_t* I_out, void* ws, cudaStream_t st);
+// D_sh[s] / I_sh[s]: shard s's range result (local ids) with lims lims_sh [G, nq + 1] (device); glims [nq + 1] (device)
+// the global lims; max_n the largest shard total.  Out: the global result, (score desc, id asc) per query.
+int launch_multi_range_merge(const float* const* D_sh, const int64_t* const* I_sh, const int64_t* lims_sh,
+                             const int64_t* glims, int G, int64_t nq, int64_t max_n, int64_t id_offset, float* D_out,
+                             int64_t* I_out, cudaStream_t st);
+
 // pool.cu
 int launch_pool_normalize(const void* hidden, const void* mask, float* out, void* out_lp, float* pooled_norm,
                           int64_t B, int64_t S, int64_t H, int64_t sb, int64_t ss, int64_t mb,

@@ -74,25 +74,6 @@ __device__ __forceinline__ int ld_acquire_sys(const int* p) {
     return v;
 }
 
-// (key, id) total order of the result lists: larger key first, then lower id
-__device__ __forceinline__ bool item_before(uint32_t ka, int64_t ia, uint32_t kb, int64_t ib) {
-    return (ka > kb) || (ka == kb && ia < ib);
-}
-
-// number of items of the sorted list (keys[0..n), ids[0..n)) that come before (key, id)
-__device__ __forceinline__ int count_before(const uint32_t* keys, const int64_t* ids, int n, uint32_t key, int64_t id) {
-    int lo = 0, hi = n;
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (item_before(keys[mid], ids[mid], key, id)) lo = mid + 1; else hi = mid;
-    }
-    return lo;
-}
-
-__device__ __forceinline__ void group_barrier(int id, int n_threads) {
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n_threads) : "memory");
-}
-
 constexpr int kExchangeThreads = 512;
 
 // Advances the epoch ON THE DEVICE (one thread) and clears the flag word of the new parity.  The epoch only has to
@@ -197,14 +178,11 @@ __global__ void __launch_bounds__(kExchangeThreads, 2) exchange_merge_kernel(con
     const int gt = threadIdx.x - grp * gthreads;
     int* n_valid = n_valid_all[grp];
     if (a.tree) {
-        // Pairwise merge tree (log2 G rounds): two sorted lists are merged by giving every element the rank
-        // "own position + number of elements of the sibling list that precede it" (one binary search) and
-        // keeping ranks < k — the top-k of a union is in the union of the top-k's, so truncating after
-        // every round is exact.  O(G k log k) steps per query instead of O(G^2 k log k).
+        // pairwise merge tree (common.cuh::merge_tree): O(G k log k) steps per query instead of O(G^2 k log k)
         int64_t* ids_buf = reinterpret_cast<int64_t*>(xsmem) + (size_t)grp * 2 * L;                               // [2][L]
         uint32_t* keys_buf = reinterpret_cast<uint32_t*>(reinterpret_cast<int64_t*>(xsmem) + (size_t)n_groups * 2 * L) +
                              (size_t)grp * 2 * L;                                                                    // [2][L]
-        int* nv[2] = {n_valid, n_valid + kMaxRanks};
+        int* const nv[2] = {n_valid, n_valid + kMaxRanks};
         for (int64_t q = q_lo + grp; q < q_hi; q += n_groups) {
             if (gt < G) nv[0][gt] = 0;
             group_barrier(1 + grp, gthreads);
@@ -219,32 +197,7 @@ __global__ void __launch_bounds__(kExchangeThreads, 2) exchange_merge_kernel(con
                 if (key != 0u) atomicAdd(&nv[0][g], 1);  // valid items form a prefix of each list
             }
             group_barrier(1 + grp, gthreads);
-            int cur = 0;
-            for (int n_lists = G; n_lists > 1; n_lists = (n_lists + 1) >> 1) {
-                const uint32_t* kin = keys_buf + (size_t)cur * L;
-                const int64_t* iin = ids_buf + (size_t)cur * L;
-                uint32_t* kout = keys_buf + (size_t)(cur ^ 1) * L;
-                int64_t* iout = ids_buf + (size_t)(cur ^ 1) * L;
-                const int* nin = nv[cur];
-                int* nout = nv[cur ^ 1];
-                for (int i = gt; i < n_lists * k; i += gthreads) {
-                    const int l = i / k, j = i - l * k;
-                    const int mate = l ^ 1;
-                    const int n_own = nin[l];
-                    const int n_mate = (mate < n_lists) ? nin[mate] : 0;
-                    if (j == 0 && (l & 1) == 0) nout[l >> 1] = (n_own + n_mate < k) ? (n_own + n_mate) : k;
-                    if (j >= n_own) continue;
-                    const uint32_t key = kin[i];
-                    const int64_t id = iin[i];
-                    const int r = j + (n_mate ? count_before(kin + mate * k, iin + mate * k, n_mate, key, id) : 0);
-                    if (r < k) {
-                        kout[(l >> 1) * k + r] = key;
-                        iout[(l >> 1) * k + r] = id;
-                    }
-                }
-                group_barrier(1 + grp, gthreads);
-                cur ^= 1;
-            }
+            const int cur = merge_tree(keys_buf, ids_buf, nv, G, k, gt, gthreads, 1 + grp);
             const int total = nv[cur][0];
             for (int j = gt; j < k; j += gthreads) {
                 const bool ok = j < total;

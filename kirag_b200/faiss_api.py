@@ -19,7 +19,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from typing import Optional, Tuple
+from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -45,33 +45,74 @@ def _master_flags(master: Optional[str]) -> int:
     return _lib.INDEX_HOST_MASTER if master == "host" else 0
 
 
+def _resolve_devices(device: Optional[int], devices) -> Optional[List[int]]:
+    """The device list of a multi-device index, or None for a single-device one.  devices=None reads KIRAG_DEVICES
+    (comma-separated device ids, e.g. "0,1,2,3") when no device is given either; unset means a single-device index."""
+    if devices is None and device is None:
+        env = os.environ.get("KIRAG_DEVICES")
+        if env is not None:
+            try:
+                devices = [int(v) for v in env.split(",")]
+            except ValueError:
+                raise AssertionError(f"KIRAG_DEVICES must be comma-separated device ids, got {env!r}") from None
+    if devices is None:
+        return None
+    assert device is None, "give either device or devices, not both"
+    devices = [int(v) for v in devices]
+    assert len(devices) >= 1, "devices must name at least one device"
+    assert all(v >= 0 for v in devices), f"device ids must be non-negative, got {devices}"
+    return devices
+
+
 class IndexFlatIP:
     """Exact inner-product index; corpus lives in HBM (fp32 master + bf16 shadow).  master="host" keeps the fp32 master
-    in pinned host memory instead (only the shadow in HBM), with bit-identical results."""
+    in pinned host memory instead (only the shadow in HBM), with bit-identical results.  devices=[...] stripes the rows
+    over several GPUs (repeats allowed), searched at once and merged on devices[0]; results are bit-identical to a
+    single-device index with the same rows."""
 
     metric_type = METRIC_INNER_PRODUCT
     is_trained = True
 
     def __init__(self, d: int, device: Optional[int] = None, master: Optional[str] = None,
-                 _handle: Optional[int] = None):
+                 devices: Optional[Sequence[int]] = None, _handle: Optional[int] = None):
         self._h = None
         self._pending = None
         self.last_stats: dict = {}
         self._flags = _master_flags(master)
+        self._devices = _resolve_devices(device, devices)
         self._lib = _lib.load()
+        if self._devices is not None:
+            device = self._devices[0]
+        self.device = _lib.default_device() if device is None else int(device)
         if _handle is not None:
             self._h = ctypes.c_void_p(_handle)
             self.d = int(self._lib.kirag_index_dim(self._h))
-            self.device = _lib.default_device() if device is None else int(device)
             return
         d = int(d)
         assert d > 0, "dimension must be positive"
         self.d = d
-        self.device = _lib.default_device() if device is None else int(device)
+        self._h = self._create()
+
+    def _create(self) -> ctypes.c_void_p:
         h = ctypes.c_void_p()
-        _lib.check(self._lib.kirag_index_create_ex(d, METRIC_INNER_PRODUCT, self.device, self._flags, ctypes.byref(h)),
-                   "IndexFlatIP")
-        self._h = h
+        if self._devices is None:
+            rc = self._lib.kirag_index_create_ex(self.d, METRIC_INNER_PRODUCT, self.device, self._flags, ctypes.byref(h))
+        else:
+            devs = (ctypes.c_int * len(self._devices))(*self._devices)
+            rc = self._lib.kirag_index_create_multi(self.d, METRIC_INNER_PRODUCT, devs, len(self._devices), self._flags,
+                                                    ctypes.byref(h))
+        _lib.check(rc, "IndexFlatIP")
+        return h
+
+    @property
+    def devices(self) -> List[int]:
+        """The devices of the shards, home device first ([device] for a single-device index)."""
+        return list(self._devices) if self._devices is not None else [self.device]
+
+    def _single_device(self, what: str) -> None:
+        if self._devices is not None:
+            raise RuntimeError(f"{what} is not supported on a multi-device index (no CUDA graph or asynchronous search "
+                               "across devices)")
 
     @property
     def master(self) -> str:
@@ -178,10 +219,7 @@ class IndexFlatIP:
 
     def reset(self) -> None:
         self._destroy()
-        h = ctypes.c_void_p()
-        _lib.check(self._lib.kirag_index_create_ex(self.d, METRIC_INNER_PRODUCT, self.device, self._flags,
-                                                   ctypes.byref(h)), "reset")
-        self._h = h
+        self._h = self._create()
 
     # -- device-resident entry points (additions, not part of faiss) --------
     def _own_tensor(self, t, what: str):
@@ -259,6 +297,7 @@ class IndexFlatIP:
         passed.  Call finish() (after whatever else was enqueued behind it) to complete the search."""
         import torch
 
+        self._single_device("search_device_async")
         q = self._own_tensor(q, "search_device_async")
         k = int(k)
         assert k > 0, "k must be positive"
@@ -278,6 +317,7 @@ class IndexFlatIP:
 
     def pending_flags_ptr(self) -> int:
         """Device address of the pending search's per-query certificate flags (0 if there is nothing to verify)."""
+        self._single_device("pending_flags_ptr")
         p = ctypes.c_void_p()
         _lib.check(self._lib.kirag_index_search_flags(self._h, ctypes.byref(p)), "search_flags")
         return int(p.value or 0)
@@ -285,6 +325,7 @@ class IndexFlatIP:
     def finish(self) -> int:
         """Second half of search_device_async: verifies the certificates, re-answers flagged queries in place.
         Returns the number of queries whose rows of (D, I) were rewritten."""
+        self._single_device("finish")
         stats = _lib.SearchStats()
         changed = ctypes.c_int64(0)
         _lib.check(self._lib.kirag_index_search_finish(self._h, ctypes.byref(stats), ctypes.byref(changed)), "finish")
@@ -296,6 +337,7 @@ class IndexFlatIP:
     def state_token(self) -> int:
         """Changes whenever something a captured search baked into its kernel arguments does (rows added, a workspace
         grown by a larger call): a graph is replayed only while the token is the one read after its capture."""
+        self._single_device("state_token")
         tok = ctypes.c_uint64(0)
         _lib.check(self._lib.kirag_index_state_token(self._h, ctypes.byref(tok)), "state_token")
         return int(tok.value)
@@ -307,6 +349,7 @@ class IndexFlatIP:
         (`q` to fill, `D`/`I` results), the graph, its stream and the state token."""
         import torch
 
+        self._single_device("capture_search")
         dev = torch.device("cuda", self.device)
         q = torch.nn.functional.normalize(torch.randn((nq, self.d), dtype=torch.float32, device=dev), dim=1)
         self.search_device(q, k, id_offset=id_offset)  # warm the workspaces: the capture itself must not allocate
@@ -327,6 +370,7 @@ class IndexFlatIP:
 
     def replay_search(self, cap) -> None:
         """Launch a captured search on its stream and mark it pending (finish() completes it)."""
+        self._single_device("replay_search")
         cap["graph"].replay()
         _lib.check(self._lib.kirag_index_search_rearm(self._h, ctypes.c_void_p(cap["stream"].cuda_stream)), "search_rearm")
         self._pending = (cap["q"], cap["D"], cap["I"])
@@ -337,6 +381,7 @@ class IndexFlatIP:
         next call with the same (nq, k)."""
         import torch
 
+        self._single_device("search_device_graph")
         q = self._own_tensor(q, "search_device_graph")
         key = (int(q.shape[0]), int(k), int(id_offset))
         cache = self.__dict__.setdefault("_graphs", {})
@@ -353,6 +398,7 @@ class IndexFlatIP:
 
     def debug_scores(self, x) -> np.ndarray:
         """Dense approximate (bf16 tcgen05) scores [ntotal, nq] — test hook."""
+        self._single_device("debug_scores")
         x = np.ascontiguousarray(x, dtype=np.float32)
         out = np.empty((self.ntotal, x.shape[0]), dtype=np.float32)
         _lib.check(self._lib.kirag_index_debug_scores(self._h, _ptr(x), x.shape[0], _ptr(out)), "debug_scores")
@@ -391,14 +437,21 @@ def write_index(index: IndexFlatIP, path) -> None:
     _lib.check(index._lib.kirag_index_save(index._h, os.fspath(path).encode()), "write_index")
 
 
-def read_index(path, flags: int = 0, device: Optional[int] = None, master: Optional[str] = None) -> IndexFlatIP:
-    """`flags` are FAISS IO flags (IO_FLAG_MMAP is accepted and ignored); `master` as for IndexFlatIP."""
+def read_index(path, flags: int = 0, device: Optional[int] = None, master: Optional[str] = None,
+               devices: Optional[Sequence[int]] = None) -> IndexFlatIP:
+    """`flags` are FAISS IO flags (IO_FLAG_MMAP is accepted and ignored); `master` and `devices` as for IndexFlatIP."""
     index_flags = _master_flags(master)
+    devs = _resolve_devices(device, devices)
     lib = _lib.load()
-    dev = _lib.default_device() if device is None else int(device)
     h = ctypes.c_void_p()
-    _lib.check(lib.kirag_index_load_ex(os.fspath(path).encode(), dev, index_flags, ctypes.byref(h)), "read_index")
-    return IndexFlatIP(0, device=dev, master="host" if index_flags else "device", _handle=h.value)
+    if devs is None:
+        dev = _lib.default_device() if device is None else int(device)
+        _lib.check(lib.kirag_index_load_ex(os.fspath(path).encode(), dev, index_flags, ctypes.byref(h)), "read_index")
+        return IndexFlatIP(0, device=dev, master="host" if index_flags else "device", _handle=h.value)
+    arr = (ctypes.c_int * len(devs))(*devs)
+    _lib.check(lib.kirag_index_load_multi(os.fspath(path).encode(), arr, len(devs), index_flags, ctypes.byref(h)),
+               "read_index")
+    return IndexFlatIP(0, master="host" if index_flags else "device", devices=devs, _handle=h.value)
 
 
 def omp_get_max_threads() -> int:

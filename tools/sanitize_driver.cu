@@ -3,7 +3,8 @@
 // under the tool.  Built and run by tools/sanitize.sh on the GPU box; every case checks its result against a host
 // computation, so a "passed" under the sanitizer is also a correctness pass.
 //
-//   ./sanitize_driver [case]     case = scan | search | pool | exchange | topk | host_rescore | host_exact | all (default)
+//   ./sanitize_driver [case]     case = scan | search | pool | exchange | topk | host_rescore | host_exact | multi_merge |
+//                                       all (default)
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -340,6 +341,51 @@ static void case_host_exact() {
     CK(kirag_index_destroy(h));
 }
 
+// multi-device index with three shards on device 0: the top-k merge (shared-memory and workspace variants), ids remapped
+// from the 128-row stripes, and the range merge; checked against the host answer and against a single-device index
+static void case_multi_merge() {
+    std::mt19937 rng(8);
+    const int n = 5000, d = 64, nq = 6;
+    auto xb = unit_rows(rng, n, d);
+    auto xq = unit_rows(rng, nq, d);
+    const int devs[3] = {0, 0, 0};
+    kirag_index_t* m = nullptr;
+    kirag_index_t* s = nullptr;
+    CK(kirag_index_create_multi(d, KIRAG_METRIC_INNER_PRODUCT, devs, 3, 0, &m));
+    CK(kirag_index_create(d, KIRAG_METRIC_INNER_PRODUCT, 0, &s));
+    CK(kirag_index_add(m, xb.data(), 1000, 0, nullptr));
+    CK(kirag_index_add(m, xb.data() + (size_t)1000 * d, n - 1000, 0, nullptr));
+    CK(kirag_index_add(s, xb.data(), n, 0, nullptr));
+    for (int k : {10, 2048}) {  // 2048: G*k too large for shared memory, the merge runs in its global workspace
+        std::vector<float> D((size_t)nq * k), Ds((size_t)nq * k);
+        std::vector<int64_t> I((size_t)nq * k), Is((size_t)nq * k), Ih;
+        CK(kirag_index_search_ex(m, xq.data(), nq, k, D.data(), I.data(), 0, 7, KIRAG_PATH_AUTO, nullptr, nullptr));
+        CK(kirag_index_search_ex(s, xq.data(), nq, k, Ds.data(), Is.data(), 0, 7, KIRAG_PATH_AUTO, nullptr, nullptr));
+        host_topk(xb, n, xq, nq, d, std::min(k, 10), &Ih);
+        int diff = 0, differ = 0;
+        for (int q = 0; q < nq; ++q)
+            for (int j = 0; j < std::min(k, 10); ++j) diff += I[(size_t)q * k + j] - 7 != Ih[(size_t)q * std::min(k, 10) + j];
+        for (size_t i = 0; i < I.size(); ++i) differ += I[i] != Is[i] || memcmp(&D[i], &Ds[i], 4) != 0;
+        printf("multi merge k=%d: ids vs host fp64 %d, entries differing from one device %d %s\n", k, diff, differ,
+               diff <= 1 && differ == 0 ? "ok" : "BAD");
+        if (diff > 1 || differ) exit(3);
+    }
+    std::vector<int64_t> lims(nq + 1), lims_s(nq + 1);
+    CK(kirag_index_range_search(m, xq.data(), nq, 0.2f, 0, 3, KIRAG_PATH_AUTO, lims.data(), nullptr, nullptr));
+    std::vector<float> D((size_t)lims[nq]);
+    std::vector<int64_t> I((size_t)lims[nq]);
+    CK(kirag_index_range_fetch(m, D.data(), I.data(), 0, nullptr));
+    CK(kirag_index_range_search(s, xq.data(), nq, 0.2f, 0, 3, KIRAG_PATH_AUTO, lims_s.data(), nullptr, nullptr));
+    std::vector<float> Ds((size_t)lims_s[nq]);
+    std::vector<int64_t> Is((size_t)lims_s[nq]);
+    CK(kirag_index_range_fetch(s, Ds.data(), Is.data(), 0, nullptr));
+    const bool same = lims == lims_s && I == Is && memcmp(D.data(), Ds.data(), D.size() * 4) == 0;
+    printf("multi range merge: %lld entries, equal to one device: %s\n", (long long)lims[nq], same ? "ok" : "BAD");
+    if (!same || lims[nq] == 0) exit(3);
+    CK(kirag_index_destroy(m));
+    CK(kirag_index_destroy(s));
+}
+
 int main(int argc, char** argv) {
     const std::string which = argc > 1 ? argv[1] : "all";
     if (which == "scan" || which == "all") case_scan();
@@ -349,6 +395,7 @@ int main(int argc, char** argv) {
     if (which == "topk" || which == "all") case_topk();
     if (which == "host_rescore" || which == "all") case_host_rescore();
     if (which == "host_exact" || which == "all") case_host_exact();
+    if (which == "multi_merge" || which == "all") case_multi_merge();
     CU(cudaDeviceSynchronize());
     printf("sanitize_driver %s: passed\n", which.c_str());
     return 0;
