@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define KIRAG_ABI_VERSION 9
+#define KIRAG_ABI_VERSION 10
 
 /* metric ids; only inner product is implemented, as only inner product is
  * ever constructed by the reference (retrieve.py:112, faiss_index_corpus.py:29) */
@@ -137,8 +137,8 @@ int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_
  * worker thread per shard, started here and joined by kirag_index_destroy: a call hands every shard its part, all
  * shards run at once (each on its own stream), the calling thread waits for them and merges.  Results are bit-identical
  * to a single-device index with the same rows.
- * Accepted: add, ntotal, dim, reserve, search, search_ex, range_search, range_fetch, reconstruct, save, storage_bytes
- * (summed over shards), destroy.  An error: search_async, search_finish, search_flags, search_rearm, state_token (no CUDA
+ * Accepted: add, remove_ids, remove_range, ntotal, dim, reserve, search, search_ex, range_search, range_fetch,
+ * reconstruct, save, storage_bytes (summed over shards), destroy.  An error: search_async, search_finish, search_flags, search_rearm, state_token (no CUDA
  * graph across devices), device_ptrs, debug_scores. */
 int kirag_index_create_multi(int d, int metric, const int* devices, int n_devices, int flags, kirag_index_t** out);
 
@@ -166,6 +166,28 @@ int kirag_index_reserve(kirag_index_t* h, int64_t n_total);
  * x: row-major float32 [n, d]; host pointer (x_is_device == 0) or device
  * pointer on the index's device.  Rows get implicit ids ntotal .. ntotal+n-1. */
 int kirag_index_add(kirag_index_t* h, const float* x, int64_t n, int x_is_device, void* stream);
+
+/* index.remove_ids(x)                       (faiss IndexFlatCodes::remove_ids; no reference call site)
+ * Removes every row whose id is selected; the remaining rows move down and keep their order, so the id of every row
+ * after a removed one shifts.  *n_removed (may be NULL) = rows removed.  remove_ids: the n_ids ids of a HOST array;
+ * ids < 0 or >= ntotal select nothing, a repeated id is removed once.  remove_range: the ids imin <= id < imax.
+ * The rows are compacted in place on the device (the work is proportional to the rows after the first removed one);
+ * storage stays mapped.  The norm maxima and the centre measured over the larger row set are kept (valid bounds for a
+ * subset); an index left empty returns to a fresh index's state.  A pending asynchronous search is completed first and
+ * a held range-search result is dropped; the state token changes with ntotal.  Synchronous.  Single-device,
+ * host-master and multi-device handles.  A failure part-way (a CUDA error) leaves the index holding a prefix of the
+ * kept rows. */
+int kirag_index_remove_ids(kirag_index_t* h, const int64_t* ids, int64_t n_ids, int64_t* n_removed, void* stream);
+int kirag_index_remove_range(kirag_index_t* h, int64_t imin, int64_t imax, int64_t* n_removed, void* stream);
+
+/* Test hook (host only, no device needed): the piece plan of a removal from an index of ntotal rows over G shards
+ * (d columns) whose 128-row groups keep kept_counts[(ntotal + 127) / 128] rows and whose first removed row is
+ * first_removed.  budget_rows: new rows per piece, a multiple of 128 G (<= 0: the library's staging budget).
+ * summary_out[5] = {rows removed, first rewritten row (first_removed, or ntotal if nothing is removed), new ntotal,
+ * number of pieces, budget}; pieces_out[4 i ..] = {j0, j1, i0, i1} of the first max_pieces pieces: new rows [j0, j1)
+ * gathered from the old rows [i0, i1). */
+int kirag_debug_remove_plan(const int32_t* kept_counts, int64_t ntotal, int64_t first_removed, int G, int d,
+                            int64_t budget_rows, int64_t* summary_out, int64_t* pieces_out, int64_t max_pieces);
 
 /* index.ntotal                              retriever/index.py:74,79 */
 int64_t kirag_index_ntotal(const kirag_index_t* h);

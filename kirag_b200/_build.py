@@ -14,7 +14,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(HERE, "libkirag_b200.so")
-SOURCES = ["api.cu", "convert.cu", "scan_exact.cu", "rescore.cu", "select.cu", "pool.cu", "scan_tc.cu", "exchange.cu", "range.cu", "multi.cu"]
+SOURCES = ["api.cu", "convert.cu", "scan_exact.cu", "rescore.cu", "select.cu", "pool.cu", "scan_tc.cu", "exchange.cu", "range.cu", "multi.cu", "compact.cu"]
 HEADERS = ["common.cuh", os.path.join("..", "..", "include", "kirag_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

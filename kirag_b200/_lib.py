@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("KIRAG_B200_LIB") or os.path.join(HERE, "libkirag_b200.so")
 
 # constants mirrored from the header
-ABI_VERSION = 9
+ABI_VERSION = 10
 INDEX_HOST_MASTER = 1
 METRIC_INNER_PRODUCT = 0
 METRIC_L2 = 1
@@ -68,6 +68,10 @@ SIGNATURES = {
     "kirag_index_destroy": (c_int, [c_void_p]),
     "kirag_index_reserve": (c_int, [c_void_p, c_int64]),
     "kirag_index_add": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p]),
+    "kirag_index_remove_ids": (c_int, [c_void_p, c_void_p, c_int64, POINTER(c_int64), c_void_p]),
+    "kirag_index_remove_range": (c_int, [c_void_p, c_int64, c_int64, POINTER(c_int64), c_void_p]),
+    "kirag_debug_remove_plan": (c_int, [c_void_p, c_int64, c_int64, c_int, c_int, c_int64, c_void_p, c_void_p,
+                                        c_int64]),
     "kirag_index_ntotal": (c_int64, [c_void_p]),
     "kirag_index_dim": (c_int, [c_void_p]),
     "kirag_index_search": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_int, c_int64, c_void_p]),

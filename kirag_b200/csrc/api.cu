@@ -454,6 +454,9 @@ struct kirag_index {
     DevBuf ritems, ritems2, rcount, rcursor, roff, rtab, rD, rI;
     int64_t range_n = 0;
     bool range_valid = false;
+    // row removal (kirag_index_remove_ids / _range), on the home device of a multi-device index: the id list, the
+    // removal bitmap, the kept count and the first new row of every 128-row group, the staging of the gathered rows
+    DevBuf rm_ids, rm_bits, rm_kept, rm_base, rm_stage;
 };
 
 static int64_t round_up(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
@@ -1671,6 +1674,17 @@ static int finalize_rows(kirag_index* h, int64_t r0, int64_t n, const float* src
     return 0;
 }
 
+// Returns a single-device index to a fresh index's state: no rows, centre undecided, norm maxima zero.  Storage and
+// workspaces stay mapped.
+static int forget_rows(kirag_index* h, cudaStream_t st) {
+    h->ntotal = 0;
+    h->maxnorm = h->maxerr = h->maxnorm_x = h->center_norm = 0.f;
+    h->center_decided = false;
+    if (h->center) { cudaFree(h->center); h->center = nullptr; }
+    KIRAG_CUDA_OK(cudaMemsetAsync(h->maxnorm2_bits, 0, 12, st));
+    return 0;
+}
+
 // ------------------------------------------------------------ multi-device index ----
 // kirag_index_create_multi: G shard indexes, rows striped over them (common.cuh::stripe_*), one persistent worker
 // thread per shard.  A call hands one job to every worker; each makes the ordinary single-device call on its shard on
@@ -1874,6 +1888,136 @@ static int multi_reconstruct(const kirag_index* h, int64_t i0, int64_t n, float*
                 return 0;
             })) return 1;
     }
+    return 0;
+}
+
+// ------------------------------------------------------------ row removal ----
+// kirag_index_remove_ids / _range (DESIGN.md, "Row removal"): FAISS's IndexFlatCodes::remove_ids, the kept rows move
+// down in order.  Rows below the first removed row r_min keep their id, shard and local row, so only the new rows
+// [r_min, ntotal') are written.  A removal bitmap and the kept count of every 128-row group are built on the (home)
+// device; from the counts the host plans pieces of new rows, each gathered densely from the shard masters into a
+// staging buffer (compact.cu) and appended through the ordinary add path after the index has been truncated to r_min
+// rows.  In place is safe: a kept old row i becomes new row rank(i) <= i and new row j lands where old row j
+// lived, so a piece writes only rows below the sources of every later piece.
+struct RemovePiece { int64_t j0, j1, i0, i1; };  // new rows [j0, j1) come from the old rows [i0, i1)
+struct RemovePlan {
+    int64_t n_removed = 0, j_start = 0, n_new = 0;
+    std::vector<RemovePiece> pieces;
+};
+
+// new rows per piece: about kStageBytes of staging, whole stripe rounds (128 G rows)
+static int64_t remove_piece_rows(int G, int d) {
+    const int64_t R = (int64_t)kStripeRows * G;
+    const int64_t b = (int64_t)(kStageBytes / ((size_t)d * 4)) / R * R;
+    return b < R ? R : b;
+}
+
+// kept[g]: kept rows of the 128-row group g of the n old rows; first_removed: the first removed row (it lies in the
+// first group with kept[g] below its size).  Every piece but the last ends on a round boundary and holds at most
+// `budget` rows (a multiple of 128 G); its source range is whole groups, from the group of new row j0 to the group of
+// new row j1 - 1.
+static void plan_removal(const int* kept, int64_t n, int G, int64_t budget, int64_t first_removed, RemovePlan* plan) {
+    const int64_t ng = (n + kTileRows - 1) / kTileRows, R = (int64_t)kStripeRows * G;
+    auto group_rows = [&](int64_t g) { return n - g * kTileRows < kTileRows ? n - g * kTileRows : (int64_t)kTileRows; };
+    plan->pieces.clear();
+    int64_t t0 = 0, n_new = 0;
+    while (t0 < ng && kept[t0] == group_rows(t0)) ++t0;
+    for (int64_t g = 0; g < ng; ++g) n_new += kept[g];
+    plan->n_new = n_new;
+    plan->n_removed = n - n_new;
+    plan->j_start = t0 < ng ? first_removed : n;
+    int64_t g = t0, base = t0 * kTileRows;  // base: kept rows of the groups before g
+    for (int64_t j0 = plan->j_start; j0 < n_new;) {
+        int64_t j1 = (j0 + budget) / R * R;
+        if (j1 > n_new) j1 = n_new;
+        while (base + kept[g] <= j0) base += kept[g++];
+        const int64_t g_lo = g;
+        while (base + kept[g] < j1) base += kept[g++];
+        plan->pieces.push_back({j0, j1, g_lo * kTileRows, (g + 1) * kTileRows < n ? (g + 1) * kTileRows : n});
+        j0 = j1;
+    }
+}
+
+// The index keeps its first n rows.  Only the row count changes: storage and the certificate constants stay.
+static int truncate_rows(kirag_index* h, int64_t n) {
+    if (!h->multi) {
+        if (finish_pending(h, nullptr, nullptr)) return 1;
+        h->ntotal = n;
+        return 0;
+    }
+    MultiIndex* m = h->multi;
+    multi_drop_range(m);
+    for (int s = 0; s < m->G; ++s)
+        if (truncate_rows(m->sh[(size_t)s]->h, stripe_rows(n, s, m->G))) return 1;
+    m->ntotal = n;
+    return 0;
+}
+
+// by_range: the rows [imin, imax); else the n_ids ids of the host array ids.
+static int remove_impl(kirag_index* h, bool by_range, const int64_t* ids, int64_t n_ids, int64_t imin, int64_t imax,
+                       int64_t* n_removed, cudaStream_t st) {
+    KIRAG_CHECK(h != nullptr, "index_remove: null index");
+    KIRAG_CHECK(by_range || (n_ids >= 0 && (n_ids == 0 || ids)), "index_remove_ids: bad id list");
+    if (n_removed) *n_removed = 0;
+    const int64_t n = kirag_index_ntotal(h);
+    const int64_t lo = imin > 0 ? imin : 0, hi = imax < n ? imax : n;
+    if (n == 0 || (by_range ? lo >= hi : n_ids == 0)) return 0;
+    MultiIndex* m = h->multi;
+    const int G = m ? m->G : 1, d = h->d;
+    // the rows are about to be read: nothing may still be searching them
+    if (m) multi_drop_range(m);
+    else if (finish_pending(h, nullptr, nullptr)) return 1;
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return 1;
+    const int64_t ng = (n + kTileRows - 1) / kTileRows;
+    if (h->rm_bits.ensure((size_t)ng * 16) || h->rm_kept.ensure((size_t)ng * 4) || h->rm_base.ensure((size_t)ng * 8))
+        return 1;
+    if (!by_range) {
+        if (h->rm_ids.ensure((size_t)n_ids * 8)) return 1;
+        KIRAG_CUDA_OK(cudaMemcpyAsync(h->rm_ids.p, ids, (size_t)n_ids * 8, cudaMemcpyHostToDevice, st));
+    }
+    if (launch_removal_counts(by_range ? nullptr : h->rm_ids.as<int64_t>(), n_ids, lo, hi, n, h->rm_bits.as<uint32_t>(),
+                              h->rm_kept.as<int>(), st)) return 1;
+    std::vector<int> kept((size_t)ng);
+    KIRAG_CUDA_OK(cudaMemcpyAsync(kept.data(), h->rm_kept.p, (size_t)ng * 4, cudaMemcpyDeviceToHost, st));
+    KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    int64_t t0 = 0;
+    while (t0 < ng && kept[(size_t)t0] == (n - t0 * kTileRows < kTileRows ? n - t0 * kTileRows : kTileRows)) ++t0;
+    if (t0 == ng) return 0;  // nothing selected
+    uint32_t words[4];
+    KIRAG_CUDA_OK(cudaMemcpyAsync(words, h->rm_bits.as<uint32_t>() + t0 * 4, 16, cudaMemcpyDeviceToHost, st));
+    KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    int64_t first_removed = t0 * kTileRows;
+    for (int w = 0; w < 4; ++w) {
+        if (words[w]) { first_removed += w * 32 + __builtin_ctz(words[w]); break; }
+    }
+    const int64_t budget = remove_piece_rows(G, d);
+    RemovePlan plan;
+    plan_removal(kept.data(), n, G, budget, first_removed, &plan);
+    std::vector<int64_t> base((size_t)ng);
+    for (int64_t g = 0, acc = 0; g < ng; ++g) { base[(size_t)g] = acc; acc += kept[(size_t)g]; }
+    KIRAG_CUDA_OK(cudaMemcpyAsync(h->rm_base.p, base.data(), (size_t)ng * 8, cudaMemcpyHostToDevice, st));
+    if (h->rm_stage.ensure((size_t)budget * d * 4)) return 1;
+    ShardMasters masters{};
+    for (int s = 0; s < G; ++s) masters.p[s] = m ? m->sh[(size_t)s]->h->master : h->master;
+    if (truncate_rows(h, plan.j_start)) return 1;
+    for (const RemovePiece& p : plan.pieces) {
+        // the write-back of the previous piece has completed: add() returns with its streams synchronised
+        if (launch_gather_kept(masters, G, d, h->rm_bits.as<uint32_t>(), h->rm_base.as<int64_t>(), p.i0, p.i1, p.j0,
+                               p.j1, h->rm_stage.as<float>(), (m ? m->sh[0]->h : h)->num_sms, st)) return 1;
+        if (kirag_index_add(h, h->rm_stage.as<float>(), p.j1 - p.j0, 1, st)) return 1;
+    }
+    KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    // an index (or shard) left empty is a fresh one: rows added later decide the centre again
+    for (int s = 0; s < G; ++s) {
+        kirag_index* sh = m ? m->sh[(size_t)s]->h : h;
+        if (sh->ntotal == 0) {
+            DeviceGuard sg(sh->device);
+            if (!sg.ok || forget_rows(sh, nullptr)) return 1;
+            KIRAG_CUDA_OK(cudaStreamSynchronize(nullptr));
+        }
+    }
+    if (n_removed) *n_removed = plan.n_removed;
     return 0;
 }
 
@@ -2268,8 +2412,11 @@ int kirag_index_shards(const kirag_index_t* h, int* devices_out, int64_t* rows_o
 
 int kirag_index_destroy(kirag_index_t* h) {
     if (!h) return 0;
+    DevBuf* rm_bufs[] = {&h->rm_ids, &h->rm_bits, &h->rm_kept, &h->rm_base, &h->rm_stage};
     if (h->multi) {
         multi_destroy(h->multi);
+        DeviceGuard guard(h->device);
+        for (DevBuf* b : rm_bufs) b->release();
         delete h;
         return 0;
     }
@@ -2298,6 +2445,7 @@ int kirag_index_destroy(kirag_index_t* h) {
                       &h->D_tmp, &h->I_tmp, &h->ritems, &h->ritems2, &h->rcount, &h->rcursor, &h->roff, &h->rtab,
                       &h->rD, &h->rI};
     for (DevBuf* b : bufs) b->release();
+    for (DevBuf* b : rm_bufs) b->release();
     if (h->host_flags) cudaFreeHost(h->host_flags);
     if (h->pending_ev) cudaEventDestroy(h->pending_ev);
     delete h;
@@ -2339,6 +2487,14 @@ int kirag_index_add(kirag_index_t* h, const float* x, int64_t n, int x_is_device
     }
     KIRAG_CUDA_OK(cudaMemcpyAsync(dst, x, bytes, x_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
     return finalize_rows(h, h->ntotal, n, dst, st);
+}
+
+int kirag_index_remove_ids(kirag_index_t* h, const int64_t* ids, int64_t n_ids, int64_t* n_removed, void* stream) {
+    return remove_impl(h, false, ids, n_ids, 0, 0, n_removed, (cudaStream_t)stream);
+}
+
+int kirag_index_remove_range(kirag_index_t* h, int64_t imin, int64_t imax, int64_t* n_removed, void* stream) {
+    return remove_impl(h, true, nullptr, 0, imin, imax, n_removed, (cudaStream_t)stream);
 }
 
 int64_t kirag_index_ntotal(const kirag_index_t* h) { return h ? (h->multi ? h->multi->ntotal : h->ntotal) : -1; }
@@ -2884,6 +3040,40 @@ int kirag_debug_stripe_rows(int64_t ntotal, int G, int64_t* rows_out) {
     return 0;
 }
 
+int kirag_debug_remove_plan(const int32_t* kept_counts, int64_t ntotal, int64_t first_removed, int G, int d,
+                            int64_t budget_rows, int64_t* summary_out, int64_t* pieces_out, int64_t max_pieces) {
+    KIRAG_CHECK(ntotal >= 0 && G >= 1 && G <= kMaxShards && d > 0 && summary_out && (max_pieces == 0 || pieces_out) &&
+                    (ntotal == 0 || kept_counts),
+                "debug_remove_plan: bad argument");
+    const int64_t R = (int64_t)kStripeRows * G;
+    KIRAG_CHECK(budget_rows <= 0 || budget_rows % R == 0, "debug_remove_plan: budget %lld is not a multiple of %lld rows",
+                (long long)budget_rows, (long long)R);
+    const int64_t ng = (ntotal + kTileRows - 1) / kTileRows;
+    int64_t t0 = -1;
+    for (int64_t g = 0; g < ng; ++g) {
+        const int64_t rows = ntotal - g * kTileRows < kTileRows ? ntotal - g * kTileRows : kTileRows;
+        KIRAG_CHECK(kept_counts[g] >= 0 && kept_counts[g] <= rows, "debug_remove_plan: kept count of group %lld out of range",
+                    (long long)g);
+        if (t0 < 0 && kept_counts[g] < rows) t0 = g;
+    }
+    KIRAG_CHECK(t0 < 0 || (first_removed >= t0 * kTileRows && first_removed < (t0 + 1) * kTileRows &&
+                           first_removed < ntotal),
+                "debug_remove_plan: first removed row %lld is not in group %lld, the first with a removed row",
+                (long long)first_removed, (long long)t0);
+    RemovePlan plan;
+    const int64_t budget = budget_rows > 0 ? budget_rows : remove_piece_rows(G, d);
+    plan_removal(kept_counts, ntotal, G, budget, first_removed, &plan);
+    const int64_t np = (int64_t)plan.pieces.size();
+    const int64_t summary[5] = {plan.n_removed, plan.j_start, plan.n_new, np, budget};
+    memcpy(summary_out, summary, sizeof(summary));
+    for (int64_t i = 0; i < np && i < max_pieces; ++i) {
+        const RemovePiece& p = plan.pieces[(size_t)i];
+        const int64_t row[4] = {p.j0, p.j1, p.i0, p.i1};
+        memcpy(pieces_out + 4 * i, row, sizeof(row));
+    }
+    return 0;
+}
+
 int kirag_merge_topk(const float* D_all, const int64_t* I_all, int G, int64_t nq, int k, float* D_out,
                      int64_t* I_out, int ptrs_are_device, int device, void* stream) {
     KIRAG_CHECK(G > 0 && k > 0 && nq >= 0, "merge_topk: bad shape G=%d nq=%lld k=%d", G, (long long)nq, k);
@@ -2978,12 +3168,7 @@ int kirag_topk_ip(const float* q, int64_t nq, const float* t, int64_t nt, int d,
         }
         return 0;
     }
-    // forget the previous call's rows (capacity and workspaces stay)
-    h->ntotal = 0;
-    h->maxnorm = h->maxerr = h->maxnorm_x = h->center_norm = 0.f;
-    h->center_decided = false;
-    if (h->center) { cudaFree(h->center); h->center = nullptr; }
-    KIRAG_CUDA_OK(cudaMemsetAsync(h->maxnorm2_bits, 0, 12, st));
+    if (forget_rows(h, st)) return 1;  // the previous call's rows (capacity and workspaces stay)
     int rc = 0;
     if (nt > 0 && ptrs_are_device && (reinterpret_cast<uintptr_t>(t) & 15) == 0) {
         // device-resident candidates: the caller's matrix IS the fp32 master for the duration of this (synchronous)

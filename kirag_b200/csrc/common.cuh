@@ -385,6 +385,19 @@ int launch_multi_range_merge(const float* const* D_sh, const int64_t* const* I_s
                              const int64_t* glims, int G, int64_t nq, int64_t max_n, int64_t id_offset, float* D_out,
                              int64_t* I_out, cudaStream_t st);
 
+// compact.cu — row removal.  bits: (n_rows + 127) / 128 * 16 bytes, zeroed here, then bit r set for every removed old
+// row r: the ids in ids[0..n_ids) that lie in [0, n_rows), or with ids == null the rows [lo, hi) (0 <= lo <= hi <=
+// n_rows).  kept [(n_rows + 127) / 128]: rows of each 128-row group that stay.
+int launch_removal_counts(const int64_t* ids, int64_t n_ids, int64_t lo, int64_t hi, int64_t n_rows, uint32_t* bits,
+                          int* kept, cudaStream_t st);
+// the fp32 master of every shard, readable from the launching device (peer access, or a mapped host master)
+struct ShardMasters { const float* p[kMaxShards]; };
+// Kept old rows of [i0, i1) whose new row number lies in [j0, j1) -> out[(new - j0) * d ...], new = group_base[i / 128]
+// (kept rows of the groups before) + kept rows before i in its group.  Old row i is read from shard stripe_shard(i, G)
+// at local row stripe_local(i, G).
+int launch_gather_kept(const ShardMasters& masters, int G, int d, const uint32_t* bits, const int64_t* group_base,
+                       int64_t i0, int64_t i1, int64_t j0, int64_t j1, float* out, int num_sms, cudaStream_t st);
+
 // pool.cu
 int launch_pool_normalize(const void* hidden, const void* mask, float* out, void* out_lp, float* pooled_norm,
                           int64_t B, int64_t S, int64_t H, int64_t sb, int64_t ss, int64_t mb,

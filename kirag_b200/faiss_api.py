@@ -6,6 +6,7 @@ Reference call sites (all in /root/reference/retriever/index.py):
     faiss.IndexPQ, METRIC_INNER_PRODUCT :21       -> exist, IndexPQ raises on construction
     index.is_trained / index.train  :30-31        -> True / no-op
     index.add(x)                    :32           -> kirag_index_add
+    index.remove_ids(x)             (no call site) -> kirag_index_remove_ids / kirag_index_remove_range
     index.search(x, k)              :47           -> kirag_index_search
     index.range_search(x, radius)   (no call site) -> kirag_index_range_search + kirag_index_range_fetch
     faiss.write_index(index, path)  :62           -> kirag_index_save   ("IxFI" container)
@@ -62,6 +63,28 @@ def _resolve_devices(device: Optional[int], devices) -> Optional[List[int]]:
     assert len(devices) >= 1, "devices must name at least one device"
     assert all(v >= 0 for v in devices), f"device ids must be non-negative, got {devices}"
     return devices
+
+
+class IDSelectorRange:
+    """faiss.IDSelectorRange: selects the ids imin <= id < imax."""
+
+    def __init__(self, imin: int, imax: int):
+        self.imin = int(imin)
+        self.imax = int(imax)
+
+
+class IDSelectorBatch:
+    """faiss.IDSelectorBatch: selects the ids of an integer array (converted and flattened like remove_ids does)."""
+
+    def __init__(self, ids):
+        self.ids = _id_array(ids)
+
+
+def _id_array(x) -> np.ndarray:
+    """An integer array-like as FAISS converts it: np.ascontiguousarray(x, dtype=np.int64), flattened."""
+    a = np.asarray(x)
+    assert a.size == 0 or a.dtype.kind in "iu", f"expected an integer array or an IDSelector, got {type(x).__name__}"
+    return np.ascontiguousarray(a, dtype=np.int64).ravel()
 
 
 class IndexFlatIP:
@@ -145,6 +168,19 @@ class IndexFlatIP:
         if n == 0:
             return
         _lib.check(self._lib.kirag_index_add(self._h, _ptr(x), n, 0, None), "add")
+
+    def remove_ids(self, x) -> int:
+        """faiss IndexFlatIP.remove_ids: removes every row whose id is selected by x (an integer array, an
+        IDSelectorBatch or an IDSelectorRange); the remaining rows move down in order, so later ids shift.  Ids < 0 or
+        >= ntotal select nothing, a repeated id counts once.  Returns the number of rows removed."""
+        n = ctypes.c_int64(0)
+        if isinstance(x, IDSelectorRange):
+            _lib.check(self._lib.kirag_index_remove_range(self._h, x.imin, x.imax, ctypes.byref(n), None), "remove_ids")
+        else:
+            ids = x.ids if isinstance(x, IDSelectorBatch) else _id_array(x)
+            _lib.check(self._lib.kirag_index_remove_ids(self._h, _ptr(ids), ids.size, ctypes.byref(n), None),
+                       "remove_ids")
+        return int(n.value)
 
     def search(self, x, k: int) -> Tuple[np.ndarray, np.ndarray]:
         x = np.ascontiguousarray(x, dtype=np.float32)

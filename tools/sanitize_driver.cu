@@ -4,7 +4,7 @@
 // computation, so a "passed" under the sanitizer is also a correctness pass.
 //
 //   ./sanitize_driver [case]     case = scan | search | pool | exchange | topk | host_rescore | host_exact | multi_merge |
-//                                       all (default)
+//                                       remove_compact | all (default)
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -386,6 +386,49 @@ static void case_multi_merge() {
     CK(kirag_index_destroy(s));
 }
 
+// row removal on small shapes: the removal bitmap (ids with duplicates and ids outside the index, and a range), the kept
+// counts and the gather kernel, on a single-device index (d = 100: the scalar gather; d = 64: the 16-byte gather) and
+// on three shards of one GPU; the rows left are checked against the host's compaction
+static void case_remove_compact() {
+    std::mt19937 rng(9);
+    for (int d : {100, 64}) {
+        for (int G : {1, 3}) {
+            const int n = 3000;
+            auto xb = unit_rows(rng, n, d);
+            kirag_index_t* h = nullptr;
+            const int devs[3] = {0, 0, 0};
+            if (G == 1) CK(kirag_index_create(d, KIRAG_METRIC_INNER_PRODUCT, 0, &h));
+            else CK(kirag_index_create_multi(d, KIRAG_METRIC_INNER_PRODUCT, devs, G, 0, &h));
+            CK(kirag_index_add(h, xb.data(), n, 0, nullptr));
+            std::vector<char> keep(n, 1);
+            std::vector<int64_t> ids = {5, 5, -2, n, 129, 2999, 1000};
+            for (int i = 1500; i < 1800; i += 3) ids.push_back(i);
+            for (int64_t i : ids)
+                if (i >= 0 && i < n) keep[(size_t)i] = 0;
+            int64_t removed = -1, want = 0;
+            for (char c : keep) want += !c;
+            CK(kirag_index_remove_ids(h, ids.data(), (int64_t)ids.size(), &removed, nullptr));
+            std::vector<float> rows;
+            for (int i = 0; i < n; ++i)
+                if (keep[(size_t)i]) rows.insert(rows.end(), xb.begin() + (size_t)i * d, xb.begin() + (size_t)(i + 1) * d);
+            // then a range, in the new ids
+            const int64_t lo = 200, hi = 700;
+            int64_t removed_r = -1;
+            CK(kirag_index_remove_range(h, lo, hi, &removed_r, nullptr));
+            rows.erase(rows.begin() + lo * d, rows.begin() + hi * d);
+            const int64_t nt = kirag_index_ntotal(h);
+            std::vector<float> got((size_t)nt * d);
+            CK(kirag_index_reconstruct(h, 0, nt, got.data(), 0, nullptr));
+            const bool ok = removed == want && removed_r == hi - lo && nt == (int64_t)(rows.size() / d) &&
+                            memcmp(got.data(), rows.data(), rows.size() * 4) == 0;
+            printf("remove compact d=%d G=%d: %lld + %lld rows removed, %lld left %s\n", d, G, (long long)removed,
+                   (long long)removed_r, (long long)nt, ok ? "ok" : "BAD");
+            if (!ok) exit(3);
+            CK(kirag_index_destroy(h));
+        }
+    }
+}
+
 int main(int argc, char** argv) {
     const std::string which = argc > 1 ? argv[1] : "all";
     if (which == "scan" || which == "all") case_scan();
@@ -396,6 +439,7 @@ int main(int argc, char** argv) {
     if (which == "host_rescore" || which == "all") case_host_rescore();
     if (which == "host_exact" || which == "all") case_host_exact();
     if (which == "multi_merge" || which == "all") case_multi_merge();
+    if (which == "remove_compact" || which == "all") case_remove_compact();
     CU(cudaDeviceSynchronize());
     printf("sanitize_driver %s: passed\n", which.c_str());
     return 0;
