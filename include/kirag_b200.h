@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define KIRAG_ABI_VERSION 10
+#define KIRAG_ABI_VERSION 11
 
 /* metric ids; only inner product is implemented, as only inner product is
  * ever constructed by the reference (retrieve.py:112, faiss_index_corpus.py:29) */
@@ -48,6 +48,14 @@ extern "C" {
                                    * HBM.  Needs the bf16 shadow (d % 64 == 0).  Rescoring reads only the rows that can
                                    * still reach the top-k over PCIe; the exact fp32 scan stages the master through HBM
                                    * in chunks.  Results are bit-identical to an index with a device master. */
+#define KIRAG_INDEX_ID_MAP 16     /* faiss.IndexIDMap over the flat index: every row carries a caller-given int64 id
+                                   * (kirag_index_add_with_ids; any value, negative and repeated ones included) kept in an
+                                   * id table on the (home) device, one int64 per row.  search / range_search return
+                                   * table[row] where the plain index returns row (order unchanged: score desc, row asc;
+                                   * padding -1 stays -1; id_offset must be 0); remove_ids / remove_range select by id
+                                   * value; save writes FAISS's "IxMp" container.  kirag_index_add is an error.  May be
+                                   * combined with KIRAG_INDEX_HOST_MASTER (the table stays in HBM).  Not a load flag:
+                                   * the file decides. */
 
 /* search path selectors for kirag_index_search_ex() */
 #define KIRAG_PATH_AUTO 0   /* tcgen05 bf16 filter scan + fp32 rescoring, certified; exact fp32 scan for uncertified queries */
@@ -121,8 +129,8 @@ int kirag_profile_read_timeline(int* tags_out, double* ms_since_first, int64_t m
  * Same as kirag_index_create_ex(d, metric, device, 0, out). */
 int kirag_index_create(int d, int metric, int device, kirag_index_t** out);
 
-/* flags: 0 or KIRAG_INDEX_HOST_MASTER.  Unknown flag bits and KIRAG_INDEX_HOST_MASTER with d % 64 != 0 are rejected
- * before any device is looked at. */
+/* flags: KIRAG_INDEX_HOST_MASTER and / or KIRAG_INDEX_ID_MAP.  Unknown flag bits and KIRAG_INDEX_HOST_MASTER with
+ * d % 64 != 0 are rejected before any device is looked at. */
 int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_t** out);
 
 /* Multi-device index: the rows are striped over n_devices shards (1 <= n_devices <= 16), 128 rows at a time: global
@@ -137,7 +145,8 @@ int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_
  * worker thread per shard, started here and joined by kirag_index_destroy: a call hands every shard its part, all
  * shards run at once (each on its own stream), the calling thread waits for them and merges.  Results are bit-identical
  * to a single-device index with the same rows.
- * Accepted: add, remove_ids, remove_range, ntotal, dim, reserve, search, search_ex, range_search, range_fetch,
+ * flags may include KIRAG_INDEX_ID_MAP: the table lives on the home device and the merges map the global rows.
+ * Accepted: add, add_with_ids, remove_ids, remove_ids_ex, remove_range, id_map, flags, ntotal, dim, reserve, search, search_ex, range_search, range_fetch,
  * reconstruct, save, storage_bytes (summed over shards), destroy.  An error: search_async, search_finish, search_flags, search_rearm, state_token (no CUDA
  * graph across devices), device_ptrs, debug_scores. */
 int kirag_index_create_multi(int d, int metric, const int* devices, int n_devices, int flags, kirag_index_t** out);
@@ -156,6 +165,9 @@ int kirag_debug_stripe_map(int G, const int64_t* global_ids, int64_t n, int* sha
                            int64_t* global_out);
 int kirag_debug_stripe_rows(int64_t ntotal, int G, int64_t* rows_out);
 
+/* The KIRAG_INDEX_* flags of a handle (what it was created or loaded with); -1 on a null handle. */
+int kirag_index_flags(const kirag_index_t* h);
+
 /* destructor of the faiss index object */
 int kirag_index_destroy(kirag_index_t* h);
 
@@ -166,6 +178,12 @@ int kirag_index_reserve(kirag_index_t* h, int64_t n_total);
  * x: row-major float32 [n, d]; host pointer (x_is_device == 0) or device
  * pointer on the index's device.  Rows get implicit ids ntotal .. ntotal+n-1. */
 int kirag_index_add(kirag_index_t* h, const float* x, int64_t n, int x_is_device, void* stream);
+
+/* index.add_with_ids(x, ids)                (faiss IndexIDMap::add_with_ids; KIRAG_INDEX_ID_MAP handles only)
+ * x: float32 [n, d], ids: int64 [n], both host (ptrs_are_device == 0) or both on the (home) device.  The ids are
+ * appended to the id table, then the rows are added as kirag_index_add does.  An error on a handle without the flag. */
+int kirag_index_add_with_ids(kirag_index_t* h, const float* x, const int64_t* ids, int64_t n, int ptrs_are_device,
+                             void* stream);
 
 /* index.remove_ids(x)                       (faiss IndexFlatCodes::remove_ids; no reference call site)
  * Removes every row whose id is selected; the remaining rows move down and keep their order, so the id of every row
@@ -179,6 +197,17 @@ int kirag_index_add(kirag_index_t* h, const float* x, int64_t n, int x_is_device
  * kept rows. */
 int kirag_index_remove_ids(kirag_index_t* h, const int64_t* ids, int64_t n_ids, int64_t* n_removed, void* stream);
 int kirag_index_remove_range(kirag_index_t* h, int64_t imin, int64_t imax, int64_t* n_removed, void* stream);
+/* Same as kirag_index_remove_ids with the ids on the host (ids_are_device == 0) or on the (home) device (read on
+ * `stream`).  On a KIRAG_INDEX_ID_MAP handle these three select by id VALUE (faiss IndexIDMap::remove_ids): every row
+ * whose id is in the list, or in [imin, imax), goes, all rows of a repeated id included; the kept rows keep their ids
+ * and their order.  The batch is sorted on the device and every row binary-searches its id; the id table is compacted
+ * before the rows move. */
+int kirag_index_remove_ids_ex(kirag_index_t* h, const int64_t* ids, int64_t n_ids, int ids_are_device,
+                              int64_t* n_removed, void* stream);
+
+/* faiss.vector_to_array(index.id_map): ids of rows [i0, i0 + n) of a KIRAG_INDEX_ID_MAP handle into out (host, or the
+ * (home) device with out_is_device). */
+int kirag_index_id_map(const kirag_index_t* h, int64_t i0, int64_t n, int64_t* out, int out_is_device, void* stream);
 
 /* Test hook (host only, no device needed): the piece plan of a removal from an index of ntotal rows over G shards
  * (d columns) whose 128-row groups keep kept_counts[(ntotal + 127) / 128] rows and whose first removed row is
@@ -281,19 +310,23 @@ int kirag_index_reconstruct(const kirag_index_t* h, int64_t i0, int64_t n, float
                             int out_is_device, void* stream);
 
 /* faiss.write_index(index, path)            retriever/index.py:62
- * Writes the FAISS "IxFI" flat-index container (see DESIGN.md). */
+ * Writes the FAISS "IxFI" flat-index container, or "IxMp" (the IxFI block + the ids) for a KIRAG_INDEX_ID_MAP handle
+ * (see DESIGN.md). */
 int kirag_index_save(const kirag_index_t* h, const char* path);
 
 /* faiss.read_index(path, flags)             retriever/index.py:73
  * Same as kirag_index_load_ex(path, device, 0, out). */
 int kirag_index_load(const char* path, int device, kirag_index_t** out);
 
-/* flags as for kirag_index_create_ex (these are index flags, not FAISS IO flags).  The file format does not depend on
- * where the master lives: a file written by either kind of index loads into either kind. */
+/* flags as for kirag_index_create_ex (these are index flags, not FAISS IO flags) except KIRAG_INDEX_ID_MAP, which
+ * the file decides: IxFI gives a plain handle, IxMp over IxFI a KIRAG_INDEX_ID_MAP one.  IxM2 (IndexIDMap2), another
+ * sub-index, an id count other than ntotal and a file size that does not match are reported before any device is
+ * touched.  The file format does not depend on where the master lives: a file written by either kind of index loads
+ * into either kind. */
 int kirag_index_load_ex(const char* path, int device, int flags, kirag_index_t** out);
 
-/* Bytes of corpus storage currently mapped (device) or pinned (host): fp32 master plus bf16 shadow, workspaces not
- * counted.  Either output may be NULL. */
+/* Bytes of corpus storage currently mapped (device) or pinned (host): fp32 master plus bf16 shadow, plus the id table
+ * of a KIRAG_INDEX_ID_MAP handle (device), workspaces not counted.  Either output may be NULL. */
 int kirag_index_storage_bytes(const kirag_index_t* h, int64_t* device_bytes, int64_t* host_bytes);
 
 /* Raw device pointers of the index storage (for zero-copy integration and

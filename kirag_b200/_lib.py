@@ -16,8 +16,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("KIRAG_B200_LIB") or os.path.join(HERE, "libkirag_b200.so")
 
 # constants mirrored from the header
-ABI_VERSION = 10
+ABI_VERSION = 11
 INDEX_HOST_MASTER = 1
+INDEX_ID_MAP = 16
 METRIC_INNER_PRODUCT = 0
 METRIC_L2 = 1
 PATH_AUTO, PATH_EXACT, PATH_FAST = 0, 1, 2
@@ -68,6 +69,10 @@ SIGNATURES = {
     "kirag_index_destroy": (c_int, [c_void_p]),
     "kirag_index_reserve": (c_int, [c_void_p, c_int64]),
     "kirag_index_add": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p]),
+    "kirag_index_add_with_ids": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p]),
+    "kirag_index_flags": (c_int, [c_void_p]),
+    "kirag_index_remove_ids_ex": (c_int, [c_void_p, c_void_p, c_int64, c_int, POINTER(c_int64), c_void_p]),
+    "kirag_index_id_map": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int, c_void_p]),
     "kirag_index_remove_ids": (c_int, [c_void_p, c_void_p, c_int64, POINTER(c_int64), c_void_p]),
     "kirag_index_remove_range": (c_int, [c_void_p, c_int64, c_int64, POINTER(c_int64), c_void_p]),
     "kirag_debug_remove_plan": (c_int, [c_void_p, c_int64, c_int64, c_int, c_int, c_int64, c_void_p, c_void_p,

@@ -15,8 +15,9 @@ import types
 from . import faiss_api
 
 _EXPORTED = [
-    "IndexFlatIP", "IndexFlatL2", "IndexPQ", "IDSelectorBatch", "IDSelectorRange", "METRIC_INNER_PRODUCT", "METRIC_L2",
-    "IO_FLAG_MMAP", "IO_FLAG_READ_ONLY", "write_index", "read_index", "omp_get_max_threads", "get_num_gpus",
+    "IndexFlatIP", "IndexFlatL2", "IndexPQ", "IndexIDMap", "IDSelectorBatch", "IDSelectorRange", "METRIC_INNER_PRODUCT",
+    "METRIC_L2", "IO_FLAG_MMAP", "IO_FLAG_READ_ONLY", "write_index", "read_index", "vector_to_array",
+    "omp_get_max_threads", "get_num_gpus",
 ]
 
 

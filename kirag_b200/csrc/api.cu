@@ -415,6 +415,22 @@ struct PendingSearch {
 
 struct MultiIndex;
 
+// The id table of an index created with KIRAG_INDEX_ID_MAP: one int64 external id per global row, on the (home)
+// device, table[0, ntotal) describing the rows held.  It grows like the shadow — a reserved virtual range mapped chunk
+// by chunk, the base never moves — so a captured search keeps a valid pointer until the state token changes; without
+// the virtual-memory API it is reallocated and copied.
+struct IdTable {
+    VmBuffer vm;
+    int64_t* p = nullptr;
+    size_t bytes = 0;  // usable bytes from p
+    void release() {
+        if (vm.active()) vm.release();
+        else if (p) cudaFree(p);
+        p = nullptr;
+        bytes = 0;
+    }
+};
+
 struct kirag_index {
     MultiIndex* multi = nullptr;  // a multi-device index (kirag_index_create_multi): the shards hold everything else
     int d = 0;
@@ -457,6 +473,12 @@ struct kirag_index {
     // row removal (kirag_index_remove_ids / _range), on the home device of a multi-device index: the id list, the
     // removal bitmap, the kept count and the first new row of every 128-row group, the staging of the gathered rows
     DevBuf rm_ids, rm_bits, rm_kept, rm_base, rm_stage;
+    // KIRAG_INDEX_ID_MAP (single-device or multi-device handle; the shards of a multi-device index carry no table):
+    // the id table, and for a removal by external id the sorted selection, the sort's workspace and the staging of
+    // the compacted table
+    bool id_map = false;
+    IdTable ids;
+    DevBuf rm_sorted, rm_sort_tmp, rm_id_stage;
 };
 
 static int64_t round_up(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
@@ -468,6 +490,7 @@ static int multi_range_search(kirag_index* h, const float* q, int64_t nq, float 
                               int64_t id_offset, int path, int64_t* lims_out, kirag_search_stats_t* stats,
                               cudaStream_t st);
 static int multi_range_fetch(kirag_index* h, float* D, int64_t* I, int ptrs_are_device, cudaStream_t st);
+static int add_impl(kirag_index_t* h, const float* x, int64_t n, int x_is_device, void* stream);
 
 static int env_int(const char* name, int dflt) {
     const char* v = getenv(name);
@@ -624,6 +647,49 @@ static int index_grow(kirag_index* h, int64_t need_rows, cudaStream_t st) {
     return 0;
 }
 
+// Makes table rows [0, rows) usable (rows already there keep their ids).  Called on the (home) device.
+static int ids_grow(kirag_index* h, int64_t rows, cudaStream_t st) {
+    IdTable& t = h->ids;
+    const size_t need = (size_t)rows * 8;
+    if (need <= t.bytes) return 0;
+    const size_t want = std::max(need, t.bytes + t.bytes / 4);
+    if (!t.p && vmm_api().ok) {
+        // address space for as many rows as the devices could ever hold: a row takes at least 2 d bytes of HBM
+        size_t free_b = 0, total_b = 0;
+        const int G = h->multi ? kirag_index_shards(h, nullptr, nullptr, 0) : 1;
+        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && total_b > 0 &&
+            t.vm.reserve(h->device, ((size_t)G * (total_b / ((size_t)h->d * 2)) + kTileRows) * 8) == 0)
+            t.p = static_cast<int64_t*>(t.vm.ptr());
+        cudaGetLastError();
+    }
+    if (t.vm.active()) {
+        if (t.vm.ensure(want) && t.vm.ensure(need)) {
+            set_error("id table for %lld rows does not fit in device memory", (long long)rows);
+            return 1;
+        }
+        t.bytes = t.vm.mapped;
+        return 0;
+    }
+    int64_t* nb = nullptr;
+    KIRAG_CUDA_OK(cudaMalloc((void**)&nb, want));
+    const int64_t live = kirag_index_ntotal(h);
+    if (t.p && live > 0) {
+        if (cudaMemcpyAsync(nb, t.p, (size_t)live * 8, cudaMemcpyDeviceToDevice, st) != cudaSuccess ||
+            cudaStreamSynchronize(st) != cudaSuccess) {
+            cudaFree(nb);
+            set_error("device copy while growing the id table failed: %s", cudaGetErrorString(cudaGetLastError()));
+            return 1;
+        }
+    }
+    if (t.p) cudaFree(t.p);
+    t.p = nb;
+    t.bytes = want;
+    return 0;
+}
+
+// How the writers of I of handle h (single-device, or the home of a multi-device index) turn a row into an id.
+static IdOut out_ids(const kirag_index* h, int64_t id_offset) { return IdOut{id_offset, h->id_map ? h->ids.p : nullptr}; }
+
 // ------------------------------------------------------------ exact path ----
 // Top-k of gq <= kExactNQ queries from their dense scores (rows [0, n) of dense, leading dimension ld) into D / I:
 // row g0 + i of the output block (out_row0 + g0 + i, or qmap_dev[g0 + i] if given).
@@ -653,7 +719,7 @@ static int select_dense_topk(kirag_index* h, const float* dense, int64_t ld, int
         }
         if (launch_final(cur, cur_stride, nullptr, nullptr, cur_count, cur_count, gq, k,
                          qmap_dev ? D : D + (out_row0 + g0) * k, qmap_dev ? I : I + (out_row0 + g0) * k,
-                         id_offset, nullptr, nullptr, nullptr, nullptr, 0.f, 0.f, 0, nullptr, nullptr,
+                         out_ids(h, id_offset), nullptr, nullptr, nullptr, nullptr, 0.f, 0.f, 0, nullptr, nullptr,
                          qmap_dev ? qmap_dev + g0 : nullptr, st)) return 1;
     }
     return 0;
@@ -943,8 +1009,8 @@ static int fast_search(kirag_index* h, const float* qd, int64_t nq, int k, float
     if (fuse_tail) {
         ++levels;
         if (launch_tail_fused(h->cand.as<Cand>(), cap, h->cnt.as<int>(), cap, (int)nq, fp.kprime, h->tau.as<float>(),
-                              h->overflow.as<int>(), h->master, d, qd, h->rescored.as<float>(), k, D, I, id_offset,
-                              h->qnorm.as<float>(), h->qnorm.as<float>() + nq, qcdot, ce.a, ce.b, h->flags.as<int>(),
+                              h->overflow.as<int>(), h->master, d, qd, h->rescored.as<float>(), k, D, I,
+                              out_ids(h, id_offset), h->qnorm.as<float>(), h->qnorm.as<float>() + nq, qcdot, ce.a, ce.b, h->flags.as<int>(),
                               h->num_sms, st)) return 1;
         prof_mark(51, st);
         if (levels_out) *levels_out = levels;
@@ -959,7 +1025,7 @@ static int fast_search(kirag_index* h, const float* qd, int64_t nq, int k, float
                                         h->qnorm.as<float>() + nq, ce.a, ce.b, st)) return 1;
     prof_mark(50, st);
     if (launch_final(h->cand.as<Cand>(), cap, h->rescored.as<float>(), h->cnt.as<int>(), 0, fp.kprime,
-                     (int)nq, k, D, I, id_offset, h->tau.as<float>(), h->qnorm.as<float>(), h->qnorm.as<float>() + nq,
+                     (int)nq, k, D, I, out_ids(h, id_offset), h->tau.as<float>(), h->qnorm.as<float>(), h->qnorm.as<float>() + nq,
                      qcdot, ce.a, ce.b, check_cert, h->overflow.as<int>(), h->flags.as<int>(), nullptr, st)) return 1;
     prof_mark(51, st);
     if (levels_out) *levels_out = levels;
@@ -1036,7 +1102,7 @@ static int rescan_search(kirag_index* h, const float* qsel, const float* qnorm_a
         KIRAG_CUDA_OK(cudaMemcpyAsync(counts.data(), h->cnt.p, (size_t)nb * 4, cudaMemcpyDeviceToHost, st));
     }
     if (launch_final(h->cand.as<Cand>(), cap, h->rescored.as<float>(), h->cnt.as<int>(), 0, cap, (int)nb, k, D, I,
-                     id_offset, nullptr, nullptr, nullptr, nullptr, 0.f, 0.f, 0, nullptr, nullptr, qmap_dev, st)) return 1;
+                     out_ids(h, id_offset), nullptr, nullptr, nullptr, nullptr, 0.f, 0.f, 0, nullptr, nullptr, qmap_dev, st)) return 1;
     KIRAG_CUDA_OK(cudaStreamSynchronize(st));
     for (int64_t i = 0; i < nb; ++i)
         if (counts[(size_t)i] > cap) still_bad->push_back((int)i);
@@ -1230,6 +1296,7 @@ static int search_impl(kirag_index* h, const float* q, int64_t nq, int k, float*
     KIRAG_CHECK(k <= 2048, "search: k=%d exceeds the supported maximum of 2048", k);
     KIRAG_CHECK(nq >= 0, "search: negative nq");
     KIRAG_CHECK(path >= 0 && path <= 2, "search: unknown path %d", path);
+    KIRAG_CHECK(!(h->id_map && id_offset), "search: id_offset must be 0 on an id-map index (got %lld)", (long long)id_offset);
     if (h->multi) return multi_search(h, q, nq, k, D, I, ptrs_are_device, id_offset, path, stats, st);
     if (finish_pending(h, nullptr, nullptr)) return 1;  // an unfinished asynchronous search owns the workspaces
     if (stats) memset(stats, 0, sizeof(*stats));
@@ -1547,7 +1614,7 @@ static int range_emit_chunk(kirag_index* h, RangeChunk& rc, int64_t cq, int64_t 
     KIRAG_CUDA_OK(cudaMemcpyAsync(h->roff.p, rc.src_off.data(), (size_t)cq * 8, cudaMemcpyHostToDevice, st));
     KIRAG_CUDA_OK(cudaMemcpyAsync(h->roff.as<int64_t>() + cq, lims.data(), ((size_t)cq + 1) * 8, cudaMemcpyHostToDevice, st));
     if (launch_range_emit(h->ritems.as<uint64_t>(), h->ritems2.as<uint64_t>(), cq, h->roff.as<int64_t>(),
-                          h->roff.as<int64_t>() + cq, n_seg, longest, total_long, h->rtab.as<int64_t>(), id_offset,
+                          h->roff.as<int64_t>() + cq, n_seg, longest, total_long, h->rtab.as<int64_t>(), out_ids(h, id_offset),
                           h->rD.as<float>() + base, h->rI.as<int64_t>() + base, st)) return 1;
     KIRAG_CUDA_OK(cudaStreamSynchronize(st));  // the host vectors above are read by the copies
     return 0;
@@ -1560,6 +1627,8 @@ static int range_search_impl(kirag_index* h, const float* q, int64_t nq, float r
     KIRAG_CHECK(h != nullptr, "range_search: null index");
     KIRAG_CHECK(lims_out != nullptr, "range_search: null lims");
     KIRAG_CHECK(path >= 0 && path <= 2, "range_search: unknown path %d", path);
+    KIRAG_CHECK(!(h->id_map && id_offset), "range_search: id_offset must be 0 on an id-map index (got %lld)",
+                (long long)id_offset);
     if (h->multi) return multi_range_search(h, q, nq, radius, q_is_device, id_offset, path, lims_out, stats, st);
     if (finish_pending(h, nullptr, nullptr)) return 1;  // also drops the previous range result
     if (stats) memset(stats, 0, sizeof(*stats));
@@ -1953,14 +2022,16 @@ static int truncate_rows(kirag_index* h, int64_t n) {
     return 0;
 }
 
-// by_range: the rows [imin, imax); else the n_ids ids of the host array ids.
-static int remove_impl(kirag_index* h, bool by_range, const int64_t* ids, int64_t n_ids, int64_t imin, int64_t imax,
-                       int64_t* n_removed, cudaStream_t st) {
+// by_range: the ids [imin, imax); else the n_ids ids of the array ids (host, or the (home) device with ids_are_device).
+// The ids are row numbers, or the external ids of the id table on an id-map index.
+static int remove_impl(kirag_index* h, bool by_range, const int64_t* ids, int64_t n_ids, bool ids_are_device,
+                       int64_t imin, int64_t imax, int64_t* n_removed, cudaStream_t st) {
     KIRAG_CHECK(h != nullptr, "index_remove: null index");
     KIRAG_CHECK(by_range || (n_ids >= 0 && (n_ids == 0 || ids)), "index_remove_ids: bad id list");
     if (n_removed) *n_removed = 0;
     const int64_t n = kirag_index_ntotal(h);
-    const int64_t lo = imin > 0 ? imin : 0, hi = imax < n ? imax : n;
+    const bool by_id = h->id_map;
+    const int64_t lo = by_id ? imin : (imin > 0 ? imin : 0), hi = by_id ? imax : (imax < n ? imax : n);
     if (n == 0 || (by_range ? lo >= hi : n_ids == 0)) return 0;
     MultiIndex* m = h->multi;
     const int G = m ? m->G : 1, d = h->d;
@@ -1972,12 +2043,25 @@ static int remove_impl(kirag_index* h, bool by_range, const int64_t* ids, int64_
     const int64_t ng = (n + kTileRows - 1) / kTileRows;
     if (h->rm_bits.ensure((size_t)ng * 16) || h->rm_kept.ensure((size_t)ng * 4) || h->rm_base.ensure((size_t)ng * 8))
         return 1;
-    if (!by_range) {
+    const int64_t* ids_dev = ids;
+    if (!by_range && !ids_are_device) {
         if (h->rm_ids.ensure((size_t)n_ids * 8)) return 1;
         KIRAG_CUDA_OK(cudaMemcpyAsync(h->rm_ids.p, ids, (size_t)n_ids * 8, cudaMemcpyHostToDevice, st));
+        ids_dev = h->rm_ids.as<int64_t>();
     }
-    if (launch_removal_counts(by_range ? nullptr : h->rm_ids.as<int64_t>(), n_ids, lo, hi, n, h->rm_bits.as<uint32_t>(),
-                              h->rm_kept.as<int>(), st)) return 1;
+    if (by_id) {
+        // membership of a batch: every row binary-searches its id in the sorted selection
+        const int64_t* sel = nullptr;
+        if (!by_range) {
+            const size_t tmp = sort_ids_temp_bytes(n_ids);
+            if (h->rm_sorted.ensure((size_t)n_ids * 8) || h->rm_sort_tmp.ensure(tmp)) return 1;
+            if (launch_sort_ids(ids_dev, h->rm_sorted.as<int64_t>(), n_ids, h->rm_sort_tmp.p, tmp, st)) return 1;
+            sel = h->rm_sorted.as<int64_t>();
+        }
+        if (launch_removal_counts_by_id(h->ids.p, n, sel, n_ids, lo, hi, h->rm_bits.as<uint32_t>(), h->rm_kept.as<int>(),
+                                        st)) return 1;
+    } else if (launch_removal_counts(by_range ? nullptr : ids_dev, n_ids, lo, hi, n, h->rm_bits.as<uint32_t>(),
+                                     h->rm_kept.as<int>(), st)) return 1;
     std::vector<int> kept((size_t)ng);
     KIRAG_CUDA_OK(cudaMemcpyAsync(kept.data(), h->rm_kept.p, (size_t)ng * 4, cudaMemcpyDeviceToHost, st));
     KIRAG_CUDA_OK(cudaStreamSynchronize(st));
@@ -2000,12 +2084,21 @@ static int remove_impl(kirag_index* h, bool by_range, const int64_t* ids, int64_
     if (h->rm_stage.ensure((size_t)budget * d * 4)) return 1;
     ShardMasters masters{};
     for (int s = 0; s < G; ++s) masters.p[s] = m ? m->sh[(size_t)s]->h->master : h->master;
+    if (by_id && plan.n_new > plan.j_start) {
+        // the table follows before any row moves, so that table[0, ntotal) describes the rows held at every step
+        const int64_t moved = plan.n_new - plan.j_start;
+        if (h->rm_id_stage.ensure((size_t)moved * 8)) return 1;
+        if (launch_compact_ids(h->ids.p, h->rm_bits.as<uint32_t>(), h->rm_base.as<int64_t>(), plan.j_start, n,
+                               plan.j_start, h->rm_id_stage.as<int64_t>(), st)) return 1;
+        KIRAG_CUDA_OK(cudaMemcpyAsync(h->ids.p + plan.j_start, h->rm_id_stage.p, (size_t)moved * 8,
+                                      cudaMemcpyDeviceToDevice, st));
+    }
     if (truncate_rows(h, plan.j_start)) return 1;
     for (const RemovePiece& p : plan.pieces) {
         // the write-back of the previous piece has completed: add() returns with its streams synchronised
         if (launch_gather_kept(masters, G, d, h->rm_bits.as<uint32_t>(), h->rm_base.as<int64_t>(), p.i0, p.i1, p.j0,
                                p.j1, h->rm_stage.as<float>(), (m ? m->sh[0]->h : h)->num_sms, st)) return 1;
-        if (kirag_index_add(h, h->rm_stage.as<float>(), p.j1 - p.j0, 1, st)) return 1;
+        if (add_impl(h, h->rm_stage.as<float>(), p.j1 - p.j0, 1, st)) return 1;
     }
     KIRAG_CUDA_OK(cudaStreamSynchronize(st));
     // an index (or shard) left empty is a fresh one: rows added later decide the centre again
@@ -2091,7 +2184,7 @@ static int multi_search(kirag_index* h, const float* q, int64_t nq, int k, float
         }
         const size_t ws = multi_merge_ws_bytes(G, k, cq);
         if (ws && m->ws.ensure(ws)) return 1;
-        if (launch_multi_merge(Dsh, Ish, G, cq, k, id_offset, Dd, Id, m->ws.p, st)) return 1;
+        if (launch_multi_merge(Dsh, Ish, G, cq, k, out_ids(h, id_offset), Dd, Id, m->ws.p, st)) return 1;
         if (!ptrs_are_device) {
             KIRAG_CUDA_OK(cudaMemcpyAsync(D + q0 * k, Dd, (size_t)cq * k * 4, cudaMemcpyDeviceToHost, st));
             KIRAG_CUDA_OK(cudaMemcpyAsync(I + q0 * k, Id, (size_t)cq * k * 8, cudaMemcpyDeviceToHost, st));
@@ -2173,8 +2266,8 @@ static int multi_range_fetch(kirag_index* h, float* D, int64_t* I, int ptrs_are_
         const int64_t* Ish[kMaxShards];
         for (int s = 0; s < G; ++s) { Dsh[s] = m->sh[(size_t)s]->rD.as<float>(); Ish[s] = m->sh[(size_t)s]->rI.as<int64_t>(); }
         const int64_t* lims = m->lims_dev.as<int64_t>();
-        if (launch_multi_range_merge(Dsh, Ish, lims, lims + (size_t)G * (nq + 1), G, nq, m->range_max, m->range_id_offset,
-                                     Dd, Id, st)) return 1;
+        if (launch_multi_range_merge(Dsh, Ish, lims, lims + (size_t)G * (nq + 1), G, nq, m->range_max,
+                                     out_ids(h, m->range_id_offset), Dd, Id, st)) return 1;
         if (!ptrs_are_device) {
             KIRAG_CUDA_OK(cudaMemcpyAsync(D, Dd, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
             KIRAG_CUDA_OK(cudaMemcpyAsync(I, Id, (size_t)total * 8, cudaMemcpyDeviceToHost, st));
@@ -2272,8 +2365,8 @@ static int check_index_args(const char* what, int d, int metric, int flags) {
     KIRAG_CHECK(d > 0 && d <= 16384, "%s: unsupported dimension %d", what, d);
     KIRAG_CHECK(metric == KIRAG_METRIC_INNER_PRODUCT, "%s: only the inner-product metric is implemented (got %d)", what,
                 metric);
-    KIRAG_CHECK((flags & ~KIRAG_INDEX_HOST_MASTER) == 0, "%s: unknown flag bits 0x%x", what,
-                (unsigned)(flags & ~KIRAG_INDEX_HOST_MASTER));
+    const int known = KIRAG_INDEX_HOST_MASTER | KIRAG_INDEX_ID_MAP;
+    KIRAG_CHECK((flags & ~known) == 0, "%s: unknown flag bits 0x%x", what, (unsigned)(flags & ~known));
     // without a shadow every search would be an fp32 scan of the master over PCIe
     KIRAG_CHECK(!(flags & KIRAG_INDEX_HOST_MASTER) || scan_tc_supported(d),
                 "%s: host master needs the bf16 shadow (d %% 64 == 0, got d=%d)", what, d);
@@ -2314,6 +2407,7 @@ int kirag_index_create_ex(int d, int metric, int device, int flags, kirag_index_
     h->device = device;
     h->num_sms = num_sms;
     h->host_master = (flags & KIRAG_INDEX_HOST_MASTER) != 0;
+    h->id_map = (flags & KIRAG_INDEX_ID_MAP) != 0;
     if (cudaMalloc((void**)&h->maxnorm2_bits, 12) != cudaSuccess || cudaMemset(h->maxnorm2_bits, 0, 12) != cudaSuccess) {
         set_error("index_create: cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
         delete h;
@@ -2365,7 +2459,8 @@ int kirag_index_create_multi(int d, int metric, const int* devices, int n_device
         }
         if (!sh) { multi_destroy(m); set_error("index_create_multi: out of host memory"); return 1; }
         sh->device = devices[s];
-        if (kirag_index_create_ex(d, metric, devices[s], flags, &sh->h)) { multi_destroy(m); return 1; }
+        // the table lives with the home handle: the merges map the global rows
+        if (kirag_index_create_ex(d, metric, devices[s], flags & ~KIRAG_INDEX_ID_MAP, &sh->h)) { multi_destroy(m); return 1; }
         DeviceGuard guard(devices[s]);
         if (!guard.ok || cudaStreamCreateWithFlags(&sh->st, cudaStreamNonBlocking) != cudaSuccess) {
             set_error("index_create_multi: cudaStreamCreate on device %d failed: %s", devices[s],
@@ -2391,6 +2486,7 @@ int kirag_index_create_multi(int d, int metric, const int* devices, int n_device
     h->metric = metric;
     h->device = home;
     h->host_master = (flags & KIRAG_INDEX_HOST_MASTER) != 0;
+    h->id_map = (flags & KIRAG_INDEX_ID_MAP) != 0;
     *out = h;
     return 0;
 }
@@ -2412,11 +2508,13 @@ int kirag_index_shards(const kirag_index_t* h, int* devices_out, int64_t* rows_o
 
 int kirag_index_destroy(kirag_index_t* h) {
     if (!h) return 0;
-    DevBuf* rm_bufs[] = {&h->rm_ids, &h->rm_bits, &h->rm_kept, &h->rm_base, &h->rm_stage};
+    DevBuf* rm_bufs[] = {&h->rm_ids, &h->rm_bits, &h->rm_kept, &h->rm_base, &h->rm_stage, &h->rm_sorted, &h->rm_sort_tmp,
+                         &h->rm_id_stage};
     if (h->multi) {
         multi_destroy(h->multi);
         DeviceGuard guard(h->device);
         for (DevBuf* b : rm_bufs) b->release();
+        h->ids.release();
         delete h;
         return 0;
     }
@@ -2446,6 +2544,7 @@ int kirag_index_destroy(kirag_index_t* h) {
                       &h->rD, &h->rI};
     for (DevBuf* b : bufs) b->release();
     for (DevBuf* b : rm_bufs) b->release();
+    h->ids.release();
     if (h->host_flags) cudaFreeHost(h->host_flags);
     if (h->pending_ev) cudaEventDestroy(h->pending_ev);
     delete h;
@@ -2461,8 +2560,11 @@ int kirag_index_reserve(kirag_index_t* h, int64_t n_total) {
     return index_grow(h, n_total, 0);
 }
 
-int kirag_index_add(kirag_index_t* h, const float* x, int64_t n, int x_is_device, void* stream) {
-    KIRAG_CHECK(h != nullptr, "index_add: null index");
+}  // extern "C"
+
+// Appends rows to any handle, id-map or not (the id table, if any, is the caller's business): kirag_index_add,
+// kirag_index_add_with_ids, the write-back of a removal and the load of a multi-device index.
+static int add_impl(kirag_index_t* h, const float* x, int64_t n, int x_is_device, void* stream) {
     KIRAG_CHECK(n >= 0, "index_add: negative n");
     if (n == 0) return 0;
     KIRAG_CHECK(x != nullptr, "index_add: null data");
@@ -2489,12 +2591,67 @@ int kirag_index_add(kirag_index_t* h, const float* x, int64_t n, int x_is_device
     return finalize_rows(h, h->ntotal, n, dst, st);
 }
 
+extern "C" {
+
+int kirag_index_add(kirag_index_t* h, const float* x, int64_t n, int x_is_device, void* stream) {
+    KIRAG_CHECK(h != nullptr, "index_add: null index");
+    KIRAG_CHECK(!h->id_map, "index_add: add does not work on IndexIDMap, use add_with_ids");
+    return add_impl(h, x, n, x_is_device, stream);
+}
+
+int kirag_index_add_with_ids(kirag_index_t* h, const float* x, const int64_t* ids, int64_t n, int ptrs_are_device,
+                             void* stream) {
+    KIRAG_CHECK(h != nullptr, "index_add_with_ids: null index");
+    KIRAG_CHECK(h->id_map, "index_add_with_ids: add_with_ids not implemented for this type of index (created without "
+                           "KIRAG_INDEX_ID_MAP)");
+    KIRAG_CHECK(n >= 0, "index_add_with_ids: negative n");
+    if (n == 0) return 0;
+    KIRAG_CHECK(x != nullptr && ids != nullptr, "index_add_with_ids: null data");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!h->multi && finish_pending(h, nullptr, nullptr)) return 1;  // a pending search may still read the table
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return 1;
+    const int64_t n0 = kirag_index_ntotal(h);
+    // the table first: a failure in add leaves ids past ntotal, which describe nothing
+    if (ids_grow(h, n0 + n, st)) return 1;
+    KIRAG_CUDA_OK(cudaMemcpyAsync(h->ids.p + n0, ids, (size_t)n * 8,
+                                  ptrs_are_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
+    if (!ptrs_are_device) KIRAG_CUDA_OK(cudaStreamSynchronize(st));  // the caller may free ids on return
+    return add_impl(h, x, n, ptrs_are_device, stream);
+}
+
 int kirag_index_remove_ids(kirag_index_t* h, const int64_t* ids, int64_t n_ids, int64_t* n_removed, void* stream) {
-    return remove_impl(h, false, ids, n_ids, 0, 0, n_removed, (cudaStream_t)stream);
+    return remove_impl(h, false, ids, n_ids, false, 0, 0, n_removed, (cudaStream_t)stream);
+}
+
+int kirag_index_remove_ids_ex(kirag_index_t* h, const int64_t* ids, int64_t n_ids, int ids_are_device, int64_t* n_removed,
+                              void* stream) {
+    return remove_impl(h, false, ids, n_ids, ids_are_device != 0, 0, 0, n_removed, (cudaStream_t)stream);
 }
 
 int kirag_index_remove_range(kirag_index_t* h, int64_t imin, int64_t imax, int64_t* n_removed, void* stream) {
-    return remove_impl(h, true, nullptr, 0, imin, imax, n_removed, (cudaStream_t)stream);
+    return remove_impl(h, true, nullptr, 0, false, imin, imax, n_removed, (cudaStream_t)stream);
+}
+
+int kirag_index_id_map(const kirag_index_t* h, int64_t i0, int64_t n, int64_t* out, int out_is_device, void* stream) {
+    KIRAG_CHECK(h != nullptr && (n == 0 || out != nullptr), "index_id_map: null argument");
+    KIRAG_CHECK(h->id_map, "index_id_map: the index has no id table (created without KIRAG_INDEX_ID_MAP)");
+    const int64_t ntotal = kirag_index_ntotal(h);
+    KIRAG_CHECK(i0 >= 0 && n >= 0 && i0 + n <= ntotal, "index_id_map: rows [%lld,%lld) out of range (ntotal=%lld)",
+                (long long)i0, (long long)(i0 + n), (long long)ntotal);
+    if (n == 0) return 0;
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return 1;
+    cudaStream_t st = (cudaStream_t)stream;
+    KIRAG_CUDA_OK(cudaMemcpyAsync(out, h->ids.p + i0, (size_t)n * 8,
+                                  out_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
+    if (!out_is_device) KIRAG_CUDA_OK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+int kirag_index_flags(const kirag_index_t* h) {
+    if (!h) { set_error("index_flags: null index"); return -1; }
+    return (h->host_master ? KIRAG_INDEX_HOST_MASTER : 0) | (h->id_map ? KIRAG_INDEX_ID_MAP : 0);
 }
 
 int64_t kirag_index_ntotal(const kirag_index_t* h) { return h ? (h->multi ? h->multi->ntotal : h->ntotal) : -1; }
@@ -2533,6 +2690,8 @@ int kirag_index_search_async(kirag_index_t* h, const float* q, int64_t nq, int k
     KIRAG_CHECK(h != nullptr, "search_async: null index");
     KIRAG_CHECK(!h->multi, "search_async: not supported on a multi-device index");
     KIRAG_CHECK(k > 0 && k <= 2048, "search_async: k=%d not in [1, 2048]", k);
+    KIRAG_CHECK(!(h->id_map && id_offset), "search_async: id_offset must be 0 on an id-map index (got %lld)",
+                (long long)id_offset);
     KIRAG_CHECK(nq >= 0 && nq <= kQChunk, "search_async: nq=%lld not in [0, %lld] (split larger batches)", (long long)nq,
                 (long long)kQChunk);
     if (finish_pending(h, nullptr, nullptr)) return 1;
@@ -2589,6 +2748,7 @@ int kirag_index_state_token(const kirag_index_t* h, uint64_t* token) {
     mix((uint64_t)(uintptr_t)h->master);
     mix((uint64_t)(uintptr_t)h->shadow);
     mix((uint64_t)(uintptr_t)h->center);
+    mix((uint64_t)(uintptr_t)h->ids.p);
     uint32_t f[4];
     memcpy(&f[0], &h->maxnorm, 4); memcpy(&f[1], &h->maxerr, 4); memcpy(&f[2], &h->maxnorm_x, 4); memcpy(&f[3], &h->center_norm, 4);
     mix(((uint64_t)f[0] << 32) | f[1]);
@@ -2740,7 +2900,7 @@ int kirag_index_storage_bytes(const kirag_index_t* h, int64_t* device_bytes, int
             dev_sum += db;
             host_sum += hb;
         }
-        if (device_bytes) *device_bytes = dev_sum;
+        if (device_bytes) *device_bytes = dev_sum + (int64_t)h->ids.bytes;
         if (host_bytes) *host_bytes = host_sum;
         return 0;
     }
@@ -2748,7 +2908,7 @@ int kirag_index_storage_bytes(const kirag_index_t* h, int64_t* device_bytes, int
     size_t dev = 0;
     if (h->use_vmm) dev = (h->host_master ? 0 : h->vm_master.mapped) + h->vm_shadow.mapped;
     else dev = (h->host_master || !h->master ? 0 : (size_t)h->capacity * row_m) + (h->shadow ? (size_t)h->capacity * row_s : 0);
-    if (device_bytes) *device_bytes = (int64_t)dev;
+    if (device_bytes) *device_bytes = (int64_t)(dev + h->ids.bytes);
     if (host_bytes) *host_bytes = (int64_t)h->hm.mapped;
     return 0;
 }
@@ -2762,30 +2922,45 @@ int kirag_index_device_ptrs(const kirag_index_t* h, const float** master_f32, co
 }
 
 // ---- FAISS "IxFI" container (faiss 1.8.0 index_write.cpp: write_index_header
-//      + WRITEXBVECTOR(codes)); restated from the published format -------------
+//      + WRITEXBVECTOR(codes)) and the "IxMp" container of IndexIDMap (write_index_header, the sub-index's complete
+//      block, WRITEVECTOR(id_map)); restated from the published format -------------
 static const size_t kIoChunkRows = 65536;
-static const uint32_t kIxFI = (uint32_t)'I' | ((uint32_t)'x' << 8) | ((uint32_t)'F' << 16) | ((uint32_t)'I' << 24);
+static constexpr uint32_t fourcc(const char* c) {
+    return (uint32_t)c[0] | ((uint32_t)c[1] << 8) | ((uint32_t)c[2] << 16) | ((uint32_t)c[3] << 24);
+}
+static const uint32_t kIxFI = fourcc("IxFI"), kIxMp = fourcc("IxMp"), kIxM2 = fourcc("IxM2");
 
-static bool write_ixfi_header(FILE* f, int32_t d, int64_t ntotal) {
+// faiss write_index_header after the fourcc: d, ntotal, two dummies, is_trained, metric (inner product)
+static bool write_index_header(FILE* f, int32_t d, int64_t ntotal) {
     const int64_t dummy = (int64_t)1 << 20;
     const uint8_t trained = 1;
     const int32_t metric = 0;  // METRIC_INNER_PRODUCT
+    return fwrite(&d, 4, 1, f) == 1 && fwrite(&ntotal, 8, 1, f) == 1 && fwrite(&dummy, 8, 1, f) == 1 &&
+           fwrite(&dummy, 8, 1, f) == 1 && fwrite(&trained, 1, 1, f) == 1 && fwrite(&metric, 4, 1, f) == 1;
+}
+
+static bool write_ixfi_header(FILE* f, int32_t d, int64_t ntotal) {
     const uint64_t words = (uint64_t)ntotal * (uint64_t)d;
-    return fwrite(&kIxFI, 4, 1, f) == 1 && fwrite(&d, 4, 1, f) == 1 && fwrite(&ntotal, 8, 1, f) == 1 &&
-           fwrite(&dummy, 8, 1, f) == 1 && fwrite(&dummy, 8, 1, f) == 1 && fwrite(&trained, 1, 1, f) == 1 &&
-           fwrite(&metric, 4, 1, f) == 1 && fwrite(&words, 8, 1, f) == 1;
+    return fwrite(&kIxFI, 4, 1, f) == 1 && write_index_header(f, d, ntotal) && fwrite(&words, 8, 1, f) == 1;
+}
+
+// faiss read_index_header after the fourcc (metric_arg is read for metrics > 1)
+static bool read_index_header(FILE* f, int32_t* d, int64_t* ntotal, int32_t* metric) {
+    int64_t dummy = 0;
+    uint8_t trained = 0;
+    bool ok = fread(d, 4, 1, f) == 1 && fread(ntotal, 8, 1, f) == 1 && fread(&dummy, 8, 1, f) == 1 &&
+              fread(&dummy, 8, 1, f) == 1 && fread(&trained, 1, 1, f) == 1 && fread(metric, 4, 1, f) == 1;
+    if (ok && *metric > 1) { float arg; ok = fread(&arg, 4, 1, f) == 1; }
+    return ok;
 }
 
 // Reads the header up to the payload; 0 ok, 1 (error set) not an IxFI file or an inconsistent header.
 static int read_ixfi_header(FILE* f, const char* path, int32_t* d_out, int64_t* ntotal_out) {
-    uint32_t fourcc = 0; int32_t d = 0; int64_t ntotal = 0, dummy = 0; uint8_t trained = 0; int32_t metric = 0;
+    uint32_t fourcc = 0; int32_t d = 0; int64_t ntotal = 0; int32_t metric = 0;
     uint64_t words = 0;
-    bool ok = fread(&fourcc, 4, 1, f) == 1 && fread(&d, 4, 1, f) == 1 && fread(&ntotal, 8, 1, f) == 1 &&
-              fread(&dummy, 8, 1, f) == 1 && fread(&dummy, 8, 1, f) == 1 && fread(&trained, 1, 1, f) == 1 &&
-              fread(&metric, 4, 1, f) == 1;
+    bool ok = fread(&fourcc, 4, 1, f) == 1;
     KIRAG_CHECK(ok && fourcc == kIxFI, "index_load: %s is not an IxFI (IndexFlatIP) file (fourcc 0x%08x)", path, fourcc);
-    if (metric > 1) { float arg; ok = ok && fread(&arg, 4, 1, f) == 1; }
-    ok = ok && fread(&words, 8, 1, f) == 1;
+    ok = read_index_header(f, &d, &ntotal, &metric) && fread(&words, 8, 1, f) == 1;
     KIRAG_CHECK(ok && metric == 0 && d > 0 && ntotal >= 0 && words == (uint64_t)ntotal * (uint64_t)d,
                 "index_load: %s has an inconsistent header (d=%d ntotal=%lld metric=%d words=%llu)", path, d,
                 (long long)ntotal, metric, (unsigned long long)words);
@@ -2794,12 +2969,73 @@ static int read_ixfi_header(FILE* f, const char* path, int32_t* d_out, int64_t* 
     return 0;
 }
 
-int kirag_index_save(const kirag_index_t* h, const char* path) {
-    KIRAG_CHECK(h != nullptr && path != nullptr, "index_save: null argument");
+// The header of a file for kirag_index_load_*: an IxFI file, or an IxMp file (IndexIDMap) whose sub-index is an IxFI
+// block (*id_map = true; its id vector follows the rows).  Every check of the file is made here, before any device is
+// touched, and the file is left at the first byte of the rows.
+static int read_load_header(FILE* f, const char* path, int32_t* d_out, int64_t* ntotal_out, bool* id_map) {
+    *id_map = false;
+    uint32_t outer = 0;
+    KIRAG_CHECK(fread(&outer, 4, 1, f) == 1, "index_load: %s is empty", path);
+    KIRAG_CHECK(outer != kIxM2, "index_load: %s is an IndexIDMap2 file (IxM2), which is not supported; IndexIDMap (IxMp) "
+                                "over IndexFlatIP is", path);
+    if (outer != kIxMp) {
+        KIRAG_CHECK(fseeko(f, 0, SEEK_SET) == 0, "index_load: cannot seek in %s", path);
+        return read_ixfi_header(f, path, d_out, ntotal_out);
+    }
+    int32_t d = 0, metric = 0;
+    int64_t ntotal = 0;
+    KIRAG_CHECK(read_index_header(f, &d, &ntotal, &metric) && metric == 0 && d > 0 && ntotal >= 0,
+                "index_load: %s has an inconsistent IxMp header (d=%d ntotal=%lld metric=%d)", path, d,
+                (long long)ntotal, metric);
+    const off_t sub_at = ftello(f);
+    uint32_t sub = 0;
+    KIRAG_CHECK(fread(&sub, 4, 1, f) == 1 && sub == kIxFI,
+                "index_load: the sub-index of the IndexIDMap file %s is not an IxFI (IndexFlatIP) block (fourcc "
+                "0x%08x); only IndexIDMap over IndexFlatIP is supported", path, sub);
+    KIRAG_CHECK(fseeko(f, sub_at, SEEK_SET) == 0, "index_load: cannot seek in %s", path);
+    int32_t sd = 0;
+    int64_t sn = 0;
+    if (read_ixfi_header(f, path, &sd, &sn)) return 1;
+    KIRAG_CHECK(sd == d && sn == ntotal, "index_load: %s: the IxMp header (d=%d ntotal=%lld) and its IxFI block (d=%d "
+                                         "ntotal=%lld) disagree", path, d, (long long)ntotal, sd, (long long)sn);
+    const off_t rows_at = ftello(f);
+    const off_t ids_at = rows_at + (off_t)ntotal * d * 4;
+    uint64_t n_ids = 0;
+    KIRAG_CHECK(fseeko(f, ids_at, SEEK_SET) == 0 && fread(&n_ids, 8, 1, f) == 1,
+                "index_load: %s is truncated: no id vector after the %lld rows", path, (long long)ntotal);
+    KIRAG_CHECK(n_ids == (uint64_t)ntotal, "index_load: %s holds %llu ids for %lld rows", path,
+                (unsigned long long)n_ids, (long long)ntotal);
+    KIRAG_CHECK(fseeko(f, 0, SEEK_END) == 0, "index_load: cannot seek in %s", path);
+    const off_t size = ftello(f), want = ids_at + 8 + (off_t)ntotal * 8;
+    KIRAG_CHECK(size == want, "index_load: %s has %lld bytes; an IxMp file of %lld rows x %d has %lld", path,
+                (long long)size, (long long)ntotal, d, (long long)want);
+    KIRAG_CHECK(fseeko(f, rows_at, SEEK_SET) == 0, "index_load: cannot seek in %s", path);
+    *d_out = d;
+    *ntotal_out = ntotal;
+    *id_map = true;
+    return 0;
+}
+
+// The id vector of an IxMp file (f at its count, checked by read_load_header) into the table of h.
+static int load_ids(kirag_index* h, FILE* f, const char* path, int64_t ntotal) {
+    uint64_t n = 0;
+    KIRAG_CHECK(fread(&n, 8, 1, f) == 1 && n == (uint64_t)ntotal, "index_load: %s: reading the id count failed", path);
+    if (ntotal == 0) return 0;
     DeviceGuard guard(h->device);
     if (!guard.ok) return 1;
-    FILE* f = fopen(path, "wb");
-    KIRAG_CHECK(f != nullptr, "index_save: cannot open %s for writing", path);
+    if (ids_grow(h, ntotal, nullptr)) return 1;
+    std::vector<int64_t> buf((size_t)std::min<int64_t>(ntotal, (int64_t)1 << 20));
+    for (int64_t r = 0; r < ntotal; r += (int64_t)buf.size()) {
+        const size_t rows = (size_t)std::min<int64_t>(ntotal - r, (int64_t)buf.size());
+        KIRAG_CHECK(fread(buf.data(), 8, rows, f) == rows, "index_load: %s is truncated in its id vector", path);
+        KIRAG_CUDA_OK(cudaMemcpyAsync(h->ids.p + r, buf.data(), rows * 8, cudaMemcpyHostToDevice, nullptr));
+        KIRAG_CUDA_OK(cudaStreamSynchronize(nullptr));
+    }
+    return 0;
+}
+
+// The IxFI block of h (single- or multi-device) to f.  false: failed (error set where the cause is known).
+static bool save_ixfi(const kirag_index* h, FILE* f) {
     if (h->multi) {
         // the same bytes as a single-device index with the same rows: every shard reconstructs its part of a piece,
         // the stripes are interleaved in a pinned host buffer, the piece is written
@@ -2817,14 +3053,7 @@ int kirag_index_save(const kirag_index_t* h, const char* path) {
             ok = fwrite(buf, (size_t)h->d * 4, (size_t)rows, f) == (size_t)rows;
         }
         if (buf) cudaFreeHost(buf);
-        if (fclose(f) != 0) ok = false;
-        if (!ok) {
-            char why[512];
-            snprintf(why, sizeof(why), "%s", kirag_last_error());  // set_error writes the buffer kirag_last_error reads
-            set_error("index_save: write to %s failed: %s", path, why);
-            return 1;
-        }
-        return 0;
+        return ok;
     }
     const int32_t d = h->d;
     const int64_t ntotal = h->ntotal;
@@ -2835,9 +3064,7 @@ int kirag_index_save(const kirag_index_t* h, const char* path) {
             const size_t n_el = (size_t)((ntotal - r < (int64_t)kIoChunkRows) ? (ntotal - r) : (int64_t)kIoChunkRows) * d;
             ok = fwrite(h->master + r * d, 4, n_el, f) == n_el;
         }
-        if (fclose(f) != 0) ok = false;
-        KIRAG_CHECK(ok, "index_save: write to %s failed", path);
-        return 0;
+        return ok;
     }
     // two pinned buffers: the device -> host copy of piece i+1 runs while piece i is being written
     float* stage[2] = {nullptr, nullptr};
@@ -2879,8 +3106,41 @@ int kirag_index_save(const kirag_index_t* h, const char* path) {
         if (copied[i]) cudaEventDestroy(copied[i]);
     }
     if (st) cudaStreamDestroy(st);
+    return ok;
+}
+
+// faiss WRITEVECTOR(id_map): u64 count, then the ids of the table in row order
+static bool save_ids(const kirag_index* h, FILE* f) {
+    const int64_t ntotal = kirag_index_ntotal(h);
+    const uint64_t n = (uint64_t)ntotal;
+    if (fwrite(&n, 8, 1, f) != 1) return false;
+    std::vector<int64_t> buf((size_t)std::min<int64_t>(ntotal, (int64_t)1 << 20));
+    for (int64_t r = 0; r < ntotal; r += (int64_t)buf.size()) {
+        const size_t rows = (size_t)std::min<int64_t>(ntotal - r, (int64_t)buf.size());
+        if (kirag_index_id_map(h, r, (int64_t)rows, buf.data(), 0, nullptr)) return false;
+        if (fwrite(buf.data(), 8, rows, f) != rows) return false;
+    }
+    return true;
+}
+
+int kirag_index_save(const kirag_index_t* h, const char* path) {
+    KIRAG_CHECK(h != nullptr && path != nullptr, "index_save: null argument");
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return 1;
+    FILE* f = fopen(path, "wb");
+    KIRAG_CHECK(f != nullptr, "index_save: cannot open %s for writing", path);
+    set_error("%s", "");
+    bool ok = true;
+    if (h->id_map) ok = fwrite(&kIxMp, 4, 1, f) == 1 && write_index_header(f, h->d, kirag_index_ntotal(h));
+    ok = ok && save_ixfi(h, f);
+    if (h->id_map) ok = ok && save_ids(h, f);
     if (fclose(f) != 0) ok = false;
-    KIRAG_CHECK(ok, "index_save: write to %s failed", path);
+    if (!ok) {
+        char why[512];
+        snprintf(why, sizeof(why), "%s", kirag_last_error());  // set_error writes the buffer kirag_last_error reads
+        set_error("index_save: write to %s failed%s%s", path, why[0] ? ": " : "", why);
+        return 1;
+    }
     return 0;
 }
 
@@ -2890,7 +3150,8 @@ int kirag_index_save(const kirag_index_t* h, const char* path) {
 // for the piece that used the same buffer two pieces ago), then ONE convert pass builds the bf16 shadow.  The
 // IO_FLAG_MMAP the reference passes asks FAISS not to read the file eagerly; it has no meaning for a device-resident
 // index and is accepted and ignored.  A host-master index (flags) reads the payload straight into its pinned master
-// and streams it to the device once for the convert pass.
+// and streams it to the device once for the convert pass.  An IxMp file gives an id-map handle: the rows as above,
+// then the id vector into its table.
 int kirag_index_load(const char* path, int device, kirag_index_t** out) {
     return kirag_index_load_ex(path, device, 0, out);
 }
@@ -2898,13 +3159,19 @@ int kirag_index_load(const char* path, int device, kirag_index_t** out) {
 int kirag_index_load_ex(const char* path, int device, int flags, kirag_index_t** out) {
     KIRAG_CHECK(path != nullptr && out != nullptr, "index_load: null argument");
     *out = nullptr;
+    KIRAG_CHECK(!(flags & KIRAG_INDEX_ID_MAP), "index_load: KIRAG_INDEX_ID_MAP is not a load flag (the file decides: "
+                                               "IxMp gives an id-map index, IxFI a plain one)");
     FILE* f = fopen(path, "rb");
     KIRAG_CHECK(f != nullptr, "index_load: cannot open %s", path);
     int32_t d = 0;
     int64_t ntotal = 0;
-    if (read_ixfi_header(f, path, &d, &ntotal)) { fclose(f); return 1; }
+    bool id_map = false;
+    if (read_load_header(f, path, &d, &ntotal, &id_map)) { fclose(f); return 1; }
     kirag_index_t* h = nullptr;
-    if (kirag_index_create_ex(d, KIRAG_METRIC_INNER_PRODUCT, device, flags, &h)) { fclose(f); return 1; }
+    if (kirag_index_create_ex(d, KIRAG_METRIC_INNER_PRODUCT, device, flags | (id_map ? KIRAG_INDEX_ID_MAP : 0), &h)) {
+        fclose(f);
+        return 1;
+    }
     if (ntotal == 0) { fclose(f); *out = h; return 0; }
     DeviceGuard guard(device);
     float* stage[2] = {nullptr, nullptr};
@@ -2960,6 +3227,7 @@ int kirag_index_load_ex(const char* path, int device, int flags, kirag_index_t**
         if (finalize_rows(h, 0, ntotal, h->master, st)) break;
         rc = 0;
     } while (0);
+    if (rc == 0 && id_map && load_ids(h, f, path, ntotal)) rc = 1;
     for (int i = 0; i < 2; ++i) {
         if (stage[i]) cudaFreeHost(stage[i]);
         if (done[i]) cudaEventDestroy(done[i]);
@@ -2976,13 +3244,17 @@ int kirag_index_load_ex(const char* path, int device, int flags, kirag_index_t**
 int kirag_index_load_multi(const char* path, const int* devices, int n_devices, int flags, kirag_index_t** out) {
     KIRAG_CHECK(path != nullptr && out != nullptr, "index_load: null argument");
     *out = nullptr;
+    KIRAG_CHECK(!(flags & KIRAG_INDEX_ID_MAP), "index_load: KIRAG_INDEX_ID_MAP is not a load flag (the file decides: "
+                                               "IxMp gives an id-map index, IxFI a plain one)");
     FILE* f = fopen(path, "rb");
     KIRAG_CHECK(f != nullptr, "index_load: cannot open %s", path);
     int32_t d = 0;
     int64_t ntotal = 0;
+    bool id_map = false;
     kirag_index_t* h = nullptr;
-    if (read_ixfi_header(f, path, &d, &ntotal) ||
-        kirag_index_create_multi(d, KIRAG_METRIC_INNER_PRODUCT, devices, n_devices, flags, &h)) {
+    if (read_load_header(f, path, &d, &ntotal, &id_map) ||
+        kirag_index_create_multi(d, KIRAG_METRIC_INNER_PRODUCT, devices, n_devices,
+                                 flags | (id_map ? KIRAG_INDEX_ID_MAP : 0), &h)) {
         fclose(f);
         return 1;
     }
@@ -3006,10 +3278,11 @@ int kirag_index_load_multi(const char* path, const int* devices, int n_devices, 
             if (fread(buf, row_bytes, (size_t)rows, f) != (size_t)rows) {
                 set_error("index_load: %s is truncated", path);
                 ok = false;
-            } else if (kirag_index_add(h, buf, rows, 0, nullptr)) {
+            } else if (add_impl(h, buf, rows, 0, nullptr)) {
                 ok = false;
             }
         }
+        if (ok && id_map && load_ids(h, f, path, ntotal)) ok = false;
         if (ok) rc = 0;
     } while (0);
     if (buf) cudaFreeHost(buf);

@@ -283,6 +283,16 @@ __host__ __device__ __forceinline__ int64_t stripe_rows(int64_t n, int s, int G)
     return n / span * kStripeRows + (rem < 0 ? 0 : rem > kStripeRows ? kStripeRows : rem);
 }
 
+// ------------------------------------------------------------ result ids ---
+// Every writer of a result id I takes it through this descriptor: map[row] for an index with an id table
+// (KIRAG_INDEX_ID_MAP: the caller's external ids, FAISS's IndexIDMap), else row + offset (the row-sharded search's
+// global id).  The table is indexed by the global row; a multi-device merge maps after the stripe -> global remap.
+struct IdOut {
+    int64_t offset;
+    const int64_t* map;  // null: no id table
+};
+__device__ __forceinline__ int64_t out_id(const IdOut& o, int64_t row) { return o.map ? __ldg(o.map + row) : row + o.offset; }
+
 // ------------------------------------------------------ kernel launchers ---
 // convert.cu
 // center: corpus rows are stored as bf16(x - center) (row_cdot == nullptr); for query rows pass row_cdot to get
@@ -321,10 +331,10 @@ int launch_compact_topm(Cand* buf, int64_t stride, int* cnt, int cap, int nq, in
 // last compaction + fp32 rescoring + final sort + certificate in ONE cluster kernel (small query batches)
 int launch_tail_fused(Cand* buf, int64_t stride, int* cnt, int cap, int nq, int m, float* tau, int* overflow,
                       const float* master, int d, const float* q, float* rescored, int k, float* D, int64_t* I,
-                      int64_t id_offset, const float* qnorm, const float* qerr, const float* qcdot, float eps_a, float eps_b,
+                      IdOut ids, const float* qnorm, const float* qerr, const float* qcdot, float eps_a, float eps_b,
                       int* flags, int num_sms, cudaStream_t st);
 int launch_final(const Cand* cand, int64_t cand_stride, const float* rescored, const int* cnt,
-                 int fixed_count, int m_in, int nq, int k, float* D, int64_t* I, int64_t id_offset,
+                 int fixed_count, int m_in, int nq, int k, float* D, int64_t* I, IdOut ids,
                  const float* tau, const float* qnorm, const float* qerr, const float* qcdot, float eps_a, float eps_b,
                  int check_cert, const int* overflow, int* flags, const int* qmap, cudaStream_t st);
 int launch_merge(const float* D_all, const int64_t* I_all, int G, int64_t nq, int k, float* D_out,
@@ -364,25 +374,26 @@ int launch_range_count_dense(const float* scores, int64_t ld, int64_t n, int nq,
                              cudaStream_t st);
 int launch_range_collect_dense(const float* scores, int64_t ld, int64_t n, int nq, float radius,
                                unsigned long long* cursor, uint64_t* items, cudaStream_t st);
-// Query q's items[src_off[q] .. + lims[q+1] - lims[q]) -> D / I [lims[q], lims[q+1]) by (score desc, id asc), ids +
-// id_offset.  Segments of at most kRangeRun items: one CTA each.  The n_seg longer ones are listed in the device table
+// Query q's items[src_off[q] .. + lims[q+1] - lims[q]) -> D / I [lims[q], lims[q+1]) by (score desc, row asc), ids
+// out_id(ids, row).  Segments of at most kRangeRun items: one CTA each.  The n_seg longer ones are listed in the device table
 // tab = seg_src [n_seg] (item offset), seg_dst [n_seg] (result offset), seg_len [n_seg], seg_e0 [n_seg + 1] (prefix of
 // the lengths, total_long in all); they are sorted in items / items2 (same offsets).  Stream-ordered.
 int launch_range_emit(uint64_t* items, uint64_t* items2, int64_t nq, const int64_t* src_off, const int64_t* lims,
-                      int n_seg, int64_t longest, int64_t total_long, const int64_t* tab, int64_t id_offset, float* D,
+                      int n_seg, int64_t longest, int64_t total_long, const int64_t* tab, IdOut ids, float* D,
                       int64_t* I, cudaStream_t st);
 // multi.cu — merges of a multi-device index's shard results on the home device (shard buffers read in place, through
 // peer pointers)
 constexpr int kMaxShards = 16;
-// D_sh[s] / I_sh[s]: shard s's top-k [nq, k] (local ids, padding id -1).  Out: the global top-k [nq, k] with global
-// ids + id_offset, padding (-FLT_MAX, -1).  ws: workspace of multi_merge_ws_bytes(G, k, nq) bytes (may be null if 0).
+// D_sh[s] / I_sh[s]: shard s's top-k [nq, k] (local ids, padding id -1).  Out: the global top-k [nq, k] by (score
+// desc, global row asc), ids out_id(ids, global row), padding (-FLT_MAX, -1).  ws: workspace of multi_merge_ws_bytes(G, k, nq) bytes (may be null if 0).
 size_t multi_merge_ws_bytes(int G, int k, int64_t nq);
-int launch_multi_merge(const float* const* D_sh, const int64_t* const* I_sh, int G, int64_t nq, int k, int64_t id_offset,
+int launch_multi_merge(const float* const* D_sh, const int64_t* const* I_sh, int G, int64_t nq, int k, IdOut ids,
                        float* D_out, int64_t* I_out, void* ws, cudaStream_t st);
 // D_sh[s] / I_sh[s]: shard s's range result (local ids) with lims lims_sh [G, nq + 1] (device); glims [nq + 1] (device)
-// the global lims; max_n the largest shard total.  Out: the global result, (score desc, id asc) per query.
+// the global lims; max_n the largest shard total.  Out: the global result, (score desc, global row asc) per query,
+// ids out_id(ids, global row).
 int launch_multi_range_merge(const float* const* D_sh, const int64_t* const* I_sh, const int64_t* lims_sh,
-                             const int64_t* glims, int G, int64_t nq, int64_t max_n, int64_t id_offset, float* D_out,
+                             const int64_t* glims, int G, int64_t nq, int64_t max_n, IdOut ids, float* D_out,
                              int64_t* I_out, cudaStream_t st);
 
 // compact.cu — row removal.  bits: (n_rows + 127) / 128 * 16 bytes, zeroed here, then bit r set for every removed old
@@ -390,6 +401,17 @@ int launch_multi_range_merge(const float* const* D_sh, const int64_t* const* I_s
 // n_rows).  kept [(n_rows + 127) / 128]: rows of each 128-row group that stay.
 int launch_removal_counts(const int64_t* ids, int64_t n_ids, int64_t lo, int64_t hi, int64_t n_rows, uint32_t* bits,
                           int* kept, cudaStream_t st);
+// The same bitmap and counts for an index with an id table: old row r is removed when its id table[r] is selected —
+// with sel == null the ids lo <= id < hi, else the ids of sel[0..n_sel), sorted ascending (launch_sort_ids).
+int launch_removal_counts_by_id(const int64_t* table, int64_t n_rows, const int64_t* sel, int64_t n_sel, int64_t lo,
+                                int64_t hi, uint32_t* bits, int* kept, cudaStream_t st);
+// out[0..n) = in[0..n) sorted ascending (CUB radix sort).  temp: sort_ids_temp_bytes(n) bytes.
+size_t sort_ids_temp_bytes(int64_t n);
+int launch_sort_ids(const int64_t* in, int64_t* out, int64_t n, void* temp, size_t temp_bytes, cudaStream_t st);
+// The id table follows the rows: the id of every kept old row of [i0, n_rows) goes to out[new - j0] (new row number as
+// for launch_gather_kept).
+int launch_compact_ids(const int64_t* table, const uint32_t* bits, const int64_t* group_base, int64_t i0, int64_t n_rows,
+                       int64_t j0, int64_t* out, cudaStream_t st);
 // the fp32 master of every shard, readable from the launching device (peer access, or a mapped host master)
 struct ShardMasters { const float* p[kMaxShards]; };
 // Kept old rows of [i0, i1) whose new row number lies in [j0, j1) -> out[(new - j0) * d ...], new = group_base[i / 128]

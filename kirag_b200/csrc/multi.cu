@@ -3,7 +3,8 @@
 // place through peer pointers; no [G, nq, k] gather comes first.
 //   top-k   the G sorted [nq, k] lists are read, local ids are remapped to global ones by the stripe arithmetic
 //           (common.cuh::stripe_global) and the lists are merged by the rank-based pairwise tree
-//           (common.cuh::merge_tree, shared with the exchange of the row-sharded search);
+//           (common.cuh::merge_tree, shared with the exchange of the row-sharded search); the merged global rows are
+//           written through common.cuh::out_id (offset or id table);
 //   range   one thread per shard entry computes its global position: global lims[q] + own position + for every other
 //           shard the number of its entries of query q that precede it (one binary search each, on global ids).
 #include "common.cuh"
@@ -20,7 +21,8 @@ struct MultiMergeArgs {
     const float* D[kMaxShards];
     const int64_t* I[kMaxShards];
     int G, k, n_groups;
-    int64_t nq, id_offset;
+    int64_t nq;
+    IdOut ids;
     float* D_out;
     int64_t* I_out;
     uint8_t* ws;  // null: the lists live in shared memory
@@ -49,7 +51,7 @@ __global__ void __launch_bounds__(kMultiMergeThreads) multi_merge_kernel(const M
             uint32_t key = 0u;
             if (id >= 0) key = score_key(a.D[s][q * k + j]);
             if (key != 0u) {
-                id = stripe_global(id, s, G) + a.id_offset;
+                id = stripe_global(id, s, G);
                 atomicAdd(&nv[0][s], 1);  // valid items form a prefix of each list
             }
             keys_buf[i] = key;
@@ -65,6 +67,14 @@ __global__ void __launch_bounds__(kMultiMergeThreads) multi_merge_kernel(const M
         }
         group_barrier(1 + grp, gthreads);
     }
+    // global rows -> ids, each thread over the entries it wrote above.  A separate pass: mapping in the loop above made
+    // ptxas spill a pointer across the merge.
+    if (!a.ids.map && !a.ids.offset) return;
+    for (int64_t q = (int64_t)blockIdx.x * n_groups + grp; q < a.nq; q += (int64_t)gridDim.x * n_groups)
+        for (int j = gt; j < k; j += gthreads) {
+            const int64_t row = a.I_out[q * k + j];
+            if (row >= 0) a.I_out[q * k + j] = out_id(a.ids, row);
+        }
 }
 
 // thread groups per CTA when the two list buffers of a group fit shared memory; 0 when they do not
@@ -81,13 +91,13 @@ size_t multi_merge_ws_bytes(int G, int k, int64_t nq) {
     return (size_t)blocks * 2 * G * k * 12;
 }
 
-int launch_multi_merge(const float* const* D_sh, const int64_t* const* I_sh, int G, int64_t nq, int k, int64_t id_offset,
+int launch_multi_merge(const float* const* D_sh, const int64_t* const* I_sh, int G, int64_t nq, int k, IdOut ids,
                        float* D_out, int64_t* I_out, void* ws, cudaStream_t st) {
     KIRAG_CHECK(G >= 1 && G <= kMaxShards && k >= 1 && nq >= 0, "multi_merge: bad shape G=%d k=%d", G, k);
     if (nq == 0) return 0;
     MultiMergeArgs a{};
     for (int s = 0; s < G; ++s) { a.D[s] = D_sh[s]; a.I[s] = I_sh[s]; }
-    a.G = G; a.k = k; a.nq = nq; a.id_offset = id_offset; a.D_out = D_out; a.I_out = I_out;
+    a.G = G; a.k = k; a.nq = nq; a.ids = ids; a.D_out = D_out; a.I_out = I_out;
     const int groups = multi_merge_groups(G, k);
     size_t smem = 0;
     int64_t blocks;
@@ -116,7 +126,8 @@ struct MultiRangeArgs {
     const int64_t* lims;   // [G, nq + 1]
     const int64_t* glims;  // [nq + 1]
     int G;
-    int64_t nq, id_offset;
+    int64_t nq;
+    IdOut ids;
     float* D_out;
     int64_t* I_out;
 };
@@ -154,17 +165,17 @@ __global__ void multi_range_merge_kernel(const MultiRangeArgs a) {
         pos += count_before_shard(a, t, lt[q], lt[q + 1], key, gid);
     }
     a.D_out[pos] = score;
-    a.I_out[pos] = gid + a.id_offset;
+    a.I_out[pos] = out_id(a.ids, gid);
 }
 
 int launch_multi_range_merge(const float* const* D_sh, const int64_t* const* I_sh, const int64_t* lims_sh,
-                             const int64_t* glims, int G, int64_t nq, int64_t max_n, int64_t id_offset, float* D_out,
+                             const int64_t* glims, int G, int64_t nq, int64_t max_n, IdOut ids, float* D_out,
                              int64_t* I_out, cudaStream_t st) {
     KIRAG_CHECK(G >= 1 && G <= kMaxShards && nq >= 0 && max_n >= 0, "multi_range_merge: bad shape G=%d", G);
     if (nq == 0 || max_n == 0) return 0;
     MultiRangeArgs a{};
     for (int s = 0; s < G; ++s) { a.D[s] = D_sh[s]; a.I[s] = I_sh[s]; }
-    a.lims = lims_sh; a.glims = glims; a.G = G; a.nq = nq; a.id_offset = id_offset; a.D_out = D_out; a.I_out = I_out;
+    a.lims = lims_sh; a.glims = glims; a.G = G; a.nq = nq; a.ids = ids; a.D_out = D_out; a.I_out = I_out;
     multi_range_merge_kernel<<<dim3((unsigned)((max_n + 255) / 256), (unsigned)G), 256, 0, st>>>(a);
     KIRAG_LAUNCH_OK("multi_range_merge_kernel");
     return 0;

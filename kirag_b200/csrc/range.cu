@@ -10,7 +10,7 @@
 //                          of a flat item array; positions inside a segment are reserved with atomics, so the
 //                          segment is unordered until it is sorted below
 //   range_emit_kernel      segments of at most kRangeRun items: one CTA sorts the segment in shared memory (bitonic)
-//                          and writes D / I (row + id_offset) at the query's offset of the result
+//                          and writes D / I (out_id of the row) at the query's offset of the result
 //   longer segments        range_sort_runs_kernel sorts runs of kRangeRun items in place, range_merge_kernel merges
 //                          neighbouring runs by rank (own position + binary-search rank in the sibling run, the way
 //                          exchange.cu merges shard lists) until one run is left, range_write_kernel writes D / I
@@ -125,22 +125,22 @@ __device__ __forceinline__ void load_and_sort(uint64_t* sm, const uint64_t* src,
     bitonic_sort_desc(sm, P);
 }
 
-__device__ __forceinline__ void write_result(uint64_t it, int64_t id_offset, float* D, int64_t* I) {
+__device__ __forceinline__ void write_result(uint64_t it, const IdOut& ids, float* D, int64_t* I) {
     *D = key_score(item_key(it));
-    *I = (int64_t)item_id(it) + id_offset;
+    *I = out_id(ids, item_id(it));
 }
 
 // grid nq: the segments of at most kRangeRun items
 __global__ void __launch_bounds__(kRangeSortThreads) range_emit_kernel(const uint64_t* __restrict__ items,
                                                                        const int64_t* __restrict__ src_off,
-                                                                       const int64_t* __restrict__ lims, int64_t id_offset,
+                                                                       const int64_t* __restrict__ lims, const IdOut ids,
                                                                        float* __restrict__ D, int64_t* __restrict__ I) {
     extern __shared__ uint64_t sm[];
     const int64_t q = blockIdx.x;
     const int64_t lo = lims[q], len = lims[q + 1] - lo;
     if (len == 0 || len > kRangeRun) return;
     load_and_sort(sm, items + src_off[q], (int)len);
-    for (int j = threadIdx.x; j < (int)len; j += blockDim.x) write_result(sm[j], id_offset, D + lo + j, I + lo + j);
+    for (int j = threadIdx.x; j < (int)len; j += blockDim.x) write_result(sm[j], ids, D + lo + j, I + lo + j);
 }
 
 // grid (runs of the longest segment, long segments): run blockIdx.x of segment blockIdx.y, sorted in place
@@ -195,12 +195,12 @@ __global__ void range_merge_kernel(const uint64_t* __restrict__ src, uint64_t* _
 
 __global__ void range_write_kernel(const uint64_t* __restrict__ items, const int64_t* __restrict__ seg_src,
                                    const int64_t* __restrict__ seg_dst, const int64_t* __restrict__ seg_e0, int n_seg,
-                                   int64_t total, int64_t id_offset, float* __restrict__ D, int64_t* __restrict__ I) {
+                                   int64_t total, const IdOut ids, float* __restrict__ D, int64_t* __restrict__ I) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= total) return;
     const int s = find_segment(seg_e0, n_seg, t);
     const int64_t e = t - seg_e0[s];
-    write_result(items[seg_src[s] + e], id_offset, D + seg_dst[s] + e, I + seg_dst[s] + e);
+    write_result(items[seg_src[s] + e], ids, D + seg_dst[s] + e, I + seg_dst[s] + e);
 }
 
 // ------------------------------------------------------------------ hosts ----
@@ -264,12 +264,12 @@ int launch_range_collect_dense(const float* scores, int64_t ld, int64_t n, int n
 }
 
 int launch_range_emit(uint64_t* items, uint64_t* items2, int64_t nq, const int64_t* src_off, const int64_t* lims,
-                      int n_seg, int64_t longest, int64_t total_long, const int64_t* tab, int64_t id_offset, float* D,
+                      int n_seg, int64_t longest, int64_t total_long, const int64_t* tab, IdOut ids, float* D,
                       int64_t* I, cudaStream_t st) {
     if (nq <= 0) return 0;
     const size_t smem = (size_t)kRangeRun * sizeof(uint64_t);
     if (ensure_dynamic_smem(range_emit_kernel, smem) || ensure_dynamic_smem(range_sort_runs_kernel, smem)) return 1;
-    range_emit_kernel<<<(unsigned)nq, kRangeSortThreads, smem, st>>>(items, src_off, lims, id_offset, D, I);
+    range_emit_kernel<<<(unsigned)nq, kRangeSortThreads, smem, st>>>(items, src_off, lims, ids, D, I);
     KIRAG_LAUNCH_OK("range_emit_kernel");
     if (n_seg == 0) return 0;
     KIRAG_CHECK(n_seg <= 65535, "range_emit: %d long segments in one call", n_seg);
@@ -289,7 +289,7 @@ int launch_range_emit(uint64_t* items, uint64_t* items2, int64_t nq, const int64
         KIRAG_LAUNCH_OK("range_merge_kernel");
         uint64_t* t = cur; cur = nxt; nxt = t;
     }
-    range_write_kernel<<<blocks, 256, 0, st>>>(cur, d_src, d_dst, d_e0, n_seg, total_long, id_offset, D, I);
+    range_write_kernel<<<blocks, 256, 0, st>>>(cur, d_src, d_dst, d_e0, n_seg, total_long, ids, D, I);
     KIRAG_LAUNCH_OK("range_write_kernel");
     return 0;
 }

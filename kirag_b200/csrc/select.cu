@@ -348,7 +348,7 @@ compact_topm_kernel(Cand* __restrict__ buf, int64_t stride, int* __restrict__ cn
 // items[0..P) hold the packed (canonical score, row) pairs of query q (0 = absent); sorts them, writes row qo of
 // D / I and evaluates the certificate.  Called by all threads of a CTA.
 __device__ __forceinline__ void final_body(uint64_t* items, int P, int q, int64_t qo, int k, float* __restrict__ D,
-                                           int64_t* __restrict__ I, int64_t id_offset, const float* __restrict__ tau,
+                                           int64_t* __restrict__ I, const IdOut& ids, const float* __restrict__ tau,
                                            const float* __restrict__ qnorm, const float* __restrict__ qerr,
                                            const float* __restrict__ qcdot, float eps_a,
                                            float eps_b, int check_cert, const int* __restrict__ overflow,
@@ -359,7 +359,7 @@ __device__ __forceinline__ void final_body(uint64_t* items, int P, int q, int64_
         int64_t id = -1;
         if (j < P && item_key(items[j]) != 0u) {
             s = key_score(item_key(items[j]));
-            id = (int64_t)item_id(items[j]) + id_offset;
+            id = out_id(ids, item_id(items[j]));
         }
         D[qo * k + j] = s;
         I[qo * k + j] = id;
@@ -391,7 +391,7 @@ __device__ __forceinline__ void final_body(uint64_t* items, int P, int q, int64_
 __global__ void __launch_bounds__(1024)
 final_kernel(const Cand* __restrict__ cand, int64_t cand_stride, const float* __restrict__ rescored,
              const int* __restrict__ cnt, int fixed_count, int m_in, int k, float* __restrict__ D,
-             int64_t* __restrict__ I, int64_t id_offset, const float* __restrict__ tau,
+             int64_t* __restrict__ I, const IdOut ids, const float* __restrict__ tau,
              const float* __restrict__ qnorm, const float* __restrict__ qerr, const float* __restrict__ qcdot,
              float eps_a, float eps_b, int check_cert,
              const int* __restrict__ overflow, int* __restrict__ flags,
@@ -415,7 +415,7 @@ final_kernel(const Cand* __restrict__ cand, int64_t cand_stride, const float* __
     }
     __syncthreads();
     const int64_t qo = qmap ? qmap[q] : q;
-    final_body(items, P, q, qo, k, D, I, id_offset, tau, qnorm, qerr, qcdot, eps_a, eps_b, check_cert, overflow, flags);
+    final_body(items, P, q, qo, k, D, I, ids, tau, qnorm, qerr, qcdot, eps_a, eps_b, check_cert, overflow, flags);
 }
 
 // ---- fused tail of a small-batch search --------------------------------------------------
@@ -438,7 +438,7 @@ __global__ void __launch_bounds__(kCompactThreadsWide, 1)
 tail_fused_kernel(Cand* __restrict__ buf, int64_t stride, int* __restrict__ cnt, int cap, int m,
                   float* __restrict__ tau, int* __restrict__ overflow, const float* __restrict__ master, int d,
                   const float* __restrict__ qmat, int vec4, float* __restrict__ rescored, int k,
-                  float* __restrict__ D, int64_t* __restrict__ I, int64_t id_offset, const float* __restrict__ qnorm,
+                  float* __restrict__ D, int64_t* __restrict__ I, const IdOut ids, const float* __restrict__ qnorm,
                   const float* __restrict__ qerr, const float* __restrict__ qcdot, float eps_a, float eps_b,
                   int* __restrict__ flags) {
     __shared__ CompactSmem sm;
@@ -494,7 +494,7 @@ tail_fused_kernel(Cand* __restrict__ buf, int64_t stride, int* __restrict__ cnt,
         items[i] = it;
     }
     __syncthreads();
-    final_body(items, P, q, q, k, D, I, id_offset, tau, qnorm, qerr, qcdot, eps_a, eps_b, 1, overflow, flags);
+    final_body(items, P, q, q, k, D, I, ids, tau, qnorm, qerr, qcdot, eps_a, eps_b, 1, overflow, flags);
 }
 
 // ---- multi-GPU merge ---------------------------------------------------------
@@ -625,7 +625,7 @@ int launch_compact_topm(Cand* buf, int64_t stride, int* cnt, int cap, int nq, in
 }
 
 int launch_final(const Cand* cand, int64_t cand_stride, const float* rescored, const int* cnt,
-                 int fixed_count, int m_in, int nq, int k, float* D, int64_t* I, int64_t id_offset,
+                 int fixed_count, int m_in, int nq, int k, float* D, int64_t* I, IdOut ids,
                  const float* tau, const float* qnorm, const float* qerr, const float* qcdot, float eps_a, float eps_b,
                  int check_cert, const int* overflow, int* flags, const int* qmap, cudaStream_t st) {
     KIRAG_CHECK(m_in <= kSelectSeg, "final: m_in=%d > %d", m_in, kSelectSeg);
@@ -633,7 +633,7 @@ int launch_final(const Cand* cand, int64_t cand_stride, const float* rescored, c
     const size_t smem = (size_t)P * 8;
     if (ensure_smem(final_kernel, (size_t)kSelectSeg * 8)) return 1;
     KIRAG_CUDA_OK(launch_chained(final_kernel, dim3((unsigned)nq), dim3(sort_threads(P)), smem, st, cand, cand_stride,
-                                 rescored, cnt, fixed_count, m_in, k, D, I, id_offset, tau, qnorm, qerr, qcdot, eps_a, eps_b,
+                                 rescored, cnt, fixed_count, m_in, k, D, I, ids, tau, qnorm, qerr, qcdot, eps_a, eps_b,
                                  check_cert, overflow, flags, qmap));
     KIRAG_LAUNCH_OK("final_kernel");
     return 0;
@@ -641,7 +641,7 @@ int launch_final(const Cand* cand, int64_t cand_stride, const float* rescored, c
 
 int launch_tail_fused(Cand* buf, int64_t stride, int* cnt, int cap, int nq, int m, float* tau, int* overflow,
                       const float* master, int d, const float* q, float* rescored, int k, float* D, int64_t* I,
-                      int64_t id_offset, const float* qnorm, const float* qerr, const float* qcdot, float eps_a, float eps_b,
+                      IdOut ids, const float* qnorm, const float* qerr, const float* qcdot, float eps_a, float eps_b,
                       int* flags, int num_sms, cudaStream_t st) {
     KIRAG_CHECK(cap <= kWideCap && m <= cap && m <= kTailMaxM, "tail_fused: cap=%d m=%d out of range", cap, m);
     if (nq <= 0) return 0;
@@ -665,7 +665,7 @@ int launch_tail_fused(Cand* buf, int64_t stride, int* cnt, int cap, int nq, int 
     cfg.attrs = attr;
     cfg.numAttrs = pdl_enabled() ? 2 : 1;
     KIRAG_CUDA_OK(cudaLaunchKernelEx(&cfg, tail_fused_kernel, buf, stride, cnt, cap, m, tau, overflow, master, d, q, vec4,
-                                     rescored, k, D, I, id_offset, qnorm, qerr, qcdot, eps_a, eps_b, flags));
+                                     rescored, k, D, I, ids, qnorm, qerr, qcdot, eps_a, eps_b, flags));
     KIRAG_LAUNCH_OK("tail_fused_kernel");
     return 0;
 }

@@ -9,9 +9,17 @@ Reference call sites (all in /root/reference/retriever/index.py):
     index.remove_ids(x)             (no call site) -> kirag_index_remove_ids / kirag_index_remove_range
     index.search(x, k)              :47           -> kirag_index_search
     index.range_search(x, radius)   (no call site) -> kirag_index_range_search + kirag_index_range_fetch
-    faiss.write_index(index, path)  :62           -> kirag_index_save   ("IxFI" container)
-    faiss.read_index(path, flags)   :73           -> kirag_index_load
+    faiss.write_index(index, path)  :62           -> kirag_index_save   ("IxFI" container, "IxMp" for an IndexIDMap)
+    faiss.read_index(path, flags)   :73           -> kirag_index_load   (IndexFlatIP, or IndexIDMap for an IxMp file)
     index.ntotal                    :74, :79      -> kirag_index_ntotal
+
+FAISS's way of attaching the caller's ids to a flat index (no reference call site; the reference keeps its own
+row -> passage table, retriever/index.py:24,82):
+    faiss.IndexIDMap(faiss.IndexFlatIP(d))           -> IndexIDMap: the handle is recreated with KIRAG_INDEX_ID_MAP
+    index.add_with_ids(x, ids)                       -> kirag_index_add_with_ids (int64 ids into the device id table)
+    index.search / range_search                      -> the ids of the table, mapped by the kernels that write I
+    index.remove_ids(x)                              -> selects by id value; nothing else shifts
+    faiss.vector_to_array(index.id_map)              -> kirag_index_id_map
 
 Error behaviour follows FAISS's SWIG wrapper: shape / k problems are
 AssertionError, library failures are RuntimeError.  There is no CPU path.
@@ -85,6 +93,16 @@ def _id_array(x) -> np.ndarray:
     a = np.asarray(x)
     assert a.size == 0 or a.dtype.kind in "iu", f"expected an integer array or an IDSelector, got {type(x).__name__}"
     return np.ascontiguousarray(a, dtype=np.int64).ravel()
+
+
+def _id_pairs(x, ids, d: int) -> Tuple[np.ndarray, np.ndarray]:
+    """(x, ids) as FAISS's add_with_ids converts them: float32 [n, d] and int64 of shape (n,)."""
+    x = np.ascontiguousarray(x, dtype=np.float32)
+    assert x.ndim == 2, "add_with_ids expects a 2-D array"
+    assert x.shape[1] == d, f"add_with_ids: vectors have dimension {x.shape[1]}, index has {d}"
+    ids = np.ascontiguousarray(ids, dtype=np.int64)
+    assert ids.shape == (x.shape[0],), "not same nb of vectors as ids"
+    return x, ids
 
 
 class IndexFlatIP:
@@ -169,6 +187,11 @@ class IndexFlatIP:
             return
         _lib.check(self._lib.kirag_index_add(self._h, _ptr(x), n, 0, None), "add")
 
+    def add_with_ids(self, x, ids) -> None:
+        """Raises as FAISS's IndexFlat does: a flat index has no ids of its own (wrap it in IndexIDMap)."""
+        x, ids = _id_pairs(x, ids, self.d)
+        _lib.check(self._lib.kirag_index_add_with_ids(self._h, _ptr(x), _ptr(ids), x.shape[0], 0, None), "add_with_ids")
+
     def remove_ids(self, x) -> int:
         """faiss IndexFlatIP.remove_ids: removes every row whose id is selected by x (an integer array, an
         IDSelectorBatch or an IDSelectorRange); the remaining rows move down in order, so later ids shift.  Ids < 0 or
@@ -180,6 +203,21 @@ class IndexFlatIP:
             ids = x.ids if isinstance(x, IDSelectorBatch) else _id_array(x)
             _lib.check(self._lib.kirag_index_remove_ids(self._h, _ptr(ids), ids.size, ctypes.byref(n), None),
                        "remove_ids")
+        return int(n.value)
+
+    def remove_ids_device(self, ids) -> int:
+        """remove_ids with the ids in an integer CUDA tensor on this index's (home) device, read on the current
+        stream.  Selects by position on a plain index, by id value on an id map."""
+        import torch
+
+        assert ids.is_cuda and ids.device.index == self.device, \
+            f"remove_ids_device: expected a CUDA tensor on cuda:{self.device}"
+        assert not ids.dtype.is_floating_point and ids.dtype != torch.bool, "remove_ids_device: integer ids only"
+        ids = ids.reshape(-1).to(torch.int64).contiguous()
+        n = ctypes.c_int64(0)
+        st = torch.cuda.current_stream(ids.device).cuda_stream
+        _lib.check(self._lib.kirag_index_remove_ids_ex(self._h, ctypes.c_void_p(ids.data_ptr()), ids.numel(), 1,
+                                                       ctypes.byref(n), ctypes.c_void_p(st)), "remove_ids_device")
         return int(n.value)
 
     def search(self, x, k: int) -> Tuple[np.ndarray, np.ndarray]:
@@ -453,6 +491,134 @@ class IndexFlatIP:
             pass
 
 
+class IndexIDMap:
+    """faiss.IndexIDMap over an IndexFlatIP: every row carries an int64 id of the caller's (any value, negative and
+    repeated ones included), kept in a table on the device.  search / range_search return those ids (order as the
+    plain index: score desc, then insertion order), remove_ids selects by id value and nothing else shifts,
+    write_index writes FAISS's IxMp file.  The sub-index must be empty; its handle is recreated with the id table
+    (device, devices and master kept) and shared with this object, which keeps it as `.index` (rows stay reachable
+    by position through index.reconstruct_n; searches through either object return the ids)."""
+
+    def __init__(self, index: IndexFlatIP, _loaded: bool = False):
+        assert isinstance(index, IndexFlatIP), "IndexIDMap: the sub-index must be a kirag_b200 IndexFlatIP"
+        if not _loaded:
+            if index.ntotal != 0:
+                raise RuntimeError("IndexIDMap: index must be empty on input")
+            index._flags |= _lib.INDEX_ID_MAP
+            index.reset()
+        self.index = index
+
+    metric_type = METRIC_INNER_PRODUCT
+    is_trained = True
+
+    @property
+    def d(self) -> int:
+        return self.index.d
+
+    @property
+    def ntotal(self) -> int:
+        return self.index.ntotal
+
+    @property
+    def device(self) -> int:
+        return self.index.device
+
+    @property
+    def devices(self) -> List[int]:
+        return self.index.devices
+
+    @property
+    def last_stats(self) -> dict:
+        return self.index.last_stats
+
+    def train(self, x) -> None:
+        return None
+
+    def add(self, x) -> None:
+        raise RuntimeError("add does not work on IndexIDMap, use add_with_ids")
+
+    def add_with_ids(self, x, ids) -> None:
+        x, ids = _id_pairs(x, ids, self.d)
+        if x.shape[0]:
+            _lib.check(self.index._lib.kirag_index_add_with_ids(self.index._h, _ptr(x), _ptr(ids), x.shape[0], 0, None),
+                       "add_with_ids")
+
+    def search(self, x, k: int) -> Tuple[np.ndarray, np.ndarray]:
+        return self.index.search(x, k)
+
+    def search_ex(self, x, k: int, path: int = _lib.PATH_AUTO):
+        return self.index.search_ex(x, k, path=path)
+
+    def range_search(self, x, radius: float) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        return self.index.range_search(x, radius)
+
+    def remove_ids(self, x) -> int:
+        """Removes every row whose id is selected by x (an integer array or IDSelectorBatch: membership;
+        IDSelectorRange(imin, imax): imin <= id < imax), every row of a repeated id included.  Returns the rows
+        removed."""
+        return self.index.remove_ids(x)
+
+    def reset(self) -> None:
+        self.index.reset()
+
+    def reconstruct(self, key: int):
+        raise RuntimeError("reconstruct not implemented for this type of index (IndexIDMap has no reverse map; use "
+                           "IndexIDMap.index.reconstruct_n for rows by position)")
+
+    @property
+    def id_map(self) -> np.ndarray:
+        """The ids in row order (int64)."""
+        n = self.ntotal
+        out = np.empty(n, dtype=np.int64)
+        if n:
+            _lib.check(self.index._lib.kirag_index_id_map(self.index._h, 0, n, _ptr(out), 0, None), "id_map")
+        return out
+
+    def storage_bytes(self) -> dict:
+        return self.index.storage_bytes()
+
+    # -- device-resident entry points (as on IndexFlatIP) ---------------------------------------------------------
+    def add_with_ids_device(self, x, ids) -> None:
+        """x: float32 CUDA tensor [n, d], ids: integer CUDA tensor [n], both on this index's (home) device."""
+        import torch
+
+        assert str(x.dtype) == "torch.float32", "add_with_ids_device: float32 only (faiss add() semantics)"
+        x = self.index._own_tensor(x, "add_with_ids_device")
+        assert ids.is_cuda and ids.device == x.device, "add_with_ids_device: ids must be a CUDA tensor on the index's device"
+        ids = ids.to(torch.int64).contiguous()
+        assert tuple(ids.shape) == (x.shape[0],), "not same nb of vectors as ids"
+        st = torch.cuda.current_stream(x.device).cuda_stream
+        _lib.check(self.index._lib.kirag_index_add_with_ids(self.index._h, ctypes.c_void_p(x.data_ptr()),
+                                                            ctypes.c_void_p(ids.data_ptr()), x.shape[0], 1,
+                                                            ctypes.c_void_p(st)), "add_with_ids_device")
+
+    def search_device(self, q, k: int, path: int = _lib.PATH_AUTO):
+        return self.index.search_device(q, k, path=path)
+
+    def range_search_device(self, q, radius: float, path: int = _lib.PATH_AUTO):
+        return self.index.range_search_device(q, radius, path=path)
+
+    def remove_ids_device(self, ids) -> int:
+        return self.index.remove_ids_device(ids)
+
+    def search_device_async(self, q, k: int):
+        return self.index.search_device_async(q, k)
+
+    def finish(self) -> int:
+        return self.index.finish()
+
+    def search_device_graph(self, q, k: int):
+        return self.index.search_device_graph(q, k)
+
+    def state_token(self) -> int:
+        return self.index.state_token()
+
+
+def vector_to_array(v) -> np.ndarray:
+    """faiss.vector_to_array: a copy of the vector as a numpy array (IndexIDMap.id_map already is one)."""
+    return np.array(v, copy=True)
+
+
 class IndexFlatL2:
     """Present because retriever/index.py:14 names it at import time; never constructed by KiRAG."""
 
@@ -468,14 +634,17 @@ class IndexPQ:
         raise NotImplementedError("kirag_b200 implements the exact flat index only (IndexPQ is unused by KiRAG)")
 
 
-def write_index(index: IndexFlatIP, path) -> None:
-    assert isinstance(index, IndexFlatIP), "write_index: not a kirag_b200 IndexFlatIP"
+def write_index(index, path) -> None:
+    if isinstance(index, IndexIDMap):
+        index = index.index
+    assert isinstance(index, IndexFlatIP), "write_index: not a kirag_b200 IndexFlatIP or IndexIDMap"
     _lib.check(index._lib.kirag_index_save(index._h, os.fspath(path).encode()), "write_index")
 
 
 def read_index(path, flags: int = 0, device: Optional[int] = None, master: Optional[str] = None,
-               devices: Optional[Sequence[int]] = None) -> IndexFlatIP:
-    """`flags` are FAISS IO flags (IO_FLAG_MMAP is accepted and ignored); `master` and `devices` as for IndexFlatIP."""
+               devices: Optional[Sequence[int]] = None):
+    """`flags` are FAISS IO flags (IO_FLAG_MMAP is accepted and ignored); `master` and `devices` as for IndexFlatIP.
+    An IxFI file gives an IndexFlatIP, an IxMp file an IndexIDMap over one."""
     index_flags = _master_flags(master)
     devs = _resolve_devices(device, devices)
     lib = _lib.load()
@@ -483,11 +652,16 @@ def read_index(path, flags: int = 0, device: Optional[int] = None, master: Optio
     if devs is None:
         dev = _lib.default_device() if device is None else int(device)
         _lib.check(lib.kirag_index_load_ex(os.fspath(path).encode(), dev, index_flags, ctypes.byref(h)), "read_index")
-        return IndexFlatIP(0, device=dev, master="host" if index_flags else "device", _handle=h.value)
-    arr = (ctypes.c_int * len(devs))(*devs)
-    _lib.check(lib.kirag_index_load_multi(os.fspath(path).encode(), arr, len(devs), index_flags, ctypes.byref(h)),
-               "read_index")
-    return IndexFlatIP(0, master="host" if index_flags else "device", devices=devs, _handle=h.value)
+        ix = IndexFlatIP(0, device=dev, master="host" if index_flags else "device", _handle=h.value)
+    else:
+        arr = (ctypes.c_int * len(devs))(*devs)
+        _lib.check(lib.kirag_index_load_multi(os.fspath(path).encode(), arr, len(devs), index_flags, ctypes.byref(h)),
+                   "read_index")
+        ix = IndexFlatIP(0, master="host" if index_flags else "device", devices=devs, _handle=h.value)
+    if lib.kirag_index_flags(ix._h) & _lib.INDEX_ID_MAP:
+        ix._flags |= _lib.INDEX_ID_MAP  # reset() keeps the table
+        return IndexIDMap(ix, _loaded=True)
+    return ix
 
 
 def omp_get_max_threads() -> int:

@@ -246,6 +246,11 @@ class ShardedFlatIP:
 
             local_index = IndexFlatIP(d, device=device, master=master)
             local_index.reserve(max(self.hi - self.lo, 1))
+        from .faiss_api import IndexIDMap
+
+        if isinstance(local_index, IndexIDMap) or getattr(local_index, "_flags", 0) & _lib.INDEX_ID_MAP:
+            raise RuntimeError("ShardedFlatIP: the local index is an IndexIDMap; the row-sharded search returns global "
+                               "row numbers and does not support id maps")
         self.index = local_index
         self.merge_fn = merge_fn or merge_topk_device
         # "peer": fused NVLink exchange+merge kernel; "nccl": all-gather + merge kernel.  An injected

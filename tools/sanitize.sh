@@ -9,7 +9,7 @@ nvcc -O2 -std=c++17 -o $OUT/sanitize_driver tools/sanitize_driver.cu -Lkirag_b20
 $OUT/sanitize_driver all > $OUT/r2_sanitize_plain.log 2>&1
 echo "plain rc=$?"; tail -3 $OUT/r2_sanitize_plain.log
 for tool in memcheck racecheck synccheck initcheck; do
-  for c in scan search pool exchange topk host_rescore host_exact multi_merge remove_compact; do
+  for c in scan search pool exchange topk host_rescore host_exact multi_merge remove_compact id_map; do
     timeout 900 compute-sanitizer --tool $tool --error-exitcode 9 --print-limit 20 $OUT/sanitize_driver $c > $OUT/r2_sanitize_${tool}_$c.log 2>&1
     rc=$?
     echo "$tool $c rc=$rc: $(grep -E 'ERROR SUMMARY|RACECHECK SUMMARY|passed' $OUT/r2_sanitize_${tool}_$c.log | tr '\n' ' ')"

@@ -4,7 +4,7 @@
 // computation, so a "passed" under the sanitizer is also a correctness pass.
 //
 //   ./sanitize_driver [case]     case = scan | search | pool | exchange | topk | host_rescore | host_exact | multi_merge |
-//                                       remove_compact | all (default)
+//                                       remove_compact | id_map | all (default)
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -429,6 +429,56 @@ static void case_remove_compact() {
     }
 }
 
+// id map (KIRAG_INDEX_ID_MAP) on small shapes, single-device and three shards of one GPU: add with ids (negative and
+// repeated ids), a search whose ids must be the ids of the host's top-k rows (d = 64: the filter path and the fused tail
+// or final kernel; the multi-device merge), then a batch removal by id (the device sort and the binary-search marking)
+// and a range removal by id value, each checked against the host's restatement of the table
+static void case_id_map() {
+    std::mt19937 rng(10);
+    const int n = 3000, d = 64, nq = 4, k = 10;
+    for (int G : {1, 3}) {
+        auto xb = unit_rows(rng, n, d);
+        auto xq = unit_rows(rng, nq, d);
+        std::vector<int64_t> ids((size_t)n);
+        for (int i = 0; i < n; ++i) ids[(size_t)i] = ((int64_t)(i * 7919 % n) - 1000) * 1000003;
+        for (int i = 0; i < 40; ++i) ids[(size_t)(2000 + i)] = ids[(size_t)i];  // repeated ids
+        kirag_index_t* h = nullptr;
+        const int devs[3] = {0, 0, 0};
+        if (G == 1) CK(kirag_index_create_ex(d, KIRAG_METRIC_INNER_PRODUCT, 0, KIRAG_INDEX_ID_MAP, &h));
+        else CK(kirag_index_create_multi(d, KIRAG_METRIC_INNER_PRODUCT, devs, G, KIRAG_INDEX_ID_MAP, &h));
+        CK(kirag_index_add_with_ids(h, xb.data(), ids.data(), n, 0, nullptr));
+        std::vector<float> D((size_t)nq * k);
+        std::vector<int64_t> I((size_t)nq * k), Ih;
+        CK(kirag_index_search(h, xq.data(), nq, k, D.data(), I.data(), 0, 0, nullptr));
+        host_topk(xb, n, xq, nq, d, k, &Ih);
+        bool ok = true;
+        for (size_t j = 0; j < I.size(); ++j) ok = ok && I[j] == ids[(size_t)Ih[j]];
+        // batch by id (with an absent id and a repeat), then a range of id values
+        std::vector<int64_t> sel = {ids[5], ids[5], ids[77], 123456789, ids[2999]};
+        for (int i = 1500; i < 1800; i += 3) sel.push_back(ids[(size_t)i]);
+        std::vector<int64_t> keep_ids;
+        for (int64_t v : ids)
+            if (std::find(sel.begin(), sel.end(), v) == sel.end()) keep_ids.push_back(v);
+        int64_t removed = -1;
+        CK(kirag_index_remove_ids(h, sel.data(), (int64_t)sel.size(), &removed, nullptr));
+        ok = ok && removed == n - (int64_t)keep_ids.size();
+        const int64_t lo = -300LL * 1000003, hi = 200LL * 1000003;
+        std::vector<int64_t> left;
+        for (int64_t v : keep_ids)
+            if (v < lo || v >= hi) left.push_back(v);
+        int64_t removed_r = -1;
+        CK(kirag_index_remove_range(h, lo, hi, &removed_r, nullptr));
+        const int64_t nt = kirag_index_ntotal(h);
+        std::vector<int64_t> table((size_t)nt);
+        CK(kirag_index_id_map(h, 0, nt, table.data(), 0, nullptr));
+        ok = ok && removed_r == (int64_t)(keep_ids.size() - left.size()) && table == left;
+        printf("id map G=%d: search mapped, %lld + %lld rows removed by id, %lld left %s\n", G, (long long)removed,
+               (long long)removed_r, (long long)nt, ok ? "ok" : "BAD");
+        if (!ok) exit(3);
+        CK(kirag_index_destroy(h));
+    }
+}
+
 int main(int argc, char** argv) {
     const std::string which = argc > 1 ? argv[1] : "all";
     if (which == "scan" || which == "all") case_scan();
@@ -440,6 +490,7 @@ int main(int argc, char** argv) {
     if (which == "host_exact" || which == "all") case_host_exact();
     if (which == "multi_merge" || which == "all") case_multi_merge();
     if (which == "remove_compact" || which == "all") case_remove_compact();
+    if (which == "id_map" || which == "all") case_id_map();
     CU(cudaDeviceSynchronize());
     printf("sanitize_driver %s: passed\n", which.c_str());
     return 0;
